@@ -2,6 +2,7 @@
 """bench.py — the hot path's headline metric on B200 (see BASELINE.json, SURVEY.md §8d, DESIGN.md §6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg1]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one pass of the per-pixel multi-dataset label-space path over one synthetic batch:
@@ -21,6 +22,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from, which may be read-only
 
 import numpy as np
 import torch
@@ -98,7 +100,19 @@ def parse():
                     help="do not pin the rank to the CPUs of its GPU's NUMA node (A/B of the e2e arm)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-kernel-times", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (rank 0): "
+                         "loss, miou, confusion (the flat int64 histograms of every dataset, as float64) and the "
+                         "gradients d logits_uni, d bi_graph<i> (--bi-graphs dense) and d aux<i> (--with-aux) as "
+                         "float32.  A gradient of more than %d elements is stored at a fixed, seeded sample of "
+                         "positions, so two builds run with the same arguments can be compared output for output"
+                         % DUMP_MAX_ELEMS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def measured_peak():
@@ -164,6 +178,26 @@ def make_batch(workload, device, seed, images=None, logits="randn"):
             raw[b][torch.rand(H, W, generator=dgen, device=device) < 0.03] = 250                  # void -> 255
     return dict(n_cats=n_cats, c_uni=c_uni, ids=ids, h=h, w=w, H=H, W=W, x=x, raw=raw, pred=pred, graphs=graphs,
                 luts=luts)
+
+
+DUMP_MAX_ELEMS = 1 << 20  # 4 MB of float32 per array: d logits_uni plus seven aux heads stay far below 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """np.save every array as out_dir/<name>.npy; integers as float64, the rest as float32.  An array of more than
+    DUMP_MAX_ELEMS elements is reduced to the elements at DUMP_MAX_ELEMS flat positions drawn with a seed that depends
+    only on its size, so the same arguments select the same positions in every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if t is None:  # a tensor that received no gradient
+            continue
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            pos = np.random.default_rng(t.numel()).choice(t.numel(), DUMP_MAX_ELEMS, replace=False)
+            pos.sort()
+            t = t.reshape(-1)[torch.from_numpy(pos).to(t.device)]
+        t = t.to(torch.float32 if t.is_floating_point() else torch.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def dataset_slices(ids):
@@ -425,6 +459,13 @@ def run_ours(args, rank, world, local_rank):
             step(bt["raw"], x, bt["pred"])
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:  # before the checks and the other loops below overwrite the step's results
+        outputs = {"loss": out["loss"], "miou": out["miou"], "confusion": hist_flat, "dlogits_uni": x.grad}
+        if args.bi_graphs == "dense":
+            outputs.update({f"dbi_graph{d}": g.grad for d, g in enumerate(graphs)})
+        if aux is not None:
+            outputs.update({f"daux{d}": t.grad for d, t in enumerate(aux)})
+        dump_outputs(args.dump_outputs, outputs)
     ms = e0.elapsed_time(e1)
     gpu_launches = launches["n"]
     ms = dist_utils.max_over_ranks(ms, dev)

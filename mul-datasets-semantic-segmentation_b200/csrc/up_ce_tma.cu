@@ -491,7 +491,7 @@ up_ce_bwd_tma_kernel(const __grid_constant__ TmaMaps maps, const BwdArgs a) {
   const int x = xa + warp * kOwnPerWarp + lane - 1;
   // staged column of this cell.  The TMA box must start at or left of the halo cell xa-1, and its
   // innermost start coordinate has to be a multiple of 16 bytes: an unaligned (or negative) start
-  // raises "illegal instruction" on B200 (tests/probes/tma_coord_alignment.cu).  xa is a multiple
+  // raises "illegal instruction" on B200 (fp32, SWIZZLE_NONE, driver 580, CUDA 12.9).  xa is a multiple
   // of 124, so the box starts 4 cells left of xa (at 0 for the first CTA of a row).
   static_assert((kNW * kOwnPerWarp) % 4 == 0, "box start must stay 16-byte aligned");
   const int box_x0 = xa > 0 ? xa - 4 : 0;

@@ -193,9 +193,9 @@ def test_label_transform_planner_draws_the_reference_stream():
 
 
 # ---- round 2: the drop-in really drops in (VERDICT r1 weak #2 / ADVICE high) -----------------------------------------
-REFERENCE = "/root/reference"
-needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "lib")),
-                                     reason="the reference checkout exists in the build container only")
+REFERENCE = os.environ.get("MDSEG_REFERENCE_ROOT", "")
+needs_reference = pytest.mark.skipif(not REFERENCE or not os.path.isdir(os.path.join(REFERENCE, "lib")),
+                                     reason="needs a checkout of the reference project under $MDSEG_REFERENCE_ROOT")
 
 _TRAINER_IMPORTS = """
 import sys, types, torch
@@ -224,13 +224,13 @@ print(CrossDatasetsCELoss_AdvGNN.__module__, CrossDatasetsCELoss.__module__, Cro
 
 @needs_reference
 @pytest.mark.parametrize("which", ["all_three", "leaf_modules_only"])
-def test_install_then_the_trainers_import_lines(which):
+def test_install_then_the_trainers_import_lines(which, tmp_path):
     """After install() the reference's own import lines work — both with the loss module aliased (native
     CrossDatasetsCELoss*, the rest passed through) and with only the two leaf modules aliased (the reference's own
     lib/loss/loss_cross_datasets.py then imports MdsOhemNLLPlusLoss etc. from the drop-in, :6)."""
     args = "" if which == "all_three" else "only=['lib.loss.ohem_ce_loss', 'lib.class_remap']"
     code = _TRAINER_IMPORTS.format(root=ROOT, ref=REFERENCE, install_args=args)
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path)
     assert r.returncode == 0, r.stderr[-2000:]
     adv, ce, legacy, modname = r.stdout.split()
     if which == "all_three":
@@ -241,7 +241,7 @@ def test_install_then_the_trainers_import_lines(which):
 
 
 @needs_reference
-def test_reference_methods_run_on_the_dropin_classremap():
+def test_reference_methods_run_on_the_dropin_classremap(tmp_path):
     """lib/test/test_class_remap.py:43-95 (the reference's own MultiProtoRemapping test body, CPU tensors) against the
     drop-in ClassRemapOneHotLabel: the method is the reference's, grafted onto the drop-in instance."""
     code = f"""
@@ -270,11 +270,11 @@ assert all(torch.equal(x, y) for x, y in zip(a, b))
 assert ours.getAnyClassRemap(2, 0) == theirs.getAnyClassRemap(2, 0) == [2, 3]
 print('ok')
 """
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path)
     assert r.returncode == 0 and r.stdout.strip() == "ok", r.stderr[-2000:]
 
 
-def test_dropin_superset_without_a_reference_checkout():
+def test_dropin_superset_without_a_reference_checkout(tmp_path):
     """No checkout on sys.path: the native names work, a passed-through name raises an AttributeError that says why."""
     code = f"""
 import sys
@@ -290,7 +290,8 @@ except AttributeError as e:
     assert 'pass-through is unavailable' in str(e), e
     print('ok')
 """
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+    env = {k: v for k, v in os.environ.items() if k != "MDSEG_REFERENCE_ROOT"}
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path, env=env)
     assert r.returncode == 0 and r.stdout.strip() == "ok", r.stderr[-2000:] + r.stdout
 
 
@@ -318,3 +319,34 @@ def test_bench_reference_arm_contract_and_no_cpu_fallback():
         r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tiny", "--steps", "1"],
                            capture_output=True, text=True, env=env, timeout=600)
         assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
+
+
+def test_bench_steps_and_dump_outputs(tmp_path):
+    """--steps is the number of timed steps, so fewer than one is refused.  dump_outputs() stores integers as float64
+    and the rest as float32, and keeps an array above DUMP_MAX_ELEMS as the same sorted sample of positions in every
+    run."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=600)
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+    code = f"""
+import sys, torch
+sys.path.insert(0, {ROOT!r})
+import bench
+n = bench.DUMP_MAX_ELEMS + 1000
+for d in ("a", "b"):
+    bench.dump_outputs({str(tmp_path)!r} + "/" + d, {{"big": torch.arange(n, dtype=torch.float32).reshape(8, -1),
+                                                      "hist": torch.arange(6).view(2, 3) << 40,
+                                                      "half": torch.ones(3, dtype=torch.bfloat16), "none": None}})
+print(bench.DUMP_MAX_ELEMS)
+"""
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    cap = int(r.stdout.split()[-1])
+    assert sorted(os.listdir(tmp_path / "a")) == ["big.npy", "half.npy", "hist.npy"]
+    big = np.load(tmp_path / "a" / "big.npy")
+    assert big.dtype == np.float32 and big.shape == (cap,)
+    assert np.all(np.diff(big) > 0) and big[0] >= 0 and big[-1] < cap + 1000  # distinct positions, in order
+    assert np.array_equal(big, np.load(tmp_path / "b" / "big.npy"))
+    hist = np.load(tmp_path / "a" / "hist.npy")
+    assert hist.dtype == np.float64 and np.array_equal(hist, (np.arange(6).reshape(2, 3) << 40).astype(np.float64))
+    assert np.load(tmp_path / "a" / "half.npy").dtype == np.float32
