@@ -313,6 +313,36 @@ int mdseg_proj_bwd_graph_tc(const void* x, int dtype, const float* dyA, const fl
                             float* dG, long long dg_stride, void* workspace,
                             size_t workspace_bytes, void* stream);
 
+/* ---- a5 for channels_last (NHWC) unified logits -------------------------------
+ * The projection of mdseg_proj_fwd with x [n_images, h, w, C_uni] pixel-major (what a model run with
+ * memory_format=torch.channels_last produces); y and cmax_out are the same NCHW outputs, bit-identical to
+ * mdseg_proj_fwd on the NCHW copy of x.  Sparse graphs only (dense graphs take mdseg_proj_fwd_tc on NCHW),
+ * C_uni <= MDSEG_NHWC_MAX_CUNI and every C_ds <= MDSEG_NHWC_MAX_CDS. */
+#define MDSEG_NHWC_MAX_CUNI 1536
+#define MDSEG_NHWC_MAX_CDS 768
+int mdseg_proj_fwd_nhwc(const void* x, int dtype, const mdseg_graph_table* graphs /*host*/,
+                        const int32_t* dataset_ids, int n_images, int h, int w,
+                        float* y, int y_cmax, float* cmax_out, int32_t* err_flag, void* stream);
+
+/* The adjoint of mdseg_proj_bwd written pixel-major: dx [n_images, h, w, C_uni] in `dtype`, fully overwritten
+ * (zeros for images whose dataset id is out of range), bit-identical to mdseg_proj_bwd given the same dy.
+ * Same graph limits as mdseg_proj_fwd_nhwc. */
+int mdseg_proj_bwd_nhwc(const float* dyA, const float* dyB, int y_cmax,
+                        const mdseg_graph_table* graphs /*host*/,
+                        const int32_t* dataset_ids, int n_images, int h, int w,
+                        void* dx, int dtype, void* stream);
+
+/* Layout moves of the aux heads' channels_last sources.  `nhwc` lists the heads as [n_images, h, w, C_d]
+ * (image_stride in elements); `planar` lists where image b's rows go as [C_d, h, w] planes at
+ * base[d] + b * image_stride[d] (one shared buffer [n_images, max C_d, h, w] or one per head), same dtype.
+ * mdseg_nhwc_to_planar copies the rows of each image's own head d = dataset_ids[b] (0 when NULL).
+ * mdseg_planar_to_nhwc writes every head's NHWC tensor: the planar rows for the image's own head, zeros for
+ * every other head. */
+int mdseg_nhwc_to_planar(const mdseg_src_table* nhwc /*host*/, const int32_t* dataset_ids, int n_images, int h,
+                         int w, const mdseg_src_table* planar /*host*/, void* stream);
+int mdseg_planar_to_nhwc(const mdseg_src_table* planar /*host*/, const int32_t* dataset_ids, int n_images, int h,
+                         int w, const mdseg_src_table* nhwc /*host*/, void* stream);
+
 /* ---- a6 + a7 (+ a10): fused bilinear upsample (align_corners=True) + CE -------
  * For every label pixel (Y,X) of image b: interpolate the C low-res logits of
  * the image's source (see mdseg_src_table) to (Y,X) exactly as

@@ -11,6 +11,8 @@ What runs where:
   * the per-pixel work (SURVEY.md §8 rows a5-a10) goes through libmdseg_b200.so:
       - SEG stage (is_adv=False, 0/1 graphs): projection + bilinear up-sampling + CE + one OHEM selection over the
         batch from the LOW-resolution unified logits (:1006-1007, :1074), aux heads from ``preds['aux']`` (:1051-1056);
+        channels_last ``preds['seg']`` / ``preds['aux']`` (a model run with memory_format=torch.channels_last) are
+        taken as they are, without a layout copy, and get channels_last gradients;
       - GNN stage (is_adv=True, trainable soft / hard graph pairs): the same fused loss once per graph set, blended
         by ``max_rate`` (:1063-1071), with gradients to the logits AND to every ``bi_graphs[i]`` (tcgen05 split-K
         ``d bi_graph``); aux heads from the dataset prototypes (:941-951, :1044-1048) through the fused

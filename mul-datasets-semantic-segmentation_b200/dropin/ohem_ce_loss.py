@@ -51,7 +51,8 @@ class MdsOhemCELoss(nn.Module):
     def forward_fused(self, logits_uni, labels, dataset_ids, bi_graphs):
         """Projection + bilinear up-sampling + CE + one OHEM selection from the LOW-resolution unified logits
         [B, C_uni, h, w] (loss_cross_datasets.py:1006-1007 + :1074 in one autograd node; no host sync once the graphs' descriptors are
-        cached, see ops.mds_proj_ohem_ce)."""
+        cached, see ops.mds_proj_ohem_ce).  channels_last logits with 0/1 graphs are taken as they are (no layout copy)
+        and get a channels_last gradient."""
         return ops.mds_proj_ohem_ce(logits_uni, labels, dataset_ids, list(bi_graphs), float(self.thresh),
                                     self.ignore_lb)
 

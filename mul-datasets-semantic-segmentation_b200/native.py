@@ -16,6 +16,7 @@ U8, I32, I64 = 10, 11, 12
 NCHW, NHWC = 0, 1
 ERR_LABEL_RANGE, ERR_PRED_RANGE, ERR_TOPK_RANGE, ERR_DATASET_ID, ERR_GRAPH_KIND = 1, 2, 4, 8, 16
 MAX_DATASETS = 32
+NHWC_MAX_CUNI, NHWC_MAX_CDS = 1536, 768  # graph limits of mdseg_proj_fwd_nhwc / mdseg_proj_bwd_nhwc
 
 
 class OhemState(C.Structure):
@@ -105,6 +106,10 @@ SIGNATURES = {
     "mdseg_proj_bwd_graph_tc_workspace_bytes": (C.c_size_t, [C.POINTER(GraphTable), _I, _I, _I]),
     "mdseg_proj_bwd_graph_tc": (_I, [_P, _I, _P, _P, _I, C.POINTER(GraphTable), _P, _I, _I, _I, _P, C.c_longlong, _P,
                                      C.c_size_t, _P]),
+    "mdseg_proj_fwd_nhwc": (_I, [_P, _I, C.POINTER(GraphTable), _P, _I, _I, _I, _P, _I, _P, _P, _P]),
+    "mdseg_proj_bwd_nhwc": (_I, [_P, _P, _I, C.POINTER(GraphTable), _P, _I, _I, _I, _P, _I, _P]),
+    "mdseg_nhwc_to_planar": (_I, [C.POINTER(SrcTable), _P, _I, _I, _I, C.POINTER(SrcTable), _P]),
+    "mdseg_planar_to_nhwc": (_I, [C.POINTER(SrcTable), _P, _I, _I, _I, C.POINTER(SrcTable), _P]),
     "mdseg_up_ce_fwd": (_I, [C.POINTER(SrcTable), _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "mdseg_up_ce_bwd": (_I, [C.POINTER(SrcTable), _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _F,
                              C.POINTER(SrcTable), C.POINTER(SrcTable), _P]),

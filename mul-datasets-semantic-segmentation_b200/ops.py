@@ -524,13 +524,27 @@ def _src_table(bases, strides, Cs, dtype, seg_per_dataset, c_alloc=None, cmax=No
     return t
 
 
+def _channels_last(x):
+    """A 4-D tensor that is channels_last-contiguous and not NCHW-contiguous (the layout decision of ohem_ce: shapes that
+    are both, C = 1 or h * w = 1, count as NCHW)."""
+    return x.dim() == 4 and not x.is_contiguous() and x.is_contiguous(memory_format=torch.channels_last)
+
+
+def _nhwc_proj_ok(x, tab):
+    """channels_last logits with sparse graphs inside the limits of mdseg_proj_fwd_nhwc / mdseg_proj_bwd_nhwc: the
+    projection reads x as it is.  Anything else (dense graphs included) takes the NCHW kernels on x.contiguous()."""
+    return (_channels_last(x) and tab.C_uni <= N.NHWC_MAX_CUNI
+            and all(not tab.g[i].dense and tab.g[i].C_ds <= N.NHWC_MAX_CDS for i in range(tab.n_datasets)))
+
+
 # ---- a5 projection alone (model-side eval einsum, semseg.py:342-345) --------------------------------
 def project(logits_uni, graphs, dataset_ids=None, cache=None):
-    """fp32 [B, max C_ds, h, w]: einsum('bchw,nc->bnhw') with the graph of each image's dataset."""
+    """fp32 [B, max C_ds, h, w]: einsum('bchw,nc->bnhw') with the graph of each image's dataset.  channels_last logits
+    with sparse graphs are read as they are (no layout copy)."""
     _require_cuda(logits_uni)
-    x = logits_uni.contiguous()
-    B, Cu, h, w = x.shape
     tab, keep = (cache or _default_graphs).table(list(graphs))
+    x = logits_uni if _nhwc_proj_ok(logits_uni, tab) else logits_uni.contiguous()
+    B, Cu, h, w = x.shape
     if tab.C_uni != Cu:
         raise ValueError(f"graphs have C_uni={tab.C_uni}, logits have {Cu}")
     cmax = max(g.shape[0] for g in graphs)
@@ -542,8 +556,13 @@ def project(logits_uni, graphs, dataset_ids=None, cache=None):
 
 def _proj_fwd(x, tab, ids, B, h, w, y, cmax, ymax, ef, graphs=None):
     """mdseg_proj_fwd, or mdseg_proj_fwd_tc (dense graphs on the tensor cores) when a graph is dense; 16-bit logits
-    with all-dense graphs take the TMA-fed kernel (mdseg_proj_fwd_tc16)."""
+    with all-dense graphs take the TMA-fed kernel (mdseg_proj_fwd_tc16); channels_last x (callers pass it only when
+    _nhwc_proj_ok) takes mdseg_proj_fwd_nhwc."""
     n = tab.n_datasets
+    if _channels_last(x):
+        N.call("mdseg_proj_fwd_nhwc", _ptr(x), _DT[x.dtype], C.byref(tab), _ptr(ids), B, h, w, _ptr(y), cmax, _ptr(ymax),
+               _ptr(ef), _stream())
+        return
     if (graphs is not None and x.dtype in (torch.bfloat16, torch.float16) and (h * w) % 8 == 0 and x.data_ptr() % 16 == 0
             and all(tab.g[i].dense and 8 <= tab.g[i].C_ds <= 1024 for i in range(n)) and tab.C_uni >= 32):
         ldb = (tab.C_uni + 7) // 8 * 8
@@ -679,7 +698,8 @@ def prototype_head(feats, proto):
 
 # ---- a5+a6+a7+a8+a9: the fused multi-dataset loss ------------------------------------------------------
 class _MdsProjOhemCE(torch.autograd.Function):
-    """MdsOhemCELoss(project -> upsample -> CE) of loss_cross_datasets.py:1006-1007,1074 in four kernels."""
+    """MdsOhemCELoss(project -> upsample -> CE) of loss_cross_datasets.py:1006-1007,1074 in four kernels.  channels_last
+    logits with sparse graphs are projected as they are and get a channels_last gradient (mdseg_proj_*_nhwc)."""
 
     @staticmethod
     def forward(ctx, logits_uni, labels, dataset_ids, thresh, ignore, cache, per_dataset, *graphs):
@@ -687,7 +707,6 @@ class _MdsProjOhemCE(torch.autograd.Function):
         x = logits_uni
         if x.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             x = x.float()
-        x = x.contiguous()
         B, Cu, h, w = x.shape
         labels = _labels(labels)
         if labels.dim() != 3 or labels.shape[0] != B:
@@ -698,6 +717,8 @@ class _MdsProjOhemCE(torch.autograd.Function):
         tab, keep = cache.table(list(graphs))
         if tab.C_uni != Cu:
             raise ValueError(f"graphs have C_uni={tab.C_uni}, logits have {Cu}")
+        if not _nhwc_proj_ok(x, tab):
+            x = x.contiguous()
         Cs = [g.shape[0] for g in graphs]
         cmax = max(Cs)
         ids = _ids32(dataset_ids, B, dev)
@@ -735,6 +756,16 @@ class _MdsProjOhemCE(torch.autograd.Function):
         src = _src_table([y.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, per_dataset, c_alloc=cmax, cmax=scratch,
                          cmax_ready=True)
         want_dg = any(ctx.needs_input_grad[7 + i] for i in range(n))
+        if not want_dg and _channels_last(x):
+            # channels_last logits (sparse graphs, see forward): d loss / d y from the upsample + CE adjoint, then the
+            # broadcast through G^T written pixel-major
+            dx = None
+            if ctx.needs_input_grad[0]:
+                dyA, dyB = _mds_dy(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, y, Cs, cmax)
+                dx = torch.empty_like(x)  # channels_last
+                N.call("mdseg_proj_bwd_nhwc", _ptr(dyA), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dx),
+                       _DT[x.dtype], _stream())
+            return (dx, None, None, None, None, None, None, *([None] * n))
         if not want_dg:
             # one call: softmax recompute + adjoint of the upsample + broadcast through G^T (fused when it applies)
             dx = None
@@ -781,22 +812,7 @@ class _MdsProjOhemCE(torch.autograd.Function):
                    _ptr(dG), _ptr(ws2), nb, _stream())
             dgs = [dG[i, :Cs[i]].to(graphs[i].dtype) if ctx.needs_input_grad[7 + i] else None for i in range(n)]
             return (dx, None, None, None, None, None, None, *dgs)
-        if fused_direct:
-            # the fused single-pass kernel with the identity in place of G^T: one gradient plane d loss / d y
-            dyA, dyB = torch.empty_like(y), None  # only the first C_ds planes of an image are written — and read
-            dst = _src_table([dyA.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
-            nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-            N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W,
-                   ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes,
-                   _stream())
-        else:
-            dyA = torch.empty_like(y)
-            dyB = torch.empty_like(y)
-            dA = _src_table([dyA.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
-            dB = _src_table([dyB.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
-            N.call("mdseg_up_ce_bwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
-                   _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dA), C.byref(dB), _stream())
+        dyA, dyB = _mds_dy(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, y, Cs, cmax)
         dx = None
         if ctx.needs_input_grad[0]:
             dx = torch.empty_like(x)
@@ -824,6 +840,29 @@ class _MdsProjOhemCE(torch.autograd.Function):
                 if ctx.needs_input_grad[7 + i]:
                     dgs[i] = dG[i, :Cs[i] * Cu].view(Cs[i], Cu).to(graphs[i].dtype)
         return (dx, None, None, None, None, None, None, *dgs)
+
+
+def _mds_dy(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, y, Cs, cmax):
+    """d loss / d y of the fused loss as fp32 planes shaped like y: (dyA, None) from the fused single-pass kernel with
+    the identity in place of G^T when it applies, else the two planes (dyA, dyB) of mdseg_up_ce_bwd, whose sum it is."""
+    B, h, w, H, W = shape
+    n = len(Cs)
+    dev = y.device
+    if N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W):
+        dyA, dyB = torch.empty_like(y), None  # only the first C_ds planes of an image are written — and read
+        dst = _src_table([dyA.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
+        nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W,
+               ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
+    else:
+        dyA = torch.empty_like(y)
+        dyB = torch.empty_like(y)
+        dA = _src_table([dyA.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
+        dB = _src_table([dyB.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
+        N.call("mdseg_up_ce_bwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
+               _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dA), C.byref(dB), _stream())
+    return dyA, dyB
 
 
 def mds_proj_ohem_ce(logits_uni, labels, dataset_ids, graphs, thresh, ignore=255, cache=None, per_dataset=False):
@@ -1135,6 +1174,10 @@ def mds_nll_plus(logits_uni, labels, dataset_ids, graphs, thresh, ignore=255, ca
 
 # ---- a10: per-dataset aux heads (upsample + OhemCE, one selection per dataset) ---------------------------
 class _UpOhemCE(torch.autograd.Function):
+    """channels_last sources (all of them) are not copied: the rows of each head's own images are gathered into one
+    planar buffer [B, max C_i, h, w] (mdseg_nhwc_to_planar) and the gradients come back channels_last
+    (mdseg_planar_to_nhwc)."""
+
     @staticmethod
     def forward(ctx, labels, dataset_ids, thresh, ignore, seg_per_dataset, *srcs):
         labels = _labels(labels)
@@ -1146,7 +1189,10 @@ class _UpOhemCE(torch.autograd.Function):
         dt = srcs[0].dtype
         if dt not in (torch.float32, torch.bfloat16, torch.float16):
             dt = torch.float32
-        srcs = [s.to(dt).contiguous() for s in srcs]
+        srcs = [s.to(dt) for s in srcs]
+        nhwc = all(_channels_last(s) for s in srcs)
+        if not nhwc:
+            srcs = [s.contiguous() for s in srcs]
         h, w = srcs[0].shape[2:]
         for s in srcs:
             if s.shape[0] != B or tuple(s.shape[2:]) != (h, w):
@@ -1154,7 +1200,17 @@ class _UpOhemCE(torch.autograd.Function):
         Cs = [s.shape[1] for s in srcs]
         ids = _ids32(dataset_ids, B, dev) if n > 1 else None
         smax = torch.empty(B, h, w, dtype=torch.float32, device=dev) if dt == torch.float32 else None
-        src = _src_table([s.data_ptr() for s in srcs], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset, cmax=smax)
+        if nhwc:
+            cm = max(Cs)
+            planar = torch.empty(B, cm, h, w, dtype=dt, device=dev)
+            src = _src_table([planar.data_ptr()] * n, [cm * h * w] * n, Cs, _DT[dt], seg_per_dataset, c_alloc=cm,
+                             cmax=smax)
+            nt = _src_table([s.data_ptr() for s in srcs], [s.stride(0) for s in srcs], Cs, _DT[dt], seg_per_dataset)
+            N.call("mdseg_nhwc_to_planar", C.byref(nt), _ptr(ids), B, h, w, C.byref(src), _stream())
+            srcs = [planar]
+        else:
+            src = _src_table([s.data_ptr() for s in srcs], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset,
+                             cmax=smax)
         n_seg = n if seg_per_dataset else 1
         P = B * H * W
         loss_px = torch.empty(P, dtype=torch.float32, device=dev)
@@ -1164,19 +1220,23 @@ class _UpOhemCE(torch.autograd.Function):
                _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(err_flag(dev)), _stream())
         out = _select(loss_px, B, H * W, ids if seg_per_dataset else None, st, n_seg)
         ctx.save_for_backward(labels, ids, loss_px, lse_px, st, *srcs)
-        ctx.meta = (int(ignore), bool(seg_per_dataset), Cs, dt, (h, w, H, W))
+        ctx.meta = (int(ignore), bool(seg_per_dataset), Cs, dt, (h, w, H, W), nhwc)
         ctx.states = st
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         labels, ids, loss_px, lse_px, st, *srcs = ctx.saved_tensors
-        ignore, seg_per_dataset, Cs, dt, (h, w, H, W) = ctx.meta
+        ignore, seg_per_dataset, Cs, dt, (h, w, H, W), nhwc = ctx.meta
         B = labels.shape[0]
-        n = len(srcs)
+        n = len(Cs)
         n_seg = n if seg_per_dataset else 1
         g = _grad_scalar(grad_out, n_seg)
         scratch = torch.empty(1, dtype=torch.float32, device=labels.device) if dt == torch.float32 else None
+        if nhwc:
+            return (None, None, None, None, None,
+                    *_up_ohem_ce_bwd_nhwc(srcs[0], labels, ids, loss_px, lse_px, st, g, scratch, ignore, seg_per_dataset,
+                                          Cs, dt, (h, w, H, W)))
         src = _src_table([s.data_ptr() for s in srcs], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset,
                          cmax=scratch, cmax_ready=True)
         # images of other datasets get a zero gradient (their rows are never selected, :1051): zero-initialised
@@ -1190,9 +1250,36 @@ class _UpOhemCE(torch.autograd.Function):
         return (None, None, None, None, None, *grads)
 
 
+def _up_ohem_ce_bwd_nhwc(planar, labels, ids, loss_px, lse_px, st, g, scratch, ignore, seg_per_dataset, Cs, dt, shape):
+    """Gradients of _UpOhemCE's channels_last sources: d loss / d (planar rows) from mdseg_up_ce_bwd_direct, scattered
+    into channels_last tensors (zeros for the images of other datasets)."""
+    h, w, H, W = shape
+    B, cm = planar.shape[:2]
+    n = len(Cs)
+    dev = planar.device
+    src = _src_table([planar.data_ptr()] * n, [cm * h * w] * n, Cs, _DT[dt], seg_per_dataset, c_alloc=cm, cmax=scratch,
+                     cmax_ready=True)
+    if N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W):
+        dp = torch.empty_like(planar)  # the rows of image b's own head are written — and read
+        dst = _src_table([dp.data_ptr()] * n, [cm * h * w] * n, Cs, _DT[dt], seg_per_dataset, c_alloc=cm)
+    else:  # the generic route adds two planes per head: dense [B, C_d, h, w] destinations
+        dp = [torch.empty(B, c, h, w, dtype=dt, device=dev) for c in Cs]
+        dst = _src_table([t.data_ptr() for t in dp], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset)
+    nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W,
+           ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
+    del ws
+    grads = [torch.empty((B, c, h, w), dtype=dt, device=dev, memory_format=torch.channels_last) for c in Cs]
+    gt = _src_table([t.data_ptr() for t in grads], [t.stride(0) for t in grads], Cs, _DT[dt], seg_per_dataset)
+    N.call("mdseg_planar_to_nhwc", C.byref(dst), _ptr(ids), B, h, w, C.byref(gt), _stream())
+    return grads
+
+
 def up_ohem_ce(srcs, labels, dataset_ids, thresh, ignore=255, seg_per_dataset=True):
     """Per-dataset OhemCE(upsample(srcs[d][ids==d]), labels[ids==d]) as a vector [n_datasets]
-    (seg_per_dataset) or one selection over all images ([1]).  srcs[d]: [B, C_d, h, w] over ALL images."""
+    (seg_per_dataset) or one selection over all images ([1]).  srcs[d]: [B, C_d, h, w] over ALL images; channels_last
+    sources are read without a layout copy and get channels_last gradients."""
     return _UpOhemCE.apply(labels, dataset_ids, float(thresh), int(ignore), bool(seg_per_dataset), *srcs)
 
 
