@@ -565,6 +565,25 @@ size_t mdseg_proj_bwd_graph_tc16_workspace_bytes(int n_images, int C_uni, int64_
 int mdseg_proj_bwd_graph_tc16(const void* dy16, const void* x, int dtype, int n_images, int C_uni, int64_t hw, int y_cmax,
                               const int32_t* dataset_ids, int n_datasets, float* dG, void* workspace, size_t workspace_bytes,
                               void* stream);
+/* The same three GEMMs with channels_last (pixel-major) x / feats [n_images, hw, C_uni], bf16 / fp16, C_uni % 8 == 0
+ * (16-byte TMA pixel stride), 16-byte-aligned bases; the planar operands (y, dy16) keep hw % 8 == 0.  Arguments,
+ * padding and workspace sizes as for the planar entry points; every output is bit-identical to theirs on x made
+ * NCHW-contiguous (same products, same K order, same reduction order).
+ * mdseg_proj_fwd_tc16_nhwc: x pixel-major (a K-major UMMA operand), y planar fp32 [n_images, y_cmax, hw].  With one
+ *   graph and dataset_ids = NULL it is the prototype head (mdseg_head_fwd_tc16 with fp32 output).
+ * mdseg_proj_bwd_tc16_nhwc: dx written pixel-major [n_images, hw, C_uni] (fp32 or the dtype of dy16); zero rows for
+ *   images whose dataset id is out of range.  With one operand and dataset_ids = NULL it is d feats of the head.
+ * mdseg_proj_bwd_graph_tc16_nhwc: x pixel-major (an MN-major UMMA operand).  dataset_ids = NULL with n_datasets = 1
+ *   sums over every image: d prototype of the head, dW [y_cmax, C_uni] (mdseg_head_dw_tc16). */
+int mdseg_proj_fwd_tc16_nhwc(const void* x, int dtype, int n_images, int C_uni, int64_t hw, const void* const* graphs_t,
+                             int ldb, const int* C_ds /*host*/, int n_datasets, const int32_t* dataset_ids, float* y,
+                             int y_cmax, void* stream);
+int mdseg_proj_bwd_tc16_nhwc(const void* dy16, int dtype, int n_images, int y_cmax, int64_t hw,
+                             const void* const* graphs_tt, int ldb, int C_uni, int n_datasets, const int32_t* dataset_ids,
+                             void* dx, int dx_dtype, void* stream);
+int mdseg_proj_bwd_graph_tc16_nhwc(const void* dy16, const void* x, int dtype, int n_images, int C_uni, int64_t hw,
+                                   int y_cmax, const int32_t* dataset_ids, int n_datasets, float* dG, void* workspace,
+                                   size_t workspace_bytes, void* stream);
 
 /* ---- MscEvalCrop (evaluate.py:650-753): sliding-window evaluation ------------------------------------------
  * probs[c, y0 + y, x0 + x] += g(softmax_c(logits)[c, y, x] (+ softmax_c(logits_flip)[c, y, cw - 1 - x])) for one chip

@@ -15,6 +15,16 @@
 //     warp stores 32 consecutive pixels of one prototype plane per instruction).
 //   * two CTAs per SM (two 40 KB stages and 256 TMEM columns each): one CTA's epilogue overlaps the other's main loop.
 // The N tiles of one pixel tile are neighbouring CTAs (blockIdx.x), so the second read of A comes from L2.
+//
+// Pixel-major (channels_last, NHWC) variants, chosen at compile time so that the MMA issue loop never branches on them:
+//   * kAK: A = x [n_images, hw, K] — the channel is contiguous, i.e. A is K-MAJOR, exactly like B: one TMA box
+//     [128 pixels][64 channels] (16 KB, the same kABytes) per stage, 128-byte swizzle, a_major = K.
+//   * kOutPM: the output is [n_images, hw, out_cstride] — a TMEM lane is a pixel and its columns are channels, so an
+//     epilogue thread writes 16 consecutive channels of its pixel (32 B in 16 bit, 64 B in fp32) as 16-byte stores.
+//   * head_tc16_dw_kernel<true> reads feats [n_images, hw, K] as its B operand (N = channels, K = pixels): MN-MAJOR,
+//     staged as ceil(NT / 64) TMA boxes [64 pixels][64 channels], the layout the forward uses for its MN-major A.
+// The tensor cores see the same 16-bit products in the same K order as on the planar layout, so every output of the
+// pixel-major variants is bit-identical to the planar entry point on x.contiguous().
 #include <cuda.h>
 
 #include "common.cuh"
@@ -78,7 +88,7 @@ struct alignas(64) BMaps {
 };
 
 struct HeadArgs {
-  void* out;          // [n_images, out_cstride, hw] fp32 or the feature dtype
+  void* out;          // [n_images, out_cstride, hw] (kOutPM: [n_images, hw, out_cstride]) fp32 or the feature dtype
   long long hw;
   const int32_t* dataset_ids;  // NULL: every image uses B operand 0
   int Nd[MDSEG_MAX_DATASETS], NTd[MDSEG_MAX_DATASETS];  // output rows / N tile width per B operand
@@ -86,7 +96,27 @@ struct HeadArgs {
   int zero_N, zero_NT;  // zero_N > 0: images of no dataset get zeros in their zero_N output rows (tiles of zero_NT)
 };
 
+// 16 channels of one pixel, pixel-major output: whole 16-byte stores (o is 32-byte aligned)
 template <typename TO>
+__device__ __forceinline__ void store16_pm(TO* o, const uint32_t* r) {
+  uint4* v = reinterpret_cast<uint4*>(o);
+  if constexpr (sizeof(TO) == 4) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) v[i] = make_uint4(r[4 * i], r[4 * i + 1], r[4 * i + 2], r[4 * i + 3]);
+  } else {
+    uint32_t w[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const TO lo = from_f32<TO>(__uint_as_float(r[2 * i])), hi = from_f32<TO>(__uint_as_float(r[2 * i + 1]));
+      w[i] = (uint32_t)(*reinterpret_cast<const unsigned short*>(&lo)) |
+             ((uint32_t)(*reinterpret_cast<const unsigned short*>(&hi)) << 16);
+    }
+    v[0] = make_uint4(w[0], w[1], w[2], w[3]);
+    v[1] = make_uint4(w[4], w[5], w[6], w[7]);
+  }
+}
+
+template <typename TO, bool kAK, bool kOutPM>
 __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_constant__ CUtensorMap mapA,
                                                                 const __grid_constant__ BMaps mapsB,
                                                                 const __grid_constant__ HeadArgs a) {
@@ -102,11 +132,20 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
   if (d < 0 || d >= a.n_datasets) {                 // uniform per CTA: an image of no dataset
     if (a.zero_N > 0) {                             // gradient route: its rows are zero (else the caller zero-fills)
       const int n0 = nz * a.zero_NT;
-      TO* ob = (TO*)a.out + ((long long)b * a.out_cstride + n0) * a.hw;
-      for (int i = threadIdx.x; i < a.zero_NT * kM; i += kThreads) {
-        const int c = i / kM;
-        const long long p = p0 + (i - c * kM);
-        if (n0 + c < a.zero_N && p < a.hw) ob[(long long)c * a.hw + p] = from_f32<TO>(0.f);
+      if constexpr (kOutPM) {  // rows [p0, p0 + 128) x channels [n0, n0 + zero_NT): consecutive threads, consecutive channels
+        TO* ob = (TO*)a.out + (long long)b * a.hw * a.out_cstride + n0;
+        for (int i = threadIdx.x; i < a.zero_NT * kM; i += kThreads) {
+          const int r = i / a.zero_NT, c = i - r * a.zero_NT;
+          const long long p = p0 + r;
+          if (n0 + c < a.zero_N && p < a.hw) ob[p * a.out_cstride + c] = from_f32<TO>(0.f);
+        }
+      } else {
+        TO* ob = (TO*)a.out + ((long long)b * a.out_cstride + n0) * a.hw;
+        for (int i = threadIdx.x; i < a.zero_NT * kM; i += kThreads) {
+          const int c = i / kM;
+          const long long p = p0 + (i - c * kM);
+          if (n0 + c < a.zero_N && p < a.hw) ob[(long long)c * a.hw + p] = from_f32<TO>(0.f);
+        }
       }
     }
     return;
@@ -143,15 +182,19 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
         if (kb >= kNStages) bar_wait(&empty[s], (uint32_t)((kb / kNStages - 1) & 1));
         unsigned char* st = smem + (size_t)s * stage_bytes;
         bar_expect(&full[s], stage_bytes);
-        tma3(st, &mapA, &full[s], (int)p0, kb * kKB, b);                      // pixels p0 .. p0+63
-        tma3(st + kKB * 128, &mapA, &full[s], (int)p0 + 64, kb * kKB, b);     // pixels p0+64 .. p0+127
+        if constexpr (kAK) {
+          tma3(st, &mapA, &full[s], kb * kKB, (int)p0, b);                    // [128 pixels][64 channels]
+        } else {
+          tma3(st, &mapA, &full[s], (int)p0, kb * kKB, b);                    // pixels p0 .. p0+63
+          tma3(st + kKB * 128, &mapA, &full[s], (int)p0 + 64, kb * kKB, b);   // pixels p0+64 .. p0+127
+        }
         tma2(st + kABytes, &mapB, &full[s], kb * kKB, nz * NT);
       }
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      // instruction descriptor: fp32 accumulate, A MN-major (bit 15), B K-major, N = NT, M = 128
-      const uint32_t idesc = (1u << 4) | ((uint32_t)a.fmt << 7) | ((uint32_t)a.fmt << 10) | (1u << 15) |
+      // instruction descriptor: fp32 accumulate, A MN-major (bit 15; clear for kAK), B K-major, N = NT, M = 128
+      const uint32_t idesc = (1u << 4) | ((uint32_t)a.fmt << 7) | ((uint32_t)a.fmt << 10) | (kAK ? 0u : (1u << 15)) |
                              ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(kM >> 4) << 24);
       for (int kb = 0; kb < a.n_kb; ++kb) {
         const int s = kb % kNStages;
@@ -160,8 +203,9 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
         const uint32_t aA = sa(smem + (size_t)s * stage_bytes), aB = aA + kABytes;
 #pragma unroll
         for (int ks = 0; ks < kKB / 16; ++ks) {
-          // A (MN-major): 16 channels = two 8-row atoms of 1024 B; the second 64-pixel atom kKB * 128 B further on
-          const uint64_t ad = desc_sw128(aA + ks * 2048, kKB * 128, 1024);
+          // A (MN-major): 16 channels = two 8-row atoms of 1024 B; the second 64-pixel atom kKB * 128 B further on.
+          // A (kAK, K-major): like B — 16 channels = 32 bytes inside the swizzle row; 8-pixel groups 1024 B apart
+          const uint64_t ad = kAK ? desc_sw128(aA + ks * 32, 16, 1024) : desc_sw128(aA + ks * 2048, kKB * 128, 1024);
           // B (K-major): 16 k = 32 bytes inside the 128-byte swizzle row; 8-row groups 1024 B apart
           const uint64_t bd = desc_sw128(aB + ks * 32, 16, 1024);
           umma(tmem_d, ad, bd, idesc, (kb > 0 || ks > 0) ? 1u : 0u);
@@ -177,7 +221,7 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
     bar_wait(&acc_full, 0);
     tc_after();
     const int n0 = nz * NT;
-    TO* ob = (TO*)a.out + ((long long)b * a.out_cstride + n0) * a.hw;
+    TO* ob = (TO*)a.out + ((long long)b * a.out_cstride + n0) * a.hw;  // planar output
     // 16 accumulator columns per TMEM load, two register sets: the load of the next 16 columns is in flight while the
     // current ones are stored (a load + wait + 16 stores in lockstep left the four epilogue warps waiting on TMEM
     // latency for about half of the epilogue).  The wait names the registers it releases, so no use can move above it.
@@ -197,7 +241,17 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
                  "+r"(R[8]), "+r"(R[9]), "+r"(R[10]), "+r"(R[11]), "+r"(R[12]), "+r"(R[13]), "+r"(R[14]), "+r"(R[15])   \
                :: "memory")
 #define MDSEG_H16_ST(R, C0)                                                                                            \
-  if (p < a.hw) {                                                                                                      \
+  if constexpr (kOutPM) {                                                                                              \
+    if (p < a.hw) {                                                                                                    \
+      TO* o = (TO*)a.out + ((long long)b * a.hw + p) * a.out_cstride + n0 + (C0);                                      \
+      if (n0 + (C0) + 16 <= Nout) {                                                                                    \
+        store16_pm<TO>(o, R);                                                                                          \
+      } else {                                                                                                         \
+        _Pragma("unroll") for (int i = 0; i < 16; ++i)                                                                 \
+          if (n0 + (C0) + i < Nout) o[i] = from_f32<TO>(__uint_as_float(R[i]));                                        \
+      }                                                                                                                \
+    }                                                                                                                  \
+  } else if (p < a.hw) {                                                                                               \
     TO* o = ob + (long long)(C0) * a.hw + p;                                                                           \
     if (n0 + (C0) + 16 <= Nout) { /* whole group inside the output: no per-column test */                              \
       _Pragma("unroll") for (int i = 0; i < 16; ++i) { *o = from_f32<TO>(__uint_as_float(R[i])); o += a.hw; }          \
@@ -234,12 +288,15 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
 // A CTA takes one 128-row tile of prototypes, one NT-column tile of feature channels and one slab of the pixels of
 // one image; its fp32 partial goes to a workspace slot and a second kernel adds the slots in a fixed order
 // (deterministic).  The tile CTAs of one slab are neighbours in the grid, so operand re-reads hit L2.
+// kBMN: feats is pixel-major [n_images, hw, K], so B is MN-major (the channel is contiguous): ceil(NT / 64) TMA boxes
+// [64 pixels][64 channels] per stage, b_major = MN.  Columns of the last box past NT are loaded and never read.
 struct DwArgs {
   float* part;        // [n_slabs_total][m_tiles][n_tiles][128][NT]
   long long hw, slab; // pixels per image, pixels per slab (multiple of 64)
   int slabs_per_image, m_tiles, n_tiles, NT, fmt;
 };
 
+template <bool kBMN>
 __global__ void __launch_bounds__(kThreads, 2) head_tc16_dw_kernel(const __grid_constant__ CUtensorMap mapA,
                                                                    const __grid_constant__ CUtensorMap mapB,
                                                                    const __grid_constant__ DwArgs a) {
@@ -256,7 +313,8 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_dw_kernel(const __grid_
   const int n_kb = (int)((p_end - p_beg + 63) / 64);
   const int NT = a.NT;
   constexpr uint32_t a_bytes = 128 * 128;  // [128 prototype rows][64 px x 2 B]
-  const uint32_t stage_bytes = a_bytes + (uint32_t)NT * 128u;
+  const int n_boxes = (NT + 63) / 64;  // kBMN: 64-channel boxes of B per stage
+  const uint32_t stage_bytes = a_bytes + (kBMN ? (uint32_t)n_boxes * 8192u : (uint32_t)NT * 128u);
   uint32_t tmem_cols = 32;
   while ((int)tmem_cols < NT) tmem_cols <<= 1;
 
@@ -287,14 +345,19 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_dw_kernel(const __grid_
         // pixels beyond the slab but inside the image would be counted twice: slabs are whole 64-pixel chunks, and
         // pixels beyond the image are zero-filled by TMA
         tma3(st, &mapA, &full[s], (int)(p_beg + (long long)kb * 64), mt * 128, b);
-        tma3(st + a_bytes, &mapB, &full[s], (int)(p_beg + (long long)kb * 64), nt * NT, b);
+        if constexpr (kBMN) {
+          for (int j = 0; j < n_boxes; ++j)
+            tma3(st + a_bytes + j * 8192, &mapB, &full[s], nt * NT + 64 * j, (int)(p_beg + (long long)kb * 64), b);
+        } else {
+          tma3(st + a_bytes, &mapB, &full[s], (int)(p_beg + (long long)kb * 64), nt * NT, b);
+        }
       }
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      // fp32 accumulate, both operands K-major, N = NT, M = 128
-      const uint32_t idesc = (1u << 4) | ((uint32_t)a.fmt << 7) | ((uint32_t)a.fmt << 10) | ((uint32_t)(NT >> 3) << 17) |
-                             ((uint32_t)(kM >> 4) << 24);
+      // fp32 accumulate, A K-major, B K-major (kBMN: MN-major, bit 16), N = NT, M = 128
+      const uint32_t idesc = (1u << 4) | ((uint32_t)a.fmt << 7) | ((uint32_t)a.fmt << 10) | (kBMN ? (1u << 16) : 0u) |
+                             ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(kM >> 4) << 24);
       for (int kb = 0; kb < n_kb; ++kb) {
         const int s = kb % kNStages;
         bar_wait(&full[s], (uint32_t)((kb / kNStages) & 1));
@@ -302,7 +365,9 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_dw_kernel(const __grid_
         const uint32_t aA = sa(smem + (size_t)s * stage_bytes), aB = aA + a_bytes;
 #pragma unroll
         for (int ks = 0; ks < 4; ++ks)
-          umma(tmem_d, desc_sw128(aA + ks * 32, 16, 1024), desc_sw128(aB + ks * 32, 16, 1024), idesc,
+          // kBMN: 16 pixels = two 8-row atoms of 1024 B; the next 64-channel atom one 8 KB box further on
+          umma(tmem_d, desc_sw128(aA + ks * 32, 16, 1024),
+               kBMN ? desc_sw128(aB + ks * 2048, 64 * 128, 1024) : desc_sw128(aB + ks * 32, 16, 1024), idesc,
                (kb > 0 || ks > 0) ? 1u : 0u);
         tc_commit(&empty[s]);
         if (kb == n_kb - 1) tc_commit(&acc_full);
@@ -377,18 +442,33 @@ extern "C" int mdseg_head_tc16_tile(int N) {
 
 namespace mdseg {
 namespace {
-// A = x [n_images, K, hw] (16-bit, MN-major by TMA); B operand d = bt[d]: [n_tiles(d) * NT(d), ldb] in the same dtype
+template <typename TO, bool kAK, bool kOutPM>
+int launch_head16_kernel(const CUtensorMap& mapA, const BMaps& mapsB, const HeadArgs& a, dim3 grid, size_t smem,
+                         cudaStream_t s) {
+  auto k = head_tc16_kernel<TO, kAK, kOutPM>;
+  MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k<<<grid, kThreads, smem, s>>>(mapA, mapsB, a);
+  return 0;
+}
+
+// A = x [n_images, K, hw] (16-bit, MN-major by TMA) or, a_pm, [n_images, hw, K] (K-major); B operand d = bt[d]:
+// [n_tiles(d) * NT(d), ldb] in the same dtype.  out: [n_images, out_cstride, hw] or, out_pm, [n_images, hw, out_cstride]
 int launch_head16(const void* x, int dtype, int n_images, int K, int64_t hw, const void* const* bt, int ldb, const int* Nd,
                   int n_b, const int32_t* dataset_ids, void* out, int out_cstride, int out_dtype, cudaStream_t s,
-                  const char* who, int zero_N = 0) {
+                  const char* who, int zero_N = 0, bool a_pm = false, bool out_pm = false) {
   MDSEG_REQUIRE(dtype == MDSEG_BF16 || dtype == MDSEG_F16, "%s: inputs must be bf16 or fp16", who);
   MDSEG_REQUIRE(out_dtype == MDSEG_F32 || out_dtype == dtype, "%s: output is fp32 or the input dtype", who);
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && K > 0 && hw > 0 && n_b > 0 && n_b <= MDSEG_MAX_DATASETS, "%s: bad shape", who);
   MDSEG_REQUIRE(ldb >= K && ldb % 8 == 0 && hw % 8 == 0,
                 "%s: ldb and h * w must be multiples of 8 (16-byte TMA strides), ldb >= K", who);
+  MDSEG_REQUIRE(!a_pm || K % 8 == 0, "%s: the channel count of pixel-major x must be a multiple of 8 (16-byte TMA pixel "
+                "stride)", who);
+  MDSEG_REQUIRE(!out_pm || out_cstride % 8 == 0, "%s: the channel count of a pixel-major output must be a multiple of 8",
+                who);
   if (n_images == 0) return 0;
   MDSEG_REQUIRE(x && out && bt && Nd, "%s: null pointer", who);
   MDSEG_REQUIRE(((uintptr_t)x & 15) == 0, "%s: operands must be 16-byte aligned", who);
+  MDSEG_REQUIRE(!out_pm || ((uintptr_t)out & 15) == 0, "%s: a pixel-major output must be 16-byte aligned", who);
   EncodeTiledFn enc = encode_fn();
   MDSEG_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available in this driver");
   static thread_local bool ctx_bound = false;
@@ -402,6 +482,11 @@ int launch_head16(const void* x, int dtype, int n_images, int K, int64_t hw, con
     cuuint64_t dims[3] = {(cuuint64_t)hw, (cuuint64_t)K, (cuuint64_t)n_images};
     cuuint64_t strides[2] = {(cuuint64_t)hw * 2, (cuuint64_t)K * hw * 2};
     cuuint32_t box[3] = {64, (cuuint32_t)kKB, 1};
+    if (a_pm) {  // [n_images, hw, K]: one box of [128 pixels][64 channels]
+      dims[0] = (cuuint64_t)K; dims[1] = (cuuint64_t)hw;
+      strides[0] = (cuuint64_t)K * 2;
+      box[0] = (cuuint32_t)kKB; box[1] = (cuuint32_t)kM;
+    }
     cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = enc(&mapA, dt, 3, const_cast<void*>(x), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -435,15 +520,19 @@ int launch_head16(const void* x, int dtype, int n_images, int K, int64_t hw, con
   if (tiles_max == 0) return 0;
   const size_t smem = (size_t)kNStages * (kABytes + (size_t)nt_max * 128) + 1024;
   const dim3 grid((unsigned)tiles_max, (unsigned)((hw + kM - 1) / kM), (unsigned)n_images);
-#define MDSEG_H16_LAUNCH(TO)                                                                              \
-  do {                                                                                                    \
-    auto k = head_tc16_kernel<TO>;                                                                        \
-    MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));       \
-    k<<<grid, kThreads, smem, s>>>(mapA, mapsB, a);                                                       \
-  } while (0)
-  if (out_dtype == MDSEG_F32) MDSEG_H16_LAUNCH(float);
-  else if (dtype == MDSEG_BF16) MDSEG_H16_LAUNCH(__nv_bfloat16);
-  else MDSEG_H16_LAUNCH(__half);
+  // the variants in use: planar in and out; pixel-major x with planar fp32 y (forward); planar dy with a pixel-major
+  // gradient (adjoint)
+  MDSEG_REQUIRE(!(a_pm && out_pm) && (!a_pm || out_dtype == MDSEG_F32), "%s: unsupported layout combination", who);
+#define MDSEG_H16_LAUNCH(TO, AK, PM) \
+  do { if (launch_head16_kernel<TO, AK, PM>(mapA, mapsB, a, grid, smem, s)) return 1; } while (0)
+  if (a_pm) MDSEG_H16_LAUNCH(float, true, false);
+  else if (out_pm) {
+    if (out_dtype == MDSEG_F32) MDSEG_H16_LAUNCH(float, false, true);
+    else if (dtype == MDSEG_BF16) MDSEG_H16_LAUNCH(__nv_bfloat16, false, true);
+    else MDSEG_H16_LAUNCH(__half, false, true);
+  } else if (out_dtype == MDSEG_F32) MDSEG_H16_LAUNCH(float, false, false);
+  else if (dtype == MDSEG_BF16) MDSEG_H16_LAUNCH(__nv_bfloat16, false, false);
+  else MDSEG_H16_LAUNCH(__half, false, false);
 #undef MDSEG_H16_LAUNCH
   MDSEG_LAUNCH_OK();
   return 0;
@@ -485,12 +574,15 @@ extern "C" size_t mdseg_head_dw_tc16_workspace_bytes(int n_images, int K, int64_
   return (size_t)n_images * spi * m_tiles * n_tiles * 128 * NT * 4 + 256;
 }
 
+// feats_pm: feats is pixel-major [n_images, hw, K] (channels_last), read as an MN-major B operand
 static int head_dw_tc16_impl(const void* dy16, const void* feats, int dtype, int n_images, int K, int64_t hw, int N,
                              const int32_t* dataset_ids, int n_datasets, float* dW, void* workspace, size_t workspace_bytes,
-                             void* stream) {
+                             void* stream, bool feats_pm = false) {
   using namespace mdseg;
   MDSEG_REQUIRE(dtype == MDSEG_BF16 || dtype == MDSEG_F16, "mdseg_head_dw_tc16: operands must be bf16 or fp16");
   MDSEG_REQUIRE(n_images > 0 && n_images <= 65535 && K > 0 && N > 0 && hw > 0 && hw % 8 == 0, "mdseg_head_dw_tc16: bad shape");
+  MDSEG_REQUIRE(!feats_pm || K % 8 == 0,
+                "mdseg_proj_bwd_graph_tc16_nhwc: the channel count must be a multiple of 8 (16-byte TMA pixel stride)");
   MDSEG_REQUIRE(dy16 && feats && dW && workspace, "mdseg_head_dw_tc16: null pointer");
   MDSEG_REQUIRE((((uintptr_t)dy16 | (uintptr_t)feats) & 15) == 0, "mdseg_head_dw_tc16: operands must be 16-byte aligned");
   MDSEG_REQUIRE(workspace_bytes >= mdseg_head_dw_tc16_workspace_bytes(n_images, K, hw, N),
@@ -527,15 +619,27 @@ static int head_dw_tc16_impl(const void* dy16, const void* feats, int dtype, int
     cuuint64_t dims[3] = {(cuuint64_t)hw, (cuuint64_t)K, (cuuint64_t)n_images};
     cuuint64_t strides[2] = {(cuuint64_t)hw * 2, (cuuint64_t)K * hw * 2};
     cuuint32_t box[3] = {64, (cuuint32_t)a.NT, 1};
+    if (feats_pm) {  // [n_images, hw, K]: boxes of [64 pixels][64 channels]
+      dims[0] = (cuuint64_t)K; dims[1] = (cuuint64_t)hw;
+      strides[0] = (cuuint64_t)K * 2;
+      box[0] = 64; box[1] = 64;
+    }
     CUresult r = enc(&mapB, dt, 3, const_cast<void*>(feats), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     MDSEG_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed for the features (CUresult %d)", (int)r);
   }
   const int n_slabs_total = n_images * a.slabs_per_image;
-  const size_t smem = (size_t)kNStages * (128 * 128 + (size_t)a.NT * 128) + 1024;
+  const size_t b_bytes = feats_pm ? (size_t)((a.NT + 63) / 64) * 8192 : (size_t)a.NT * 128;
+  const size_t smem = (size_t)kNStages * (128 * 128 + b_bytes) + 1024;
   cudaStream_t s = (cudaStream_t)stream;
-  MDSEG_CUDA_OK(cudaFuncSetAttribute(head_tc16_dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  head_tc16_dw_kernel<<<dim3((unsigned)(a.m_tiles * a.n_tiles), (unsigned)n_slabs_total), kThreads, smem, s>>>(mapA, mapB, a);
+  const dim3 grid((unsigned)(a.m_tiles * a.n_tiles), (unsigned)n_slabs_total);
+  if (feats_pm) {
+    MDSEG_CUDA_OK(cudaFuncSetAttribute(head_tc16_dw_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    head_tc16_dw_kernel<true><<<grid, kThreads, smem, s>>>(mapA, mapB, a);
+  } else {
+    MDSEG_CUDA_OK(cudaFuncSetAttribute(head_tc16_dw_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    head_tc16_dw_kernel<false><<<grid, kThreads, smem, s>>>(mapA, mapB, a);
+  }
   MDSEG_LAUNCH_OK();
   head_tc16_dw_reduce_kernel<<<dim3((unsigned)(((long long)N * K + 255) / 256), (unsigned)(dataset_ids ? n_datasets : 1)),
                                256, 0, s>>>(a, n_slabs_total, N, K, dataset_ids, dW);
@@ -569,4 +673,34 @@ extern "C" int mdseg_proj_bwd_tc16(const void* dy16, int dtype, int n_images, in
   for (int d = 0; d < n_datasets; ++d) Nd[d] = C_uni;
   return mdseg::launch_head16(dy16, dtype, n_images, y_cmax, hw, graphs_tt, ldb, Nd, n_datasets, dataset_ids, dx, C_uni,
                               dx_dtype, (cudaStream_t)stream, "mdseg_proj_bwd_tc16", /*zero_N=*/C_uni);
+}
+
+// ---- channels_last (pixel-major) x / feats: the same kernels with K-major A, MN-major B or a pixel-major output ------
+extern "C" int mdseg_proj_fwd_tc16_nhwc(const void* x, int dtype, int n_images, int C_uni, int64_t hw,
+                                        const void* const* graphs_t, int ldb, const int* C_ds, int n_datasets,
+                                        const int32_t* dataset_ids, float* y, int y_cmax, void* stream) {
+  for (int d = 0; d < n_datasets && d < MDSEG_MAX_DATASETS; ++d)
+    MDSEG_REQUIRE(!C_ds || C_ds[d] <= y_cmax, "mdseg_proj_fwd_tc16_nhwc: y_cmax %d < C_ds %d", y_cmax, C_ds[d]);
+  return mdseg::launch_head16(x, dtype, n_images, C_uni, hw, graphs_t, ldb, C_ds, n_datasets, dataset_ids, y, y_cmax, MDSEG_F32,
+                              (cudaStream_t)stream, "mdseg_proj_fwd_tc16_nhwc", 0, /*a_pm=*/true, /*out_pm=*/false);
+}
+
+extern "C" int mdseg_proj_bwd_tc16_nhwc(const void* dy16, int dtype, int n_images, int y_cmax, int64_t hw,
+                                        const void* const* graphs_tt, int ldb, int C_uni, int n_datasets,
+                                        const int32_t* dataset_ids, void* dx, int dx_dtype, void* stream) {
+  MDSEG_REQUIRE(C_uni > 0 && n_datasets > 0 && n_datasets <= MDSEG_MAX_DATASETS, "mdseg_proj_bwd_tc16_nhwc: bad shape");
+  int Nd[MDSEG_MAX_DATASETS];
+  for (int d = 0; d < n_datasets; ++d) Nd[d] = C_uni;
+  return mdseg::launch_head16(dy16, dtype, n_images, y_cmax, hw, graphs_tt, ldb, Nd, n_datasets, dataset_ids, dx, C_uni,
+                              dx_dtype, (cudaStream_t)stream, "mdseg_proj_bwd_tc16_nhwc", /*zero_N=*/C_uni,
+                              /*a_pm=*/false, /*out_pm=*/true);
+}
+
+extern "C" int mdseg_proj_bwd_graph_tc16_nhwc(const void* dy16, const void* x, int dtype, int n_images, int C_uni,
+                                              int64_t hw, int y_cmax, const int32_t* dataset_ids, int n_datasets, float* dG,
+                                              void* workspace, size_t workspace_bytes, void* stream) {
+  MDSEG_REQUIRE(n_datasets > 0 && n_datasets <= MDSEG_MAX_DATASETS && (dataset_ids || n_datasets == 1),
+                "mdseg_proj_bwd_graph_tc16_nhwc: 1..%d datasets, dataset ids unless there is one", MDSEG_MAX_DATASETS);
+  return head_dw_tc16_impl(dy16, x, dtype, n_images, C_uni, hw, y_cmax, dataset_ids, n_datasets, dG, workspace,
+                           workspace_bytes, stream, /*feats_pm=*/true);
 }

@@ -261,7 +261,8 @@ def target_bipart_from_hist(hist, bipart_graph, ignore_index=255):
 def eval_find_use_and_unuse_label(configer, net, dls=None):
     """evaluate.py:1788-1930 — per dataset the rectangular ``[n_cats, C_uni]`` histogram of the labels against the
     arg-max of the UNIFIED logits (prototype einsum -> bilinear up-sampling -> soft-max -> arg-max), then the
-    bucket rules that produce ``target_bi_graph`` for the GNN stage.  The prototype einsum runs on tcgen05 (ops.prototype_head);
+    bucket rules that produce ``target_bi_graph`` for the GNN stage.  The prototype einsum runs on tcgen05 (ops.prototype_head;
+    a channels_last bf16 / fp16 embedding is read as it is, without a layout copy);
     up-sampling + arg-max (soft-max is monotone, no [C_uni, H, W] tensor) and the histogram run in libmdseg_b200.so.
     `dls` defaults to the reference's ``get_data_loader(configer, aux_mode='train', distributed=..., stage=2)``."""
     org_aux = net.aux_mode

@@ -16,7 +16,9 @@ What runs where:
       - GNN stage (is_adv=True, trainable soft / hard graph pairs): the same fused loss once per graph set, blended
         by ``max_rate`` (:1063-1071), with gradients to the logits AND to every ``bi_graphs[i]`` (tcgen05 split-K
         ``d bi_graph``); aux heads from the dataset prototypes (:941-951, :1044-1048) through the fused
-        up-sample + OhemCE(0.7) kernels;
+        up-sample + OhemCE(0.7) kernels; channels_last bf16 / fp16 features (``preds['seg']``, K % 8 == 0) are taken as
+        they are by the prototype head and the folded / dense-graph losses and get a channels_last gradient (the
+        ``feats.index_select`` rows of the aux prototypes are a gathered copy either way);
   * the prototype contractions ``einsum('bchw,nc->bnhw', feats, unify_prototype[...])`` (:950, :961, :971) — the
     producer of the unified logits, SURVEY §8 f2 — run on the tcgen05 tensor cores.  With ``FOLD_PROTOTYPES`` (the
     default) the unified head and the bipartite projection behind it are ONE contraction with

@@ -537,6 +537,18 @@ def _nhwc_proj_ok(x, tab):
             and all(not tab.g[i].dense and tab.g[i].C_ds <= N.NHWC_MAX_CDS for i in range(tab.n_datasets)))
 
 
+def _nhwc_tc16_ok(x, tab=None):
+    """channels_last 16-bit features / logits that the TMA-fed tcgen05 kernels read as they are (the *_tc16_nhwc entry
+    points): the channel count a multiple of 8 (16-byte TMA pixel stride), a 16-byte-aligned base, h * w a multiple of
+    8 (the planar y / dy) and, with a graph table, all graphs dense with 8 <= C_ds <= 1024 and C_uni >= 32 (the tc16
+    envelope of the projection).  Anything else (fp32, odd channel counts, storage offsets) takes x.contiguous()."""
+    if not (_channels_last(x) and x.dtype in (torch.bfloat16, torch.float16) and x.shape[1] % 8 == 0
+            and x.data_ptr() % 16 == 0 and (x.shape[2] * x.shape[3]) % 8 == 0):
+        return False
+    return tab is None or (tab.C_uni >= 32 and all(tab.g[i].dense and 8 <= tab.g[i].C_ds <= 1024
+                                                   for i in range(tab.n_datasets)))
+
+
 # ---- a5 projection alone (model-side eval einsum, semseg.py:342-345) --------------------------------
 def project(logits_uni, graphs, dataset_ids=None, cache=None):
     """fp32 [B, max C_ds, h, w]: einsum('bchw,nc->bnhw') with the graph of each image's dataset.  channels_last logits
@@ -557,14 +569,16 @@ def project(logits_uni, graphs, dataset_ids=None, cache=None):
 def _proj_fwd(x, tab, ids, B, h, w, y, cmax, ymax, ef, graphs=None):
     """mdseg_proj_fwd, or mdseg_proj_fwd_tc (dense graphs on the tensor cores) when a graph is dense; 16-bit logits
     with all-dense graphs take the TMA-fed kernel (mdseg_proj_fwd_tc16); channels_last x (callers pass it only when
-    _nhwc_proj_ok) takes mdseg_proj_fwd_nhwc."""
+    _nhwc_proj_ok or _nhwc_tc16_ok) takes mdseg_proj_fwd_nhwc (sparse graphs) or mdseg_proj_fwd_tc16_nhwc (dense)."""
     n = tab.n_datasets
-    if _channels_last(x):
+    nhwc = _channels_last(x)
+    if nhwc and not all(tab.g[i].dense for i in range(n)):
         N.call("mdseg_proj_fwd_nhwc", _ptr(x), _DT[x.dtype], C.byref(tab), _ptr(ids), B, h, w, _ptr(y), cmax, _ptr(ymax),
                _ptr(ef), _stream())
         return
-    if (graphs is not None and x.dtype in (torch.bfloat16, torch.float16) and (h * w) % 8 == 0 and x.data_ptr() % 16 == 0
-            and all(tab.g[i].dense and 8 <= tab.g[i].C_ds <= 1024 for i in range(n)) and tab.C_uni >= 32):
+    if nhwc or (graphs is not None and x.dtype in (torch.bfloat16, torch.float16) and (h * w) % 8 == 0
+                and x.data_ptr() % 16 == 0 and all(tab.g[i].dense and 8 <= tab.g[i].C_ds <= 1024 for i in range(n))
+                and tab.C_uni >= 32):
         ldb = (tab.C_uni + 7) // 8 * 8
         ptrs, cds = (C.c_void_p * n)(), (C.c_int * n)()
         rows = []
@@ -577,8 +591,8 @@ def _proj_fwd(x, tab, ids, B, h, w, y, cmax, ymax, ef, graphs=None):
             gt[o:o + g.shape[0], :tab.C_uni] = g.detach().to(x.dtype)
             ptrs[i], cds[i] = gt.data_ptr() + o * ldb * gt.element_size(), g.shape[0]
             o += rows[i]
-        N.call("mdseg_proj_fwd_tc16", _ptr(x), _DT[x.dtype], B, tab.C_uni, h * w, ptrs, ldb, cds, n, _ptr(ids), _ptr(y), cmax,
-               _stream())
+        N.call("mdseg_proj_fwd_tc16_nhwc" if nhwc else "mdseg_proj_fwd_tc16", _ptr(x), _DT[x.dtype], B, tab.C_uni, h * w,
+               ptrs, ldb, cds, n, _ptr(ids), _ptr(y), cmax, _stream())
         return
     if any(tab.g[i].dense for i in range(tab.n_datasets)):
         nbytes = N.lib.mdseg_proj_fwd_tc_workspace_bytes(C.byref(tab), _DT[x.dtype])
@@ -605,17 +619,29 @@ def _tc16_ok(x):
     return x.dtype in (torch.bfloat16, torch.float16) and (x.shape[2] * x.shape[3]) % 8 == 0 and x.data_ptr() % 16 == 0
 
 
+def _head_operand(wgt, dtype):
+    """wgt fp32 [n_rows, K] (any strides) as the B operand of the tc16 kernels: dtype, rows padded to whole N tiles,
+    K padded to ldb (a multiple of 8), zeros in the padding.  -> (wt, ldb)"""
+    n_rows, K = wgt.shape
+    nt = N.lib.mdseg_head_tc16_tile(n_rows)
+    ldb = (K + 7) // 8 * 8
+    wt = torch.zeros(((n_rows + nt - 1) // nt) * nt, ldb, dtype=dtype, device=wgt.device)
+    wt[:n_rows, :K] = wgt.to(dtype)
+    return wt, ldb
+
+
 def _head_tc16(a, wgt, out):
     """out[b, n, p] = sum_k a[b, k, p] * wgt[n, k] with 16-bit `a` [B, K, h, w]; wgt: fp32 [n_rows, K] (any strides);
     out: fp32 or a's dtype.  mdseg_head_fwd_tc16 (TMA + tcgen05)."""
     B, K, h, w = a.shape
     n_rows = wgt.shape[0]
-    nt = N.lib.mdseg_head_tc16_tile(n_rows)
-    ldb = (K + 7) // 8 * 8
-    wt = torch.zeros(((n_rows + nt - 1) // nt) * nt, ldb, dtype=a.dtype, device=a.device)
-    wt[:n_rows, :K] = wgt.to(a.dtype)
+    wt, ldb = _head_operand(wgt, a.dtype)
     N.call("mdseg_head_fwd_tc16", _ptr(a), _DT[a.dtype], B, K, h * w, _ptr(wt), ldb, n_rows, _ptr(out), _DT[out.dtype],
            _stream())
+
+
+def _one(t):
+    return (C.c_void_p * 1)(t.data_ptr())
 
 
 class _PrototypeHead(torch.autograd.Function):
@@ -624,7 +650,9 @@ class _PrototypeHead(torch.autograd.Function):
     [128 px, N] x [N, K] tcgen05 GEMM per CTA (mdseg_proj_fwd_tc with the prototypes in the role of the dense graph,
     N tiled by 256).  Backward: d feats = proto^T dlogits (mdseg_proj_bwd_tc), d proto = dlogits feats^T as a split-K
     GEMM over the pixels (mdseg_proj_bwd_graph_tc).  fp32 inputs: three bf16 terms per operand (1e-5 bar);
-    bf16 / fp16 inputs: one product in their own type, like autocast.  Output fp32."""
+    bf16 / fp16 inputs: one product in their own type, like autocast.  Output fp32 NCHW.  channels_last 16-bit features
+    (_nhwc_tc16_ok) are read as they are by the *_tc16_nhwc kernels and get a channels_last gradient, bit-identical to
+    the NCHW route; other channels_last features are copied to NCHW first."""
 
     @staticmethod
     def forward(ctx, feats, proto):
@@ -632,7 +660,8 @@ class _PrototypeHead(torch.autograd.Function):
         x = feats
         if x.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             x = x.float()
-        x = x.contiguous()
+        if not _nhwc_tc16_ok(x):
+            x = x.contiguous()
         B, K, h, w = x.shape
         if proto.dim() != 2 or proto.shape[1] != K:
             raise ValueError(f"prototypes must be [N, {K}]")
@@ -641,6 +670,12 @@ class _PrototypeHead(torch.autograd.Function):
         y = torch.empty(B, Nn, h, w, dtype=torch.float32, device=x.device)
         ctx.save_for_backward(x, wgt)
         ctx.proto_dtype = proto.dtype
+        if _channels_last(x):
+            # channels_last 16-bit features: K-major A operand, one dense "graph" = the prototypes
+            wt, ldb = _head_operand(wgt, x.dtype)
+            N.call("mdseg_proj_fwd_tc16_nhwc", _ptr(x), _DT[x.dtype], B, K, h * w, _one(wt), ldb, (C.c_int * 1)(Nn), 1,
+                   None, _ptr(y), Nn, _stream())
+            return y
         if _tc16_ok(x):
             # 16-bit features: TMA-fed MN-major operands, warp-specialised (csrc/head_tc16.cu)
             _head_tc16(x, wgt, y)
@@ -660,6 +695,23 @@ class _PrototypeHead(torch.autograd.Function):
         dy = dy.to(torch.float32).contiguous()
         tab = _dense_table(wgt)
         dx = dw = None
+        if _channels_last(x):
+            # channels_last 16-bit features (see forward): d feats written pixel-major, d proto with the features as an
+            # MN-major operand; the same products and reduction order as the NCHW branch below
+            dyh = dy.to(x.dtype)
+            if ctx.needs_input_grad[0]:
+                wt, ldb = _head_operand(wgt.t(), x.dtype)
+                dx = torch.empty_like(x)  # channels_last
+                N.call("mdseg_proj_bwd_tc16_nhwc", _ptr(dyh), _DT[x.dtype], B, Nn, h * w, _one(wt), ldb, K, 1, None,
+                       _ptr(dx), _DT[x.dtype], _stream())
+            if ctx.needs_input_grad[1]:
+                dG = torch.empty(Nn, K, dtype=torch.float32, device=x.device)
+                nb = N.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, K, h * w, Nn)
+                ws = torch.empty(nb, dtype=torch.uint8, device=x.device)
+                N.call("mdseg_proj_bwd_graph_tc16_nhwc", _ptr(dyh), _ptr(x), _DT[x.dtype], B, K, h * w, Nn, None, 1,
+                       _ptr(dG), _ptr(ws), nb, _stream())
+                dw = dG.to(ctx.proto_dtype)
+            return dx, dw
         if _tc16_ok(x):
             # 16-bit features: both gradients on the TMA-fed kernels.  The incoming gradient is rounded to the feature
             # dtype first (what the reference's autocast backward does to it).
@@ -692,14 +744,17 @@ class _PrototypeHead(torch.autograd.Function):
 
 
 def prototype_head(feats, proto):
-    """einsum('bchw,nc->bnhw', feats [B, K, h, w], proto [N, K]) -> fp32 [B, N, h, w] on the tensor cores."""
+    """einsum('bchw,nc->bnhw', feats [B, K, h, w], proto [N, K]) -> fp32 [B, N, h, w] (NCHW) on the tensor cores.
+    channels_last bf16 / fp16 features with K % 8 == 0 are read without a layout copy."""
     return _PrototypeHead.apply(feats, proto)
 
 
 # ---- a5+a6+a7+a8+a9: the fused multi-dataset loss ------------------------------------------------------
 class _MdsProjOhemCE(torch.autograd.Function):
     """MdsOhemCELoss(project -> upsample -> CE) of loss_cross_datasets.py:1006-1007,1074 in four kernels.  channels_last
-    logits with sparse graphs are projected as they are and get a channels_last gradient (mdseg_proj_*_nhwc)."""
+    logits with sparse graphs are projected as they are and get a channels_last gradient (mdseg_proj_*_nhwc); so are
+    channels_last 16-bit logits / features with dense graphs (folded prototypes, trainable graphs) when the backward takes
+    the tc16 route (mdseg_proj_*_tc16_nhwc)."""
 
     @staticmethod
     def forward(ctx, logits_uni, labels, dataset_ids, thresh, ignore, cache, per_dataset, *graphs):
@@ -717,8 +772,6 @@ class _MdsProjOhemCE(torch.autograd.Function):
         tab, keep = cache.table(list(graphs))
         if tab.C_uni != Cu:
             raise ValueError(f"graphs have C_uni={tab.C_uni}, logits have {Cu}")
-        if not _nhwc_proj_ok(x, tab):
-            x = x.contiguous()
         Cs = [g.shape[0] for g in graphs]
         cmax = max(Cs)
         ids = _ids32(dataset_ids, B, dev)
@@ -726,10 +779,12 @@ class _MdsProjOhemCE(torch.autograd.Function):
         y = torch.empty(B, cmax, h, w, dtype=torch.float32, device=dev)
         ymax = torch.empty(B, h, w, dtype=torch.float32, device=dev)  # channel maximum of y: the softmax shift
         all_sparse = all(not tab.g[i].dense for i in range(len(Cs)))
-        _proj_fwd(x, tab, ids, B, h, w, y, cmax, ymax, ef, graphs=graphs)
         n_seg = len(Cs) if per_dataset else 1
         src = _src_table([y.data_ptr()] * len(Cs), [cmax * h * w] * len(Cs), Cs, N.F32, per_dataset, c_alloc=cmax,
                          cmax=ymax, cmax_ready=all_sparse)
+        if not (_nhwc_proj_ok(x, tab) or (_nhwc_tc16_ok(x, tab) and _tc16_bwd_nhwc_ok(ctx, len(Cs), src, h, w, H, W))):
+            x = x.contiguous()
+        _proj_fwd(x, tab, ids, B, h, w, y, cmax, ymax, ef, graphs=graphs)
         P = B * H * W
         loss_px = torch.empty(P, dtype=torch.float32, device=dev)
         lse_px = torch.empty(P, dtype=torch.float32, device=dev)
@@ -793,6 +848,7 @@ class _MdsProjOhemCE(torch.autograd.Function):
             if ids is None:
                 ids = torch.zeros(B, dtype=torch.int32, device=dev)
             dx = None
+            nhwc = _channels_last(x)  # channels_last x (see forward): dx written pixel-major, x read pixel-major
             if ctx.needs_input_grad[0]:
                 ldb = (cmax + 7) // 8 * 8
                 nt = N.lib.mdseg_head_tc16_tile(Cu)
@@ -803,13 +859,13 @@ class _MdsProjOhemCE(torch.autograd.Function):
                     gt[i, :Cu, :Cs[i]] = gph.detach().t().to(x.dtype)
                     ptrs[i] = gt[i].data_ptr()
                 dx = torch.empty_like(x)
-                N.call("mdseg_proj_bwd_tc16", _ptr(dy16), _DT[x.dtype], B, cmax, h * w, ptrs, ldb, Cu, n, _ptr(ids),
-                       _ptr(dx), _DT[x.dtype], _stream())
+                N.call("mdseg_proj_bwd_tc16_nhwc" if nhwc else "mdseg_proj_bwd_tc16", _ptr(dy16), _DT[x.dtype], B, cmax,
+                       h * w, ptrs, ldb, Cu, n, _ptr(ids), _ptr(dx), _DT[x.dtype], _stream())
             dG = torch.empty(n, cmax, Cu, dtype=torch.float32, device=dev)
             nb = N.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, Cu, h * w, cmax)
             ws2 = torch.empty(nb, dtype=torch.uint8, device=dev)
-            N.call("mdseg_proj_bwd_graph_tc16", _ptr(dy16), _ptr(x), _DT[x.dtype], B, Cu, h * w, cmax, _ptr(ids), n,
-                   _ptr(dG), _ptr(ws2), nb, _stream())
+            N.call("mdseg_proj_bwd_graph_tc16_nhwc" if nhwc else "mdseg_proj_bwd_graph_tc16", _ptr(dy16), _ptr(x),
+                   _DT[x.dtype], B, Cu, h * w, cmax, _ptr(ids), n, _ptr(dG), _ptr(ws2), nb, _stream())
             dgs = [dG[i, :Cs[i]].to(graphs[i].dtype) if ctx.needs_input_grad[7 + i] else None for i in range(n)]
             return (dx, None, None, None, None, None, None, *dgs)
         dyA, dyB = _mds_dy(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, y, Cs, cmax)
@@ -840,6 +896,16 @@ class _MdsProjOhemCE(torch.autograd.Function):
                 if ctx.needs_input_grad[7 + i]:
                     dgs[i] = dG[i, :Cs[i] * Cu].view(Cs[i], Cu).to(graphs[i].dtype)
         return (dx, None, None, None, None, None, None, *dgs)
+
+
+def _tc16_bwd_nhwc_ok(ctx, n, src, h, w, H, W):
+    """_MdsProjOhemCE with dense graphs (x passed _nhwc_tc16_ok): the backward reads x only on its tc16 branch — taken
+    when a graph wants a gradient and the upsample + CE adjoint is the fused kernel — or never runs (no input wants a
+    gradient).  A d x without d graphs goes through mdseg_mds_bwd, which writes dx planar, so x is copied then."""
+    want_dg = any(ctx.needs_input_grad[7 + i] for i in range(n))
+    if not want_dg:
+        return not ctx.needs_input_grad[0]
+    return bool(N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W))
 
 
 def _mds_dy(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, y, Cs, cmax):
@@ -883,14 +949,14 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
     graph pair, lib/loss/loss_cross_datasets.py:996-1004,1063-1071): ONE projection with the graphs of a dataset
     stacked to [H * C_ds, C_uni], H fused CE / OHEM passes on the slices of y, and in the backward one adjoint and one
     d-graph GEMM over the stacked gradient planes — x is read once per direction instead of H times and its gradient
-    is written once instead of H times and added.  Dense graphs only (tensor-core routes); `graphs` is head-major."""
+    is written once instead of H times and added.  Dense graphs only (tensor-core routes); `graphs` is head-major.
+    channels_last 16-bit x (_nhwc_tc16_ok) is read as it is and gets a channels_last gradient."""
 
     @staticmethod
     def forward(ctx, x, labels, dataset_ids, thresh, ignore, n_heads, *graphs):
         _require_cuda(x, labels)
         if x.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             x = x.float()
-        x = x.contiguous()
         B, Cu, h, w = x.shape
         labels = _labels(labels)
         H, W = labels.shape[1:]
@@ -902,6 +968,8 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
         stacked = [torch.cat([graphs[k * n + d].detach().to(torch.float32) for k in range(n_heads)], 0) for d in range(n)]
         cache = BipartiteGraphs(assume_dense=True)
         tab, keep = cache.table(stacked)
+        if not _nhwc_tc16_ok(x, tab):  # the backward's tc16 branch holds exactly when this does
+            x = x.contiguous()
         ids = _ids32(dataset_ids, B, dev)
         ef = err_flag(dev)
         y = torch.empty(B, cmax2, h, w, dtype=torch.float32, device=dev)
@@ -952,6 +1020,7 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
         dx = None
         if tc16:
             ids_ = ids if ids is not None else torch.zeros(B, dtype=torch.int32, device=dev)
+            nhwc = _channels_last(x)
             if ctx.needs_input_grad[0]:
                 ldb = (cmax2 + 7) // 8 * 8
                 nt = N.lib.mdseg_head_tc16_tile(Cu)
@@ -962,13 +1031,13 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
                     gt[i, :Cu, :Cs2[i]] = gph.t().to(x.dtype)
                     ptrs[i] = gt[i].data_ptr()
                 dx = torch.empty_like(x)
-                N.call("mdseg_proj_bwd_tc16", _ptr(dy), _DT[x.dtype], B, cmax2, h * w, ptrs, ldb, Cu, n, _ptr(ids_),
-                       _ptr(dx), _DT[x.dtype], _stream())
+                N.call("mdseg_proj_bwd_tc16_nhwc" if nhwc else "mdseg_proj_bwd_tc16", _ptr(dy), _DT[x.dtype], B, cmax2,
+                       h * w, ptrs, ldb, Cu, n, _ptr(ids_), _ptr(dx), _DT[x.dtype], _stream())
             dG = torch.empty(n, cmax2, Cu, dtype=torch.float32, device=dev)
             nb = N.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, Cu, h * w, cmax2)
             ws2 = torch.empty(nb, dtype=torch.uint8, device=dev)
-            N.call("mdseg_proj_bwd_graph_tc16", _ptr(dy), _ptr(x), _DT[x.dtype], B, Cu, h * w, cmax2, _ptr(ids_), n,
-                   _ptr(dG), _ptr(ws2), nb, _stream())
+            N.call("mdseg_proj_bwd_graph_tc16_nhwc" if nhwc else "mdseg_proj_bwd_graph_tc16", _ptr(dy), _ptr(x),
+                   _DT[x.dtype], B, Cu, h * w, cmax2, _ptr(ids_), n, _ptr(dG), _ptr(ws2), nb, _stream())
         else:
             cache = BipartiteGraphs(assume_dense=True)
             tab, keep = cache.table(list(stacked))
@@ -998,7 +1067,8 @@ def mds_proj_ohem_ce_heads(x, labels, dataset_ids, graph_sets, thresh, ignore=25
     """Vector [H] of MdsOhemCELoss values, one per graph set, sharing ONE pass over x per direction (see
     _MdsProjOhemCEHeads).  graph_sets: H lists of n_datasets dense [C_ds, C_uni] matrices (the same C_ds in every set).
     Falls back to H independent fused losses when the stacked route does not apply (graphs that are not all in the
-    tensor-core envelope, geometry outside the fused backward)."""
+    tensor-core envelope, geometry outside the fused backward).  channels_last 16-bit x inside _nhwc_tc16_ok is read
+    without a layout copy on both routes (the fallback's losses pick their layout one by one)."""
     sets = [list(gs) for gs in graph_sets]
     n = len(sets[0])
     B, Cu, h, w = x.shape
