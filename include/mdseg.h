@@ -483,6 +483,36 @@ typedef struct mdseg_label_view {
 int mdseg_label_pipeline(const mdseg_label_view* views /*device*/, int n_images, const uint8_t* luts, int n_luts,
                          void* out, int out_dtype, int out_h, int out_w, int pad_value, void* stream);
 
+/*
+ * Image branch of the same training transforms as ONE gather (SURVEY.md §8 f3).  Replaces, per sample and on a
+ * DataLoader worker in the reference, after cv2.imread(p)[:, :, ::-1]:  cv2.resize(im, (im_w, im_h)) (INTER_LINEAR,
+ * uint8) -> np.pad(..., 0) -> crop -> horizontal flip -> ColorJitter(brightness, contrast, saturation) ->
+ * ToTensor(mean, std), fp32.  The crop / pad / flip integers are those of mdseg_label_view for the same sample.
+ * Out-of-image pixels are colour (0, 0, 0) and then go through the jitter and the table, as in the reference.
+ * Brightness and contrast are one composed byte table (`lut`), saturation multiplies by the matrix with `sat_diag` on
+ * the diagonal and `sat_off` elsewhere (fp32 FMA chain in input-channel order, / 3, clip, truncate), and ToTensor is a
+ * float table per channel and byte.  The INTER_LINEAR arithmetic is OpenCV's fixed-point one, bit for bit.
+ */
+typedef struct mdseg_image_view {
+  const uint8_t* src;       /* decoded image, uint8 [src_h, src_w, 3] interleaved (pixel stride 3), device memory */
+  long long src_row_stride; /* bytes between source rows */
+  int src_h, src_w;
+  int im_h, im_w;           /* size after the resize */
+  int pad_top, pad_left;    /* rows / columns of padding in front of the resized image */
+  int crop_y, crop_x;       /* crop origin inside the padded image */
+  int flip;                 /* != 0: columns reversed after the crop */
+  int swap_rb;              /* != 0: the source is BGR (cv2.imread), output channel c reads source channel 2 - c */
+  int norm;                 /* row of `norm`; a value outside [0, n_norm) reads row 0 */
+  int saturate;             /* != 0: apply the saturation matrix after `lut` */
+  float sat_diag, sat_off;  /* float32(1 + 2r), float32(1 - r) */
+  uint8_t lut[256];         /* brightness then contrast, composed; identity when jitter is off */
+} mdseg_image_view;
+
+/* out: fp32, [n_images, 3, out_h, out_w] (MDSEG_NCHW) or [n_images, out_h, out_w, 3] (MDSEG_NHWC, the storage of a
+ * channels_last tensor), 16-byte aligned; out_w % 16 == 0.  norm: [n_norm][3][256] fp32, n_norm >= 1. */
+int mdseg_image_pipeline(const mdseg_image_view* views /*device*/, int n_images, const float* norm, int n_norm,
+                         float* out, int out_layout, int out_h, int out_w, void* stream);
+
 /* ---- f4: NLLPlus loss (soft-max in the unified space, projection of PROBABILITIES, up-sampling, -log) ----------
  * Replaces AdjNLLPlusLoss.forward (lib/loss/loss_helper.py:647-668) as driven by MdsOhemNLLPlusLoss
  * (lib/loss/ohem_ce_loss.py:92-146):

@@ -72,6 +72,14 @@ class LabelView(C.Structure):
                 ("crop_y", C.c_int), ("crop_x", C.c_int), ("flip", C.c_int), ("lut", C.c_int)]
 
 
+class ImageView(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("src_row_stride", C.c_longlong), ("src_h", C.c_int), ("src_w", C.c_int),
+                ("im_h", C.c_int), ("im_w", C.c_int), ("pad_top", C.c_int), ("pad_left", C.c_int),
+                ("crop_y", C.c_int), ("crop_x", C.c_int), ("flip", C.c_int), ("swap_rb", C.c_int),
+                ("norm", C.c_int), ("saturate", C.c_int), ("sat_diag", C.c_float), ("sat_off", C.c_float),
+                ("lut", C.c_uint8 * 256)]
+
+
 class GraphTable(C.Structure):
     _fields_ = [("g", SparseGraph * MAX_DATASETS), ("n_datasets", C.c_int), ("C_uni", C.c_int)]
 
@@ -127,6 +135,7 @@ SIGNATURES = {
     "mdseg_argmax_hist": (_I, [_P, _I, _L, _P, _P, _I, _P, _P, _I, _P, _P]),
     "mdseg_label_nearest": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P]),
     "mdseg_label_pipeline": (_I, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _P]),
+    "mdseg_image_pipeline": (_I, [_P, _I, _P, _I, _P, _I, _I, _I, _P]),
     "mdseg_graph_build_onehot_ints": (C.c_size_t, [_I, _I]),
     "mdseg_graph_build_onehot": (_I, [_P, _I, _I, _P, _P, _P]),
     "mdseg_head_tc16_tile": (_I, [_I]),

@@ -1528,6 +1528,90 @@ def label_pipeline(srcs, plans, out_size, luts=None, lut_ids=None, out_dtype=tor
     return out
 
 
+# ---- f3: image branch of the data pipeline (resize -> pad -> crop -> flip -> ColorJitter -> ToTensor) in one gather
+def to_tensor_tables(mean_std, device):
+    """ToTensor(mean, std) (lib/transform_cv2.py) as fp32 [n, 3, 256] tables on `device`, one per (mean, std) pair:
+    table[k, c, v] is what the reference's `torch.from_numpy(im.astype(np.float32)).div_(255).sub_(mean).div_(std)`
+    gives a byte v in channel c — built with exactly those torch ops, so the lookup is bit-exact by construction."""
+    rows = []
+    for mean, std in mean_std:
+        t = torch.arange(256, dtype=torch.float32).repeat(3, 1)[:, None, :].div_(255)   # [3, 1, 256] like [3, H, W]
+        m = torch.as_tensor(mean, dtype=t.dtype)[:, None, None]
+        s = torch.as_tensor(std, dtype=t.dtype)[:, None, None]
+        rows.append(t.sub_(m).div_(s)[:, 0, :])
+    return torch.stack(rows).to(device)
+
+
+_DEFAULT_TABLES = {}
+
+
+def image_pipeline(srcs, plans, out_size, jitter=None, norms=None, norm_ids=None, bgr=True,
+                   memory_format=torch.contiguous_format):
+    """out[b] = ToTensor(ColorJitter(flip(crop(pad(cv2.resize(srcs[b], INTER_LINEAR)))))) for a batch of decoded
+    uint8 images (lib/transform_cv2.py: RandomResizedCrop, RandomHorizontalFlip, ColorJitter, ToTensor) without
+    materialising any intermediate.
+
+    srcs: list of uint8 CUDA tensors [H_b, W_b, 3] (any row stride, pixel stride 3), BGR as cv2.imread returns them
+    when `bgr` (the reference's [:, :, ::-1] view is folded into the gather), RGB otherwise; plans: one dict per image
+    with ``im_h, im_w, pad_top, pad_left, crop_y, crop_x, flip`` (the same plans ``label_pipeline`` takes);
+    out_size = (crop_h, crop_w), crop_w % 16 == 0; jitter: None, or one entry per image — None or a dict with
+    ``lut`` (uint8[256], brightness then contrast) and ``sat`` (None or float32 (1 + 2r, 1 - r)) as
+    ``dropin.label_transform.ColorJitterPlan`` draws them; norms: fp32 [n, 3, 256] from ``to_tensor_tables`` (None:
+    ToTensor's default mean 0 / std 1), norm_ids[b] selects the row (None: row 0).
+    Returns fp32 [B, 3, crop_h, crop_w], NCHW-contiguous or channels_last (`memory_format`)."""
+    _require_cuda(*srcs)
+    if len(srcs) != len(plans) or not srcs:
+        raise ValueError("image_pipeline: one plan per source image")
+    if jitter is not None and len(jitter) != len(srcs):
+        raise ValueError("image_pipeline: one jitter entry per source image")
+    if memory_format not in (torch.contiguous_format, torch.channels_last):
+        raise ValueError("image_pipeline: memory_format must be torch.contiguous_format or torch.channels_last")
+    dev = srcs[0].device
+    if norms is None:
+        if dev not in _DEFAULT_TABLES:
+            _DEFAULT_TABLES[dev] = to_tensor_tables([((0., 0., 0.), (1., 1., 1.))], dev)
+        norms = _DEFAULT_TABLES[dev]
+    if not (isinstance(norms, torch.Tensor) and norms.dtype == torch.float32 and norms.device == dev
+            and norms.dim() == 3 and norms.shape[1:] == (3, 256) and norms.shape[0] > 0 and norms.is_contiguous()):
+        raise TypeError("image_pipeline: norms must be a contiguous fp32 [n, 3, 256] tensor on the sources' device")
+    table = image_views(srcs, plans, jitter, norm_ids, norms.shape[0], bgr)
+    Ho, Wo = int(out_size[0]), int(out_size[1])
+    out = torch.empty(len(srcs), 3, Ho, Wo, dtype=torch.float32, device=dev, memory_format=memory_format)
+    layout = N.NHWC if memory_format == torch.channels_last else N.NCHW
+    N.call("mdseg_image_pipeline", _ptr(table), len(srcs), _ptr(norms), norms.shape[0], _ptr(out), layout, Ho, Wo,
+           _stream())
+    return out
+
+
+def image_views(srcs, plans, jitter, norm_ids, n_norm, bgr):
+    """The device array of mdseg_image_view that ``image_pipeline`` passes to the kernel, LUTs inside, uploaded in
+    one host-to-device copy; validates the sources, plans, jitter entries and norm indices."""
+    views = (N.ImageView * len(srcs))()
+    for b, (t, pl) in enumerate(zip(srcs, plans)):
+        if t.dtype != torch.uint8 or t.dim() != 3 or t.shape[2] != 3 or t.stride(2) != 1 or t.stride(1) != 3:
+            raise TypeError("image_pipeline: sources must be uint8 [H, W, 3] with pixel stride 3")
+        v = views[b]
+        v.src, v.src_row_stride, v.src_h, v.src_w = t.data_ptr(), t.stride(0), t.shape[0], t.shape[1]
+        v.im_h, v.im_w = int(pl["im_h"]), int(pl["im_w"])
+        v.pad_top, v.pad_left = int(pl.get("pad_top", 0)), int(pl.get("pad_left", 0))
+        v.crop_y, v.crop_x, v.flip = int(pl.get("crop_y", 0)), int(pl.get("crop_x", 0)), int(bool(pl.get("flip", False)))
+        if v.im_h <= 0 or v.im_w <= 0 or v.src_h <= 0 or v.src_w <= 0:
+            raise ValueError("image_pipeline: empty source or resized image")
+        v.swap_rb = int(bool(bgr))
+        v.norm = int(norm_ids[b]) if norm_ids is not None else 0
+        if not 0 <= v.norm < n_norm:
+            raise ValueError(f"image_pipeline: norm_ids[{b}] = {v.norm} outside [0, {n_norm})")
+        jt = jitter[b] if jitter is not None else None
+        lut = np.arange(256, dtype=np.uint8) if jt is None or jt.get("lut") is None else np.ascontiguousarray(jt["lut"])
+        if lut.dtype != np.uint8 or lut.shape != (256,):
+            raise TypeError("image_pipeline: a jitter lut must be uint8[256]")
+        C.memmove(v.lut, lut.ctypes.data, 256)
+        sat = None if jt is None else jt.get("sat")
+        v.saturate = int(sat is not None)
+        v.sat_diag, v.sat_off = (float(sat[0]), float(sat[1])) if sat is not None else (0.0, 0.0)
+    return torch.from_numpy(np.frombuffer(bytes(views), dtype=np.uint8).copy()).to(srcs[0].device, non_blocking=True)
+
+
 def neg_log(p):
     """-log(p) in fp32, as torch computes OhemCELoss.thresh (ohem_ce_loss.py:17)."""
     return float(-torch.log(torch.tensor(p, dtype=torch.float)))
