@@ -39,7 +39,7 @@ enum {
   MDSEG_I64 = 12
 };
 
-/* logits layouts */
+/* layouts of logits and features */
 enum { MDSEG_NCHW = 0, MDSEG_NHWC = 1 };
 
 /* err_flag bits */
@@ -553,67 +553,42 @@ int mdseg_up_nll_bwd(const mdseg_src_table* src /*host*/, const int32_t* dataset
 size_t mdseg_graph_build_onehot_ints(int C_ds, int C_uni);
 int mdseg_graph_build_onehot(const float* G, int C_ds, int C_uni, int* buf, int32_t* err_flag, void* stream);
 
-/* ---- f2: the prototype head for 16-bit features on TMA + tcgen05 --------------------------------------------
- * out[b, n, p] = sum_k feats[b, k, p] * proto[n, k]: torch.einsum('bchw,nc->bnhw', feats, unify_prototype)
- * (lib/models/semseg.py:325-333,342-343; lib/loss/loss_cross_datasets.py:950,961,971) under amp.autocast.
- * feats: [n_images, K, hw] bf16 / fp16 (NCHW; hw % 8 == 0, 16-byte aligned).  proto_t: the prototypes converted to
- * the feature dtype, row-major [n_tiles * NT, ldb] (ldb >= K, ldb % 8 == 0, columns >= K zero) with
- * NT = mdseg_head_tc16_tile(N), rows >= N zero.  The same call gives d feats = dlogits x prototypes^T (K = the
- * number of prototypes, proto_t = the transposed prototypes).
- * out: [n_images, N, hw] fp32 or the feature dtype.  The features are read by TMA as MN-major UMMA operands — no
- * thread touches them. */
+/* ---- f2: the prototype head and the dense projection for 16-bit operands on TMA + tcgen05 ------------------------
+ * y[b, n, p] = sum_c G_d[n, c] x[b, c, p], d = dataset_ids[b], and its two adjoints.  With one operand and
+ * dataset_ids = NULL this is the prototype head torch.einsum('bchw,nc->bnhw', feats, unify_prototype)
+ * (lib/models/semseg.py:325-333,342-343; lib/loss/loss_cross_datasets.py:950,961,971) under amp.autocast, the
+ * prototypes in the role of G; with one operand per dataset it is the DENSE bipartite projection of 16-bit unified
+ * logits (GNN stage, loss_cross_datasets.py:997-1006); with folded prototypes (bi_graph @ unify_prototype in the role of
+ * G, the features in the role of x) it is both at once.
+ * x: bf16 / fp16, hw % 8 == 0, 16-byte aligned, in `layout`: MDSEG_NCHW [n_images, C_uni, hw] (read by TMA as an
+ * MN-major UMMA operand — no thread touches it) or MDSEG_NHWC [n_images, hw, C_uni] (channels_last; C_uni % 8 == 0, the
+ * 16-byte TMA pixel stride).  y and dy16 are planar in either layout.  Every output for MDSEG_NHWC is bit-identical to
+ * the one for MDSEG_NCHW on x made NCHW-contiguous (same products, same K order, same reduction order).
+ * graphs_t / graphs_tt: host arrays of n_datasets device pointers; operand d in the dtype of x, row-major
+ * [n_tiles * NT, ldb] with NT = mdseg_head_tc16_tile(rows) (ldb % 8 == 0, rows and columns past the matrix zero);
+ * a NULL entry skips the dataset. */
 int mdseg_head_tc16_tile(int N);
-/* The DENSE bipartite projection (GNN stage, loss_cross_datasets.py:997-1006) of 16-bit unified logits on the same
- * kernel: y[b, n, p] = sum_c G_d[n, c] x[b, c, p], d = dataset_ids[b].  graphs_t: host array of n_datasets device
- * pointers, graph d converted to the logits' dtype and padded like proto_t above ([n_tiles * NT(C_ds[d]), ldb]); a NULL
- * entry skips the dataset.  y: fp32 [n_images, y_cmax, hw]; rows of images whose dataset is skipped are untouched. */
-int mdseg_proj_fwd_tc16(const void* x, int dtype, int n_images, int C_uni, int64_t hw, const void* const* graphs_t, int ldb,
-                        const int* C_ds /*host*/, int n_datasets, const int32_t* dataset_ids, float* y, int y_cmax,
-                        void* stream);
-/* d prototype: dW[n, k] = sum_{b, p} dy16[b, n, p] * feats[b, k, p] — split-K over pixel slabs, both operands read by
- * TMA as K-major UMMA operands (the pixel is the contiguous index of both), fixed-order reduction of the per-slab
- * partials in `workspace` (deterministic).  dy16: the gradient w.r.t. the head's output in the feature dtype,
- * [n_images, N, hw]; dW: fp32 [N, K], fully overwritten. */
-size_t mdseg_head_dw_tc16_workspace_bytes(int n_images, int K, int64_t hw, int N);
-int mdseg_head_dw_tc16(const void* dy16, const void* feats, int dtype, int n_images, int K, int64_t hw, int N, float* dW,
-                       void* workspace, size_t workspace_bytes, void* stream);
-int mdseg_head_fwd_tc16(const void* feats, int dtype, int n_images, int K, int64_t hw, const void* proto_t, int ldb,
-                        int N, void* out, int out_dtype, void* stream);
-/* The two adjoints of mdseg_proj_fwd_tc16 (autograd replay of the einsum at loss_cross_datasets.py:997-1006 under
- * amp.autocast; with folded prototypes — bi_graph @ unify_prototype in the role of the graph and the features in the
- * role of x — also of the head einsum :971) on the same TMA-fed tcgen05 kernels.
+/* graphs_t[d] = G_d [C_ds[d], C_uni] (ldb >= C_uni).  y: fp32 [n_images, y_cmax, hw]; rows of images whose dataset is
+ * skipped are untouched. */
+int mdseg_proj_fwd_tc16(const void* x, int dtype, int layout, int n_images, int C_uni, int64_t hw,
+                        const void* const* graphs_t, int ldb, const int* C_ds /*host*/, int n_datasets,
+                        const int32_t* dataset_ids, float* y, int y_cmax, void* stream);
+/* The two adjoints (autograd replay of the einsums under amp.autocast).
  * dy16: [n_images, y_cmax, hw] in the dtype of x, planes >= C_ds[dataset] of an image ZERO.
- * mdseg_proj_bwd_tc16: dx[b, c, p] = sum_n G_d[n, c] dy16[b, n, p].  graphs_tt[d]: G_d transposed, in that dtype,
- * [n_tiles * NT(C_uni), ldb] (ldb >= y_cmax, ldb % 8 == 0, rows >= C_uni and columns >= C_ds zero).  dx: [n_images, C_uni,
- * hw] fp32 or that dtype, fully written (zeros for images whose dataset id is out of range).
+ * mdseg_proj_bwd_tc16: dx[b, c, p] = sum_n G_d[n, c] dy16[b, n, p].  graphs_tt[d] = G_d transposed, [C_uni, C_ds[d]]
+ * (ldb >= y_cmax).  dx: fp32 or the dtype of dy16, in `layout`, fully written (zeros for images whose dataset id is out
+ * of range).
  * mdseg_proj_bwd_graph_tc16: dG[d][n, c] = sum over the images b of dataset d and pixels p of dy16[b, n, p] x[b, c, p]:
- * split-K over pixel slabs, fixed-order reduction per dataset (deterministic).  dG: fp32 [n_datasets, y_cmax, C_uni],
- * fully overwritten (zeros for a dataset without images). */
-int mdseg_proj_bwd_tc16(const void* dy16, int dtype, int n_images, int y_cmax, int64_t hw, const void* const* graphs_tt,
-                        int ldb, int C_uni, int n_datasets, const int32_t* dataset_ids, void* dx, int dx_dtype, void* stream);
+ * split-K over pixel slabs, fixed-order reduction per dataset of the per-slab partials in `workspace` (deterministic).
+ * dG: fp32 [n_datasets, y_cmax, C_uni], fully overwritten (zeros for a dataset without images).  dataset_ids = NULL
+ * with n_datasets = 1 sums over every image (d prototype of the head). */
+int mdseg_proj_bwd_tc16(const void* dy16, int dtype, int layout, int n_images, int y_cmax, int64_t hw,
+                        const void* const* graphs_tt, int ldb, int C_uni, int n_datasets, const int32_t* dataset_ids,
+                        void* dx, int dx_dtype, void* stream);
 size_t mdseg_proj_bwd_graph_tc16_workspace_bytes(int n_images, int C_uni, int64_t hw, int y_cmax);
-int mdseg_proj_bwd_graph_tc16(const void* dy16, const void* x, int dtype, int n_images, int C_uni, int64_t hw, int y_cmax,
-                              const int32_t* dataset_ids, int n_datasets, float* dG, void* workspace, size_t workspace_bytes,
-                              void* stream);
-/* The same three GEMMs with channels_last (pixel-major) x / feats [n_images, hw, C_uni], bf16 / fp16, C_uni % 8 == 0
- * (16-byte TMA pixel stride), 16-byte-aligned bases; the planar operands (y, dy16) keep hw % 8 == 0.  Arguments,
- * padding and workspace sizes as for the planar entry points; every output is bit-identical to theirs on x made
- * NCHW-contiguous (same products, same K order, same reduction order).
- * mdseg_proj_fwd_tc16_nhwc: x pixel-major (a K-major UMMA operand), y planar fp32 [n_images, y_cmax, hw].  With one
- *   graph and dataset_ids = NULL it is the prototype head (mdseg_head_fwd_tc16 with fp32 output).
- * mdseg_proj_bwd_tc16_nhwc: dx written pixel-major [n_images, hw, C_uni] (fp32 or the dtype of dy16); zero rows for
- *   images whose dataset id is out of range.  With one operand and dataset_ids = NULL it is d feats of the head.
- * mdseg_proj_bwd_graph_tc16_nhwc: x pixel-major (an MN-major UMMA operand).  dataset_ids = NULL with n_datasets = 1
- *   sums over every image: d prototype of the head, dW [y_cmax, C_uni] (mdseg_head_dw_tc16). */
-int mdseg_proj_fwd_tc16_nhwc(const void* x, int dtype, int n_images, int C_uni, int64_t hw, const void* const* graphs_t,
-                             int ldb, const int* C_ds /*host*/, int n_datasets, const int32_t* dataset_ids, float* y,
-                             int y_cmax, void* stream);
-int mdseg_proj_bwd_tc16_nhwc(const void* dy16, int dtype, int n_images, int y_cmax, int64_t hw,
-                             const void* const* graphs_tt, int ldb, int C_uni, int n_datasets, const int32_t* dataset_ids,
-                             void* dx, int dx_dtype, void* stream);
-int mdseg_proj_bwd_graph_tc16_nhwc(const void* dy16, const void* x, int dtype, int n_images, int C_uni, int64_t hw,
-                                   int y_cmax, const int32_t* dataset_ids, int n_datasets, float* dG, void* workspace,
-                                   size_t workspace_bytes, void* stream);
+int mdseg_proj_bwd_graph_tc16(const void* dy16, const void* x, int dtype, int layout, int n_images, int C_uni, int64_t hw,
+                              int y_cmax, const int32_t* dataset_ids, int n_datasets, float* dG, void* workspace,
+                              size_t workspace_bytes, void* stream);
 
 /* ---- MscEvalCrop (evaluate.py:650-753): sliding-window evaluation ------------------------------------------
  * probs[c, y0 + y, x0 + x] += g(softmax_c(logits)[c, y, x] (+ softmax_c(logits_flip)[c, y, cw - 1 - x])) for one chip

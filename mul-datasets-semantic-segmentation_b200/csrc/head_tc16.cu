@@ -24,10 +24,9 @@
 //   * head_tc16_dw_kernel<true> reads feats [n_images, hw, K] as its B operand (N = channels, K = pixels): MN-MAJOR,
 //     staged as ceil(NT / 64) TMA boxes [64 pixels][64 channels], the layout the forward uses for its MN-major A.
 // The tensor cores see the same 16-bit products in the same K order as on the planar layout, so every output of the
-// pixel-major variants is bit-identical to the planar entry point on x.contiguous().
-#include <cuda.h>
-
-#include "common.cuh"
+// pixel-major variants is bit-identical to the planar one on x.contiguous().  The entry points take the layout of x
+// (MDSEG_NCHW / MDSEG_NHWC) as an argument and pick the variant from it.
+#include "tma_util.cuh"
 
 namespace mdseg {
 namespace {
@@ -415,19 +414,14 @@ __global__ void __launch_bounds__(256) head_tc16_dw_reduce_kernel(const DwArgs a
   dW[(long long)d * N * K + idx] = sum;
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      p = nullptr;
-    return (EncodeTiledFn)p;
-  }();
-  return fn;
+// the TMA encoder, with the primary context current on the calling thread; NULL (error set) if either is missing
+tma::EncodeTiledFn tensor_map_encoder() {
+  const tma::EncodeTiledFn enc = tma::encode_fn();
+  if (enc == nullptr) {
+    set_error("cuTensorMapEncodeTiled is not available in this driver");
+    return nullptr;
+  }
+  return tma::bind_primary_context() ? nullptr : enc;
 }
 
 }  // namespace
@@ -469,13 +463,8 @@ int launch_head16(const void* x, int dtype, int n_images, int K, int64_t hw, con
   MDSEG_REQUIRE(x && out && bt && Nd, "%s: null pointer", who);
   MDSEG_REQUIRE(((uintptr_t)x & 15) == 0, "%s: operands must be 16-byte aligned", who);
   MDSEG_REQUIRE(!out_pm || ((uintptr_t)out & 15) == 0, "%s: a pixel-major output must be 16-byte aligned", who);
-  EncodeTiledFn enc = encode_fn();
-  MDSEG_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available in this driver");
-  static thread_local bool ctx_bound = false;
-  if (!ctx_bound) {  // driver entry point: needs the primary context current on this host thread
-    MDSEG_CUDA_OK(cudaFree(nullptr));
-    ctx_bound = true;
-  }
+  const tma::EncodeTiledFn enc = tensor_map_encoder();
+  if (enc == nullptr) return 1;
   const CUtensorMapDataType dt = dtype == MDSEG_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
   CUtensorMap mapA;
   {
@@ -540,25 +529,31 @@ int launch_head16(const void* x, int dtype, int n_images, int K, int64_t hw, con
 }  // namespace
 }  // namespace mdseg
 
-extern "C" int mdseg_head_fwd_tc16(const void* feats, int dtype, int n_images, int K, int64_t hw, const void* proto_t,
-                                   int ldb, int N, void* out, int out_dtype, void* stream) {
-  MDSEG_REQUIRE(N > 0 && proto_t, "mdseg_head_fwd_tc16: bad prototypes");
-  const void* bt[1] = {proto_t};
-  const int Nd[1] = {N};
-  return mdseg::launch_head16(feats, dtype, n_images, K, hw, bt, ldb, Nd, 1, nullptr, out, N, out_dtype, (cudaStream_t)stream,
-                              "mdseg_head_fwd_tc16");
-}
+static bool layout_ok(int layout) { return layout == MDSEG_NCHW || layout == MDSEG_NHWC; }
 
-extern "C" int mdseg_proj_fwd_tc16(const void* x, int dtype, int n_images, int C_uni, int64_t hw, const void* const* graphs_t,
-                                   int ldb, const int* C_ds, int n_datasets, const int32_t* dataset_ids, float* y, int y_cmax,
-                                   void* stream) {
+extern "C" int mdseg_proj_fwd_tc16(const void* x, int dtype, int layout, int n_images, int C_uni, int64_t hw,
+                                   const void* const* graphs_t, int ldb, const int* C_ds, int n_datasets,
+                                   const int32_t* dataset_ids, float* y, int y_cmax, void* stream) {
+  MDSEG_REQUIRE(layout_ok(layout), "mdseg_proj_fwd_tc16: layout %d is neither NCHW nor NHWC", layout);
   for (int d = 0; d < n_datasets && d < MDSEG_MAX_DATASETS; ++d)
     MDSEG_REQUIRE(!C_ds || C_ds[d] <= y_cmax, "mdseg_proj_fwd_tc16: y_cmax %d < C_ds %d", y_cmax, C_ds[d]);
   return mdseg::launch_head16(x, dtype, n_images, C_uni, hw, graphs_t, ldb, C_ds, n_datasets, dataset_ids, y, y_cmax, MDSEG_F32,
-                              (cudaStream_t)stream, "mdseg_proj_fwd_tc16");
+                              (cudaStream_t)stream, "mdseg_proj_fwd_tc16", 0, /*a_pm=*/layout == MDSEG_NHWC);
 }
 
-// pixel slabs per image of the split-K d prototype GEMM: about two waves of CTAs, at least 4096 pixels per slab
+extern "C" int mdseg_proj_bwd_tc16(const void* dy16, int dtype, int layout, int n_images, int y_cmax, int64_t hw,
+                                   const void* const* graphs_tt, int ldb, int C_uni, int n_datasets,
+                                   const int32_t* dataset_ids, void* dx, int dx_dtype, void* stream) {
+  MDSEG_REQUIRE(layout_ok(layout), "mdseg_proj_bwd_tc16: layout %d is neither NCHW nor NHWC", layout);
+  MDSEG_REQUIRE(C_uni > 0 && n_datasets > 0 && n_datasets <= MDSEG_MAX_DATASETS, "mdseg_proj_bwd_tc16: bad shape");
+  int Nd[MDSEG_MAX_DATASETS];
+  for (int d = 0; d < n_datasets; ++d) Nd[d] = C_uni;
+  return mdseg::launch_head16(dy16, dtype, n_images, y_cmax, hw, graphs_tt, ldb, Nd, n_datasets, dataset_ids, dx, C_uni,
+                              dx_dtype, (cudaStream_t)stream, "mdseg_proj_bwd_tc16", /*zero_N=*/C_uni, /*a_pm=*/false,
+                              /*out_pm=*/layout == MDSEG_NHWC);
+}
+
+// pixel slabs per image of the split-K d W GEMM: about two waves of CTAs, at least 4096 pixels per slab
 static int dw_slabs_per_image(int n_images, int64_t hw, int tiles) {
   long long want = (2LL * 2 * mdseg::sm_count() + (long long)n_images * tiles - 1) / ((long long)n_images * tiles);
   const long long cap = (hw + 4095) / 4096;
@@ -566,7 +561,8 @@ static int dw_slabs_per_image(int n_images, int64_t hw, int tiles) {
   return (int)(want < 1 ? 1 : want);
 }
 
-extern "C" size_t mdseg_head_dw_tc16_workspace_bytes(int n_images, int K, int64_t hw, int N) {
+// d W = dy16 x^T below contracts over the pixels: K = C_uni (channels of x), N = y_cmax (planes of dy16)
+extern "C" size_t mdseg_proj_bwd_graph_tc16_workspace_bytes(int n_images, int K, int64_t hw, int N) {
   if (n_images <= 0 || K <= 0 || hw <= 0 || N <= 0) return 256;
   const int NT = mdseg_head_tc16_tile(K);
   const int n_tiles = (K + NT - 1) / NT, m_tiles = (N + 127) / 128;
@@ -574,26 +570,26 @@ extern "C" size_t mdseg_head_dw_tc16_workspace_bytes(int n_images, int K, int64_
   return (size_t)n_images * spi * m_tiles * n_tiles * 128 * NT * 4 + 256;
 }
 
-// feats_pm: feats is pixel-major [n_images, hw, K] (channels_last), read as an MN-major B operand
-static int head_dw_tc16_impl(const void* dy16, const void* feats, int dtype, int n_images, int K, int64_t hw, int N,
-                             const int32_t* dataset_ids, int n_datasets, float* dW, void* workspace, size_t workspace_bytes,
-                             void* stream, bool feats_pm = false) {
+// x planar [n_images, K, hw] is a K-major B operand like dy16; pixel-major [n_images, hw, K] (MDSEG_NHWC) an MN-major one
+extern "C" int mdseg_proj_bwd_graph_tc16(const void* dy16, const void* x, int dtype, int layout, int n_images, int K,
+                                         int64_t hw, int N, const int32_t* dataset_ids, int n_datasets, float* dW,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
   using namespace mdseg;
-  MDSEG_REQUIRE(dtype == MDSEG_BF16 || dtype == MDSEG_F16, "mdseg_head_dw_tc16: operands must be bf16 or fp16");
-  MDSEG_REQUIRE(n_images > 0 && n_images <= 65535 && K > 0 && N > 0 && hw > 0 && hw % 8 == 0, "mdseg_head_dw_tc16: bad shape");
-  MDSEG_REQUIRE(!feats_pm || K % 8 == 0,
-                "mdseg_proj_bwd_graph_tc16_nhwc: the channel count must be a multiple of 8 (16-byte TMA pixel stride)");
-  MDSEG_REQUIRE(dy16 && feats && dW && workspace, "mdseg_head_dw_tc16: null pointer");
-  MDSEG_REQUIRE((((uintptr_t)dy16 | (uintptr_t)feats) & 15) == 0, "mdseg_head_dw_tc16: operands must be 16-byte aligned");
-  MDSEG_REQUIRE(workspace_bytes >= mdseg_head_dw_tc16_workspace_bytes(n_images, K, hw, N),
-                "mdseg_head_dw_tc16: workspace too small");
-  EncodeTiledFn enc = encode_fn();
-  MDSEG_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available in this driver");
-  static thread_local bool ctx_bound = false;
-  if (!ctx_bound) {
-    MDSEG_CUDA_OK(cudaFree(nullptr));
-    ctx_bound = true;
-  }
+  const bool x_pm = layout == MDSEG_NHWC;
+  MDSEG_REQUIRE(layout_ok(layout), "mdseg_proj_bwd_graph_tc16: layout %d is neither NCHW nor NHWC", layout);
+  MDSEG_REQUIRE(n_datasets > 0 && n_datasets <= MDSEG_MAX_DATASETS && (dataset_ids || n_datasets == 1),
+                "mdseg_proj_bwd_graph_tc16: 1..%d datasets, dataset ids unless there is one", MDSEG_MAX_DATASETS);
+  MDSEG_REQUIRE(dtype == MDSEG_BF16 || dtype == MDSEG_F16, "mdseg_proj_bwd_graph_tc16: operands must be bf16 or fp16");
+  MDSEG_REQUIRE(n_images > 0 && n_images <= 65535 && K > 0 && N > 0 && hw > 0 && hw % 8 == 0,
+                "mdseg_proj_bwd_graph_tc16: bad shape");
+  MDSEG_REQUIRE(!x_pm || K % 8 == 0,
+                "mdseg_proj_bwd_graph_tc16: the channel count must be a multiple of 8 (16-byte TMA pixel stride)");
+  MDSEG_REQUIRE(dy16 && x && dW && workspace, "mdseg_proj_bwd_graph_tc16: null pointer");
+  MDSEG_REQUIRE((((uintptr_t)dy16 | (uintptr_t)x) & 15) == 0, "mdseg_proj_bwd_graph_tc16: operands must be 16-byte aligned");
+  MDSEG_REQUIRE(workspace_bytes >= mdseg_proj_bwd_graph_tc16_workspace_bytes(n_images, K, hw, N),
+                "mdseg_proj_bwd_graph_tc16: workspace too small");
+  const tma::EncodeTiledFn enc = tensor_map_encoder();
+  if (enc == nullptr) return 1;
   DwArgs a;
   a.NT = mdseg_head_tc16_tile(K);
   a.n_tiles = (K + a.NT - 1) / a.NT;
@@ -619,21 +615,21 @@ static int head_dw_tc16_impl(const void* dy16, const void* feats, int dtype, int
     cuuint64_t dims[3] = {(cuuint64_t)hw, (cuuint64_t)K, (cuuint64_t)n_images};
     cuuint64_t strides[2] = {(cuuint64_t)hw * 2, (cuuint64_t)K * hw * 2};
     cuuint32_t box[3] = {64, (cuuint32_t)a.NT, 1};
-    if (feats_pm) {  // [n_images, hw, K]: boxes of [64 pixels][64 channels]
+    if (x_pm) {  // [n_images, hw, K]: boxes of [64 pixels][64 channels]
       dims[0] = (cuuint64_t)K; dims[1] = (cuuint64_t)hw;
       strides[0] = (cuuint64_t)K * 2;
       box[0] = 64; box[1] = 64;
     }
-    CUresult r = enc(&mapB, dt, 3, const_cast<void*>(feats), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    CUresult r = enc(&mapB, dt, 3, const_cast<void*>(x), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     MDSEG_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed for the features (CUresult %d)", (int)r);
   }
   const int n_slabs_total = n_images * a.slabs_per_image;
-  const size_t b_bytes = feats_pm ? (size_t)((a.NT + 63) / 64) * 8192 : (size_t)a.NT * 128;
+  const size_t b_bytes = x_pm ? (size_t)((a.NT + 63) / 64) * 8192 : (size_t)a.NT * 128;
   const size_t smem = (size_t)kNStages * (128 * 128 + b_bytes) + 1024;
   cudaStream_t s = (cudaStream_t)stream;
   const dim3 grid((unsigned)(a.m_tiles * a.n_tiles), (unsigned)n_slabs_total);
-  if (feats_pm) {
+  if (x_pm) {
     MDSEG_CUDA_OK(cudaFuncSetAttribute(head_tc16_dw_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     head_tc16_dw_kernel<true><<<grid, kThreads, smem, s>>>(mapA, mapB, a);
   } else {
@@ -645,62 +641,4 @@ static int head_dw_tc16_impl(const void* dy16, const void* feats, int dtype, int
                                256, 0, s>>>(a, n_slabs_total, N, K, dataset_ids, dW);
   MDSEG_LAUNCH_OK();
   return 0;
-}
-
-extern "C" int mdseg_head_dw_tc16(const void* dy16, const void* feats, int dtype, int n_images, int K, int64_t hw, int N,
-                                  float* dW, void* workspace, size_t workspace_bytes, void* stream) {
-  return head_dw_tc16_impl(dy16, feats, dtype, n_images, K, hw, N, nullptr, 1, dW, workspace, workspace_bytes, stream);
-}
-
-extern "C" size_t mdseg_proj_bwd_graph_tc16_workspace_bytes(int n_images, int C_uni, int64_t hw, int y_cmax) {
-  return mdseg_head_dw_tc16_workspace_bytes(n_images, C_uni, hw, y_cmax);
-}
-
-extern "C" int mdseg_proj_bwd_graph_tc16(const void* dy16, const void* x, int dtype, int n_images, int C_uni, int64_t hw,
-                                         int y_cmax, const int32_t* dataset_ids, int n_datasets, float* dG, void* workspace,
-                                         size_t workspace_bytes, void* stream) {
-  MDSEG_REQUIRE(dataset_ids && n_datasets > 0 && n_datasets <= MDSEG_MAX_DATASETS,
-                "mdseg_proj_bwd_graph_tc16: dataset ids and 1..%d datasets", MDSEG_MAX_DATASETS);
-  return head_dw_tc16_impl(dy16, x, dtype, n_images, C_uni, hw, y_cmax, dataset_ids, n_datasets, dG, workspace,
-                           workspace_bytes, stream);
-}
-
-extern "C" int mdseg_proj_bwd_tc16(const void* dy16, int dtype, int n_images, int y_cmax, int64_t hw,
-                                   const void* const* graphs_tt, int ldb, int C_uni, int n_datasets,
-                                   const int32_t* dataset_ids, void* dx, int dx_dtype, void* stream) {
-  MDSEG_REQUIRE(C_uni > 0 && n_datasets > 0 && n_datasets <= MDSEG_MAX_DATASETS, "mdseg_proj_bwd_tc16: bad shape");
-  int Nd[MDSEG_MAX_DATASETS];
-  for (int d = 0; d < n_datasets; ++d) Nd[d] = C_uni;
-  return mdseg::launch_head16(dy16, dtype, n_images, y_cmax, hw, graphs_tt, ldb, Nd, n_datasets, dataset_ids, dx, C_uni,
-                              dx_dtype, (cudaStream_t)stream, "mdseg_proj_bwd_tc16", /*zero_N=*/C_uni);
-}
-
-// ---- channels_last (pixel-major) x / feats: the same kernels with K-major A, MN-major B or a pixel-major output ------
-extern "C" int mdseg_proj_fwd_tc16_nhwc(const void* x, int dtype, int n_images, int C_uni, int64_t hw,
-                                        const void* const* graphs_t, int ldb, const int* C_ds, int n_datasets,
-                                        const int32_t* dataset_ids, float* y, int y_cmax, void* stream) {
-  for (int d = 0; d < n_datasets && d < MDSEG_MAX_DATASETS; ++d)
-    MDSEG_REQUIRE(!C_ds || C_ds[d] <= y_cmax, "mdseg_proj_fwd_tc16_nhwc: y_cmax %d < C_ds %d", y_cmax, C_ds[d]);
-  return mdseg::launch_head16(x, dtype, n_images, C_uni, hw, graphs_t, ldb, C_ds, n_datasets, dataset_ids, y, y_cmax, MDSEG_F32,
-                              (cudaStream_t)stream, "mdseg_proj_fwd_tc16_nhwc", 0, /*a_pm=*/true, /*out_pm=*/false);
-}
-
-extern "C" int mdseg_proj_bwd_tc16_nhwc(const void* dy16, int dtype, int n_images, int y_cmax, int64_t hw,
-                                        const void* const* graphs_tt, int ldb, int C_uni, int n_datasets,
-                                        const int32_t* dataset_ids, void* dx, int dx_dtype, void* stream) {
-  MDSEG_REQUIRE(C_uni > 0 && n_datasets > 0 && n_datasets <= MDSEG_MAX_DATASETS, "mdseg_proj_bwd_tc16_nhwc: bad shape");
-  int Nd[MDSEG_MAX_DATASETS];
-  for (int d = 0; d < n_datasets; ++d) Nd[d] = C_uni;
-  return mdseg::launch_head16(dy16, dtype, n_images, y_cmax, hw, graphs_tt, ldb, Nd, n_datasets, dataset_ids, dx, C_uni,
-                              dx_dtype, (cudaStream_t)stream, "mdseg_proj_bwd_tc16_nhwc", /*zero_N=*/C_uni,
-                              /*a_pm=*/false, /*out_pm=*/true);
-}
-
-extern "C" int mdseg_proj_bwd_graph_tc16_nhwc(const void* dy16, const void* x, int dtype, int n_images, int C_uni,
-                                              int64_t hw, int y_cmax, const int32_t* dataset_ids, int n_datasets, float* dG,
-                                              void* workspace, size_t workspace_bytes, void* stream) {
-  MDSEG_REQUIRE(n_datasets > 0 && n_datasets <= MDSEG_MAX_DATASETS && (dataset_ids || n_datasets == 1),
-                "mdseg_proj_bwd_graph_tc16_nhwc: 1..%d datasets, dataset ids unless there is one", MDSEG_MAX_DATASETS);
-  return head_dw_tc16_impl(dy16, x, dtype, n_images, C_uni, hw, y_cmax, dataset_ids, n_datasets, dG, workspace,
-                           workspace_bytes, stream, /*feats_pm=*/true);
 }

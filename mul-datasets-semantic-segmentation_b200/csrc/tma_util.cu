@@ -3,11 +3,6 @@
 
 namespace mdseg {
 namespace tma {
-namespace {
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 EncodeTiledFn encode_fn() {
   static EncodeTiledFn fn = [] {
@@ -20,6 +15,17 @@ EncodeTiledFn encode_fn() {
   }();
   return fn;
 }
+
+int bind_primary_context() {
+  static thread_local bool bound = false;
+  if (!bound) {
+    MDSEG_CUDA_OK(cudaFree(nullptr));
+    bound = true;
+  }
+  return 0;
+}
+
+namespace {
 
 // largest number of destinations that fall into one cell (cells fold the last source index, see axis_cell)
 int max_cell_population(float scale, int n_in, int n_out) {
@@ -93,13 +99,7 @@ int make_maps(const mdseg_src_table& src, const Geom& gm, int n_images, int box_
     set_error("cuTensorMapEncodeTiled is not available in this driver");
     return 1;
   }
-  // cuTensorMapEncodeTiled is a driver entry point: it needs the primary context current on THIS
-  // host thread (autograd runs the backward on its own thread, where only runtime calls were made).
-  static thread_local bool ctx_bound = false;
-  if (!ctx_bound) {
-    MDSEG_CUDA_OK(cudaFree(nullptr));
-    ctx_bound = true;
-  }
+  if (int rc = bind_primary_context()) return rc;
   for (int i = 0; i < src.n_datasets; ++i) {
     const int calloc = src.C_alloc[i] > 0 ? src.C_alloc[i] : src.C[i];
     cuuint64_t dims[4] = {(cuuint64_t)gm.w, (cuuint64_t)gm.h, (cuuint64_t)calloc, (cuuint64_t)n_images};

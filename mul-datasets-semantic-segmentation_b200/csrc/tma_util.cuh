@@ -117,6 +117,14 @@ __device__ __forceinline__ void cell_span(const AxisMap& m, int c, int n_out, in
 }
 #endif  // __CUDACC__
 
+// host: the driver's cuTensorMapEncodeTiled, looked up once; NULL when the driver does not have it
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn encode_fn();
+// host: make the primary context current on the calling thread before a driver entry point is called (autograd runs
+// the backward on its own thread, where only runtime calls were made).  0 = OK, else set_error was called.
+int bind_primary_context();
 // host: tensor maps over the fp32 sources [n_images][C_alloc][h][w] with box (box_w, box_h, box_c, 1)
 int make_maps(const mdseg_src_table& src, const Geom& gm, int n_images, int box_w, int box_h, int box_c, Maps* out);
 // cmax[b, y, x] = max_c src[b, c, y, x] for fp32 sources with hw % 4 == 0 (src.cmax is the output plane)

@@ -576,22 +576,6 @@ up_ce_bwd_tma_kernel(const __grid_constant__ TmaMaps maps, const BwdArgs a) {
 // =================================================================================================
 // host side
 // =================================================================================================
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      p = nullptr;
-    return (EncodeTiledFn)p;
-  }();
-  return fn;
-}
-
 bool tma_applicable(const mdseg_src_table& src, const Geom& gm) {
   if (src.dtype != MDSEG_F32 || src.cmax == nullptr) return false;
   if (gm.w % 4 != 0 || gm.h < 1) return false;
@@ -600,18 +584,12 @@ bool tma_applicable(const mdseg_src_table& src, const Geom& gm) {
     if (src.C[i] > 254) return false;  // labels are staged as bytes
     if (((uintptr_t)src.base[i] & 15) != 0 || (src.image_stride[i] % 4) != 0) return false;
   }
-  return encode_fn() != nullptr;
+  return tma::encode_fn() != nullptr;
 }
 
 int make_maps(const mdseg_src_table& src, const Geom& gm, int n_images, TmaMaps* out) {
-  EncodeTiledFn enc = encode_fn();
-  // cuTensorMapEncodeTiled is a driver entry point: it needs the primary context current on THIS
-  // host thread (autograd runs the backward on its own thread, where only runtime calls were made).
-  static thread_local bool ctx_bound = false;
-  if (!ctx_bound) {
-    MDSEG_CUDA_OK(cudaFree(nullptr));
-    ctx_bound = true;
-  }
+  tma::EncodeTiledFn enc = tma::encode_fn();
+  if (int rc = tma::bind_primary_context()) return rc;
   for (int i = 0; i < src.n_datasets; ++i) {
     const int calloc = src.C_alloc[i] > 0 ? src.C_alloc[i] : src.C[i];
     cuuint64_t dims[4] = {(cuuint64_t)gm.w, (cuuint64_t)gm.h, (cuuint64_t)calloc, (cuuint64_t)n_images};

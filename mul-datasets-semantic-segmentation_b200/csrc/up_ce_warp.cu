@@ -500,10 +500,6 @@ __global__ void __launch_bounds__(32, MDSEG_FWD_OCC) up_ce_fwd_warp_kernel(const
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 }  // namespace
 
 // Return 0 = launched, -1 = not applicable (caller falls back), > 0 = error.
@@ -518,18 +514,15 @@ int up_ce_fwd_warp(const FwdArgs& fa, int label_dtype, int n_images, cudaStream_
     if (int rc = tma::channel_max(fa.src, fa.dataset_ids, n_images, (int64_t)fa.gm.h * fa.gm.w, s)) return rc;
   CUtensorMap cmap;
   {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess || !p)
-      return -1;
+    const tma::EncodeTiledFn enc = tma::encode_fn();
+    if (!enc) return -1;
     cuuint64_t dims[3] = {(cuuint64_t)fa.gm.w, (cuuint64_t)fa.gm.h, (cuuint64_t)n_images};
     cuuint64_t strides[2] = {(cuuint64_t)fa.gm.w * 4, (cuuint64_t)fa.gm.h * fa.gm.w * 4};
     cuuint32_t box[3] = {(cuuint32_t)kBoxW, 2, 1};
     cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = ((EncodeTiledFn)p)(&cmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, fa.src.cmax, dims, strides, box, estr,
-                                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                    CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = enc(&cmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, fa.src.cmax, dims, strides, box, estr,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
       set_error("cuTensorMapEncodeTiled failed for the channel-maximum plane (CUresult %d)", (int)r);
       return 1;

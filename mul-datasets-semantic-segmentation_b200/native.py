@@ -139,17 +139,11 @@ SIGNATURES = {
     "mdseg_graph_build_onehot_ints": (C.c_size_t, [_I, _I]),
     "mdseg_graph_build_onehot": (_I, [_P, _I, _I, _P, _P, _P]),
     "mdseg_head_tc16_tile": (_I, [_I]),
-    "mdseg_proj_fwd_tc16": (_I, [_P, _I, _I, _I, _L, C.POINTER(C.c_void_p), _I, C.POINTER(C.c_int), _I, _P, _P, _I, _P]),
-    "mdseg_head_dw_tc16_workspace_bytes": (C.c_size_t, [_I, _I, _L, _I]),
-    "mdseg_head_dw_tc16": (_I, [_P, _P, _I, _I, _I, _L, _I, _P, _P, C.c_size_t, _P]),
-    "mdseg_head_fwd_tc16": (_I, [_P, _I, _I, _I, _L, _P, _I, _I, _P, _I, _P]),
-    "mdseg_proj_bwd_tc16": (_I, [_P, _I, _I, _I, _L, C.POINTER(C.c_void_p), _I, _I, _I, _P, _P, _I, _P]),
+    "mdseg_proj_fwd_tc16": (_I, [_P, _I, _I, _I, _I, _L, C.POINTER(C.c_void_p), _I, C.POINTER(C.c_int), _I, _P, _P, _I,
+                                 _P]),
+    "mdseg_proj_bwd_tc16": (_I, [_P, _I, _I, _I, _I, _L, C.POINTER(C.c_void_p), _I, _I, _I, _P, _P, _I, _P]),
     "mdseg_proj_bwd_graph_tc16_workspace_bytes": (C.c_size_t, [_I, _I, _L, _I]),
-    "mdseg_proj_bwd_graph_tc16": (_I, [_P, _P, _I, _I, _I, _L, _I, _P, _I, _P, _P, C.c_size_t, _P]),
-    "mdseg_proj_fwd_tc16_nhwc": (_I, [_P, _I, _I, _I, _L, C.POINTER(C.c_void_p), _I, C.POINTER(C.c_int), _I, _P, _P, _I,
-                                      _P]),
-    "mdseg_proj_bwd_tc16_nhwc": (_I, [_P, _I, _I, _I, _L, C.POINTER(C.c_void_p), _I, _I, _I, _P, _P, _I, _P]),
-    "mdseg_proj_bwd_graph_tc16_nhwc": (_I, [_P, _P, _I, _I, _I, _L, _I, _P, _I, _P, _P, C.c_size_t, _P]),
+    "mdseg_proj_bwd_graph_tc16": (_I, [_P, _P, _I, _I, _I, _I, _L, _I, _P, _I, _P, _P, C.c_size_t, _P]),
     "mdseg_eval_chip_accum": (_I, [_P, _P, _I, _I, _I, _I, _P, _I, _I, _I, _I, _I, _P]),
     "mdseg_prob_resize_accum": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _P, _I, _I, _I, _P]),
     "mdseg_softmax_nchw": (_I, [_P, _I, _I, _I, _L, _P, _P]),

@@ -537,16 +537,47 @@ def _nhwc_proj_ok(x, tab):
             and all(not tab.g[i].dense and tab.g[i].C_ds <= N.NHWC_MAX_CDS for i in range(tab.n_datasets)))
 
 
-def _nhwc_tc16_ok(x, tab=None):
-    """channels_last 16-bit features / logits that the TMA-fed tcgen05 kernels read as they are (the *_tc16_nhwc entry
-    points): the channel count a multiple of 8 (16-byte TMA pixel stride), a 16-byte-aligned base, h * w a multiple of
-    8 (the planar y / dy) and, with a graph table, all graphs dense with 8 <= C_ds <= 1024 and C_uni >= 32 (the tc16
-    envelope of the projection).  Anything else (fp32, odd channel counts, storage offsets) takes x.contiguous()."""
-    if not (_channels_last(x) and x.dtype in (torch.bfloat16, torch.float16) and x.shape[1] % 8 == 0
-            and x.data_ptr() % 16 == 0 and (x.shape[2] * x.shape[3]) % 8 == 0):
-        return False
-    return tab is None or (tab.C_uni >= 32 and all(tab.g[i].dense and 8 <= tab.g[i].C_ds <= 1024
-                                                   for i in range(tab.n_datasets)))
+def _tc16_layout(x):
+    """The layout (N.NCHW / N.NHWC) in which the TMA-fed tcgen05 kernels (mdseg_proj_*_tc16) read 16-bit x as it lies,
+    or None: bf16 / fp16, h * w a multiple of 8 (the planar y / dy), a 16-byte-aligned base, and NCHW-contiguous or
+    channels_last with a channel count that is a multiple of 8 (16-byte TMA pixel stride)."""
+    if x.dtype not in (torch.bfloat16, torch.float16) or (x.shape[2] * x.shape[3]) % 8 or x.data_ptr() % 16:
+        return None
+    if _channels_last(x):
+        return N.NHWC if x.shape[1] % 8 == 0 else None
+    return N.NCHW if x.is_contiguous() else None
+
+
+def _tc16_envelope(c_uni, c_ds, n_heads=1):
+    """Graph sizes the projection runs on the tc16 kernels for: C_uni >= 32 and, per dataset, C_ds >= 8 and
+    n_heads * C_ds <= 1024 (the dataset's graphs of n_heads sets stacked into one operand)."""
+    return c_uni >= 32 and all(8 <= c and n_heads * c <= 1024 for c in c_ds)
+
+
+def _dense_tc16(tab):
+    """Every graph of the table dense and inside _tc16_envelope."""
+    n = tab.n_datasets
+    return all(tab.g[i].dense for i in range(n)) and _tc16_envelope(tab.C_uni, [tab.g[i].C_ds for i in range(n)])
+
+
+def _tc16_operands(mats, dtype, transpose=False):
+    """The B operands of the mdseg_proj_*_tc16 kernels for matrices M_d (or M_d^T with `transpose`) in one zero-filled
+    buffer: each in `dtype`, its rows padded to whole N tiles (mdseg_head_tc16_tile), its columns to ldb (the widest
+    matrix rounded up to a multiple of 8).  -> (buffer, host array of the operands' pointers, ldb)"""
+    mats = [m.detach().t() if transpose else m.detach() for m in mats]
+    ldb = (max(m.shape[1] for m in mats) + 7) // 8 * 8
+    rows = []
+    for m in mats:
+        nt = N.lib.mdseg_head_tc16_tile(m.shape[0])
+        rows.append((m.shape[0] + nt - 1) // nt * nt)
+    buf = torch.zeros(sum(rows), ldb, dtype=dtype, device=mats[0].device)
+    ptrs = (C.c_void_p * len(mats))()
+    o = 0
+    for i, m in enumerate(mats):
+        buf[o:o + m.shape[0], :m.shape[1]] = m.to(dtype)
+        ptrs[i] = buf.data_ptr() + o * ldb * buf.element_size()
+        o += rows[i]
+    return buf, ptrs, ldb
 
 
 # ---- a5 projection alone (model-side eval einsum, semseg.py:342-345) --------------------------------
@@ -554,7 +585,8 @@ def project(logits_uni, graphs, dataset_ids=None, cache=None):
     """fp32 [B, max C_ds, h, w]: einsum('bchw,nc->bnhw') with the graph of each image's dataset.  channels_last logits
     with sparse graphs are read as they are (no layout copy)."""
     _require_cuda(logits_uni)
-    tab, keep = (cache or _default_graphs).table(list(graphs))
+    graphs = list(graphs)
+    tab, keep = (cache or _default_graphs).table(graphs)
     x = logits_uni if _nhwc_proj_ok(logits_uni, tab) else logits_uni.contiguous()
     B, Cu, h, w = x.shape
     if tab.C_uni != Cu:
@@ -562,39 +594,26 @@ def project(logits_uni, graphs, dataset_ids=None, cache=None):
     cmax = max(g.shape[0] for g in graphs)
     ids = _ids32(dataset_ids, B, x.device)
     y = torch.empty(B, cmax, h, w, dtype=torch.float32, device=x.device)
-    _proj_fwd(x, tab, ids, B, h, w, y, cmax, None, err_flag(x.device), graphs=list(graphs))
+    _proj_fwd(x, tab, graphs, ids, y, None, err_flag(x.device), _tc16_layout(x) is not None and _dense_tc16(tab))
     return y
 
 
-def _proj_fwd(x, tab, ids, B, h, w, y, cmax, ymax, ef, graphs=None):
-    """mdseg_proj_fwd, or mdseg_proj_fwd_tc (dense graphs on the tensor cores) when a graph is dense; 16-bit logits
-    with all-dense graphs take the TMA-fed kernel (mdseg_proj_fwd_tc16); channels_last x (callers pass it only when
-    _nhwc_proj_ok or _nhwc_tc16_ok) takes mdseg_proj_fwd_nhwc (sparse graphs) or mdseg_proj_fwd_tc16_nhwc (dense)."""
-    n = tab.n_datasets
-    nhwc = _channels_last(x)
-    if nhwc and not all(tab.g[i].dense for i in range(n)):
+def _proj_fwd(x, tab, graphs, ids, y, ymax, ef, tc16):
+    """y[b] = G_d x[b], d = ids[b], into fp32 planes y [B, cmax, h, w] (and, unless tc16, their channel maximum into
+    ymax when given).  tc16 (the caller's route: 16-bit x with _tc16_layout, graphs that the backward will take the same
+    way): mdseg_proj_fwd_tc16 in x's layout.  Otherwise mdseg_proj_fwd_nhwc (channels_last x, which callers pass only
+    with sparse graphs inside _nhwc_proj_ok), mdseg_proj_fwd_tc (a dense graph, on the tensor cores) or mdseg_proj_fwd."""
+    B, _, h, w = x.shape
+    cmax = y.shape[1]
+    if tc16:
+        n = len(graphs)
+        buf, ptrs, ldb = _tc16_operands(graphs, x.dtype)
+        N.call("mdseg_proj_fwd_tc16", _ptr(x), _DT[x.dtype], _tc16_layout(x), B, x.shape[1], h * w, ptrs, ldb,
+               (C.c_int * n)(*[g.shape[0] for g in graphs]), n, _ptr(ids), _ptr(y), cmax, _stream())
+    elif _channels_last(x):
         N.call("mdseg_proj_fwd_nhwc", _ptr(x), _DT[x.dtype], C.byref(tab), _ptr(ids), B, h, w, _ptr(y), cmax, _ptr(ymax),
                _ptr(ef), _stream())
-        return
-    if nhwc or (graphs is not None and x.dtype in (torch.bfloat16, torch.float16) and (h * w) % 8 == 0
-                and x.data_ptr() % 16 == 0 and all(tab.g[i].dense and 8 <= tab.g[i].C_ds <= 1024 for i in range(n))
-                and tab.C_uni >= 32):
-        ldb = (tab.C_uni + 7) // 8 * 8
-        ptrs, cds = (C.c_void_p * n)(), (C.c_int * n)()
-        rows = []
-        for g in graphs:
-            nt = N.lib.mdseg_head_tc16_tile(g.shape[0])
-            rows.append(((g.shape[0] + nt - 1) // nt) * nt)
-        gt = torch.zeros(sum(rows), ldb, dtype=x.dtype, device=x.device)  # one zero fill for all datasets
-        o = 0
-        for i, g in enumerate(graphs):
-            gt[o:o + g.shape[0], :tab.C_uni] = g.detach().to(x.dtype)
-            ptrs[i], cds[i] = gt.data_ptr() + o * ldb * gt.element_size(), g.shape[0]
-            o += rows[i]
-        N.call("mdseg_proj_fwd_tc16_nhwc" if nhwc else "mdseg_proj_fwd_tc16", _ptr(x), _DT[x.dtype], B, tab.C_uni, h * w,
-               ptrs, ldb, cds, n, _ptr(ids), _ptr(y), cmax, _stream())
-        return
-    if any(tab.g[i].dense for i in range(tab.n_datasets)):
+    elif any(tab.g[i].dense for i in range(tab.n_datasets)):
         nbytes = N.lib.mdseg_proj_fwd_tc_workspace_bytes(C.byref(tab), _DT[x.dtype])
         ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
         N.call("mdseg_proj_fwd_tc", _ptr(x), _DT[x.dtype], C.byref(tab), _ptr(ids), B, h, w, _ptr(y), cmax, _ptr(ymax),
@@ -602,6 +621,57 @@ def _proj_fwd(x, tab, ids, B, h, w, y, cmax, ymax, ef, graphs=None):
     else:
         N.call("mdseg_proj_fwd", _ptr(x), _DT[x.dtype], C.byref(tab), _ptr(ids), B, h, w, _ptr(y), cmax, _ptr(ymax),
                _ptr(ef), _stream())
+
+
+def _proj_bwd(dy, dyB, graphs, tab, ids, dx):
+    """The adjoint of _proj_fwd: dx[b] = G_d^T (dy[b] + dyB[b]), d = ids[b], into dx (its layout and dtype).  16-bit dy
+    (the dtype of x, from a backward that took the tc16 route; dyB None): mdseg_proj_bwd_tc16.  fp32 planes:
+    mdseg_proj_bwd_nhwc (channels_last dx, sparse graphs), mdseg_proj_bwd_tc (a dense graph) or mdseg_proj_bwd."""
+    B, Cu, h, w = dx.shape
+    cmax = dy.shape[1]
+    if dy.dtype != torch.float32:
+        buf, ptrs, ldb = _tc16_operands(graphs, dy.dtype, transpose=True)
+        N.call("mdseg_proj_bwd_tc16", _ptr(dy), _DT[dy.dtype], N.NHWC if _channels_last(dx) else N.NCHW, B, cmax, h * w,
+               ptrs, ldb, Cu, len(graphs), _ptr(ids), _ptr(dx), _DT[dx.dtype], _stream())
+    elif _channels_last(dx):
+        N.call("mdseg_proj_bwd_nhwc", _ptr(dy), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dx),
+               _DT[dx.dtype], _stream())
+    elif any(tab.g[i].dense for i in range(tab.n_datasets)):
+        nb = N.lib.mdseg_proj_bwd_tc_workspace_bytes(C.byref(tab), _DT[dx.dtype])
+        ws = torch.empty(nb, dtype=torch.uint8, device=dx.device)
+        N.call("mdseg_proj_bwd_tc", _ptr(dy), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dx), _DT[dx.dtype],
+               _ptr(ws), nb, _stream())
+    else:
+        N.call("mdseg_proj_bwd", _ptr(dy), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dx), _DT[dx.dtype],
+               _stream())
+
+
+def _proj_bwd_graph(x, dy, dyB, graphs, tab, ids):
+    """The graph gradients of _proj_fwd: dG[d] = sum over the images of dataset d of (dy + dyB) x^T, fp32
+    [n_datasets, cmax, C_uni].  16-bit dy (see _proj_bwd): mdseg_proj_bwd_graph_tc16 with x in its layout.  fp32
+    planes: mdseg_proj_bwd_graph_tc (a dense graph) or mdseg_proj_bwd_graph."""
+    B, Cu, h, w = x.shape
+    n, cmax = len(graphs), dy.shape[1]
+    if dy.dtype != torch.float32:
+        if ids is None and n > 1:  # every image belongs to dataset 0; the other datasets get zeros
+            ids = torch.zeros(B, dtype=torch.int32, device=x.device)
+        dG = torch.empty(n, cmax, Cu, dtype=torch.float32, device=x.device)
+        nb = N.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, Cu, h * w, cmax)
+        ws = torch.empty(nb, dtype=torch.uint8, device=x.device)
+        N.call("mdseg_proj_bwd_graph_tc16", _ptr(dy), _ptr(x), _DT[x.dtype], _tc16_layout(x), B, Cu, h * w, cmax,
+               _ptr(ids), n, _ptr(dG), _ptr(ws), nb, _stream())
+        return dG
+    stride = cmax * Cu
+    dG = torch.zeros(n, stride, dtype=torch.float32, device=x.device)
+    if any(tab.g[i].dense for i in range(tab.n_datasets)):  # dense graphs: split-K GEMM on the tensor cores
+        nb = N.lib.mdseg_proj_bwd_graph_tc_workspace_bytes(C.byref(tab), B, h, w)
+        ws = torch.empty(nb, dtype=torch.uint8, device=x.device)
+        N.call("mdseg_proj_bwd_graph_tc", _ptr(x), _DT[x.dtype], _ptr(dy), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B,
+               h, w, _ptr(dG), stride, _ptr(ws), nb, _stream())
+    else:
+        N.call("mdseg_proj_bwd_graph", _ptr(x), _DT[x.dtype], _ptr(dy), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B, h,
+               w, _ptr(dG), stride, _stream())
+    return dG.view(n, cmax, Cu)
 
 
 # ---- f2: the prototype head (producer of the unified logits) on the tcgen05 tensor cores ---------------------------
@@ -615,44 +685,14 @@ def _dense_table(weight):
     return tab
 
 
-def _tc16_ok(x):
-    return x.dtype in (torch.bfloat16, torch.float16) and (x.shape[2] * x.shape[3]) % 8 == 0 and x.data_ptr() % 16 == 0
-
-
-def _head_operand(wgt, dtype):
-    """wgt fp32 [n_rows, K] (any strides) as the B operand of the tc16 kernels: dtype, rows padded to whole N tiles,
-    K padded to ldb (a multiple of 8), zeros in the padding.  -> (wt, ldb)"""
-    n_rows, K = wgt.shape
-    nt = N.lib.mdseg_head_tc16_tile(n_rows)
-    ldb = (K + 7) // 8 * 8
-    wt = torch.zeros(((n_rows + nt - 1) // nt) * nt, ldb, dtype=dtype, device=wgt.device)
-    wt[:n_rows, :K] = wgt.to(dtype)
-    return wt, ldb
-
-
-def _head_tc16(a, wgt, out):
-    """out[b, n, p] = sum_k a[b, k, p] * wgt[n, k] with 16-bit `a` [B, K, h, w]; wgt: fp32 [n_rows, K] (any strides);
-    out: fp32 or a's dtype.  mdseg_head_fwd_tc16 (TMA + tcgen05)."""
-    B, K, h, w = a.shape
-    n_rows = wgt.shape[0]
-    wt, ldb = _head_operand(wgt, a.dtype)
-    N.call("mdseg_head_fwd_tc16", _ptr(a), _DT[a.dtype], B, K, h * w, _ptr(wt), ldb, n_rows, _ptr(out), _DT[out.dtype],
-           _stream())
-
-
-def _one(t):
-    return (C.c_void_p * 1)(t.data_ptr())
-
-
 class _PrototypeHead(torch.autograd.Function):
     """logits[b, n, y, x] = sum_c feats[b, c, y, x] * proto[n, c]: torch.einsum('bchw,nc->bnhw', feats, unify_prototype)
-    of lib/models/semseg.py:325-333,342-343 and lib/loss/loss_cross_datasets.py:950,961,971 as a
-    [128 px, N] x [N, K] tcgen05 GEMM per CTA (mdseg_proj_fwd_tc with the prototypes in the role of the dense graph,
-    N tiled by 256).  Backward: d feats = proto^T dlogits (mdseg_proj_bwd_tc), d proto = dlogits feats^T as a split-K
-    GEMM over the pixels (mdseg_proj_bwd_graph_tc).  fp32 inputs: three bf16 terms per operand (1e-5 bar);
-    bf16 / fp16 inputs: one product in their own type, like autocast.  Output fp32 NCHW.  channels_last 16-bit features
-    (_nhwc_tc16_ok) are read as they are by the *_tc16_nhwc kernels and get a channels_last gradient, bit-identical to
-    the NCHW route; other channels_last features are copied to NCHW first."""
+    of lib/models/semseg.py:325-333,342-343 and lib/loss/loss_cross_datasets.py:950,961,971: the projection with the
+    prototypes as the one dense graph.  bf16 / fp16 features that _tc16_layout reads as they lie (NCHW or channels_last)
+    take the TMA-fed tcgen05 kernels (mdseg_proj_*_tc16, one product in their own type, like autocast; d feats in the
+    layout of feats, bit-identical between the two layouts); other features are made NCHW-contiguous and take
+    mdseg_proj_*_tc (fp32: three bf16 terms per operand, 1e-5 bar).  Backward: d feats = proto^T dlogits, d proto =
+    dlogits feats^T as a split-K GEMM over the pixels.  Output fp32 NCHW."""
 
     @staticmethod
     def forward(ctx, feats, proto):
@@ -660,86 +700,31 @@ class _PrototypeHead(torch.autograd.Function):
         x = feats
         if x.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             x = x.float()
-        if not _nhwc_tc16_ok(x):
+        if _tc16_layout(x) is None:
             x = x.contiguous()
         B, K, h, w = x.shape
         if proto.dim() != 2 or proto.shape[1] != K:
             raise ValueError(f"prototypes must be [N, {K}]")
         wgt = proto.detach().to(torch.float32).contiguous()
-        Nn = wgt.shape[0]
-        y = torch.empty(B, Nn, h, w, dtype=torch.float32, device=x.device)
+        y = torch.empty(B, wgt.shape[0], h, w, dtype=torch.float32, device=x.device)
         ctx.save_for_backward(x, wgt)
         ctx.proto_dtype = proto.dtype
-        if _channels_last(x):
-            # channels_last 16-bit features: K-major A operand, one dense "graph" = the prototypes
-            wt, ldb = _head_operand(wgt, x.dtype)
-            N.call("mdseg_proj_fwd_tc16_nhwc", _ptr(x), _DT[x.dtype], B, K, h * w, _one(wt), ldb, (C.c_int * 1)(Nn), 1,
-                   None, _ptr(y), Nn, _stream())
-            return y
-        if _tc16_ok(x):
-            # 16-bit features: TMA-fed MN-major operands, warp-specialised (csrc/head_tc16.cu)
-            _head_tc16(x, wgt, y)
-            return y
-        tab = _dense_table(wgt)
-        nbytes = N.lib.mdseg_proj_fwd_tc_workspace_bytes(C.byref(tab), _DT[x.dtype])
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
-        N.call("mdseg_proj_fwd_tc", _ptr(x), _DT[x.dtype], C.byref(tab), None, B, h, w, _ptr(y), Nn, None, _ptr(ws),
-               nbytes, _ptr(err_flag(x.device)), _stream())
+        _proj_fwd(x, _dense_table(wgt), [wgt], None, y, None, err_flag(x.device), _tc16_layout(x) is not None)
         return y
 
     @staticmethod
     def backward(ctx, dy):
         x, wgt = ctx.saved_tensors
-        B, K, h, w = x.shape
-        Nn = wgt.shape[0]
-        dy = dy.to(torch.float32).contiguous()
         tab = _dense_table(wgt)
+        dy = dy.to(torch.float32).contiguous()
+        if _tc16_layout(x) is not None:  # rounded to the feature dtype, as the reference's autocast backward does
+            dy = dy.to(x.dtype)
         dx = dw = None
-        if _channels_last(x):
-            # channels_last 16-bit features (see forward): d feats written pixel-major, d proto with the features as an
-            # MN-major operand; the same products and reduction order as the NCHW branch below
-            dyh = dy.to(x.dtype)
-            if ctx.needs_input_grad[0]:
-                wt, ldb = _head_operand(wgt.t(), x.dtype)
-                dx = torch.empty_like(x)  # channels_last
-                N.call("mdseg_proj_bwd_tc16_nhwc", _ptr(dyh), _DT[x.dtype], B, Nn, h * w, _one(wt), ldb, K, 1, None,
-                       _ptr(dx), _DT[x.dtype], _stream())
-            if ctx.needs_input_grad[1]:
-                dG = torch.empty(Nn, K, dtype=torch.float32, device=x.device)
-                nb = N.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, K, h * w, Nn)
-                ws = torch.empty(nb, dtype=torch.uint8, device=x.device)
-                N.call("mdseg_proj_bwd_graph_tc16_nhwc", _ptr(dyh), _ptr(x), _DT[x.dtype], B, K, h * w, Nn, None, 1,
-                       _ptr(dG), _ptr(ws), nb, _stream())
-                dw = dG.to(ctx.proto_dtype)
-            return dx, dw
-        if _tc16_ok(x):
-            # 16-bit features: both gradients on the TMA-fed kernels.  The incoming gradient is rounded to the feature
-            # dtype first (what the reference's autocast backward does to it).
-            dyh = dy.to(x.dtype)
-            if ctx.needs_input_grad[0]:  # d feats = dlogits x prototypes^T: the forward kernel, transposed prototypes
-                dx = torch.empty_like(x)
-                _head_tc16(dyh, wgt.t(), dx)
-            if ctx.needs_input_grad[1]:  # d prototype: split-K over the pixels, both operands K-major
-                dG = torch.empty(Nn, K, dtype=torch.float32, device=x.device)
-                nb = N.lib.mdseg_head_dw_tc16_workspace_bytes(B, K, h * w, Nn)
-                ws = torch.empty(nb, dtype=torch.uint8, device=x.device)
-                N.call("mdseg_head_dw_tc16", _ptr(dyh), _ptr(x), _DT[x.dtype], B, K, h * w, Nn, _ptr(dG), _ptr(ws), nb,
-                       _stream())
-                dw = dG.to(ctx.proto_dtype)
-            return dx, dw
         if ctx.needs_input_grad[0]:
-            dx = torch.empty_like(x)
-            nb = N.lib.mdseg_proj_bwd_tc_workspace_bytes(C.byref(tab), _DT[x.dtype])
-            ws = torch.empty(nb, dtype=torch.uint8, device=x.device)
-            N.call("mdseg_proj_bwd_tc", _ptr(dy), None, Nn, C.byref(tab), None, B, h, w, _ptr(dx), _DT[x.dtype], _ptr(ws),
-                   nb, _stream())
+            dx = torch.empty_like(x)  # the layout of x
+            _proj_bwd(dy, None, [wgt], tab, None, dx)
         if ctx.needs_input_grad[1]:
-            dG = torch.zeros(1, Nn * K, dtype=torch.float32, device=x.device)
-            nb = N.lib.mdseg_proj_bwd_graph_tc_workspace_bytes(C.byref(tab), B, h, w)
-            ws = torch.empty(nb, dtype=torch.uint8, device=x.device)
-            N.call("mdseg_proj_bwd_graph_tc", _ptr(x), _DT[x.dtype], _ptr(dy), None, Nn, C.byref(tab), None, B, h, w,
-                   _ptr(dG), Nn * K, _ptr(ws), nb, _stream())
-            dw = dG.view(Nn, K).to(ctx.proto_dtype)
+            dw = _proj_bwd_graph(x, dy, None, [wgt], tab, None)[0].to(ctx.proto_dtype)
         return dx, dw
 
 
@@ -754,7 +739,7 @@ class _MdsProjOhemCE(torch.autograd.Function):
     """MdsOhemCELoss(project -> upsample -> CE) of loss_cross_datasets.py:1006-1007,1074 in four kernels.  channels_last
     logits with sparse graphs are projected as they are and get a channels_last gradient (mdseg_proj_*_nhwc); so are
     channels_last 16-bit logits / features with dense graphs (folded prototypes, trainable graphs) when the backward takes
-    the tc16 route (mdseg_proj_*_tc16_nhwc)."""
+    the tc16 route (mdseg_proj_*_tc16 with layout NHWC)."""
 
     @staticmethod
     def forward(ctx, logits_uni, labels, dataset_ids, thresh, ignore, cache, per_dataset, *graphs):
@@ -782,9 +767,11 @@ class _MdsProjOhemCE(torch.autograd.Function):
         n_seg = len(Cs) if per_dataset else 1
         src = _src_table([y.data_ptr()] * len(Cs), [cmax * h * w] * len(Cs), Cs, N.F32, per_dataset, c_alloc=cmax,
                          cmax=ymax, cmax_ready=all_sparse)
-        if not (_nhwc_proj_ok(x, tab) or (_nhwc_tc16_ok(x, tab) and _tc16_bwd_nhwc_ok(ctx, len(Cs), src, h, w, H, W))):
+        tc16 = _dense_tc16(tab)
+        if not (_nhwc_proj_ok(x, tab)
+                or (tc16 and _tc16_layout(x) == N.NHWC and _tc16_bwd_nhwc_ok(ctx, len(Cs), src, h, w, H, W))):
             x = x.contiguous()
-        _proj_fwd(x, tab, ids, B, h, w, y, cmax, ymax, ef, graphs=graphs)
+        _proj_fwd(x, tab, graphs, ids, y, ymax, ef, tc16 and _tc16_layout(x) is not None)
         P = B * H * W
         loss_px = torch.empty(P, dtype=torch.float32, device=dev)
         lse_px = torch.empty(P, dtype=torch.float32, device=dev)
@@ -802,7 +789,7 @@ class _MdsProjOhemCE(torch.autograd.Function):
     def backward(ctx, grad_out, _grad_states=None):
         x, labels, ids, y, loss_px, lse_px, st, *graphs = ctx.saved_tensors
         ignore, cache, Cs, cmax, (h, w, H, W), per_dataset = ctx.meta
-        B, Cu = x.shape[:2]
+        B = x.shape[0]
         dev = x.device
         n = len(Cs)
         g = _grad_scalar(grad_out, n if per_dataset else 1)
@@ -810,21 +797,17 @@ class _MdsProjOhemCE(torch.autograd.Function):
         scratch = torch.empty(1, dtype=torch.float32, device=dev)  # non-NULL cmax selects the TMA kernels
         src = _src_table([y.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, per_dataset, c_alloc=cmax, cmax=scratch,
                          cmax_ready=True)
+        adj = (src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g)
         want_dg = any(ctx.needs_input_grad[7 + i] for i in range(n))
-        if not want_dg and _channels_last(x):
-            # channels_last logits (sparse graphs, see forward): d loss / d y from the upsample + CE adjoint, then the
-            # broadcast through G^T written pixel-major
-            dx = None
-            if ctx.needs_input_grad[0]:
-                dyA, dyB = _mds_dy(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, y, Cs, cmax)
-                dx = torch.empty_like(x)  # channels_last
-                N.call("mdseg_proj_bwd_nhwc", _ptr(dyA), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dx),
-                       _DT[x.dtype], _stream())
-            return (dx, None, None, None, None, None, None, *([None] * n))
+        dx = None
         if not want_dg:
-            # one call: softmax recompute + adjoint of the upsample + broadcast through G^T (fused when it applies)
-            dx = None
-            if ctx.needs_input_grad[0]:
+            if ctx.needs_input_grad[0] and _channels_last(x):
+                # channels_last logits (sparse graphs, see forward): d loss / d y from the upsample + CE adjoint, then the
+                # broadcast through G^T written pixel-major
+                dx = torch.empty_like(x)  # channels_last
+                _proj_bwd(*_mds_dy(*adj, y, Cs, cmax), graphs, tab, ids, dx)
+            elif ctx.needs_input_grad[0]:
+                # one call: softmax recompute + adjoint of the upsample + broadcast through G^T (fused when it applies)
                 nbytes = N.lib.mdseg_mds_bwd_workspace_bytes(C.byref(src), C.byref(tab), B, h, w, H, W)
                 ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
                 dx = torch.empty_like(x)
@@ -832,74 +815,25 @@ class _MdsProjOhemCE(torch.autograd.Function):
                        w, H, W, ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, _ptr(dx), _DT[x.dtype],
                        _ptr(ws), nbytes, _stream())
             return (dx, None, None, None, None, None, None, *([None] * n))
-        fused_direct = bool(N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W))
-        if (fused_direct and _tc16_ok(x) and Cu >= 32
-                and all(tab.g[i].dense and 8 <= Cs[i] <= 1024 for i in range(n))):
+        if (N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W) and _tc16_layout(x) is not None
+                and _dense_tc16(tab)):
             # 16-bit logits / features with dense graphs (AMP GNN stage, folded prototypes): d loss / d y leaves the fused
             # kernel in the dtype of x (what autocast's backward rounds it to) and both adjoints of the projection run
             # on the TMA-fed tcgen05 kernels — no register-staged conversion, one launch for all datasets each.
-            dy16 = torch.zeros(B, cmax, h, w, dtype=x.dtype, device=dev)  # planes >= C_ds of an image stay zero
-            dst = _src_table([dy16.data_ptr()] * n, [cmax * h * w] * n, Cs, _DT[x.dtype], False)
-            nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-            N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W,
-                   ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes,
-                   _stream())
-            if ids is None:
-                ids = torch.zeros(B, dtype=torch.int32, device=dev)
-            dx = None
-            nhwc = _channels_last(x)  # channels_last x (see forward): dx written pixel-major, x read pixel-major
-            if ctx.needs_input_grad[0]:
-                ldb = (cmax + 7) // 8 * 8
-                nt = N.lib.mdseg_head_tc16_tile(Cu)
-                rows = (Cu + nt - 1) // nt * nt
-                ptrs = (C.c_void_p * n)()
-                gt = torch.zeros(n, rows, ldb, dtype=x.dtype, device=dev)  # one zero fill for all datasets
-                for i, gph in enumerate(graphs):
-                    gt[i, :Cu, :Cs[i]] = gph.detach().t().to(x.dtype)
-                    ptrs[i] = gt[i].data_ptr()
-                dx = torch.empty_like(x)
-                N.call("mdseg_proj_bwd_tc16_nhwc" if nhwc else "mdseg_proj_bwd_tc16", _ptr(dy16), _DT[x.dtype], B, cmax,
-                       h * w, ptrs, ldb, Cu, n, _ptr(ids), _ptr(dx), _DT[x.dtype], _stream())
-            dG = torch.empty(n, cmax, Cu, dtype=torch.float32, device=dev)
-            nb = N.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, Cu, h * w, cmax)
-            ws2 = torch.empty(nb, dtype=torch.uint8, device=dev)
-            N.call("mdseg_proj_bwd_graph_tc16_nhwc" if nhwc else "mdseg_proj_bwd_graph_tc16", _ptr(dy16), _ptr(x),
-                   _DT[x.dtype], B, Cu, h * w, cmax, _ptr(ids), n, _ptr(dG), _ptr(ws2), nb, _stream())
-            dgs = [dG[i, :Cs[i]].to(graphs[i].dtype) if ctx.needs_input_grad[7 + i] else None for i in range(n)]
-            return (dx, None, None, None, None, None, None, *dgs)
-        dyA, dyB = _mds_dy(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, y, Cs, cmax)
-        dx = None
+            dy, dyB = torch.zeros(B, cmax, h, w, dtype=x.dtype, device=dev), None  # planes >= C_ds of an image stay 0
+            _up_ce_adjoint(*adj, _src_table([dy.data_ptr()] * n, [cmax * h * w] * n, Cs, _DT[x.dtype], False))
+        else:
+            dy, dyB = _mds_dy(*adj, y, Cs, cmax)
         if ctx.needs_input_grad[0]:
             dx = torch.empty_like(x)
-            if any(tab.g[i].dense for i in range(tab.n_datasets)):  # dense graphs: adjoint on the tensor cores
-                nb = N.lib.mdseg_proj_bwd_tc_workspace_bytes(C.byref(tab), _DT[x.dtype])
-                ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-                N.call("mdseg_proj_bwd_tc", _ptr(dyA), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dx),
-                       _DT[x.dtype], _ptr(ws), nb, _stream())
-            else:
-                N.call("mdseg_proj_bwd", _ptr(dyA), _ptr(dyB), cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dx),
-                       _DT[x.dtype], _stream())
-        dgs = [None] * n
-        if want_dg:
-            stride = cmax * Cu
-            dG = torch.zeros(n, stride, dtype=torch.float32, device=dev)
-            if any(tab.g[i].dense for i in range(tab.n_datasets)):  # dense graphs: split-K GEMM on the tensor cores
-                nb = N.lib.mdseg_proj_bwd_graph_tc_workspace_bytes(C.byref(tab), B, h, w)
-                ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-                N.call("mdseg_proj_bwd_graph_tc", _ptr(x), _DT[x.dtype], _ptr(dyA), _ptr(dyB), cmax, C.byref(tab),
-                       _ptr(ids), B, h, w, _ptr(dG), stride, _ptr(ws), nb, _stream())
-            else:
-                N.call("mdseg_proj_bwd_graph", _ptr(x), _DT[x.dtype], _ptr(dyA), _ptr(dyB), cmax, C.byref(tab),
-                       _ptr(ids), B, h, w, _ptr(dG), stride, _stream())
-            for i in range(n):
-                if ctx.needs_input_grad[7 + i]:
-                    dgs[i] = dG[i, :Cs[i] * Cu].view(Cs[i], Cu).to(graphs[i].dtype)
+            _proj_bwd(dy, dyB, graphs, tab, ids, dx)
+        dG = _proj_bwd_graph(x, dy, dyB, graphs, tab, ids)
+        dgs = [dG[i, :Cs[i]].to(graphs[i].dtype) if ctx.needs_input_grad[7 + i] else None for i in range(n)]
         return (dx, None, None, None, None, None, None, *dgs)
 
 
 def _tc16_bwd_nhwc_ok(ctx, n, src, h, w, H, W):
-    """_MdsProjOhemCE with dense graphs (x passed _nhwc_tc16_ok): the backward reads x only on its tc16 branch — taken
+    """_MdsProjOhemCE with channels_last x in the tc16 route of the forward: the backward reads x only on its tc16 branch — taken
     when a graph wants a gradient and the upsample + CE adjoint is the fused kernel — or never runs (no input wants a
     gradient).  A d x without d graphs goes through mdseg_mds_bwd, which writes dx planar, so x is copied then."""
     want_dg = any(ctx.needs_input_grad[7 + i] for i in range(n))
@@ -908,19 +842,25 @@ def _tc16_bwd_nhwc_ok(ctx, n, src, h, w, H, W):
     return bool(N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W))
 
 
+def _up_ce_adjoint(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, dst):
+    """mdseg_up_ce_bwd_direct: d loss / d (the low-resolution rows src describes) of the fused upsample + CE under the
+    selection in st, into the rows dst describes."""
+    B, h, w, H, W = shape
+    nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=labels.device)
+    N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
+           _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
+
+
 def _mds_dy(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, y, Cs, cmax):
     """d loss / d y of the fused loss as fp32 planes shaped like y: (dyA, None) from the fused single-pass kernel with
     the identity in place of G^T when it applies, else the two planes (dyA, dyB) of mdseg_up_ce_bwd, whose sum it is."""
     B, h, w, H, W = shape
     n = len(Cs)
-    dev = y.device
     if N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W):
         dyA, dyB = torch.empty_like(y), None  # only the first C_ds planes of an image are written — and read
-        dst = _src_table([dyA.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
-        nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W,
-               ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
+        _up_ce_adjoint(src, ids, labels, shape, ignore, loss_px, lse_px, st, g,
+                       _src_table([dyA.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False))
     else:
         dyA = torch.empty_like(y)
         dyB = torch.empty_like(y)
@@ -950,7 +890,8 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
     stacked to [H * C_ds, C_uni], H fused CE / OHEM passes on the slices of y, and in the backward one adjoint and one
     d-graph GEMM over the stacked gradient planes — x is read once per direction instead of H times and its gradient
     is written once instead of H times and added.  Dense graphs only (tensor-core routes); `graphs` is head-major.
-    channels_last 16-bit x (_nhwc_tc16_ok) is read as it is and gets a channels_last gradient."""
+    16-bit x that _tc16_layout reads as it lies takes the tc16 kernels in both directions when the stacked graphs are in
+    _tc16_envelope; channels_last x is then read as it is and gets a channels_last gradient."""
 
     @staticmethod
     def forward(ctx, x, labels, dataset_ids, thresh, ignore, n_heads, *graphs):
@@ -968,12 +909,14 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
         stacked = [torch.cat([graphs[k * n + d].detach().to(torch.float32) for k in range(n_heads)], 0) for d in range(n)]
         cache = BipartiteGraphs(assume_dense=True)
         tab, keep = cache.table(stacked)
-        if not _nhwc_tc16_ok(x, tab):  # the backward's tc16 branch holds exactly when this does
+        tc16 = _dense_tc16(tab)
+        if not (tc16 and _tc16_layout(x) == N.NHWC):
             x = x.contiguous()
+        tc16 = tc16 and _tc16_layout(x) is not None  # the route of both directions
         ids = _ids32(dataset_ids, B, dev)
         ef = err_flag(dev)
         y = torch.empty(B, cmax2, h, w, dtype=torch.float32, device=dev)
-        _proj_fwd(x, tab, ids, B, h, w, y, cmax2, None, ef, graphs=stacked)
+        _proj_fwd(x, tab, stacked, ids, y, None, ef, tc16)
         P = B * H * W
         outs, saved = [], []
         for k in range(n_heads):
@@ -988,20 +931,19 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
             outs.append(_select(loss_px, B, H * W, None, st, 1)[0])
             saved += [loss_px, lse_px, st]
         ctx.save_for_backward(x, labels, ids, y, *saved, *stacked)
-        ctx.meta = (int(ignore), Cs, cmax2, (h, w, H, W), n_heads, [g.dtype for g in graphs])
+        ctx.meta = (int(ignore), Cs, cmax2, (h, w, H, W), n_heads, [g.dtype for g in graphs], tc16)
         return torch.stack(outs)
 
     @staticmethod
     def backward(ctx, grad_out):
-        ignore, Cs, cmax2, (h, w, H, W), n_heads, gdt = ctx.meta
+        ignore, Cs, cmax2, (h, w, H, W), n_heads, gdt, tc16 = ctx.meta
         n = len(Cs)
         x, labels, ids, y = ctx.saved_tensors[:4]
         saved = ctx.saved_tensors[4:4 + 3 * n_heads]
         stacked = ctx.saved_tensors[4 + 3 * n_heads:]
-        B, Cu = x.shape[:2]
+        B = x.shape[0]
         dev = x.device
         g = _grad_scalar(grad_out, n_heads)
-        tc16 = _tc16_ok(x) and Cu >= 32 and all(8 <= n_heads * c <= 1024 for c in Cs)
         ddt = x.dtype if tc16 else torch.float32
         esz = 2 if tc16 else 4
         dy = torch.zeros(B, cmax2, h, w, dtype=ddt, device=dev)  # planes past the heads of an image's dataset stay zero
@@ -1011,48 +953,13 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
             src = _src_table([y.data_ptr() + k * c * h * w * 4 for c in Cs], [cmax2 * h * w] * n, Cs, N.F32, False,
                              c_alloc=[cmax2 - k * c for c in Cs], cmax=scratch, cmax_ready=True)
             dst = _src_table([dy.data_ptr() + k * c * h * w * esz for c in Cs], [cmax2 * h * w] * n, Cs, _DT[ddt], False)
-            nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-            N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W,
-                   ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g[k:k + 1]), 1.0, C.byref(dst), _ptr(ws), nbytes,
-                   _stream())
-        Cs2 = [n_heads * c for c in Cs]
+            _up_ce_adjoint(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g[k:k + 1], dst)
+        tab, keep = (None, None) if tc16 else BipartiteGraphs(assume_dense=True).table(list(stacked))
         dx = None
-        if tc16:
-            ids_ = ids if ids is not None else torch.zeros(B, dtype=torch.int32, device=dev)
-            nhwc = _channels_last(x)
-            if ctx.needs_input_grad[0]:
-                ldb = (cmax2 + 7) // 8 * 8
-                nt = N.lib.mdseg_head_tc16_tile(Cu)
-                rows = (Cu + nt - 1) // nt * nt
-                ptrs = (C.c_void_p * n)()
-                gt = torch.zeros(n, rows, ldb, dtype=x.dtype, device=dev)  # one zero fill for all datasets
-                for i, gph in enumerate(stacked):
-                    gt[i, :Cu, :Cs2[i]] = gph.t().to(x.dtype)
-                    ptrs[i] = gt[i].data_ptr()
-                dx = torch.empty_like(x)
-                N.call("mdseg_proj_bwd_tc16_nhwc" if nhwc else "mdseg_proj_bwd_tc16", _ptr(dy), _DT[x.dtype], B, cmax2,
-                       h * w, ptrs, ldb, Cu, n, _ptr(ids_), _ptr(dx), _DT[x.dtype], _stream())
-            dG = torch.empty(n, cmax2, Cu, dtype=torch.float32, device=dev)
-            nb = N.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, Cu, h * w, cmax2)
-            ws2 = torch.empty(nb, dtype=torch.uint8, device=dev)
-            N.call("mdseg_proj_bwd_graph_tc16_nhwc" if nhwc else "mdseg_proj_bwd_graph_tc16", _ptr(dy), _ptr(x),
-                   _DT[x.dtype], B, Cu, h * w, cmax2, _ptr(ids_), n, _ptr(dG), _ptr(ws2), nb, _stream())
-        else:
-            cache = BipartiteGraphs(assume_dense=True)
-            tab, keep = cache.table(list(stacked))
-            if ctx.needs_input_grad[0]:
-                dx = torch.empty_like(x)
-                nb = N.lib.mdseg_proj_bwd_tc_workspace_bytes(C.byref(tab), _DT[x.dtype])
-                ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-                N.call("mdseg_proj_bwd_tc", _ptr(dy), None, cmax2, C.byref(tab), _ptr(ids), B, h, w, _ptr(dx), _DT[x.dtype],
-                       _ptr(ws), nb, _stream())
-            dG = torch.zeros(n, cmax2 * Cu, dtype=torch.float32, device=dev)
-            nb = N.lib.mdseg_proj_bwd_graph_tc_workspace_bytes(C.byref(tab), B, h, w)
-            ws2 = torch.empty(nb, dtype=torch.uint8, device=dev)
-            N.call("mdseg_proj_bwd_graph_tc", _ptr(x), _DT[x.dtype], _ptr(dy), None, cmax2, C.byref(tab), _ptr(ids), B, h, w,
-                   _ptr(dG), cmax2 * Cu, _ptr(ws2), nb, _stream())
-            dG = dG.view(n, cmax2, Cu)
+        if ctx.needs_input_grad[0]:
+            dx = torch.empty_like(x)
+            _proj_bwd(dy, None, stacked, tab, ids, dx)
+        dG = _proj_bwd_graph(x, dy, None, stacked, tab, ids)
         dgs = []
         for k in range(n_heads):
             for d in range(n):
@@ -1067,7 +974,7 @@ def mds_proj_ohem_ce_heads(x, labels, dataset_ids, graph_sets, thresh, ignore=25
     """Vector [H] of MdsOhemCELoss values, one per graph set, sharing ONE pass over x per direction (see
     _MdsProjOhemCEHeads).  graph_sets: H lists of n_datasets dense [C_ds, C_uni] matrices (the same C_ds in every set).
     Falls back to H independent fused losses when the stacked route does not apply (graphs that are not all in the
-    tensor-core envelope, geometry outside the fused backward).  channels_last 16-bit x inside _nhwc_tc16_ok is read
+    tensor-core envelope, geometry outside the fused backward).  channels_last 16-bit x inside _tc16_layout is read
     without a layout copy on both routes (the fallback's losses pick their layout one by one)."""
     sets = [list(gs) for gs in graph_sets]
     n = len(sets[0])
@@ -1075,7 +982,7 @@ def mds_proj_ohem_ce_heads(x, labels, dataset_ids, graph_sets, thresh, ignore=25
     Hh, Ww = labels.shape[1:]
     Cs = [g.shape[0] for g in sets[0]]
     ok = (len(sets) > 1 and all(len(gs) == n and [g.shape[0] for g in gs] == Cs for gs in sets)
-          and all(8 <= c and len(sets) * c <= 1024 for c in Cs) and Cu >= 32 and x.is_cuda)
+          and _tc16_envelope(Cu, Cs, len(sets)) and x.is_cuda)
     if ok:
         probe = _src_table([x.data_ptr() & ~15] * n, [4 * h * w] * n, Cs, N.F32, False, cmax=x)
         ok = bool(N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(probe), h, w, Hh, Ww))
@@ -1177,7 +1084,7 @@ class _MdsNLLPlus(torch.autograd.Function):
         pred = torch.empty(B, Cu, h, w, dtype=torch.float32, device=dev)
         N.call("mdseg_softmax_nchw", _ptr(x), _DT[x.dtype], B, Cu, h * w, _ptr(pred), _stream())
         q = torch.empty(B, cmax, h, w, dtype=torch.float32, device=dev)
-        _proj_fwd(pred, tab, ids, B, h, w, q, cmax, None, ef)
+        _proj_fwd(pred, tab, graphs, ids, q, None, ef, False)
         src = _src_table([q.data_ptr()] * len(Cs), [cmax * h * w] * len(Cs), Cs, N.F32, False, c_alloc=cmax)
         loss_px = torch.empty(B * H * W, dtype=torch.float32, device=dev)
         st = _new_states(1, thresh, dev)
@@ -1206,31 +1113,15 @@ class _MdsNLLPlus(torch.autograd.Function):
         dx = None
         if ctx.needs_input_grad[0]:
             dpred = torch.empty_like(pred)
-            if any(tab.g[i].dense for i in range(tab.n_datasets)):
-                nb = N.lib.mdseg_proj_bwd_tc_workspace_bytes(C.byref(tab), N.F32)
-                ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-                N.call("mdseg_proj_bwd_tc", _ptr(dq), None, cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dpred), N.F32,
-                       _ptr(ws), nb, _stream())
-            else:
-                N.call("mdseg_proj_bwd", _ptr(dq), None, cmax, C.byref(tab), _ptr(ids), B, h, w, _ptr(dpred), N.F32,
-                       _stream())
+            _proj_bwd(dq, None, graphs, tab, ids, dpred)
             dx = dpred if xdt == torch.float32 else torch.empty(pred.shape, dtype=xdt, device=dev)
             N.call("mdseg_softmax_bwd_nchw", _ptr(pred), _ptr(dpred), B, Cu, h * w, _ptr(dx), _DT[xdt], _stream())
         dgs = [None] * n
         if any(ctx.needs_input_grad[6 + i] for i in range(n)):
-            stride = cmax * Cu
-            dG = torch.zeros(n, stride, dtype=torch.float32, device=dev)
-            if any(tab.g[i].dense for i in range(tab.n_datasets)):
-                nb = N.lib.mdseg_proj_bwd_graph_tc_workspace_bytes(C.byref(tab), B, h, w)
-                ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-                N.call("mdseg_proj_bwd_graph_tc", _ptr(pred), N.F32, _ptr(dq), None, cmax, C.byref(tab), _ptr(ids), B, h,
-                       w, _ptr(dG), stride, _ptr(ws), nb, _stream())
-            else:
-                N.call("mdseg_proj_bwd_graph", _ptr(pred), N.F32, _ptr(dq), None, cmax, C.byref(tab), _ptr(ids), B, h, w,
-                       _ptr(dG), stride, _stream())
+            dG = _proj_bwd_graph(pred, dq, None, graphs, tab, ids)
             for i in range(n):
                 if ctx.needs_input_grad[6 + i]:
-                    dgs[i] = dG[i, :Cs[i] * Cu].view(Cs[i], Cu).to(graphs[i].dtype)
+                    dgs[i] = dG[i, :Cs[i]].to(graphs[i].dtype)
         return (dx, None, None, None, None, None, *dgs)
 
 
@@ -1313,10 +1204,7 @@ class _UpOhemCE(torch.autograd.Function):
         # outputs, the kernel writes only the rows of a head's own images
         grads = [torch.zeros_like(s) for s in srcs]
         dst = _src_table([t.data_ptr() for t in grads], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset)
-        nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=labels.device)
-        N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W,
-               ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
+        _up_ce_adjoint(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, dst)
         return (None, None, None, None, None, *grads)
 
 
@@ -1335,11 +1223,7 @@ def _up_ohem_ce_bwd_nhwc(planar, labels, ids, loss_px, lse_px, st, g, scratch, i
     else:  # the generic route adds two planes per head: dense [B, C_d, h, w] destinations
         dp = [torch.empty(B, c, h, w, dtype=dt, device=dev) for c in Cs]
         dst = _src_table([t.data_ptr() for t in dp], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset)
-    nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
-    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-    N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W,
-           ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
-    del ws
+    _up_ce_adjoint(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, dst)
     grads = [torch.empty((B, c, h, w), dtype=dt, device=dev, memory_format=torch.channels_last) for c in Cs]
     gt = _src_table([t.data_ptr() for t in grads], [t.stride(0) for t in grads], Cs, _DT[dt], seg_per_dataset)
     N.call("mdseg_planar_to_nhwc", C.byref(dst), _ptr(ids), B, h, w, C.byref(gt), _stream())

@@ -5,9 +5,9 @@ Per dtype, forward + backward step time (median of CUDA-event timings after warm
 far above the 126 MB L2) and the peak-memory growth of one step, for
   * the folded single loss (mds_head_proj_ohem_ce), the stacked hard / soft pair (mds_head_proj_ohem_ce_heads) and
     prototype_head forward + d feats + d proto;
-  * each with (a) NCHW features, (b) channels_last features on the *_tc16_nhwc route, (c) channels_last features
+  * each with (a) NCHW features, (b) channels_last features on the tc16 route with layout NHWC, (c) channels_last features
     through the copy route: feats.contiguous() -> NCHW call -> gradient .contiguous(channels_last);
-and the three C-ABI calls of the folded loss alone (planar and pixel-major entry points, same operands).
+and the three C-ABI calls of the folded loss alone (planar and pixel-major x, same operands).
 One JSON line per measurement on stdout; the first line names the card and its power limit."""
 import ctypes as C
 import json
@@ -104,20 +104,8 @@ def calls(dt, x, xl, gs, ids):
     n, cmax = 7, max(N_CATS)
     B, hw = len(IDS), h * w
     W_d = [g.detach() @ torch.randn(C_UNI, K, device=DEV) * 0.05 for g in gs[:7]]
-    nt = N.lib.mdseg_head_tc16_tile
-    rows = max((c + nt(c) - 1) // nt(c) * nt(c) for c in N_CATS)
-    wt = torch.zeros(n, rows, K, dtype=dt, device=DEV)
-    ptrs = (C.c_void_p * n)()
-    for i, m in enumerate(W_d):
-        wt[i, :m.shape[0]] = m.to(dt)
-        ptrs[i] = wt[i].data_ptr()
-    rows_t = (K + nt(K) - 1) // nt(K) * nt(K)
-    ldb_t = (cmax + 7) // 8 * 8
-    wtt = torch.zeros(n, rows_t, ldb_t, dtype=dt, device=DEV)
-    ptrs_t = (C.c_void_p * n)()
-    for i, m in enumerate(W_d):
-        wtt[i, :K, :m.shape[0]] = m.t().to(dt)
-        ptrs_t[i] = wtt[i].data_ptr()
+    wt, ptrs, ldb = ops._tc16_operands(W_d, dt)
+    wtt, ptrs_t, ldb_t = ops._tc16_operands(W_d, dt, transpose=True)
     cds = (C.c_int * n)(*N_CATS)
     y = torch.empty(B, cmax, h, w, device=DEV)
     dy16 = (torch.randn(B, cmax, h, w, device=DEV) * 1e-3).to(dt)
@@ -128,17 +116,17 @@ def calls(dt, x, xl, gs, ids):
     ws = torch.empty(nb, dtype=torch.uint8, device=DEV)
     s = torch.cuda.current_stream().cuda_stream
     d = ops._DT[dt]
-    for suffix, xx, dd in (("", x, dx), ("_nhwc", xl, dxl)):
+    for lname, lay, xx, dd in (("NCHW", N.NCHW, x, dx), ("NHWC", N.NHWC, xl, dxl)):
         fns = {
-            "proj_fwd_tc16": lambda: N.call("mdseg_proj_fwd_tc16" + suffix, xx.data_ptr(), d, B, K, hw, ptrs, K, cds, n,
+            "proj_fwd_tc16": lambda: N.call("mdseg_proj_fwd_tc16", xx.data_ptr(), d, lay, B, K, hw, ptrs, ldb, cds, n,
                                             ids.data_ptr(), y.data_ptr(), cmax, s),
-            "proj_bwd_tc16": lambda: N.call("mdseg_proj_bwd_tc16" + suffix, dy16.data_ptr(), d, B, cmax, hw, ptrs_t, ldb_t,
+            "proj_bwd_tc16": lambda: N.call("mdseg_proj_bwd_tc16", dy16.data_ptr(), d, lay, B, cmax, hw, ptrs_t, ldb_t,
                                             K, n, ids.data_ptr(), dd.data_ptr(), d, s),
-            "proj_bwd_graph_tc16": lambda: N.call("mdseg_proj_bwd_graph_tc16" + suffix, dy16.data_ptr(), xx.data_ptr(), d,
+            "proj_bwd_graph_tc16": lambda: N.call("mdseg_proj_bwd_graph_tc16", dy16.data_ptr(), xx.data_ptr(), d, lay,
                                                   B, K, hw, cmax, ids.data_ptr(), n, dG.data_ptr(), ws.data_ptr(), nb, s),
         }
         for k, fn in fns.items():
-            emit(case=f"call {dt}", entry=f"mdseg_{k}{suffix}", ms=round(timed(fn, 3, 21), 4))
+            emit(case=f"call {dt}", entry=f"mdseg_{k}", layout=lname, ms=round(timed(fn, 3, 21), 4))
 
 
 def main():

@@ -1,7 +1,7 @@
-"""GPU: channels_last 16-bit features / logits on the TMA-fed tcgen05 kernels — mdseg_proj_fwd_tc16_nhwc,
-mdseg_proj_bwd_tc16_nhwc, mdseg_proj_bwd_graph_tc16_nhwc — and the operators that route through them (the prototype
-head, the folded and dense-graph fused losses, the stacked hard / soft pair).  Every output is compared bit for bit
-with the NCHW entry points / NCHW input on the same values."""
+"""GPU: channels_last 16-bit features / logits on the TMA-fed tcgen05 kernels — mdseg_proj_fwd_tc16,
+mdseg_proj_bwd_tc16 and mdseg_proj_bwd_graph_tc16 with layout NHWC — and the operators that route through them (the
+prototype head, the folded and dense-graph fused losses, the stacked hard / soft pair).  Every output is compared bit
+for bit with layout NCHW / NCHW input on the same values."""
 import ctypes as C
 
 import pytest
@@ -50,30 +50,10 @@ SHAPES = [(512, [19, 150, 64], 12, 20), (48, [19, 150, 64], 12, 20), (96, [19, 1
 IDS = {"sorted": [0, 0, 1, 2, 2], "shuffled": [2, 0, 1, 2, 0], "absent": [2, 0, 7, 1, 0]}  # 7: no such dataset
 
 
-def _graph_operands(ops, mats, dtype, transpose):
-    """The padded per-dataset B operands of the tc16 kernels in one buffer: G_d ([C_d, K]) or G_d^T ([K, C_d])."""
-    n = len(mats)
-    rows_of, cols = [], 0
-    for m in mats:
-        r = m.shape[1] if transpose else m.shape[0]
-        nt = ops.N.lib.mdseg_head_tc16_tile(r)
-        rows_of.append((r + nt - 1) // nt * nt)
-        cols = max(cols, m.shape[0] if transpose else m.shape[1])
-    ldb = (cols + 7) // 8 * 8
-    buf = torch.zeros(max(rows_of) * n, ldb, dtype=dtype, device=DEV)
-    ptrs = (C.c_void_p * n)()
-    for i, m in enumerate(mats):
-        mm = (m.t() if transpose else m).to(dtype)
-        o = i * max(rows_of)
-        buf[o:o + mm.shape[0], :mm.shape[1]] = mm
-        ptrs[i] = buf.data_ptr() + o * ldb * buf.element_size()
-    return buf, ptrs, ldb
-
-
 @pytest.mark.parametrize("ids_name", list(IDS))
 @pytest.mark.parametrize("shape", SHAPES, ids=[f"K{s[0]}_N{max(s[1])}" for s in SHAPES])
 @pytest.mark.parametrize("dtype", DTYPES, ids=DT_IDS)
-def test_entry_points_bit_identical(ops, native, dtype, shape, ids_name):
+def test_layout_entry_points_bit_identical(ops, native, dtype, shape, ids_name):
     K, Cs, h, w = shape
     ids = IDS[ids_name]
     B, hw, n, cmax = len(ids), h * w, len(Cs), max(Cs)
@@ -85,13 +65,13 @@ def test_entry_points_bit_identical(ops, native, dtype, shape, ids_name):
     dt = ops._DT[dtype]
 
     # forward: y = G_d x, planar fp32
-    keep, ptrs, ldb = _graph_operands(ops, mats, dtype, transpose=False)
+    keep, ptrs, ldb = ops._tc16_operands(mats, dtype)
     cds = (C.c_int * n)(*Cs)
     y0 = torch.full((B, cmax, h, w), 3.0, device=DEV)
     y1 = torch.full((B, cmax, h, w), 3.0, device=DEV)
-    native.call("mdseg_proj_fwd_tc16", x.data_ptr(), dt, B, K, hw, ptrs, ldb, cds, n, ids_t.data_ptr(), y0.data_ptr(),
-                cmax, stream())
-    native.call("mdseg_proj_fwd_tc16_nhwc", xl.data_ptr(), dt, B, K, hw, ptrs, ldb, cds, n, ids_t.data_ptr(),
+    native.call("mdseg_proj_fwd_tc16", x.data_ptr(), dt, native.NCHW, B, K, hw, ptrs, ldb, cds, n, ids_t.data_ptr(),
+                y0.data_ptr(), cmax, stream())
+    native.call("mdseg_proj_fwd_tc16", xl.data_ptr(), dt, native.NHWC, B, K, hw, ptrs, ldb, cds, n, ids_t.data_ptr(),
                 y1.data_ptr(), cmax, stream())
     torch.cuda.synchronize()
     assert torch.equal(y0, y1)
@@ -101,34 +81,34 @@ def test_entry_points_bit_identical(ops, native, dtype, shape, ids_name):
     for b, d in enumerate(ids):
         if d < n:
             dy[b, :Cs[d]] = torch.randn(Cs[d], h, w, generator=gen, device=DEV).to(dtype)
-    keep_t, ptrs_t, ldb_t = _graph_operands(ops, mats, dtype, transpose=True)
+    keep_t, ptrs_t, ldb_t = ops._tc16_operands(mats, dtype, transpose=True)
     for dx_dt in (dtype, torch.float32):
         dx0 = torch.full((B, K, h, w), 7.0, dtype=dx_dt, device=DEV)
         dx1 = torch.full((B, K, h, w), 7.0, dtype=dx_dt, device=DEV).contiguous(memory_format=CL)
-        native.call("mdseg_proj_bwd_tc16", dy.data_ptr(), dt, B, cmax, hw, ptrs_t, ldb_t, K, n, ids_t.data_ptr(),
-                    dx0.data_ptr(), ops._DT[dx_dt], stream())
-        native.call("mdseg_proj_bwd_tc16_nhwc", dy.data_ptr(), dt, B, cmax, hw, ptrs_t, ldb_t, K, n, ids_t.data_ptr(),
-                    dx1.data_ptr(), ops._DT[dx_dt], stream())
+        native.call("mdseg_proj_bwd_tc16", dy.data_ptr(), dt, native.NCHW, B, cmax, hw, ptrs_t, ldb_t, K, n,
+                    ids_t.data_ptr(), dx0.data_ptr(), ops._DT[dx_dt], stream())
+        native.call("mdseg_proj_bwd_tc16", dy.data_ptr(), dt, native.NHWC, B, cmax, hw, ptrs_t, ldb_t, K, n,
+                    ids_t.data_ptr(), dx1.data_ptr(), ops._DT[dx_dt], stream())
         torch.cuda.synchronize()
         assert torch.equal(dx0, dx1.contiguous()), dx_dt
         for b, d in enumerate(ids):
             if d >= n:
                 assert not dx1[b].any()  # zero rows for an image of no dataset
 
-    # d G_d = dy16 x^T per dataset, and the one-sum form (dataset_ids NULL) against mdseg_head_dw_tc16
+    # d G_d = dy16 x^T per dataset, and the one-sum form (dataset_ids NULL), each in both layouts
     nb = native.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, K, hw, cmax)
     ws = torch.empty(nb, dtype=torch.uint8, device=DEV)
     dG0 = torch.empty(n, cmax, K, device=DEV)
     dG1 = torch.empty(n, cmax, K, device=DEV)
-    native.call("mdseg_proj_bwd_graph_tc16", dy.data_ptr(), x.data_ptr(), dt, B, K, hw, cmax, ids_t.data_ptr(), n,
-                dG0.data_ptr(), ws.data_ptr(), nb, stream())
-    native.call("mdseg_proj_bwd_graph_tc16_nhwc", dy.data_ptr(), xl.data_ptr(), dt, B, K, hw, cmax, ids_t.data_ptr(), n,
-                dG1.data_ptr(), ws.data_ptr(), nb, stream())
+    native.call("mdseg_proj_bwd_graph_tc16", dy.data_ptr(), x.data_ptr(), dt, native.NCHW, B, K, hw, cmax,
+                ids_t.data_ptr(), n, dG0.data_ptr(), ws.data_ptr(), nb, stream())
+    native.call("mdseg_proj_bwd_graph_tc16", dy.data_ptr(), xl.data_ptr(), dt, native.NHWC, B, K, hw, cmax,
+                ids_t.data_ptr(), n, dG1.data_ptr(), ws.data_ptr(), nb, stream())
     dW0 = torch.empty(cmax, K, device=DEV)
     dW1 = torch.empty(cmax, K, device=DEV)
-    native.call("mdseg_head_dw_tc16", dy.data_ptr(), x.data_ptr(), dt, B, K, hw, cmax, dW0.data_ptr(), ws.data_ptr(), nb,
-                stream())
-    native.call("mdseg_proj_bwd_graph_tc16_nhwc", dy.data_ptr(), xl.data_ptr(), dt, B, K, hw, cmax, None, 1,
+    native.call("mdseg_proj_bwd_graph_tc16", dy.data_ptr(), x.data_ptr(), dt, native.NCHW, B, K, hw, cmax, None, 1,
+                dW0.data_ptr(), ws.data_ptr(), nb, stream())
+    native.call("mdseg_proj_bwd_graph_tc16", dy.data_ptr(), xl.data_ptr(), dt, native.NHWC, B, K, hw, cmax, None, 1,
                 dW1.data_ptr(), ws.data_ptr(), nb, stream())
     torch.cuda.synchronize()
     assert torch.equal(dG0, dG1)
@@ -137,21 +117,21 @@ def test_entry_points_bit_identical(ops, native, dtype, shape, ids_name):
     ops.check_errors(DEV)
 
 
-def test_entry_points_reject_bad_inputs(ops, native):
+def test_layout_entry_points_reject_bad_inputs(ops, native):
     x = torch.zeros(2, 60, 8, 8, dtype=torch.bfloat16, device=DEV).contiguous(memory_format=CL)
-    keep, ptrs, ldb = _graph_operands(ops, [torch.zeros(16, 60, device=DEV)], torch.bfloat16, transpose=False)
+    keep, ptrs, ldb = ops._tc16_operands([torch.zeros(16, 60, device=DEV)], torch.bfloat16)
     y = torch.empty(2, 16, 8, 8, device=DEV)
     with pytest.raises(native.MdsegError, match="multiple of 8"):  # K % 8 != 0
-        native.call("mdseg_proj_fwd_tc16_nhwc", x.data_ptr(), native.BF16, 2, 60, 64, ptrs, ldb, (C.c_int * 1)(16), 1,
-                    None, y.data_ptr(), 16, stream())
+        native.call("mdseg_proj_fwd_tc16", x.data_ptr(), native.BF16, native.NHWC, 2, 60, 64, ptrs, ldb,
+                    (C.c_int * 1)(16), 1, None, y.data_ptr(), 16, stream())
     x32 = torch.zeros(2, 64, 8, 8, device=DEV)
     with pytest.raises(native.MdsegError, match="bf16 or fp16"):
-        native.call("mdseg_proj_fwd_tc16_nhwc", x32.data_ptr(), native.F32, 2, 64, 64, ptrs, 64, (C.c_int * 1)(16), 1,
-                    None, y.data_ptr(), 16, stream())
+        native.call("mdseg_proj_fwd_tc16", x32.data_ptr(), native.F32, native.NHWC, 2, 64, 64, ptrs, 64,
+                    (C.c_int * 1)(16), 1, None, y.data_ptr(), 16, stream())
     dy = torch.zeros(2, 16, 8, 8, dtype=torch.bfloat16, device=DEV)
     with pytest.raises(native.MdsegError, match="dataset ids"):
-        native.call("mdseg_proj_bwd_graph_tc16_nhwc", dy.data_ptr(), x.data_ptr(), native.BF16, 2, 64, 64, 16, None, 2,
-                    y.data_ptr(), y.data_ptr(), 1 << 20, stream())
+        native.call("mdseg_proj_bwd_graph_tc16", dy.data_ptr(), x.data_ptr(), native.BF16, native.NHWC, 2, 64, 64, 16,
+                    None, 2, y.data_ptr(), y.data_ptr(), 1 << 20, stream())
 
 
 # ---- 2. the prototype head ------------------------------------------------------------------------------------------

@@ -95,11 +95,10 @@ def test_folded_head_loss_matches_float64_reference_order(ops, dt, tol, ids):
 @pytest.mark.parametrize("dt", [torch.bfloat16, torch.float16])
 @pytest.mark.parametrize("B,Cu,cmax,Cs,h,w", [(5, 512, 150, [19, 150, 64], 16, 24), (3, 48, 40, [40, 8], 8, 8),
                                               (4, 358, 133, [133, 26, 37, 19], 12, 20)])
-def test_proj_bwd_tc16_entry_points_match_float64(ops, dt, B, Cu, cmax, Cs, h, w):
+def test_proj_bwd_tc16_nchw_entry_points_match_float64(ops, dt, B, Cu, cmax, Cs, h, w):
     """mdseg_proj_bwd_tc16 (d x = G_d^T dy) and mdseg_proj_bwd_graph_tc16 (d G_d = sum over the dataset's images of
     dy x^T) through the C ABI, including an image whose dataset id is out of range (zero rows in d x, no contribution
     to any d G)."""
-    import ctypes as C
     from mdseg_b200 import native as N
     g = torch.Generator(device=DEV).manual_seed(B * 100 + Cu)
     n = len(Cs)
@@ -114,24 +113,16 @@ def test_proj_bwd_tc16_entry_points_match_float64(ops, dt, B, Cu, cmax, Cs, h, w
             dy[b, :Cs[d]] = torch.randn(Cs[d], h, w, generator=g, device=DEV)
     dy16 = dy.to(dt)
     dtc = {torch.bfloat16: N.BF16, torch.float16: N.F16}[dt]
-    ldb = (cmax + 7) // 8 * 8
-    nt = N.lib.mdseg_head_tc16_tile(Cu)
-    rows = (Cu + nt - 1) // nt * nt
-    ptrs, keep = (C.c_void_p * n)(), []
-    for i, m in enumerate(graphs):
-        gt = torch.zeros(rows, ldb, dtype=dt, device=DEV)
-        gt[:Cu, :Cs[i]] = m.t().to(dt)
-        keep.append(gt)
-        ptrs[i] = gt.data_ptr()
+    keep, ptrs, ldb = ops._tc16_operands(graphs, dt, transpose=True)
     dx = torch.full((B, Cu, h, w), float("nan"), dtype=dt, device=DEV)
     stream = torch.cuda.current_stream().cuda_stream
-    N.call("mdseg_proj_bwd_tc16", dy16.data_ptr(), dtc, B, cmax, h * w, ptrs, ldb, Cu, n, ids_t.data_ptr(), dx.data_ptr(),
-           dtc, stream)
+    N.call("mdseg_proj_bwd_tc16", dy16.data_ptr(), dtc, N.NCHW, B, cmax, h * w, ptrs, ldb, Cu, n, ids_t.data_ptr(),
+           dx.data_ptr(), dtc, stream)
     dG = torch.full((n, cmax, Cu), float("nan"), dtype=torch.float32, device=DEV)
     nb = N.lib.mdseg_proj_bwd_graph_tc16_workspace_bytes(B, Cu, h * w, cmax)
     ws = torch.empty(nb, dtype=torch.uint8, device=DEV)
-    N.call("mdseg_proj_bwd_graph_tc16", dy16.data_ptr(), x.data_ptr(), dtc, B, Cu, h * w, cmax, ids_t.data_ptr(), n,
-           dG.data_ptr(), ws.data_ptr(), nb, stream)
+    N.call("mdseg_proj_bwd_graph_tc16", dy16.data_ptr(), x.data_ptr(), dtc, N.NCHW, B, Cu, h * w, cmax, ids_t.data_ptr(),
+           n, dG.data_ptr(), ws.data_ptr(), nb, stream)
     torch.cuda.synchronize()
     want_dx = torch.zeros(B, Cu, h, w, dtype=torch.float64, device=DEV)
     want_dG = torch.zeros(n, cmax, Cu, dtype=torch.float64, device=DEV)
