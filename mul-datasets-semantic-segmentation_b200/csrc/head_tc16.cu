@@ -31,60 +31,13 @@
 namespace mdseg {
 namespace {
 
+using namespace tma;
+
 constexpr int kM = 128;           // pixels per tile (UMMA M)
 constexpr int kKB = 64;           // channels per stage: 64 x 2 B = one 128-byte swizzle row of B
 constexpr int kNStages = 2;
 constexpr int kThreads = 192;     // producer warp, MMA warp, four epilogue warps
 constexpr int kABytes = kKB * kM * 2;  // 16 KB: [2 pixel atoms][64 channel rows][128 B]
-
-__device__ __forceinline__ uint32_t sa(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void bar_init(uint64_t* b, int n) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(sa(b)), "r"(n));
-}
-__device__ __forceinline__ void bar_expect(uint64_t* b, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(sa(b)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bar_wait(uint64_t* b, uint32_t parity) {
-  asm volatile(
-      "{\n.reg .pred p;\nMDSEG_H16_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra MDSEG_H16_DONE;\nbra MDSEG_H16_WAIT;\nMDSEG_H16_DONE:\n}\n" ::"r"(sa(b)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void tma3(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(sa(dst)), "l"((uint64_t)m), "r"(sa(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tma2(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(sa(dst)), "l"((uint64_t)m), "r"(sa(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tc_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(sa(bar)) : "memory");
-}
-__device__ __forceinline__ void umma(uint32_t d, uint64_t ad, uint64_t bd, uint32_t idesc, uint32_t accum) {
-  asm volatile(
-      "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}\n" ::"r"(d),
-      "l"(ad), "l"(bd), "r"(idesc), "r"(accum)
-      : "memory");
-}
-// Shared-memory matrix descriptor (cute::UMMA::SmemDescriptor, version 1), 128-byte swizzle (layout type 2)
-__device__ __forceinline__ uint64_t desc_sw128(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  return (uint64_t)((saddr & 0x3ffffu) >> 4) | ((uint64_t)((lbo >> 4) & 0x3fffu) << 16) |
-         ((uint64_t)((sbo >> 4) & 0x3fffu) << 32) | (1ull << 46) | (2ull << 61);
-}
-
-struct alignas(64) BMaps {
-  CUtensorMap m[MDSEG_MAX_DATASETS];  // the B operand (prototypes, or the dense graph of dataset d)
-};
 
 struct HeadArgs {
   void* out;          // [n_images, out_cstride, hw] (kOutPM: [n_images, hw, out_cstride]) fp32 or the feature dtype
@@ -117,7 +70,7 @@ __device__ __forceinline__ void store16_pm(TO* o, const uint32_t* r) {
 
 template <typename TO, bool kAK, bool kOutPM>
 __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_constant__ CUtensorMap mapA,
-                                                                const __grid_constant__ BMaps mapsB,
+                                                                const __grid_constant__ Maps mapsB,
                                                                 const __grid_constant__ HeadArgs a) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   unsigned char* smem = reinterpret_cast<unsigned char*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -151,43 +104,42 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
   }
   const int NT = a.NTd[d], Nout = a.Nd[d];
   if (NT == 0 || nz * NT >= Nout) return;
-  const CUtensorMap& mapB = mapsB.m[d];
+  const CUtensorMap& mapB = mapsB.m[d];  // the B operand: prototypes, or the dense graph of dataset d
   const uint32_t b_bytes = (uint32_t)NT * 128u;
   const uint32_t stage_bytes = kABytes + b_bytes;
   uint32_t tmem_cols = 32;
   while ((int)tmem_cols < NT) tmem_cols <<= 1;
 
   if (threadIdx.x == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&mapA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&mapB) : "memory");
-    for (int s = 0; s < kNStages; ++s) { bar_init(&full[s], 1); bar_init(&empty[s], 1); }
-    bar_init(&acc_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    prefetch_map(&mapA);
+    prefetch_map(&mapB);
+    for (int s = 0; s < kNStages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
+    mbar_init(&acc_full, 1);
+    mbar_fence_init();
   }
   if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sa(&tmem_base_s)), "r"(tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(&tmem_base_s, tmem_cols);
+    tmem_relinquish();
   }
-  tc_before();
+  tc_fence_before();
   __syncthreads();
-  tc_after();
+  tc_fence_after();
   const uint32_t tmem_d = tmem_base_s;
 
   if (warp == 0) {
     if (lane == 0) {
       for (int kb = 0; kb < a.n_kb; ++kb) {
         const int s = kb % kNStages;
-        if (kb >= kNStages) bar_wait(&empty[s], (uint32_t)((kb / kNStages - 1) & 1));
+        if (kb >= kNStages) mbar_wait(&empty[s], (uint32_t)((kb / kNStages - 1) & 1));
         unsigned char* st = smem + (size_t)s * stage_bytes;
-        bar_expect(&full[s], stage_bytes);
+        mbar_expect_tx(&full[s], stage_bytes);
         if constexpr (kAK) {
-          tma3(st, &mapA, &full[s], kb * kKB, (int)p0, b);                    // [128 pixels][64 channels]
+          load_3d(st, &mapA, &full[s], kb * kKB, (int)p0, b);                   // [128 pixels][64 channels]
         } else {
-          tma3(st, &mapA, &full[s], (int)p0, kb * kKB, b);                    // pixels p0 .. p0+63
-          tma3(st + kKB * 128, &mapA, &full[s], (int)p0 + 64, kb * kKB, b);   // pixels p0+64 .. p0+127
+          load_3d(st, &mapA, &full[s], (int)p0, kb * kKB, b);                   // pixels p0 .. p0+63
+          load_3d(st + kKB * 128, &mapA, &full[s], (int)p0 + 64, kb * kKB, b);  // pixels p0+64 .. p0+127
         }
-        tma2(st + kABytes, &mapB, &full[s], kb * kKB, nz * NT);
+        load_2d(st + kABytes, &mapB, &full[s], kb * kKB, nz * NT);
       }
     }
   } else if (warp == 1) {
@@ -197,17 +149,18 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
                              ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(kM >> 4) << 24);
       for (int kb = 0; kb < a.n_kb; ++kb) {
         const int s = kb % kNStages;
-        bar_wait(&full[s], (uint32_t)((kb / kNStages) & 1));
-        tc_after();
-        const uint32_t aA = sa(smem + (size_t)s * stage_bytes), aB = aA + kABytes;
+        mbar_wait(&full[s], (uint32_t)((kb / kNStages) & 1));
+        tc_fence_after();
+        const uint32_t aA = smem_u32(smem + (size_t)s * stage_bytes), aB = aA + kABytes;
 #pragma unroll
         for (int ks = 0; ks < kKB / 16; ++ks) {
           // A (MN-major): 16 channels = two 8-row atoms of 1024 B; the second 64-pixel atom kKB * 128 B further on.
           // A (kAK, K-major): like B — 16 channels = 32 bytes inside the swizzle row; 8-pixel groups 1024 B apart
-          const uint64_t ad = kAK ? desc_sw128(aA + ks * 32, 16, 1024) : desc_sw128(aA + ks * 2048, kKB * 128, 1024);
+          const uint64_t ad = kAK ? umma_desc(aA + ks * 32, 16, 1024, kSwizzle128B)
+                                  : umma_desc(aA + ks * 2048, kKB * 128, 1024, kSwizzle128B);
           // B (K-major): 16 k = 32 bytes inside the 128-byte swizzle row; 8-row groups 1024 B apart
-          const uint64_t bd = desc_sw128(aB + ks * 32, 16, 1024);
-          umma(tmem_d, ad, bd, idesc, (kb > 0 || ks > 0) ? 1u : 0u);
+          const uint64_t bd = umma_desc(aB + ks * 32, 16, 1024, kSwizzle128B);
+          umma_f16(tmem_d, ad, bd, idesc, (kb > 0 || ks > 0) ? 1u : 0u);
         }
         tc_commit(&empty[s]);
         if (kb == a.n_kb - 1) tc_commit(&acc_full);
@@ -217,8 +170,8 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
     // epilogue: warp w may touch TMEM lanes 32 (w % 4) .. + 31
     const int q = warp & 3;
     const long long p = p0 + q * 32 + lane;
-    bar_wait(&acc_full, 0);
-    tc_after();
+    mbar_wait(&acc_full, 0);
+    tc_fence_after();
     const int n0 = nz * NT;
     TO* ob = (TO*)a.out + ((long long)b * a.out_cstride + n0) * a.hw;  // planar output
     // 16 accumulator columns per TMEM load, two register sets: the load of the next 16 columns is in flight while the
@@ -228,17 +181,6 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
     n_eff = n_eff > NT ? NT : (n_eff + 15) & ~15;
     const uint32_t taddr = tmem_d + ((uint32_t)(q * 32) << 16);
     uint32_t ra[16], rb[16];
-#define MDSEG_H16_LD(R, C0)                                                                                            \
-  asm volatile(                                                                                                        \
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];" \
-      : "=r"(R[0]), "=r"(R[1]), "=r"(R[2]), "=r"(R[3]), "=r"(R[4]), "=r"(R[5]), "=r"(R[6]), "=r"(R[7]), "=r"(R[8]),      \
-        "=r"(R[9]), "=r"(R[10]), "=r"(R[11]), "=r"(R[12]), "=r"(R[13]), "=r"(R[14]), "=r"(R[15])                        \
-      : "r"(taddr + (uint32_t)(C0)))
-#define MDSEG_H16_WAIT(R)                                                                                              \
-  asm volatile("tcgen05.wait::ld.sync.aligned;"                                                                        \
-               : "+r"(R[0]), "+r"(R[1]), "+r"(R[2]), "+r"(R[3]), "+r"(R[4]), "+r"(R[5]), "+r"(R[6]), "+r"(R[7]),        \
-                 "+r"(R[8]), "+r"(R[9]), "+r"(R[10]), "+r"(R[11]), "+r"(R[12]), "+r"(R[13]), "+r"(R[14]), "+r"(R[15])   \
-               :: "memory")
 #define MDSEG_H16_ST(R, C0)                                                                                            \
   if constexpr (kOutPM) {                                                                                              \
     if (p < a.hw) {                                                                                                    \
@@ -261,25 +203,23 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_kernel(const __grid_con
       }                                                                                                                \
     }                                                                                                                  \
   }
-    if (n_eff > 0) MDSEG_H16_LD(ra, 0);
+    if (n_eff > 0) tmem_ld16(taddr, ra);
     for (int c0 = 0; c0 < n_eff; c0 += 32) {
-      MDSEG_H16_WAIT(ra);
+      tmem_wait_ld(ra);
       const bool has_b = c0 + 16 < n_eff;
-      if (has_b) MDSEG_H16_LD(rb, c0 + 16);
+      if (has_b) tmem_ld16(taddr + (uint32_t)(c0 + 16), rb);
       MDSEG_H16_ST(ra, c0);
       if (has_b) {
-        MDSEG_H16_WAIT(rb);
-        if (c0 + 32 < n_eff) MDSEG_H16_LD(ra, c0 + 32);
+        tmem_wait_ld(rb);
+        if (c0 + 32 < n_eff) tmem_ld16(taddr + (uint32_t)(c0 + 32), ra);
         MDSEG_H16_ST(rb, c0 + 16);
       }
     }
-#undef MDSEG_H16_LD
-#undef MDSEG_H16_WAIT
 #undef MDSEG_H16_ST
   }
-  tc_before();
+  tc_fence_before();
   __syncthreads();
-  if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "r"(tmem_cols) : "memory");
+  if (warp == 2) tmem_dealloc(tmem_d, tmem_cols);
 }
 
 // ---- d prototype: dW[n, k] = sum over images and pixels of dy[b, n, p] * feats[b, k, p] -------------------------
@@ -318,37 +258,36 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_dw_kernel(const __grid_
   while ((int)tmem_cols < NT) tmem_cols <<= 1;
 
   if (threadIdx.x == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&mapA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&mapB) : "memory");
-    for (int s = 0; s < kNStages; ++s) { bar_init(&full[s], 1); bar_init(&empty[s], 1); }
-    bar_init(&acc_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    prefetch_map(&mapA);
+    prefetch_map(&mapB);
+    for (int s = 0; s < kNStages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
+    mbar_init(&acc_full, 1);
+    mbar_fence_init();
   }
   if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sa(&tmem_base_s)), "r"(tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(&tmem_base_s, tmem_cols);
+    tmem_relinquish();
   }
-  tc_before();
+  tc_fence_before();
   __syncthreads();
-  tc_after();
+  tc_fence_after();
   const uint32_t tmem_d = tmem_base_s;
 
   if (warp == 0) {
     if (lane == 0) {
       for (int kb = 0; kb < n_kb; ++kb) {
         const int s = kb % kNStages;
-        if (kb >= kNStages) bar_wait(&empty[s], (uint32_t)((kb / kNStages - 1) & 1));
+        if (kb >= kNStages) mbar_wait(&empty[s], (uint32_t)((kb / kNStages - 1) & 1));
         unsigned char* st = smem + (size_t)s * stage_bytes;
-        bar_expect(&full[s], stage_bytes);
+        mbar_expect_tx(&full[s], stage_bytes);
         // pixels beyond the slab but inside the image would be counted twice: slabs are whole 64-pixel chunks, and
         // pixels beyond the image are zero-filled by TMA
-        tma3(st, &mapA, &full[s], (int)(p_beg + (long long)kb * 64), mt * 128, b);
+        load_3d(st, &mapA, &full[s], (int)(p_beg + (long long)kb * 64), mt * 128, b);
         if constexpr (kBMN) {
           for (int j = 0; j < n_boxes; ++j)
-            tma3(st + a_bytes + j * 8192, &mapB, &full[s], nt * NT + 64 * j, (int)(p_beg + (long long)kb * 64), b);
+            load_3d(st + a_bytes + j * 8192, &mapB, &full[s], nt * NT + 64 * j, (int)(p_beg + (long long)kb * 64), b);
         } else {
-          tma3(st + a_bytes, &mapB, &full[s], (int)(p_beg + (long long)kb * 64), nt * NT, b);
+          load_3d(st + a_bytes, &mapB, &full[s], (int)(p_beg + (long long)kb * 64), nt * NT, b);
         }
       }
     }
@@ -359,15 +298,16 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_dw_kernel(const __grid_
                              ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(kM >> 4) << 24);
       for (int kb = 0; kb < n_kb; ++kb) {
         const int s = kb % kNStages;
-        bar_wait(&full[s], (uint32_t)((kb / kNStages) & 1));
-        tc_after();
-        const uint32_t aA = sa(smem + (size_t)s * stage_bytes), aB = aA + a_bytes;
+        mbar_wait(&full[s], (uint32_t)((kb / kNStages) & 1));
+        tc_fence_after();
+        const uint32_t aA = smem_u32(smem + (size_t)s * stage_bytes), aB = aA + a_bytes;
 #pragma unroll
         for (int ks = 0; ks < 4; ++ks)
           // kBMN: 16 pixels = two 8-row atoms of 1024 B; the next 64-channel atom one 8 KB box further on
-          umma(tmem_d, desc_sw128(aA + ks * 32, 16, 1024),
-               kBMN ? desc_sw128(aB + ks * 2048, 64 * 128, 1024) : desc_sw128(aB + ks * 32, 16, 1024), idesc,
-               (kb > 0 || ks > 0) ? 1u : 0u);
+          umma_f16(tmem_d, umma_desc(aA + ks * 32, 16, 1024, kSwizzle128B),
+                   kBMN ? umma_desc(aB + ks * 2048, 64 * 128, 1024, kSwizzle128B)
+                        : umma_desc(aB + ks * 32, 16, 1024, kSwizzle128B),
+                   idesc, (kb > 0 || ks > 0) ? 1u : 0u);
         tc_commit(&empty[s]);
         if (kb == n_kb - 1) tc_commit(&acc_full);
       }
@@ -375,25 +315,21 @@ __global__ void __launch_bounds__(kThreads, 2) head_tc16_dw_kernel(const __grid_
   } else {
     const int q = warp & 3;
     const int row = q * 32 + lane;
-    bar_wait(&acc_full, 0);
-    tc_after();
+    mbar_wait(&acc_full, 0);
+    tc_fence_after();
     float* slot = a.part + ((((long long)slab_id * a.m_tiles + mt) * a.n_tiles + nt) * 128 + row) * NT;
     for (int c0 = 0; c0 < NT; c0 += 16) {
       uint32_t r[16];
-      asm volatile(
-          "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-          : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-            "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-          : "r"(tmem_d + ((uint32_t)(q * 32) << 16) + (uint32_t)c0));
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+      tmem_ld16(tmem_d + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, r);
+      tmem_wait_ld();
       uint4* o = reinterpret_cast<uint4*>(slot + c0);
 #pragma unroll
       for (int i = 0; i < 4; ++i) o[i] = make_uint4(r[4 * i], r[4 * i + 1], r[4 * i + 2], r[4 * i + 3]);
     }
   }
-  tc_before();
+  tc_fence_before();
   __syncthreads();
-  if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "r"(tmem_cols) : "memory");
+  if (warp == 2) tmem_dealloc(tmem_d, tmem_cols);
 }
 
 // dataset_ids == NULL: one sum over every slab -> dW [N, K].  Otherwise blockIdx.y is a dataset and only the slabs of
@@ -437,7 +373,7 @@ extern "C" int mdseg_head_tc16_tile(int N) {
 namespace mdseg {
 namespace {
 template <typename TO, bool kAK, bool kOutPM>
-int launch_head16_kernel(const CUtensorMap& mapA, const BMaps& mapsB, const HeadArgs& a, dim3 grid, size_t smem,
+int launch_head16_kernel(const CUtensorMap& mapA, const Maps& mapsB, const HeadArgs& a, dim3 grid, size_t smem,
                          cudaStream_t s) {
   auto k = head_tc16_kernel<TO, kAK, kOutPM>;
   MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -481,7 +417,7 @@ int launch_head16(const void* x, int dtype, int n_images, int K, int64_t hw, con
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     MDSEG_REQUIRE(r == CUDA_SUCCESS, "%s: cuTensorMapEncodeTiled failed for the A operand (CUresult %d)", who, (int)r);
   }
-  BMaps mapsB;
+  Maps mapsB;
   HeadArgs a;
   a.out = out; a.hw = hw; a.dataset_ids = dataset_ids; a.n_datasets = n_b; a.out_cstride = out_cstride;
   a.n_kb = (K + kKB - 1) / kKB;

@@ -47,22 +47,6 @@ constexpr int kStgW28 = 160;                    // one-warp CTAs: staged label c
 constexpr int kMaxR = 5;
 constexpr int kEnt = 384;                       // (class, output channel) pairs of one class group cached in shared memory
 constexpr uint32_t kNoEnt = 0xffffffffu;
-#ifndef MDSEG_BWD_BCAST_PIPE
-#define MDSEG_BWD_BCAST_PIPE 1
-#endif
-// timing experiments only (wrong results when set): lite warps do not load their fifth-column sums / no fifth column
-#ifndef MDSEG_BWD_XP_NOLD
-#define MDSEG_BWD_XP_NOLD 0
-#endif
-#ifndef MDSEG_BWD_XP_NOUSE
-#define MDSEG_BWD_XP_NOUSE 0
-#endif
-#ifndef MDSEG_BWD_XP_NO5
-#define MDSEG_BWD_XP_NO5 0
-#endif
-#ifndef MDSEG_BWD_CHUNK_LEAN
-#define MDSEG_BWD_CHUNK_LEAN 1
-#endif
 
 // Shared-memory carve-up of ONE warp.  ROW = false: a CTA is one warp owning 28 columns (lane 0 recomputes the halo cell
 // of the strip on its left).  ROW = true: a CTA is the w / 32 warps of a whole low-res row, every lane owns a cell AND a
@@ -129,13 +113,6 @@ struct Args {
   int c_scr;
   int seg_rows, n_seg, n_strips;
 };
-
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
 
 // predicated 8-byte shared-memory store (one instruction; an `if` costs a divergent branch around the address code)
 __device__ __forceinline__ void sts2_if(uint32_t on, uint32_t addr, float a, float b) {
@@ -247,7 +224,6 @@ __device__ __forceinline__ void broadcast_chunk(const Unit& un, TO* orow, const 
   const bool col_ok = 4 * t < un.ncols;
   TO* base = orow + 4 * t;
   asm volatile("" : "+l"(base));
-#if MDSEG_BWD_BCAST_PIPE
   // four quads per round: all entry loads first, then the tile rows, then the stores — the round's shared-memory
   // latencies overlap instead of serialising load -> test -> load -> store four times
   int q = q0;
@@ -269,16 +245,6 @@ __device__ __forceinline__ void broadcast_chunk(const Unit& un, TO* orow, const 
       store4(base + (int64_t)((e & 0xffffu) * (uint32_t)hw), v);
     }
   }
-#else
-#pragma unroll 4
-  for (int q = q0; q < q1; ++q) {
-    const uint32_t e = ents[4 * q + o];
-    if (col_ok && e != kNoEnt) {
-      const float4 v = *reinterpret_cast<const float4*>(tile + (e >> 16) * OWN + 4 * t);
-      store4(base + (int64_t)((e & 0xffffu) * (uint32_t)hw), v);
-    }
-  }
-#endif
   __syncwarp();
 }
 
@@ -430,7 +396,7 @@ __device__ __forceinline__ void cell_row(const Args& a, const CUtensorMap* map, 
       Sp += 2 * kBoxW;
       if (c + 1 < cc) { n00 = Sp[0]; n01 = Sp[1]; n10 = Sp[kBoxW]; n11 = Sp[kBoxW + 1]; }
       float2 x5 = make_float2(0.f, 0.f);
-      if (!NX5 && un.has5 && !MDSEG_BWD_XP_NOLD && !MDSEG_BWD_XP_NOUSE) x5 = x5p[c];
+      if (!NX5 && un.has5) x5 = x5p[c];
       const float dv0 = v01 - v00, dv1 = v11 - v10;
       const float2 V0 = dup2(v00), DV0 = dup2(dv0), V1 = dup2(v10), DV1 = dup2(dv1);
       float2 CU2, UR2, CL2, LR2;
@@ -522,12 +488,8 @@ __device__ __forceinline__ void cell_row(const Args& a, const CUtensorMap* map, 
     __syncwarp();
     if (lane == 0 && q + kStages < un.n_loads) {  // the slot is free: every lane has read its corners
       const int qn = q + kStages;
-#if MDSEG_BWD_CHUNK_LEAN
       // a class group is one or two chunks (kCG == 2 kKC): no integer division
       const int qrow = un.n_ch == 2 ? qn >> 1 : qn, qk = un.n_ch == 2 ? qn & 1 : 0;
-#else
-      const int qrow = qn / un.n_ch, qk = qn % un.n_ch;
-#endif
       mbar_expect_tx(&bars[slot], kStageBytes + (un.c5base ? kKC * 8 : 0));
       load_4d(stages + slot * kStageFloats, map, &bars[slot], un.box_x, un.g0 + qrow, un.c_beg + qk * kKC, un.b);
       if (un.c5base)
@@ -611,7 +573,7 @@ mds_bwd_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Args a
   // fifth pixel columns: none / one lane of a row-CTA warp (sums precomputed, see cell_row) / anything else (class loop)
   const int n5 = __popc(__ballot_sync(0xffffffffu, nx > 4));
   const bool lite = ROW && a.col5 != nullptr && n5 == 1 && ((a.lite_mask >> strip) & 1u);
-  const bool nx5 = n5 > 0 && !lite && !MDSEG_BWD_XP_NO5;
+  const bool nx5 = n5 > 0 && !lite;
 
   Unit un;
   un.lane = lane; un.b = b; un.seg = seg; un.x = x; un.nx = nx; un.c_beg = c_beg; un.c_end = c_end;
@@ -627,9 +589,9 @@ mds_bwd_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Args a
   un.w_signed = wsel; un.wsign = wsel < 0.f ? -1.f : 1.f;
   un.log2w = log2f(fabsf(wsel));  // -inf when nothing is selected or the incoming gradient is 0: every term vanishes
   un.cached = false;
-  un.has5 = lite && nx > 4 && !MDSEG_BWD_XP_NO5;
+  un.has5 = lite && nx > 4;
   un.c5base = nullptr; un.c5row = 0;
-  if (lite && !MDSEG_BWD_XP_NO5 && !MDSEG_BWD_XP_NOLD) {
+  if (lite) {
     un.c5row = (int64_t)(w / 32) * a.c5s;
     un.c5base = a.col5 + ((int64_t)b * (h - 1) * (w / 32) + strip) * a.c5s + c_beg;
   }

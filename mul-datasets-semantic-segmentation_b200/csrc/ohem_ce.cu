@@ -16,7 +16,7 @@
 // Algorithmic bytes per pixel (fwd + bwd): 3*C*e + 2*L + 16 (+4 in select).
 #include <float.h>
 
-#include "common.cuh"
+#include "tma_util.cuh"
 
 namespace mdseg {
 namespace {
@@ -273,24 +273,10 @@ ce_bwd_nhwc_kernel(const T* __restrict__ logits, const L* __restrict__ labels, i
 constexpr int kTileThreads = MDSEG_TILE_THREADS;
 constexpr int kTileStageBytes = 100 * 1024;
 
-__device__ __forceinline__ uint32_t smem_u32a(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void tile_bar_init(uint64_t* b) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32a(b)));
-}
-__device__ __forceinline__ void tile_bar_wait(uint64_t* b, uint32_t parity) {
-  asm volatile(
-      "{\n.reg .pred p;\nMDSEG_TL_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra MDSEG_TL_DONE;\nbra MDSEG_TL_WAIT;\nMDSEG_TL_DONE:\n}\n" ::"r"(smem_u32a(b)),
-      "r"(parity)
-      : "memory");
-}
+// one tile of `bytes` global -> shared, completion on `bar`
 __device__ __forceinline__ void tile_load(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32a(bar)), "r"(bytes) : "memory");
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_u32a(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32a(bar))
-               : "memory");
+  tma::mbar_expect_tx(bar, bytes);
+  tma::bulk_g2s(dst, src, bytes, bar);
 }
 
 // pixels per tile for C channels of `esz` bytes, so that the tile fills (at most) one stage: a multiple of the CTA size
@@ -324,9 +310,9 @@ ce_nhwc_tile_kernel(const T* __restrict__ logits, const L* __restrict__ labels, 
   int err = 0;
 
   if (threadIdx.x == 0) {
-    tile_bar_init(&bars[0]);
-    tile_bar_init(&bars[1]);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    tma::mbar_init(&bars[0], 1);
+    tma::mbar_init(&bars[1], 1);
+    tma::mbar_fence_init();
     if ((int64_t)blockIdx.x < n_tiles)
       tile_load(tile_smem, logits + (int64_t)blockIdx.x * TP * C, tile_bytes, &bars[0]);
   }
@@ -341,7 +327,7 @@ ce_nhwc_tile_kernel(const T* __restrict__ logits, const L* __restrict__ labels, 
       if (BWD) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
       tile_load(tile_smem + (size_t)(s ^ 1) * stage_stride, logits + (tile + gridDim.x) * TP * C, tile_bytes, &bars[s ^ 1]);
     }
-    tile_bar_wait(&bars[s], (uint32_t)((it >> 1) & 1));
+    tma::mbar_wait(&bars[s], (uint32_t)((it >> 1) & 1));
     for (int j = 0; j < ppt; ++j) {
     const int px = threadIdx.x / tpc + j * kTileThreads;
     const int rot = rotate ? px % C : 0;
@@ -399,7 +385,7 @@ ce_nhwc_tile_kernel(const T* __restrict__ logits, const L* __restrict__ labels, 
       __syncthreads();
       if (threadIdx.x == 0) {
         asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dlogits + tile * TP * C),
-                     "r"(smem_u32a(buf)), "r"(tile_bytes)
+                     "r"(tma::smem_u32(buf)), "r"(tile_bytes)
                      : "memory");
         asm volatile("cp.async.bulk.commit_group;" ::: "memory");
       }

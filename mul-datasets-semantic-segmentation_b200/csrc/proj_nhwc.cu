@@ -14,7 +14,7 @@
 //  * aux heads: a gather-transpose packs the rows of each head's own images into one planar buffer in the source
 //    dtype (what mdseg_up_ce_fwd reads), and a scatter-transpose writes the gradient rows back into every head's NHWC
 //    gradient, zeros for the images of other datasets.
-#include "common.cuh"
+#include "tma_util.cuh"
 
 namespace mdseg {
 namespace {
@@ -22,8 +22,6 @@ namespace {
 constexpr int kThreads = 256;
 constexpr int kTileBytesPerChannel = 128;  // TP * sizeof(T): 32 fp32 pixels or 64 16-bit pixels per tile
 constexpr int kBwdTP = 64;                 // pixels per backward tile
-
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 // ---------------------------------------------------------------------------
 // forward: one CTA = TP pixels of one image; warp w computes the dataset classes n = w, w + 8, ...
@@ -52,21 +50,13 @@ proj_fwd_nhwc_kernel(const T* __restrict__ x, const mdseg_graph_table tab, const
   T* xs = reinterpret_cast<T*>(smem);
   if ((((uintptr_t)src | bytes) & 15) == 0) {
     if (threadIdx.x == 0) {
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(&bar)));
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(&bar)), "r"(bytes)
-                   : "memory");
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                       smem_addr(xs)),
-                   "l"(src), "r"(bytes), "r"(smem_addr(&bar))
-                   : "memory");
+      tma::mbar_init(&bar, 1);
+      tma::mbar_fence_init();
+      tma::mbar_expect_tx(&bar, bytes);
+      tma::bulk_g2s(xs, src, bytes, &bar);
     }
     __syncthreads();  // the barrier is initialised before anyone polls it
-    asm volatile(
-        "{\n.reg .pred p;\nMDSEG_PN_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], 0;\n"
-        "@p bra MDSEG_PN_DONE;\nbra MDSEG_PN_WAIT;\nMDSEG_PN_DONE:\n}\n" ::"r"(smem_addr(&bar))
-        : "memory");
+    tma::mbar_wait(&bar, 0);
   } else {  // odd C_uni * e, a storage offset or an unaligned image start: plain element copies into the same layout
     for (int e = threadIdx.x; e < np * Cu; e += kThreads) xs[e] = src[e];
     __syncthreads();

@@ -19,7 +19,7 @@
 // products of weight >= 2^-16 are accumulated (relative error ~2^-21, inside the 1e-5 parity bar without
 // giving up fp32's range); bf16 / fp16 inputs take ONE product in their own type, G rounded to it — what
 // autocast does to the reference einsum.
-#include "common.cuh"
+#include "tma_util.cuh"
 
 namespace mdseg {
 // proj.cu: the same projection without the tensor-core datasets (bit d of skip_mask = dataset d is handled here)
@@ -28,6 +28,8 @@ int proj_fwd_rest(const void* x, int dtype, const mdseg_graph_table* graphs, con
                   cudaStream_t s);
 
 namespace {
+
+using namespace tma;
 
 constexpr int kTM = 128;      // pixels per tile = UMMA M
 constexpr int kKB = 32;       // channels per shared-memory stage (two K = 16 MMA steps)
@@ -61,83 +63,17 @@ struct TcArgs {
   int n_tiles_f[MDSEG_MAX_DATASETS];
 };
 
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// ---- mbarrier / bulk copy -----------------------------------------------------------------------------
-__device__ __forceinline__ void bar_init(uint64_t* b, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(b)), "r"(count));
-}
-__device__ __forceinline__ void bar_expect_tx(uint64_t* b, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(b)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bar_wait(uint64_t* b, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "MDSEG_TC_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra MDSEG_TC_DONE;\n"
-      "bra MDSEG_TC_WAIT;\n"
-      "MDSEG_TC_DONE:\n"
-      "}\n" ::"r"(smem_addr(b)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_addr(dst)),
-               "l"(src), "r"(bytes), "r"(smem_addr(bar))
-               : "memory");
-}
-
-// ---- tcgen05 ------------------------------------------------------------------------------------------
-__device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(dst_smem)), "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_addr(bar))
-               : "memory");
-}
-// D[tmem] (+)= A[smem desc] * B[smem desc]^T, 16-bit inputs, fp32 accumulate
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accum) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
-      : "memory");
-}
 // 16 consecutive fp32 columns of this thread's TMEM lane
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
+__device__ __forceinline__ void tmem_ld16_f32(uint32_t taddr, float (&v)[16]) {
   uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld16(taddr, r);
+  tmem_wait_ld();
 #pragma unroll
   for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
 }
 
-// Shared-memory matrix descriptor, K-major, no swizzle (cute::UMMA::SmemDescriptor, version 1):
-// core matrix = 8 rows x 16 bytes stored contiguously; `sbo` = bytes between 8-row groups (M / N direction),
-// `lbo` = bytes between the core matrices adjacent in K.
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  return (uint64_t)((saddr & 0x3ffffu) >> 4) | ((uint64_t)((lbo >> 4) & 0x3fffu) << 16) |
-         ((uint64_t)((sbo >> 4) & 0x3fffu) << 32) | (1ull << 46);
-}
+// Operands are K-major without swizzle (umma_desc kNoSwizzle): a core matrix is 8 rows x 16 bytes stored contiguously,
+// `sbo` steps between 8-row groups (M / N direction), `lbo` between the core matrices adjacent in K.
 // Instruction descriptor (cute::UMMA::InstrDescriptor): fp32 accumulate, A and B K-major, M = 128
 __device__ __forceinline__ uint32_t umma_idesc(int fmt, int n) {
   return (1u << 4) | ((uint32_t)fmt << 7) | ((uint32_t)fmt << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(kTM >> 4) << 24);
@@ -275,9 +211,9 @@ __global__ void __launch_bounds__(kTcThreads, kBwd ? 4 : 2) proj_tc_kernel(const
   while ((int)tmem_cols < npad) tmem_cols <<= 1;
 
   if (tid == 0) {
-    for (int s = 0; s < kNS; ++s) { bar_init(&bar_b[s], 1); bar_init(&bar_mma[s], 1); }
-    bar_init(&bar_acc, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < kNS; ++s) { mbar_init(&bar_b[s], 1); mbar_init(&bar_mma[s], 1); }
+    mbar_init(&bar_acc, 1);
+    mbar_fence_init();
   }
   if (warp == 0) {
     tmem_alloc(&tmem_base_s, tmem_cols);
@@ -324,12 +260,12 @@ __global__ void __launch_bounds__(kTcThreads, kBwd ? 4 : 2) proj_tc_kernel(const
     for (int j = 0; j < kKB / 2; ++j) v[j] = vn[j];
     if (kc + 1 < n_chunks) load_chunk(kc + 1);
     // the MMAs of chunk kc - kStages have finished reading stage s
-    if (kc >= kNS) bar_wait(&bar_mma[s], (use - 1) & 1u);
+    if (kc >= kNS) mbar_wait(&bar_mma[s], (use - 1) & 1u);
     unsigned char* stA = sA + (size_t)s * a.a_stage_bytes;
     unsigned char* stB = sB + (size_t)s * a.b_stage_bytes;
     if (tid == 0) {
-      bar_expect_tx(&bar_b[s], b_chunk_bytes);
-      bulk_load(stB, gchunks + (size_t)kc * b_chunk_bytes, b_chunk_bytes, &bar_b[s]);
+      mbar_expect_tx(&bar_b[s], b_chunk_bytes);
+      bulk_g2s(stB, gchunks + (size_t)kc * b_chunk_bytes, b_chunk_bytes, &bar_b[s]);
     }
     // A: this thread's pixel, 16 channels -> TERMS x 2 k-groups x 16 bytes
 #pragma unroll
@@ -352,9 +288,9 @@ __global__ void __launch_bounds__(kTcThreads, kBwd ? 4 : 2) proj_tc_kernel(const
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     __syncthreads();
     if (tid == 0) {
-      bar_wait(&bar_b[s], use & 1u);
+      mbar_wait(&bar_b[s], use & 1u);
       tc_fence_after();
-      const uint32_t aA = smem_addr(stA), aB = smem_addr(stB);
+      const uint32_t aA = smem_u32(stA), aB = smem_u32(stB);
 #pragma unroll
       for (int ks = 0; ks < kKB / 16; ++ks) {
         // products in order of decreasing weight; TERMS == 1: just (0, 0)
@@ -363,8 +299,8 @@ __global__ void __launch_bounds__(kTcThreads, kBwd ? 4 : 2) proj_tc_kernel(const
         const int tb[6] = {0, 1, 0, 1, 2, 0};
 #pragma unroll
         for (int q = 0; q < kPairs; ++q) {
-          const uint64_t ad = umma_desc(aA + ta[q] * (4 * kTM * 16) + ks * 2 * (kTM * 16), kTM * 16, 128);
-          const uint64_t bd = umma_desc(aB + tb[q] * (npad * 64) + ks * 2 * (npad * 16), npad * 16, 128);
+          const uint64_t ad = umma_desc(aA + ta[q] * (4 * kTM * 16) + ks * 2 * (kTM * 16), kTM * 16, 128, kNoSwizzle);
+          const uint64_t bd = umma_desc(aB + tb[q] * (npad * 64) + ks * 2 * (npad * 16), npad * 16, 128, kNoSwizzle);
           umma_f16(tmem_d, ad, bd, idesc, (kc > 0 || ks > 0 || q > 0) ? 1u : 0u);
         }
       }
@@ -375,13 +311,13 @@ __global__ void __launch_bounds__(kTcThreads, kBwd ? 4 : 2) proj_tc_kernel(const
 
   // epilogue: warp w reads TMEM lanes 32(w % 4) .. +31 (= pixels of this tile); the two warps that share a lane
   // quarter take alternate groups of 16 columns
-  bar_wait(&bar_acc, 0);
+  mbar_wait(&bar_acc, 0);
   tc_fence_after();
   float* yb = kBwd ? nullptr : a.y + ((long long)b * a.y_cmax + u0) * a.hw;
   T* dxb = kBwd ? (T*)a.dx + ((long long)b * a.C_uni + u0) * a.hw : nullptr;
   for (int n0 = (warp >> 2) * 16; n0 < npad; n0 += 32) {
     float acc[16];
-    tmem_ld16(tmem_d + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)n0, acc);
+    tmem_ld16_f32(tmem_d + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)n0, acc);
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
       if (p_ok && n0 + i < n_out) {
@@ -647,9 +583,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) proj_tc_dgraph_kernel(const __g
   while ((int)tmem_cols < npad) tmem_cols <<= 1;
 
   if (tid == 0) {
-    for (int s = 0; s < kStagesTc; ++s) bar_init(&bar_mma[s], 1);
-    bar_init(&bar_acc, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < kStagesTc; ++s) mbar_init(&bar_mma[s], 1);
+    mbar_init(&bar_acc, 1);
+    mbar_fence_init();
   }
   if (warp == 0) {
     tmem_alloc(&tmem_base_s, tmem_cols);
@@ -746,7 +682,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) proj_tc_dgraph_kernel(const __g
 #pragma unroll
       for (int j = 0; j < kDgItems; ++j) load8(j, kc + 1, vn[j]);
     }
-    if (kc >= kStagesTc) bar_wait(&bar_mma[s], (use - 1) & 1u);
+    if (kc >= kStagesTc) mbar_wait(&bar_mma[s], (use - 1) & 1u);
     unsigned char* stA = sA + (size_t)s * a.a_stage_bytes;
     unsigned char* stB = sB + (size_t)s * a.b_stage_bytes;
 #pragma unroll
@@ -772,7 +708,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) proj_tc_dgraph_kernel(const __g
     __syncthreads();
     if (tid == 0) {
       tc_fence_after();
-      const uint32_t aA = smem_addr(stA), aB = smem_addr(stB);
+      const uint32_t aA = smem_u32(stA), aB = smem_u32(stB);
       for (int jn = 0; jn < n_tiles_n; ++jn) {
         const int col0 = jn * nt_n;
         const int nn = (npad - col0) < nt_n ? (npad - col0) : nt_n;
@@ -784,8 +720,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) proj_tc_dgraph_kernel(const __g
           const int tb[6] = {0, 1, 0, 1, 2, 0};
 #pragma unroll
           for (int q = 0; q < kPairs; ++q) {
-            const uint64_t ad = umma_desc(aA + ta[q] * (4 * kDgM * 16) + ks * 2 * (kDgM * 16), kDgM * 16, 128);
-            const uint64_t bd = umma_desc(aB + tb[q] * (4 * npad * 16) + ks * 2 * (npad * 16) + col0 * 16, npad * 16, 128);
+            const uint64_t ad = umma_desc(aA + ta[q] * (4 * kDgM * 16) + ks * 2 * (kDgM * 16), kDgM * 16, 128, kNoSwizzle);
+            const uint64_t bd =
+                umma_desc(aB + tb[q] * (4 * npad * 16) + ks * 2 * (npad * 16) + col0 * 16, npad * 16, 128, kNoSwizzle);
             umma_f16(tmem_d + (uint32_t)col0, ad, bd, idesc, (kc > 0 || ks > 0 || q > 0) ? 1u : 0u);
           }
         }
@@ -796,13 +733,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) proj_tc_dgraph_kernel(const __g
   }
 
   // epilogue: TMEM lane = class row of the M tile, columns = unified channels -> this CTA's slot of the workspace
-  bar_wait(&bar_acc, 0);
+  mbar_wait(&bar_acc, 0);
   tc_fence_after();
   float* slot = a.part + ((((long long)b * a.n_mt + mt) * a.n_nt + nz) * a.n_slabs + sl) * (long long)kDgM * npad;
   const int row = (warp & 3) * 32 + (tid & 31);
   for (int c0 = (warp >> 2) * 16; c0 < npad; c0 += 32) {
     float acc[16];
-    tmem_ld16(tmem_d + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)c0, acc);
+    tmem_ld16_f32(tmem_d + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)c0, acc);
     float4* o = reinterpret_cast<float4*>(slot + (long long)row * npad + c0);
 #pragma unroll
     for (int i = 0; i < 4; ++i) o[i] = make_float4(acc[4 * i], acc[4 * i + 1], acc[4 * i + 2], acc[4 * i + 3]);

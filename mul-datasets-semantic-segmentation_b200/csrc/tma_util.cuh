@@ -1,6 +1,6 @@
-// tma_util.cuh — mbarrier / TMA (cp.async.bulk.tensor) PTX wrappers, packed-fp32 (FFMA2/FADD2)
-// helpers and the host-side tensor-map builder shared by the warp-private fused kernels
-// (up_ce_warp.cu, mds_bwd.cu).  sm_100a only.
+// tma_util.cuh — the one copy of the mbarrier, bulk-copy, TMA (cp.async.bulk.tensor) and tcgen05 PTX wrappers every
+// kernel file uses, packed-fp32 (FFMA2/FADD2) helpers and the host-side tensor-map builder of the warp-private fused
+// kernels (up_ce_warp.cu, mds_bwd.cu).  sm_100a only.
 #pragma once
 
 #include <cuda.h>
@@ -39,7 +39,26 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       "r"(parity)
       : "memory");
 }
-// 4-D tiled load global -> shared, completion on an mbarrier.  Coordinates innermost first.
+// 1-D bulk copy global -> shared, completion on an mbarrier (addresses and size multiples of 16 bytes)
+__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                   smem_u32(dst)),
+               "l"(src), "r"(bytes), "r"(smem_u32(bar))
+               : "memory");
+}
+// tiled loads global -> shared, completion on an mbarrier.  Coordinates innermost first.
+__device__ __forceinline__ void load_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
+  asm volatile(
+      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
+      : "memory");
+}
+__device__ __forceinline__ void load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
+      : "memory");
+}
 __device__ __forceinline__ void load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2,
                                         int c3) {
   asm volatile(
@@ -49,6 +68,60 @@ __device__ __forceinline__ void load_4d(void* dst, const CUtensorMap* map, uint6
 }
 __device__ __forceinline__ void prefetch_map(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)map) : "memory");
+}
+
+// ---- tcgen05 (one CTA, cta_group::1) ----
+__device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols)
+               : "memory");
+}
+__device__ __forceinline__ void tmem_relinquish() {
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// arrive on `bar` when every MMA issued so far by this thread has retired
+__device__ __forceinline__ void tc_commit(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
+               : "memory");
+}
+// D[tmem] (+)= A[smem desc] * B[smem desc]^T, 16-bit inputs, fp32 accumulate
+__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accum) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
+      : "memory");
+}
+// 16 consecutive 32-bit columns of this thread's TMEM lane.  The registers are valid only after a tmem_wait_ld.
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr));
+}
+// wait for this thread's outstanding TMEM loads
+__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// the same wait, naming the registers it releases, so that the compiler cannot move a use of r above it
+__device__ __forceinline__ void tmem_wait_ld(uint32_t (&r)[16]) {
+  asm volatile("tcgen05.wait::ld.sync.aligned;"
+               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
+                 "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
+               :: "memory");
+}
+// Shared-memory matrix descriptor (cute::UMMA::SmemDescriptor, version 1).  `sbo` = bytes between 8-row groups,
+// `lbo` = bytes between the core matrices adjacent in the leading dimension.
+enum UmmaLayout : uint64_t { kNoSwizzle = 0, kSwizzle128B = 2 };
+__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo, UmmaLayout layout) {
+  return (uint64_t)((saddr & 0x3ffffu) >> 4) | ((uint64_t)((lbo >> 4) & 0x3fffu) << 16) |
+         ((uint64_t)((sbo >> 4) & 0x3fffu) << 32) | (1ull << 46) | ((uint64_t)layout << 61);
 }
 
 // ---- packed fp32 pairs: one issue slot for two lanes of work (FFMA2 / FADD2 / FMUL2 on sm_100) ----

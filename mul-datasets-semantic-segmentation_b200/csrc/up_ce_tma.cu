@@ -31,6 +31,8 @@
 namespace mdseg {
 namespace {
 
+using namespace tma;
+
 constexpr int kT = 128;        // threads per CTA
 constexpr int kNW = kT / 32;   // warps
 constexpr int kBoxW = 132;     // staged columns per row (528 B, multiple of 16)
@@ -42,40 +44,6 @@ constexpr int kBwdStages = 2;
 constexpr int kMaxR = 5, kMaxNX = 5;
 constexpr int kRowBuf = 32 * kMaxNX;  // label columns covered by one warp
 constexpr int kOwnPerWarp = 31;       // backward: lane 0 of every warp is a halo cell
-
-struct alignas(64) TmaMaps {
-  CUtensorMap m[MDSEG_MAX_DATASETS];
-};
-
-// ---- PTX wrappers ---------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "MDSEG_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra MDSEG_DONE;\n"
-      "bra MDSEG_WAIT;\n"
-      "MDSEG_DONE:\n"
-      "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2,
-                                            int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
 
 // ---- per-warp staging of labels / per-pixel floats -------------------------------------------
 // lab_w[j*kRowBuf + k] = label of pixel (Yb+j, Xw0+k) as a byte; 255 = ignored or invalid.
@@ -180,7 +148,7 @@ __device__ __forceinline__ void fwd_tile(const FwdArgs& a, const CUtensorMap* ma
     __syncthreads();  // everyone is done with this slot
     if (threadIdx.x == 0 && k + kFwdStages < n_chunks) {
       mbar_expect_tx(&bars[slot], kStageBytes);
-      tma_load_4d(stages + slot * kStageFloats, map, &bars[slot], xa, g, (k + kFwdStages) * kKC, b);
+      load_4d(stages + slot * kStageFloats, map, &bars[slot], xa, g, (k + kFwdStages) * kKC, b);
     }
   }
 
@@ -214,7 +182,7 @@ __device__ __forceinline__ void fwd_tile(const FwdArgs& a, const CUtensorMap* ma
 
 template <typename L>
 __global__ void __launch_bounds__(kT)
-up_ce_fwd_tma_kernel(const __grid_constant__ TmaMaps maps, const FwdArgs a) {
+up_ce_fwd_tma_kernel(const __grid_constant__ Maps maps, const FwdArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const Geom& gm = a.gm;
   const int b = blockIdx.z, g = blockIdx.y;
@@ -269,7 +237,7 @@ up_ce_fwd_tma_kernel(const __grid_constant__ TmaMaps maps, const FwdArgs a) {
     mbar_fence_init();
     for (int s = 0; s < kFwdStages && s < n_chunks; ++s) {
       mbar_expect_tx(&bars[s], kStageBytes);
-      tma_load_4d(stages + s * kStageFloats, map, &bars[s], xa, g, s * kKC, b);
+      load_4d(stages + s * kStageFloats, map, &bars[s], xa, g, s * kKC, b);
     }
   }
   // channel maxima of the two rows (zero outside the image, matching the TMA zero fill)
@@ -453,7 +421,7 @@ __device__ __forceinline__ void bwd_tile(const BwdArgs& a, const CUtensorMap* ma
     __syncthreads();  // slot and O tile free
     if (threadIdx.x == 0 && k + kBwdStages < n_chunks) {
       mbar_expect_tx(&bars[slot], kStageBytes);
-      tma_load_4d(stages + slot * kStageFloats, map, &bars[slot], box_x0, g, (k + kBwdStages) * kKC, b);
+      load_4d(stages + slot * kStageFloats, map, &bars[slot], box_x0, g, (k + kBwdStages) * kKC, b);
     }
   }
   (void)x_end;
@@ -461,7 +429,7 @@ __device__ __forceinline__ void bwd_tile(const BwdArgs& a, const CUtensorMap* ma
 
 template <typename L>
 __global__ void __launch_bounds__(kT)
-up_ce_bwd_tma_kernel(const __grid_constant__ TmaMaps maps, const BwdArgs a) {
+up_ce_bwd_tma_kernel(const __grid_constant__ Maps maps, const BwdArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const Geom& gm = a.gm;
   const int b = blockIdx.z, g = blockIdx.y;
@@ -532,7 +500,7 @@ up_ce_bwd_tma_kernel(const __grid_constant__ TmaMaps maps, const BwdArgs a) {
     mbar_fence_init();
     for (int s = 0; s < kBwdStages && s < n_chunks; ++s) {
       mbar_expect_tx(&bars[s], kStageBytes);
-      tma_load_4d(stages + s * kStageFloats, map, &bars[s], box_x0, g, s * kKC, b);
+      load_4d(stages + s * kStageFloats, map, &bars[s], box_x0, g, s * kKC, b);
     }
   }
   int err = 0;
@@ -587,33 +555,13 @@ bool tma_applicable(const mdseg_src_table& src, const Geom& gm) {
   return tma::encode_fn() != nullptr;
 }
 
-int make_maps(const mdseg_src_table& src, const Geom& gm, int n_images, TmaMaps* out) {
-  tma::EncodeTiledFn enc = tma::encode_fn();
-  if (int rc = tma::bind_primary_context()) return rc;
-  for (int i = 0; i < src.n_datasets; ++i) {
-    const int calloc = src.C_alloc[i] > 0 ? src.C_alloc[i] : src.C[i];
-    cuuint64_t dims[4] = {(cuuint64_t)gm.w, (cuuint64_t)gm.h, (cuuint64_t)calloc, (cuuint64_t)n_images};
-    cuuint64_t strides[3] = {(cuuint64_t)gm.w * 4, (cuuint64_t)gm.h * gm.w * 4, (cuuint64_t)src.image_stride[i] * 4};
-    cuuint32_t box[4] = {(cuuint32_t)kBoxW, 2, (cuuint32_t)kKC, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&out->m[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<void*>(src.base[i]), dims, strides, box,
-                     estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled failed for dataset %d (CUresult %d)", i, (int)r);
-      return 1;
-    }
-  }
-  return 0;
-}
-
 constexpr size_t kFwdSmem = (size_t)kFwdStages * kStageBytes + 2 * kBoxW * 4 + kNW * 2 * kRowBuf * 4 +
                             kNW * kMaxR * kRowBuf + kFwdStages * 8 + 64;
 constexpr size_t kBwdSmem = (size_t)(kBwdStages + 1) * kStageBytes + kNW * 2 * kRowBuf * 4 + kNW * kMaxR * kRowBuf +
                             kBwdStages * 8 + 64;
 
 template <typename L>
-int launch_fwd(const TmaMaps& maps, const FwdArgs& a, int n_images, cudaStream_t s) {
+int launch_fwd(const Maps& maps, const FwdArgs& a, int n_images, cudaStream_t s) {
   auto k = up_ce_fwd_tma_kernel<L>;
   MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
   dim3 grid((unsigned)((a.gm.w + kT - 1) / kT), (unsigned)a.gm.h, (unsigned)n_images);
@@ -622,7 +570,7 @@ int launch_fwd(const TmaMaps& maps, const FwdArgs& a, int n_images, cudaStream_t
   return 0;
 }
 template <typename L>
-int launch_bwd(const TmaMaps& maps, const BwdArgs& a, int n_images, cudaStream_t s) {
+int launch_bwd(const Maps& maps, const BwdArgs& a, int n_images, cudaStream_t s) {
   auto k = up_ce_bwd_tma_kernel<L>;
   MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmem));
   constexpr int kOwn = kNW * kOwnPerWarp;
@@ -636,8 +584,8 @@ int launch_bwd(const TmaMaps& maps, const BwdArgs& a, int n_images, cudaStream_t
 
 int up_ce_fwd_tma(const FwdArgs& a, int label_dtype, int n_images, cudaStream_t s) {
   if (!tma_applicable(a.src, a.gm)) return -1;
-  TmaMaps maps;
-  if (int rc = make_maps(a.src, a.gm, n_images, &maps)) return rc;
+  Maps maps;
+  if (int rc = tma::make_maps(a.src, a.gm, n_images, kBoxW, 2, kKC, &maps)) return rc;
   if (!a.src.cmax_ready)
     if (int rc = tma::channel_max(a.src, a.dataset_ids, n_images, (int64_t)a.gm.h * a.gm.w, s)) return rc;
   switch (label_dtype) {
@@ -650,8 +598,8 @@ int up_ce_fwd_tma(const FwdArgs& a, int label_dtype, int n_images, cudaStream_t 
 
 int up_ce_bwd_tma(const BwdArgs& a, int label_dtype, int n_images, cudaStream_t s) {
   if (!tma_applicable(a.src, a.gm)) return -1;
-  TmaMaps maps;
-  if (int rc = make_maps(a.src, a.gm, n_images, &maps)) return rc;
+  Maps maps;
+  if (int rc = tma::make_maps(a.src, a.gm, n_images, kBoxW, 2, kKC, &maps)) return rc;
   switch (label_dtype) {
     case MDSEG_U8: return launch_bwd<uint8_t>(maps, a, n_images, s);
     case MDSEG_I32: return launch_bwd<int32_t>(maps, a, n_images, s);

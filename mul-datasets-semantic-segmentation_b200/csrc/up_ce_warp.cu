@@ -36,19 +36,6 @@ constexpr int kStageBytes = kStageFloats * 4;   // 2304
 constexpr int kStgW = 176;                      // staged label columns: <= 15 alignment + 32 cells x 5
 constexpr int kMaxR = 5;
 constexpr int kSpan = 160;
-#ifndef MDSEG_FWD_LEAN_FIN
-#define MDSEG_FWD_LEAN_FIN 1
-#endif
-#ifndef MDSEG_FWD_FASTDIV
-#define MDSEG_FWD_FASTDIV 1
-#endif
-#ifndef MDSEG_FWD_CARRY
-#define MDSEG_FWD_CARRY 1
-#endif
-#ifndef MDSEG_FWD_RECUR
-#define MDSEG_FWD_RECUR 0
-#endif
-constexpr float kRecurMaxDd = 80.f;             // log2 units per cell: beyond it the row recurrence is not used
 
 struct Args {
   mdseg_src_table src;
@@ -63,18 +50,6 @@ struct Args {
   int seg_rows, n_seg, n_strips;
 };
 
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
 // T := arg where the pixel's class (fp16 pair `lab2`) equals the current class (`c2`)
 __device__ __forceinline__ void pick_label2(float2& T, float2 arg, uint32_t lab2, uint32_t c2) {
   asm("{ .reg .pred p, q;\n"
@@ -143,22 +118,6 @@ __device__ __forceinline__ void cell_row(const Args& a, const CUtensorMap* map, 
   for (int j = 0; j < RT; ++j) L1H[j] = dup2(l1h[j]);
   const float2 L1W[2] = {make_float2(l1w[0], l1w[1]), make_float2(l1w[2], l1w[3])};
   const float l1w4 = l1w[4];
-#if MDSEG_FWD_RECUR
-  // row-weight step dh = l1h[1] - l1h[0] (exact in fp32: both are differences of source coordinates inside one cell)
-  // and the deviation eta_j of the later steps from it, premultiplied by ln 2
-  float dh = l1h[1] - l1h[0];
-  float kj[RT];
-#pragma unroll
-  for (int j = 0; j < RT; ++j) {
-    kj[j] = j >= 2 ? ((l1h[j] - l1h[j - 1]) - dh) * kLn2 : 0.f;
-    asm volatile("" : "+f"(kj[j]));  // computed once per cell-row, not re-derived per class
-  }
-  asm volatile("" : "+f"(dh));
-  const float2 DH2 = dup2(dh);
-  float2 KJ[RT];
-#pragma unroll
-  for (int j = 0; j < RT; ++j) KJ[j] = dup2(kj[j]);
-#endif
 
   float2 S[RT][2], T[RT][2];
   float s4[RT], t4[RT];
@@ -169,23 +128,15 @@ __device__ __forceinline__ void cell_row(const Args& a, const CUtensorMap* map, 
     s4[j] = 0.f; t4[j] = 0.f;
   }
 
-#if MDSEG_FWD_CARRY
   uint32_t c2 = 0u;  // fp16 pair (0.0, 0.0): the class ids simply keep counting across the chunks of the cell-row
-#endif
 #pragma unroll 1
   for (int k = 0; k < un.n_ch; ++k) {
     const int q = (g - un.g0) * un.n_ch + k;
     const int c_lo = k * kKC;
     const int cc = (un.C - c_lo) < kKC ? (un.C - c_lo) : kKC;
-#if MDSEG_FWD_CARRY
     const int slot = un.slot;          // ring position and phase are carried, not derived from q by division
     mbar_wait(&bars[slot], un.phase);
     if (++un.slot == kStages) { un.slot = 0; un.phase ^= 1u; }
-#else
-    const int slot = q % kStages;
-    mbar_wait(&bars[slot], (uint32_t)((q / kStages) & 1));
-    uint32_t c2 = class_pair(c_lo);
-#endif
     const float* Sp = stages + slot * kStageFloats + un.xl;
 #pragma unroll 1
     for (int c = 0; c < cc; ++c, c2 = next_class2(c2)) {
@@ -195,52 +146,6 @@ __device__ __forceinline__ void cell_row(const Args& a, const CUtensorMap* map, 
       Sp += 2 * kBoxW;
       const float dv0 = v01 - v00, dv1 = v11 - v10;
       const float2 V0 = dup2(v00), DV0 = dup2(dv0), V1 = dup2(v10), DV1 = dup2(dv1);
-#if MDSEG_FWD_RECUR
-      // Row recurrence: inside a column the exponent is linear in the row weight, so the exponentials of rows
-      // 1.. follow from row 0 by one ratio r = 2^(dh * dd) per column — two MUFU.EX2 per column instead of one
-      // per pixel.  ATen's fp32 row weights are not an exact progression (|eta_j| <= one ulp of the source
-      // coordinate, ~1.5e-5): the ratio of step j is r * 2^(eta_j dd) = r + (ln2 eta_j)(r dd) to first order
-      // (second-order term <= 6e-7 for |dd| <= kRecurMaxDd; steeper columns take the per-pixel path below).
-      const float steep = fmaxf(fabsf(v10 - v00), fabsf(v11 - v01));
-      if (!__any_sync(0xffffffffu, steep > kRecurMaxDd)) {
-#pragma unroll
-        for (int p = 0; p < 2; ++p) {
-          const float2 h0 = fma2(L1W[p], DV0, V0);
-          const float2 dd = sub2(fma2(L1W[p], DV1, V1), h0);
-          const float2 a0 = fma2(L1H[0], dd, h0);
-          float2 E = ex2_2(a0);
-          const float2 r = ex2_2(mul2(DH2, dd));
-          const float2 rd = mul2(r, dd);
-          pick_label2(T[0][p], a0, LH[0][p], c2);
-          S[0][p] = add2(S[0][p], E);
-#pragma unroll
-          for (int j = 1; j < RT; ++j) {
-            const float2 arg = fma2(L1H[j], dd, h0);
-            pick_label2(T[j][p], arg, LH[j][p], c2);
-            E = mul2(E, j == 1 ? r : fma2(KJ[j], rd, r));
-            S[j][p] = add2(S[j][p], E);
-          }
-        }
-        if (NX5) {
-          const float h0 = fmaf(l1w4, dv0, v00);
-          const float dd = fmaf(l1w4, dv1, v10) - h0;
-          const float a0 = fmaf(l1h[0], dd, h0);
-          float E = ex2_approx(a0);
-          const float r = ex2_approx(DH2.x * dd);
-          const float rd = r * dd;
-#pragma unroll
-          for (int j = 0; j < RT; ++j) {
-            const float arg = j == 0 ? a0 : fmaf(l1h[j], dd, h0);
-            float2 t = make_float2(t4[j], 0.f);
-            pick_label2(t, make_float2(arg, 0.f), lh4[j], c2);
-            t4[j] = t.x;
-            if (j >= 1) E *= (j == 1 ? r : fmaf(KJ[j].x, rd, r));
-            s4[j] += E;
-          }
-        }
-        continue;
-      }
-#endif
 #pragma unroll
       for (int p = 0; p < 2; ++p) {
         const float2 h0 = fma2(L1W[p], DV0, V0);
@@ -268,12 +173,8 @@ __device__ __forceinline__ void cell_row(const Args& a, const CUtensorMap* map, 
     __syncwarp();
     if (lane == 0 && q + kStages < un.n_loads) {  // the slot is free: every lane has read its corners
       const int qn = q + kStages;
-#if MDSEG_FWD_FASTDIV
       const int qrow = (qn * un.inv_nch) >> 16;  // qn / n_ch by a 16-bit reciprocal (qn < 128, n_ch <= 32): no division
       const int qk = qn - qrow * un.n_ch;
-#else
-      const int qrow = qn / un.n_ch, qk = qn % un.n_ch;
-#endif
       mbar_expect_tx(&bars[slot], kStageBytes);
       load_4d(stages + slot * kStageFloats, map, &bars[slot], un.x0, un.g0 + qrow, qk * kKC, un.b);
     }
@@ -282,7 +183,6 @@ __device__ __forceinline__ void cell_row(const Args& a, const CUtensorMap* map, 
   // finalize: lse = M + log2(sum), loss = lse - z_label; rows leave through the warp's row buffer
   const float dm0 = c01 - c00, dm1 = c11 - c10;
   const int off = un.sx - (un.Xw0 - un.Xa);
-#if MDSEG_FWD_LEAN_FIN
   // straight-line and predicated: this code runs once per cell-row from a cold instruction cache, so every
   // instruction costs several cycles — no per-pixel branches, per-column terms hoisted, 32-bit row offsets
   float hm0[NX5 ? 5 : 4], dhm[NX5 ? 5 : 4];
@@ -324,38 +224,6 @@ __device__ __forceinline__ void cell_row(const Args& a, const CUtensorMap* map, 
       __syncwarp();
     }
   }
-#else
-#pragma unroll
-  for (int j = 0; j < RT; ++j) {
-    if (j < R) {
-#pragma unroll
-      for (int i = 0; i < (NX5 ? 5 : 4); ++i) {
-        if (i < un.nx) {
-          const float sv = i == 4 ? s4[j] : (i & 1 ? S[j][i >> 1].y : S[j][i >> 1].x);
-          const float tv = i == 4 ? t4[j] : (i & 1 ? T[j][i >> 1].y : T[j][i >> 1].x);
-          const uint32_t hv = i == 4 ? (lh4[j] & 0xffffu) : ((LH[j][i >> 1] >> (16 * (i & 1))) & 0xffffu);
-          const bool valid = hv != 0x5bf8u;
-          const float hm0 = fmaf(l1w[i], dm0, c00);
-          const float M2 = fmaf(l1h[j], fmaf(l1w[i], dm1, c10) - hm0, hm0);
-          const float lg = lg2_approx(sv);
-          const float l = valid ? (lg - tv) * kLn2 : 0.f;
-          rb[off + i] = l;
-          rb[kSpan + off + i] = (M2 + lg) * kLn2;
-          n_valid += valid ? 1u : 0u;
-          if (l > thresh) { ++n_hard; sum_hard += l; }
-          ++n_px;
-        }
-      }
-      __syncwarp();
-      const int64_t rowbase = ((int64_t)un.b * a.gm.H + (Ys + j)) * a.gm.W + un.Xw0;
-      for (int k = lane; k < un.nw; k += 32) {
-        a.loss_px[rowbase + k] = rb[k];
-        a.lse_px[rowbase + k] = rb[kSpan + k];
-      }
-      __syncwarp();
-    }
-  }
-#endif
 }
 
 constexpr size_t kOffCm = (size_t)kStages * kStageBytes;
