@@ -405,6 +405,29 @@ int mdseg_up_ce_bwd_direct(const mdseg_src_table* src /*host*/, const int32_t* d
                            const float* grad_out, float grad_scale, const mdseg_src_table* dst /*host*/,
                            void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- a6 + a7 (+ a10) with align_corners=False at power-of-two factors (BiSeNet heads) --------------------------
+ * Replaces a SegmentHead's trailing nn.Upsample(scale_factor=f, mode='bilinear', align_corners=False) followed by
+ * OhemCELoss (lib/loss/ohem_ce_loss.py:12-34) on the up-sampled logits, and their autograd replay: the
+ * [N, C, H, W] up-sampled tensor is never materialised.  Arguments as mdseg_up_ce_fwd / mdseg_up_ce_bwd_direct;
+ * the interpolation is ATen's align_corners=False one (half-pixel centres, source index clamped at 0).
+ * Geometry: H = fy * h and W = fx * w with fy, fx in {2, 4, 8, 16} (the axes may differ); anything else returns
+ * an error, it is not approximated.  Statistics, loss_px / lse_px and the selection contract are those of
+ * mdseg_up_ce_fwd (mdseg_ohem_select runs unchanged between the two calls). */
+int mdseg_up_ce_fwd_ac0(const mdseg_src_table* src /*host*/, const int32_t* dataset_ids, const void* labels,
+                        int label_dtype, int n_images, int h, int w, int H, int W, int ignore, float* loss_px,
+                        float* lse_px, mdseg_ohem_state* states, int32_t* err_flag, void* stream);
+/* The adjoint: d loss / d src into `dst` (any float dtype, dense [n_images, C_d, h, w] per dataset), through two
+ * fp32 planes in the workspace and mdseg_add_planes; no float atomics, bit-reproducible.  The rows of images of
+ * other datasets (or with an id outside [0, n_datasets)) are written as zeros when dataset_ids is given or there
+ * are several datasets; with one dataset and dataset_ids == NULL every row is the image's gradient. */
+size_t mdseg_up_ce_bwd_ac0_workspace_bytes(const mdseg_src_table* src /*host*/, int n_images, int h, int w, int H,
+                                           int W);
+int mdseg_up_ce_bwd_ac0(const mdseg_src_table* src /*host*/, const int32_t* dataset_ids, const void* labels,
+                        int label_dtype, int n_images, int h, int w, int H, int W, int ignore,
+                        const float* loss_px, const float* lse_px, mdseg_ohem_state* states,
+                        const float* grad_out, float grad_scale, const mdseg_src_table* dst /*host*/,
+                        void* workspace, size_t workspace_bytes, void* stream);
+
 /* out = a + b converted to out_dtype (aux heads: dlogits_aux = A + B) */
 int mdseg_add_planes(const float* a, const float* b, void* out, int out_dtype,
                      int64_t n, void* stream);

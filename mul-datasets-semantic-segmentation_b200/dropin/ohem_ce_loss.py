@@ -25,6 +25,14 @@ class OhemCELoss(nn.Module):
         """logits [N, C, H, W] (fp32 / fp16 / bf16, NCHW or channels_last), labels [N, H, W] -> 0-dim fp32."""
         return ops.ohem_ce(logits, labels, float(self.thresh), self.ignore_lb)
 
+    def forward_fused(self, logits_lowres, labels):
+        """forward(F.interpolate(logits_lowres, size=labels.shape[-2:], mode='bilinear', align_corners=False), labels)
+        without the up-sampled tensor: a BiSeNet SegmentHead's trailing nn.Upsample fused into the loss, forward and
+        backward.  logits_lowres [N, C, h, w] (NCHW or channels_last), H = f h and W = f w with f in {2, 4, 8, 16}
+        per axis; other shapes raise ValueError."""
+        return ops.up_ohem_ce([logits_lowres], labels, None, float(self.thresh), self.ignore_lb,
+                              align_corners=False)[0]
+
 
 class MdsOhemCELoss(nn.Module):
     def __init__(self, configer, thresh, ignore_lb=255):

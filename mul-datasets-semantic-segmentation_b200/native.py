@@ -128,6 +128,10 @@ SIGNATURES = {
     "mdseg_up_ce_bwd_direct_is_fused": (_I, [C.POINTER(SrcTable), _I, _I, _I, _I]),
     "mdseg_up_ce_bwd_direct": (_I, [C.POINTER(SrcTable), _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _F,
                                     C.POINTER(SrcTable), _P, C.c_size_t, _P]),
+    "mdseg_up_ce_fwd_ac0": (_I, [C.POINTER(SrcTable), _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "mdseg_up_ce_bwd_ac0_workspace_bytes": (C.c_size_t, [C.POINTER(SrcTable), _I, _I, _I, _I, _I]),
+    "mdseg_up_ce_bwd_ac0": (_I, [C.POINTER(SrcTable), _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _F,
+                                 C.POINTER(SrcTable), _P, C.c_size_t, _P]),
     "mdseg_add_planes": (_I, [_P, _P, _P, _I, _L, _P]),
     "mdseg_eval_accum": (_I, [_P, _I, _I, _I, _I, _P, _I, _I, _I, _I, _P]),
     "mdseg_eval_fused_workspace_bytes": (C.c_size_t, [_I, _I, _I]),

@@ -1140,7 +1140,7 @@ class _UpOhemCE(torch.autograd.Function):
     (mdseg_planar_to_nhwc)."""
 
     @staticmethod
-    def forward(ctx, labels, dataset_ids, thresh, ignore, seg_per_dataset, *srcs):
+    def forward(ctx, labels, dataset_ids, thresh, ignore, seg_per_dataset, ac0, *srcs):
         labels = _labels(labels)
         _require_cuda(labels, *srcs)
         labels = _compact_labels(labels, max(s.shape[1] for s in srcs), ignore)
@@ -1160,7 +1160,7 @@ class _UpOhemCE(torch.autograd.Function):
                 raise ValueError("every source must be [B, C_i, h, w] over all B images")
         Cs = [s.shape[1] for s in srcs]
         ids = _ids32(dataset_ids, B, dev) if n > 1 else None
-        smax = torch.empty(B, h, w, dtype=torch.float32, device=dev) if dt == torch.float32 else None
+        smax = torch.empty(B, h, w, dtype=torch.float32, device=dev) if dt == torch.float32 and not ac0 else None
         if nhwc:
             cm = max(Cs)
             planar = torch.empty(B, cm, h, w, dtype=dt, device=dev)
@@ -1177,64 +1177,95 @@ class _UpOhemCE(torch.autograd.Function):
         loss_px = torch.empty(P, dtype=torch.float32, device=dev)
         lse_px = torch.empty(P, dtype=torch.float32, device=dev)
         st = _new_states(n_seg, thresh, dev)
-        N.call("mdseg_up_ce_fwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, int(ignore),
-               _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(err_flag(dev)), _stream())
+        N.call("mdseg_up_ce_fwd_ac0" if ac0 else "mdseg_up_ce_fwd", C.byref(src), _ptr(ids), _ptr(labels),
+               _DT[labels.dtype], B, h, w, H, W, int(ignore), _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(err_flag(dev)),
+               _stream())
         out = _select(loss_px, B, H * W, ids if seg_per_dataset else None, st, n_seg)
         ctx.save_for_backward(labels, ids, loss_px, lse_px, st, *srcs)
-        ctx.meta = (int(ignore), bool(seg_per_dataset), Cs, dt, (h, w, H, W), nhwc)
+        ctx.meta = (int(ignore), bool(seg_per_dataset), Cs, dt, (h, w, H, W), nhwc, ac0)
         ctx.states = st
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         labels, ids, loss_px, lse_px, st, *srcs = ctx.saved_tensors
-        ignore, seg_per_dataset, Cs, dt, (h, w, H, W), nhwc = ctx.meta
+        ignore, seg_per_dataset, Cs, dt, (h, w, H, W), nhwc, ac0 = ctx.meta
         B = labels.shape[0]
         n = len(Cs)
         n_seg = n if seg_per_dataset else 1
         g = _grad_scalar(grad_out, n_seg)
         scratch = torch.empty(1, dtype=torch.float32, device=labels.device) if dt == torch.float32 else None
         if nhwc:
-            return (None, None, None, None, None,
+            return (None, None, None, None, None, None,
                     *_up_ohem_ce_bwd_nhwc(srcs[0], labels, ids, loss_px, lse_px, st, g, scratch, ignore, seg_per_dataset,
-                                          Cs, dt, (h, w, H, W)))
+                                          Cs, dt, (h, w, H, W), ac0))
         src = _src_table([s.data_ptr() for s in srcs], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset,
                          cmax=scratch, cmax_ready=True)
         # images of other datasets get a zero gradient (their rows are never selected, :1051): zero-initialised
         # outputs, the kernel writes only the rows of a head's own images
         grads = [torch.zeros_like(s) for s in srcs]
         dst = _src_table([t.data_ptr() for t in grads], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset)
-        _up_ce_adjoint(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, dst)
-        return (None, None, None, None, None, *grads)
+        (_up_ce_adjoint_ac0 if ac0 else _up_ce_adjoint)(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st,
+                                                        g, dst)
+        return (None, None, None, None, None, None, *grads)
 
 
-def _up_ohem_ce_bwd_nhwc(planar, labels, ids, loss_px, lse_px, st, g, scratch, ignore, seg_per_dataset, Cs, dt, shape):
-    """Gradients of _UpOhemCE's channels_last sources: d loss / d (planar rows) from mdseg_up_ce_bwd_direct, scattered
-    into channels_last tensors (zeros for the images of other datasets)."""
+def _up_ohem_ce_bwd_nhwc(planar, labels, ids, loss_px, lse_px, st, g, scratch, ignore, seg_per_dataset, Cs, dt, shape,
+                         ac0=False):
+    """Gradients of _UpOhemCE's channels_last sources: d loss / d (planar rows) from mdseg_up_ce_bwd_direct (or
+    mdseg_up_ce_bwd_ac0), scattered into channels_last tensors (zeros for the images of other datasets)."""
     h, w, H, W = shape
     B, cm = planar.shape[:2]
     n = len(Cs)
     dev = planar.device
     src = _src_table([planar.data_ptr()] * n, [cm * h * w] * n, Cs, _DT[dt], seg_per_dataset, c_alloc=cm, cmax=scratch,
                      cmax_ready=True)
-    if N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W):
+    if not ac0 and N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W):
         dp = torch.empty_like(planar)  # the rows of image b's own head are written — and read
         dst = _src_table([dp.data_ptr()] * n, [cm * h * w] * n, Cs, _DT[dt], seg_per_dataset, c_alloc=cm)
-    else:  # the generic route adds two planes per head: dense [B, C_d, h, w] destinations
+    else:  # the routes that add two planes per head: dense [B, C_d, h, w] destinations
         dp = [torch.empty(B, c, h, w, dtype=dt, device=dev) for c in Cs]
         dst = _src_table([t.data_ptr() for t in dp], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset)
-    _up_ce_adjoint(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, dst)
+    (_up_ce_adjoint_ac0 if ac0 else _up_ce_adjoint)(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g,
+                                                    dst)
     grads = [torch.empty((B, c, h, w), dtype=dt, device=dev, memory_format=torch.channels_last) for c in Cs]
     gt = _src_table([t.data_ptr() for t in grads], [t.stride(0) for t in grads], Cs, _DT[dt], seg_per_dataset)
     N.call("mdseg_planar_to_nhwc", C.byref(dst), _ptr(ids), B, h, w, C.byref(gt), _stream())
     return grads
 
 
-def up_ohem_ce(srcs, labels, dataset_ids, thresh, ignore=255, seg_per_dataset=True):
+def _up_ce_adjoint_ac0(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, dst):
+    """mdseg_up_ce_bwd_ac0: the align_corners=False counterpart of _up_ce_adjoint (dense destinations)."""
+    B, h, w, H, W = shape
+    nbytes = N.lib.mdseg_up_ce_bwd_ac0_workspace_bytes(C.byref(src), B, h, w, H, W)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=labels.device)
+    N.call("mdseg_up_ce_bwd_ac0", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
+           _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
+
+
+AC0_FACTORS = (2, 4, 8, 16)
+
+
+def _check_ac0_geometry(srcs, labels):
+    """align_corners=False is fused for H = f h and W = f w with f in AC0_FACTORS per axis (the BiSeNet heads' x2 ... x16
+    up-sampling); any other geometry raises instead of being approximated."""
+    H, W = labels.shape[-2:]
+    for s in srcs:
+        h, w = s.shape[-2:]
+        if not (h and w and H % h == 0 and W % w == 0 and H // h in AC0_FACTORS and W // w in AC0_FACTORS):
+            raise ValueError(f"up_ohem_ce(align_corners=False): source {tuple(s.shape)} and labels {tuple(labels.shape)} "
+                             f"are not related by a factor in {AC0_FACTORS} per axis")
+
+
+def up_ohem_ce(srcs, labels, dataset_ids, thresh, ignore=255, seg_per_dataset=True, align_corners=True):
     """Per-dataset OhemCE(upsample(srcs[d][ids==d]), labels[ids==d]) as a vector [n_datasets]
     (seg_per_dataset) or one selection over all images ([1]).  srcs[d]: [B, C_d, h, w] over ALL images; channels_last
-    sources are read without a layout copy and get channels_last gradients."""
-    return _UpOhemCE.apply(labels, dataset_ids, float(thresh), int(ignore), bool(seg_per_dataset), *srcs)
+    sources are read without a layout copy and get channels_last gradients.  `align_corners` is that of the bilinear
+    up-sampling; False (nn.Upsample's default, the BiSeNet heads) takes factors 2, 4, 8 and 16 per axis only."""
+    if not align_corners:
+        _check_ac0_geometry(srcs, labels)
+    return _UpOhemCE.apply(labels, dataset_ids, float(thresh), int(ignore), bool(seg_per_dataset), not align_corners,
+                           *srcs)
 
 
 # ---- a11: evaluator accumulation --------------------------------------------------------------------------
