@@ -924,33 +924,54 @@ void pick_lite_strips(Args& a) {
     }
 }
 
-int src_max_c(const mdseg_src_table* s) {
-  int m = 0;
-  for (int i = 0; i < s->n_datasets; ++i) m = s->C[i] > m ? s->C[i] : m;
-  return m;
+// The fused kernel covers fp32 sources at up-sampling factors in [1, 5] (tma::fast_geometry) whose label rows are whole
+// 16-byte bulk copies.
+bool fused_geometry(const mdseg_src_table* src, const Geom& gm) {
+  return gm.W % 16 == 0 && tma::fast_geometry(*src, gm);
 }
 
-}  // namespace
-}  // namespace mdseg
-
-namespace mdseg {
-namespace {
-Geom geom_of(int h, int w, int H, int W) {
-  Geom gm;
-  gm.ym.scale = axis_scale(h, H); gm.ym.n_in = h;
-  gm.xm.scale = axis_scale(w, W); gm.xm.n_in = w;
-  gm.h = h; gm.w = w; gm.H = H; gm.W = W;
-  return gm;
-}
-// the fused kernel covers fp32 sources, column-one-hot sparse graphs and up-sampling factors in [1, 5]
+// ... and, behind a projection, column-one-hot sparse graphs
 bool fused_route(const mdseg_src_table* src, const mdseg_graph_table* graphs, const Geom& gm) {
   for (int i = 0; i < src->n_datasets; ++i) {
     const mdseg_sparse_graph& g = graphs->g[i];
     if (g.dense || !g.col_onehot || !g.csr_ptr || !g.csc_ptr || g.C_ds != src->C[i]) return false;
   }
-  if (gm.W % 16 != 0) return false;  // label rows are staged with 16-byte bulk copies
-  return tma::fast_geometry(*src, gm);
+  return fused_geometry(src, gm);
 }
+
+// the fused kernel's workspace: the two seam halves of every segment, the class byte of every pixel, the fifth columns
+size_t fused_workspace_bytes(int n_images, const Geom& gm, int c_max) {
+  const int sr = pick_seg_rows(gm.h, gm.w, n_images, c_max);
+  const int n_seg = (gm.h - 1 + sr - 1) / sr;
+  return 2 * (size_t)n_images * n_seg * c_max * gm.w * 4 + (size_t)n_images * gm.H * gm.W + 1024 +
+         col5_bytes(n_images, gm.h, gm.w, c_max);
+}
+
+// The Args fields both fused entry points share, the workspace carved into them and the sources' tensor maps; the
+// caller adds the output rows, the channel lists and zero_invalid.
+int setup_fused(const char* who, const mdseg_src_table* src, const int32_t* dataset_ids, const void* labels,
+                const Geom& gm, int n_images, int ignore, const float* loss_px, const float* lse_px,
+                mdseg_ohem_state* states, const float* grad_out, float grad_scale, float* ws, Args& a, Maps* maps) {
+  MDSEG_REQUIRE(((uintptr_t)loss_px & 15) == 0 && ((uintptr_t)lse_px & 15) == 0,
+                "%s: loss_px / lse_px must be 16-byte aligned", who);
+  const int c_max = max_c(src), h = gm.h, w = gm.w;
+  a.src = *src; a.dataset_ids = dataset_ids; a.labels = labels; a.gm = gm; a.ignore = ignore;
+  a.loss_px = loss_px; a.lse_px = lse_px; a.states = states; a.grad_out = grad_out; a.grad_scale = grad_scale;
+  a.seg_rows = pick_seg_rows(h, w, n_images, c_max);
+  a.n_seg = (h - 1 + a.seg_rows - 1) / a.seg_rows;
+  a.n_strips = (w + kOwn - 1) / kOwn;
+  a.c_scr = c_max;
+  a.scrA = ws;
+  a.scrB = ws + (size_t)n_images * a.n_seg * c_max * w;
+  a.sel8 = reinterpret_cast<uint8_t*>(a.scrB + (size_t)n_images * a.n_seg * c_max * w);
+  a.col5 = col5_bytes(n_images, h, w, c_max)
+               ? reinterpret_cast<float2*>(((uintptr_t)(a.sel8 + (size_t)n_images * gm.H * gm.W) + 15) & ~(uintptr_t)15)
+               : nullptr;
+  a.c5s = (c_max + kKC - 1) / kKC * kKC;
+  pick_lite_strips(a);
+  return make_maps(a.src, gm, n_images, kBoxW, 2, kKC, maps);
+}
+
 }  // namespace
 }  // namespace mdseg
 
@@ -960,12 +981,9 @@ extern "C" size_t mdseg_mds_bwd_workspace_bytes(const mdseg_src_table* src, cons
   if (!src || !graphs || src->n_datasets <= 0 || src->n_datasets > MDSEG_MAX_DATASETS ||
       graphs->n_datasets != src->n_datasets || n_images <= 0 || h <= 0 || w <= 0 || H <= 0 || W <= 0)
     return 256;
-  const int c_max = src_max_c(src);
-  if (fused_route(src, graphs, geom_of(h, w, H, W))) {
-    const int sr = pick_seg_rows(h, w, n_images, c_max);
-    const int n_seg = (h - 1 + sr - 1) / sr;
-    return 2 * (size_t)n_images * n_seg * c_max * w * 4 + (size_t)n_images * H * W + 1024 + col5_bytes(n_images, h, w, c_max);
-  }
+  const int c_max = max_c(src);
+  const Geom gm = make_geom(h, w, H, W);
+  if (fused_route(src, graphs, gm)) return fused_workspace_bytes(n_images, gm, c_max);
   // generic route: two gradient planes + the converted dense graphs of mdseg_proj_bwd_tc
   return 2 * (size_t)n_images * c_max * h * w * 4 + 512 + mdseg_proj_bwd_tc_workspace_bytes(graphs, MDSEG_F32);
 }
@@ -984,17 +1002,15 @@ extern "C" int mdseg_mds_bwd(const mdseg_src_table* src, const mdseg_graph_table
   if (n_images == 0) return 0;
   MDSEG_REQUIRE(labels && loss_px && lse_px && states && dx && workspace, "mdseg_mds_bwd: null pointer");
   MDSEG_REQUIRE(is_float_dtype(dx_dtype), "mdseg_mds_bwd: unsupported gradient dtype %d", dx_dtype);
-  const int c_max = src_max_c(src);
+  const int c_max = max_c(src);
   MDSEG_REQUIRE(workspace_bytes >= mdseg_mds_bwd_workspace_bytes(src, graphs, n_images, h, w, H, W),
                 "mdseg_mds_bwd: workspace too small");
   cudaStream_t s = (cudaStream_t)stream;
   const int64_t hw = (int64_t)h * w;
   float* ws = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+  const Geom gm = make_geom(h, w, H, W);
 
-  const Geom gm = geom_of(h, w, H, W);
-  const bool fused = fused_route(src, graphs, gm);
-
-  if (!fused) {
+  if (!fused_route(src, graphs, gm)) {
     // generic route: adjoint of the upsample into two planes, then the projection adjoint
     float* dyA = ws;
     float* dyB = ws + (size_t)n_images * c_max * hw;
@@ -1015,11 +1031,11 @@ extern "C" int mdseg_mds_bwd(const mdseg_src_table* src, const mdseg_graph_table
                              workspace_bytes - used, stream);
   }
 
-  MDSEG_REQUIRE(((uintptr_t)loss_px & 15) == 0 && ((uintptr_t)lse_px & 15) == 0,
-                "mdseg_mds_bwd: loss_px / lse_px must be 16-byte aligned");
   Args a;
-  a.src = *src; a.dataset_ids = dataset_ids; a.labels = labels; a.gm = gm; a.ignore = ignore;
-  a.loss_px = loss_px; a.lse_px = lse_px; a.states = states; a.grad_out = grad_out; a.grad_scale = grad_scale;
+  Maps maps;
+  if (int rc = setup_fused("mdseg_mds_bwd", src, dataset_ids, labels, gm, n_images, ignore, loss_px, lse_px, states,
+                           grad_out, grad_scale, ws, a, &maps))
+    return rc;
   for (int i = 0; i < MDSEG_MAX_DATASETS; ++i) {
     a.out_base[i] = dx; a.out_image_stride[i] = (long long)graphs->C_uni * hw; a.out_channels[i] = graphs->C_uni;
     a.g[i] = GraphDev{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -1029,20 +1045,6 @@ extern "C" int mdseg_mds_bwd(const mdseg_src_table* src, const mdseg_graph_table
     }
   }
   a.zero_invalid = 1;
-  a.seg_rows = pick_seg_rows(h, w, n_images, c_max);
-  a.n_seg = (h - 1 + a.seg_rows - 1) / a.seg_rows;
-  a.n_strips = (w + kOwn - 1) / kOwn;
-  a.c_scr = c_max;
-  a.scrA = ws;
-  a.scrB = ws + (size_t)n_images * a.n_seg * c_max * w;
-  a.sel8 = reinterpret_cast<uint8_t*>(a.scrB + (size_t)n_images * a.n_seg * c_max * w);
-  a.col5 = col5_bytes(n_images, h, w, c_max)
-               ? reinterpret_cast<float2*>(((uintptr_t)(a.sel8 + (size_t)n_images * H * W) + 15) & ~(uintptr_t)15)
-               : nullptr;
-  a.c5s = (c_max + kKC - 1) / kKC * kKC;
-  pick_lite_strips(a);
-  tma::Maps maps;
-  if (int rc = tma::make_maps(a.src, gm, n_images, kBoxW, 2, kKC, &maps)) return rc;
   bool ents_fit = true;  // a class group's (class, channel) pairs, each chunk padded to quads, within kEnt
   for (int i = 0; i < src->n_datasets; ++i) ents_fit = ents_fit && graphs->g[i].nnz + 8 <= kEnt;
   switch (dx_dtype) {
@@ -1060,13 +1062,8 @@ extern "C" size_t mdseg_up_ce_bwd_direct_workspace_bytes(const mdseg_src_table* 
   if (!src || src->n_datasets <= 0 || src->n_datasets > MDSEG_MAX_DATASETS || n_images <= 0 || h <= 0 || w <= 0 ||
       H <= 0 || W <= 0)
     return 256;
-  const Geom gm = geom_of(h, w, H, W);
-  const int c_max = src_max_c(src);
-  if (gm.W % 16 == 0 && tma::fast_geometry(*src, gm)) {
-    const int sr = pick_seg_rows(h, w, n_images, c_max);
-    const int n_seg = (h - 1 + sr - 1) / sr;
-    return 2 * (size_t)n_images * n_seg * c_max * w * 4 + (size_t)n_images * H * W + 1024 + col5_bytes(n_images, h, w, c_max);
-  }
+  const Geom gm = make_geom(h, w, H, W);
+  if (fused_geometry(src, gm)) return fused_workspace_bytes(n_images, gm, max_c(src));
   size_t planes = 0;  // generic route: two fp32 planes per dataset, [n_images, C_d, h, w] each
   for (int i = 0; i < src->n_datasets; ++i) planes += 2 * (size_t)n_images * src->C[i] * h * w * 4;
   return planes + 256;
@@ -1075,8 +1072,7 @@ extern "C" size_t mdseg_up_ce_bwd_direct_workspace_bytes(const mdseg_src_table* 
 extern "C" int mdseg_up_ce_bwd_direct_is_fused(const mdseg_src_table* src, int h, int w, int H, int W) {
   using namespace mdseg;
   if (!src || src->n_datasets <= 0 || src->n_datasets > MDSEG_MAX_DATASETS || h <= 0 || w <= 0 || H <= 0 || W <= 0) return 0;
-  const Geom gm = geom_of(h, w, H, W);
-  return (gm.W % 16 == 0 && tma::fast_geometry(*src, gm)) ? 1 : 0;
+  return fused_geometry(src, make_geom(h, w, H, W)) ? 1 : 0;
 }
 
 extern "C" int mdseg_up_ce_bwd_direct(const mdseg_src_table* src, const int32_t* dataset_ids, const void* labels,
@@ -1098,11 +1094,10 @@ extern "C" int mdseg_up_ce_bwd_direct(const mdseg_src_table* src, const int32_t*
                 "mdseg_up_ce_bwd_direct: workspace too small");
   cudaStream_t s = (cudaStream_t)stream;
   const int64_t hw = (int64_t)h * w;
-  const int c_max = src_max_c(src);
-  const Geom gm = geom_of(h, w, H, W);
+  const Geom gm = make_geom(h, w, H, W);
   float* ws = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
 
-  if (!(gm.W % 16 == 0 && tma::fast_geometry(*src, gm))) {
+  if (!fused_geometry(src, gm)) {
     // generic route: two planes per dataset (zero for the images of other datasets), then their sum
     mdseg_src_table dA = *src, dB = *src;
     dA.dtype = MDSEG_F32; dB.dtype = MDSEG_F32; dA.cmax = nullptr; dB.cmax = nullptr;
@@ -1128,11 +1123,11 @@ extern "C" int mdseg_up_ce_bwd_direct(const mdseg_src_table* src, const int32_t*
     return 0;
   }
 
-  MDSEG_REQUIRE(((uintptr_t)loss_px & 15) == 0 && ((uintptr_t)lse_px & 15) == 0,
-                "mdseg_mds_bwd: loss_px / lse_px must be 16-byte aligned");
   Args a;
-  a.src = *src; a.dataset_ids = dataset_ids; a.labels = labels; a.gm = gm; a.ignore = ignore;
-  a.loss_px = loss_px; a.lse_px = lse_px; a.states = states; a.grad_out = grad_out; a.grad_scale = grad_scale;
+  Maps maps;
+  if (int rc = setup_fused("mdseg_up_ce_bwd_direct", src, dataset_ids, labels, gm, n_images, ignore, loss_px, lse_px,
+                           states, grad_out, grad_scale, ws, a, &maps))
+    return rc;
   for (int i = 0; i < MDSEG_MAX_DATASETS; ++i) {
     const bool on = i < src->n_datasets;
     a.out_base[i] = on ? const_cast<void*>(dst->base[i]) : nullptr;
@@ -1141,20 +1136,7 @@ extern "C" int mdseg_up_ce_bwd_direct(const mdseg_src_table* src, const int32_t*
     a.g[i] = GraphDev{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};  // identity: channel = class
   }
   a.zero_invalid = 0;  // rows of images that do not belong to a head stay as the caller initialised them
-  a.seg_rows = pick_seg_rows(h, w, n_images, c_max);
-  a.n_seg = (h - 1 + a.seg_rows - 1) / a.seg_rows;
-  a.n_strips = (w + kOwn - 1) / kOwn;
-  a.c_scr = c_max;
-  a.scrA = ws;
-  a.scrB = ws + (size_t)n_images * a.n_seg * c_max * w;
-  a.sel8 = reinterpret_cast<uint8_t*>(a.scrB + (size_t)n_images * a.n_seg * c_max * w);
-  a.col5 = col5_bytes(n_images, h, w, c_max)
-               ? reinterpret_cast<float2*>(((uintptr_t)(a.sel8 + (size_t)n_images * H * W) + 15) & ~(uintptr_t)15)
-               : nullptr;
-  a.c5s = (c_max + kKC - 1) / kKC * kKC;
-  pick_lite_strips(a);
-  tma::Maps maps;
-  if (int rc = tma::make_maps(a.src, gm, n_images, kBoxW, 2, kKC, &maps)) return rc;
+  const int c_max = max_c(src);
   switch (dst->dtype) {  // identity channel lists: 16 entries per class group
     case MDSEG_F32: return launch<float>(label_dtype, maps, a, n_images, c_max, true, s);
     case MDSEG_BF16: return launch<__nv_bfloat16>(label_dtype, maps, a, n_images, c_max, true, s);

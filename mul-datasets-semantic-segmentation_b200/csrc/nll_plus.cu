@@ -183,14 +183,6 @@ int launch_bwd(const NllArgs& a, int n_images, cudaStream_t s) {
   return 0;
 }
 
-Geom nll_geom(int h, int w, int H, int W) {
-  Geom gm;
-  gm.ym.scale = axis_scale(h, H); gm.ym.n_in = h;
-  gm.xm.scale = axis_scale(w, W); gm.xm.n_in = w;
-  gm.h = h; gm.w = w; gm.H = H; gm.W = W;
-  return gm;
-}
-
 }  // namespace
 }  // namespace mdseg
 
@@ -243,7 +235,7 @@ extern "C" int mdseg_up_nll_fwd(const mdseg_src_table* src, const int32_t* datas
   if (n_images == 0) return 0;
   MDSEG_REQUIRE(labels && loss_px && states, "mdseg_up_nll_fwd: null pointer");
   NllArgs a;
-  a.src = *src; a.dst = *src; a.dataset_ids = dataset_ids; a.labels = labels; a.gm = nll_geom(h, w, H, W);
+  a.src = *src; a.dst = *src; a.dataset_ids = dataset_ids; a.labels = labels; a.gm = make_geom(h, w, H, W);
   a.ignore = ignore; a.loss_px = loss_px; a.states = states; a.grad_out = nullptr; a.grad_scale = 1.f;
   a.err_flag = err_flag;
   cudaStream_t s = (cudaStream_t)stream;
@@ -268,7 +260,7 @@ extern "C" int mdseg_up_nll_bwd(const mdseg_src_table* src, const int32_t* datas
   if (n_images == 0) return 0;
   MDSEG_REQUIRE(labels && loss_px && states, "mdseg_up_nll_bwd: null pointer");
   NllArgs a;
-  a.src = *src; a.dst = *dst; a.dataset_ids = dataset_ids; a.labels = labels; a.gm = nll_geom(h, w, H, W);
+  a.src = *src; a.dst = *dst; a.dataset_ids = dataset_ids; a.labels = labels; a.gm = make_geom(h, w, H, W);
   a.ignore = ignore; a.loss_px = const_cast<float*>(loss_px); a.states = const_cast<mdseg_ohem_state*>(states);
   a.grad_out = grad_out; a.grad_scale = grad_scale; a.err_flag = nullptr;
   cudaStream_t s = (cudaStream_t)stream;

@@ -554,19 +554,6 @@ int check_src(const mdseg_src_table* s, const char* who) {
     MDSEG_REQUIRE(s->C[i] > 0 && s->base[i] != nullptr, "%s: dataset %d has no source", who, i);
   return 0;
 }
-int max_c(const mdseg_src_table* s) {
-  int m = 0;
-  for (int i = 0; i < s->n_datasets; ++i) m = s->C[i] > m ? s->C[i] : m;
-  return m;
-}
-Geom make_geom(int h, int w, int H, int W) {
-  Geom g;
-  g.ym.scale = axis_scale(h, H); g.ym.n_in = h;
-  g.xm.scale = axis_scale(w, W); g.xm.n_in = w;
-  g.h = h; g.w = w; g.H = H; g.W = W;
-  return g;
-}
-
 constexpr size_t kSmemBudget = 56 * 1024;  // per CTA: keeps 3-4 CTAs resident per SM
 
 template <typename T, typename L>

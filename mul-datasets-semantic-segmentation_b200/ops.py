@@ -241,67 +241,19 @@ def _grad_scalar(g, n=1):
     return g
 
 
-# ---- a7-a9: OhemCELoss on full-resolution logits -------------------------------------------
-class _OhemCE(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, logits, labels, thresh, ignore):
-        _require_cuda(logits, labels)
-        if logits.dim() != 4:
-            raise ValueError("logits must be [N, C, H, W]")
-        Nn, Cc, H, W = logits.shape
-        if logits.dtype not in (torch.float32, torch.bfloat16, torch.float16):
-            logits = logits.float()
-        if logits.is_contiguous():
-            layout = N.NCHW
-        elif logits.is_contiguous(memory_format=torch.channels_last):
-            layout = N.NHWC
-        else:
-            logits, layout = logits.contiguous(), N.NCHW
-        labels = _labels(labels)
-        if labels.numel() != Nn * H * W:
-            raise ValueError(f"labels {tuple(labels.shape)} do not match logits {tuple(logits.shape)}")
-        dev = logits.device
-        P = Nn * H * W
-        loss_px = torch.empty(P, dtype=torch.float32, device=dev)
-        lse_px = torch.empty(P, dtype=torch.float32, device=dev)
-        st = _new_states(1, thresh, dev)
-        N.call("mdseg_ohem_ce_fwd", _ptr(logits), _DT[logits.dtype], layout, _ptr(labels), _DT[labels.dtype], Nn, Cc,
-               H, W, int(ignore), _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(err_flag(dev)), _stream())
-        out = _select(loss_px, Nn, H * W, None, st, 1)
-        ctx.save_for_backward(logits, labels, loss_px, lse_px, st)
-        ctx.meta = (layout, int(ignore))
-        ctx.states = st
-        return out[0]
-
-    @staticmethod
-    def backward(ctx, grad_out):
-        logits, labels, loss_px, lse_px, st = ctx.saved_tensors
-        layout, ignore = ctx.meta
-        Nn, Cc, H, W = logits.shape
-        g = _grad_scalar(grad_out)
-        dl = torch.empty_like(logits)  # preserves the memory format
-        N.call("mdseg_ohem_ce_bwd", _ptr(logits), _DT[logits.dtype], layout, _ptr(labels), _DT[labels.dtype], Nn, Cc,
-               H, W, ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, _ptr(dl), _stream())
-        return dl, None, None, None
+# ---- a7-a9: OhemCELoss on full-resolution logits (one OHEM selection over one or several datasets' logits) ---------
+def _ce_operand(lg):
+    """A CE operand as mdseg_ohem_ce_* read it -> (tensor, layout): fp32 / bf16 / fp16 (anything else as fp32), read as
+    it lies when NCHW-contiguous or channels_last (the gradient then keeps that layout), else made NCHW-contiguous."""
+    if lg.dtype not in (torch.float32, torch.bfloat16, torch.float16):
+        lg = lg.float()
+    if lg.is_contiguous():
+        return lg, N.NCHW
+    if lg.is_contiguous(memory_format=torch.channels_last):
+        return lg, N.NHWC
+    return lg.contiguous(), N.NCHW
 
 
-def ohem_ce(logits, labels, thresh, ignore=255):
-    """mean over the OHEM set of CE(logits, labels); `thresh` is already -log(p) (ohem_ce_loss.py:17,21-34)."""
-    return _OhemCE.apply(logits, labels, float(thresh), int(ignore))
-
-
-def ohem_ce_with_state(logits, labels, thresh, ignore=255):
-    """Forward only; returns (loss, loss_px, OhemState) — for tests and logging (host sync)."""
-    with torch.no_grad():
-        class _Ctx:
-            def save_for_backward(self, *a):
-                self.saved = a
-        ctx = _Ctx()
-        loss = _OhemCE.forward(ctx, logits, labels, float(thresh), int(ignore))
-        return loss, ctx.saved[2], read_states(ctx.saved[4])[0]
-
-
-# ---- MdsOhemCELoss on full-resolution per-dataset logits (the reference module's own call form) ---------------
 class _MdsOhemCEFull(torch.autograd.Function):
     """One OHEM selection over the concatenation of per-dataset CE vectors (lib/loss/ohem_ce_loss.py:48-90).
     logits[k]: [B_k, C_k, H, W]; labels[k]: [B_k, H, W], in the same (ascending dataset id) order."""
@@ -312,23 +264,16 @@ class _MdsOhemCEFull(torch.autograd.Function):
         _require_cuda(*logits, *labels)
         dev = logits[0].device
         H, W = logits[0].shape[2:]
-        metas, offs, P = [], [], 0
+        metas, offs, P, n_images = [], [], 0, 0
         for k in range(n):
-            lg = logits[k]
-            if lg.dtype not in (torch.float32, torch.bfloat16, torch.float16):
-                lg = lg.float()
-            if lg.is_contiguous():
-                layout = N.NCHW
-            elif lg.is_contiguous(memory_format=torch.channels_last):
-                layout = N.NHWC
-            else:
-                lg, layout = lg.contiguous(), N.NCHW
+            lg, layout = _ce_operand(logits[k])
             if tuple(lg.shape[2:]) != (H, W) or labels[k].numel() != lg.shape[0] * H * W:
                 raise ValueError("every dataset's logits / labels must share H x W")
             logits[k] = lg
             metas.append(layout)
             offs.append(P)
             P += lg.shape[0] * H * W
+            n_images += lg.shape[0]
         loss_px = torch.empty(P, dtype=torch.float32, device=dev)
         lse_px = torch.empty(P, dtype=torch.float32, device=dev)
         st = _new_states(1, thresh, dev)
@@ -337,8 +282,8 @@ class _MdsOhemCEFull(torch.autograd.Function):
             N.call("mdseg_ohem_ce_fwd", _ptr(lg), _DT[lg.dtype], metas[k], _ptr(labels[k]), _DT[labels[k].dtype],
                    lg.shape[0], lg.shape[1], H, W, int(ignore), loss_px.data_ptr() + 4 * offs[k],
                    lse_px.data_ptr() + 4 * offs[k], _ptr(st), _ptr(err_flag(dev)), _stream())
-        out = _select(loss_px, P // (H * W), H * W, None, st, 1)
-        ctx.save_for_backward(loss_px, lse_px, st, *logits, *labels)
+        out = _select(loss_px, n_images, H * W, None, st, 1)
+        ctx.save_for_backward(*logits, *labels, loss_px, lse_px, st)  # with one entry: the layout ohem_ce always had
         ctx.meta = (n, metas, offs, int(ignore), H, W)
         ctx.states = st
         return out[0]
@@ -346,18 +291,45 @@ class _MdsOhemCEFull(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_out):
         n, metas, offs, ignore, H, W = ctx.meta
-        loss_px, lse_px, st = ctx.saved_tensors[:3]
-        logits, labels = ctx.saved_tensors[3:3 + n], ctx.saved_tensors[3 + n:]
+        logits, labels = ctx.saved_tensors[:n], ctx.saved_tensors[n:2 * n]
+        loss_px, lse_px, st = ctx.saved_tensors[2 * n:]
         g = _grad_scalar(grad_out)
         grads = []
         for k in range(n):
             lg = logits[k]
-            dl = torch.empty_like(lg)
+            dl = torch.empty_like(lg)  # preserves the memory format
             N.call("mdseg_ohem_ce_bwd", _ptr(lg), _DT[lg.dtype], metas[k], _ptr(labels[k]), _DT[labels[k].dtype],
                    lg.shape[0], lg.shape[1], H, W, ignore, loss_px.data_ptr() + 4 * offs[k],
                    lse_px.data_ptr() + 4 * offs[k], _ptr(st), _ptr(g), 1.0, _ptr(dl), _stream())
             grads.append(dl)
         return (None, None, None, *grads, *([None] * n))
+
+
+def _check_ohem_ce(logits, labels):
+    _require_cuda(logits, labels)
+    if logits.dim() != 4:
+        raise ValueError("logits must be [N, C, H, W]")
+    Nn, _, H, W = logits.shape
+    if labels.numel() != Nn * H * W:
+        raise ValueError(f"labels {tuple(labels.shape)} do not match logits {tuple(logits.shape)}")
+
+
+def ohem_ce(logits, labels, thresh, ignore=255):
+    """mean over the OHEM set of CE(logits, labels); `thresh` is already -log(p) (ohem_ce_loss.py:17,21-34)."""
+    _check_ohem_ce(logits, labels)
+    return _MdsOhemCEFull.apply(float(thresh), int(ignore), 1, logits, labels)
+
+
+def ohem_ce_with_state(logits, labels, thresh, ignore=255):
+    """Forward only; returns (loss, loss_px, OhemState) — for tests and logging (host sync)."""
+    _check_ohem_ce(logits, labels)
+    with torch.no_grad():
+        class _Ctx:
+            def save_for_backward(self, *a):
+                self.saved = a
+        ctx = _Ctx()
+        loss = _MdsOhemCEFull.forward(ctx, float(thresh), int(ignore), 1, logits, labels)
+        return loss, ctx.saved[2], read_states(ctx.saved[4])[0]
 
 
 def mds_ohem_ce_full(logits, labels, thresh, ignore=255):
@@ -522,6 +494,29 @@ def _src_table(bases, strides, Cs, dtype, seg_per_dataset, c_alloc=None, cmax=No
         ca = c_alloc[i] if isinstance(c_alloc, (list, tuple)) else c_alloc
         t.C_alloc[i] = ca if ca else c
     return t
+
+
+def _planes_table(t, Cs, seg_per_dataset=False, head=0, cmax=None, cmax_ready=False):
+    """SrcTable over ONE planes tensor t [B, c_alloc, h, w] that holds the rows of every dataset: dataset d's C_d rows
+    start at channel head * C_d (head k of the stacked heads' planes; 0 for one head)."""
+    _, ca, h, w = t.shape
+    return _src_table([t.data_ptr() + head * c * h * w * t.element_size() for c in Cs], [ca * h * w] * len(Cs), Cs,
+                      _DT[t.dtype], seg_per_dataset, c_alloc=[ca - head * c for c in Cs], cmax=cmax,
+                      cmax_ready=cmax_ready)
+
+
+def _tensors_table(ts, seg_per_dataset, cmax=None, cmax_ready=False):
+    """SrcTable over one dense [B, C_d, h, w] tensor per dataset (NCHW-contiguous or channels_last)."""
+    return _src_table([t.data_ptr() for t in ts], [t[0].numel() for t in ts], [t.shape[1] for t in ts], _DT[ts[0].dtype],
+                      seg_per_dataset, cmax=cmax, cmax_ready=cmax_ready)
+
+
+def _fused_adjoint(Cs, h, w, H, W, dtype=torch.float32):
+    """Whether mdseg_up_ce_bwd_direct takes the fused single-pass kernel (else the route of two planes per dataset) for
+    freshly allocated planes [B, max(Cs), h, w] of `dtype` holding the classes Cs.  Only the dtype, the class counts and
+    the geometry decide: an allocation is 16-byte aligned, so any aligned address stands for its base."""
+    probe = _src_table([256] * len(Cs), [max(Cs) * h * w] * len(Cs), Cs, _DT[dtype], False)
+    return bool(N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(probe), h, w, H, W))
 
 
 def _channels_last(x):
@@ -735,11 +730,77 @@ def prototype_head(feats, proto):
 
 
 # ---- a5+a6+a7+a8+a9: the fused multi-dataset loss ------------------------------------------------------
+def _up_ce_select(src, ids, labels, shape, ignore, thresh, ac0=False):
+    """mdseg_up_ce_fwd (mdseg_up_ce_fwd_ac0 with ac0) over the low-resolution rows src describes, then the OHEM
+    selection: one per dataset when src.seg_per_dataset, else one over all images.  -> (out, loss_px, lse_px, states)"""
+    B, h, w, H, W = shape
+    dev = labels.device
+    n_seg = src.n_datasets if src.seg_per_dataset else 1
+    loss_px = torch.empty(B * H * W, dtype=torch.float32, device=dev)
+    lse_px = torch.empty(B * H * W, dtype=torch.float32, device=dev)
+    st = _new_states(n_seg, thresh, dev)
+    N.call("mdseg_up_ce_fwd_ac0" if ac0 else "mdseg_up_ce_fwd", C.byref(src), _ptr(ids), _ptr(labels),
+           _DT[labels.dtype], B, h, w, H, W, int(ignore), _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(err_flag(dev)),
+           _stream())
+    out = _select(loss_px, B, H * W, ids if src.seg_per_dataset else None, st, n_seg)
+    return out, loss_px, lse_px, st
+
+
+def _up_ce_adjoint(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, dst, ac0=False):
+    """mdseg_up_ce_bwd_direct (mdseg_up_ce_bwd_ac0 with ac0): d loss / d (the low-resolution rows src describes) of the
+    upsample + CE under the selection in st, into the rows dst describes."""
+    B, h, w, H, W = shape
+    name = "mdseg_up_ce_bwd_ac0" if ac0 else "mdseg_up_ce_bwd_direct"
+    nbytes = getattr(N.lib, name + "_workspace_bytes")(C.byref(src), B, h, w, H, W)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=labels.device)
+    N.call(name, C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore, _ptr(loss_px),
+           _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
+
+
+def _mds_dy(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, y, Cs):
+    """d loss / d y of the fused loss as fp32 planes shaped like y: (dyA, None) from the fused single-pass kernel with
+    the identity in place of G^T when it applies, else the two planes (dyA, dyB) of mdseg_up_ce_bwd, whose sum it is."""
+    B, h, w, H, W = shape
+    dyA = torch.empty_like(y)  # only the first C_ds planes of an image are written — and read
+    if _fused_adjoint(Cs, h, w, H, W):
+        _up_ce_adjoint(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, _planes_table(dyA, Cs))
+        return dyA, None
+    dyB = torch.empty_like(y)
+    N.call("mdseg_up_ce_bwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
+           _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(_planes_table(dyA, Cs)),
+           C.byref(_planes_table(dyB, Cs)), _stream())
+    return dyA, dyB
+
+
+# The backward routes of _MdsProjOhemCE
+_NO_GRAD = "no gradient"             # no input wants one: the backward never runs
+_MDS_BWD = "mdseg_mds_bwd"           # d x only, NCHW x: one call
+_NHWC_BWD = "planes, nhwc adjoint"   # d x only, channels_last x (sparse graphs): d y planes, then mdseg_proj_bwd_nhwc
+_TC16_BWD = "16-bit dy, tc16"        # d graphs (and maybe d x), fused adjoint, 16-bit x, dense graphs: the tc16 adjoints
+_PLANES_BWD = "fp32 planes"          # d graphs otherwise: fp32 d y planes (_mds_dy), then _proj_bwd / _proj_bwd_graph
+
+
+def _mds_route(x, tab, Cs, geom, want_dx, want_dg):
+    """-> (the backward route of _MdsProjOhemCE, x in the layout that route and the forward read).  channels_last x is
+    kept when the projection reads it as it lies (_nhwc_proj_ok), or when it is 16-bit with dense graphs in the tc16
+    envelope and the backward either never runs or reads x on its tc16 route only; mdseg_mds_bwd writes d x planar, so
+    a d x without d graphs takes x NCHW-contiguous otherwise."""
+    tc16_nhwc = _dense_tc16(tab) and _tc16_layout(x) == N.NHWC
+    if want_dg:
+        fused = _fused_adjoint(Cs, *geom)
+        if not (_nhwc_proj_ok(x, tab) or (tc16_nhwc and fused)):
+            x = x.contiguous()
+        return (_TC16_BWD if fused and _dense_tc16(tab) and _tc16_layout(x) is not None else _PLANES_BWD), x
+    if want_dx:
+        return (_NHWC_BWD, x) if _nhwc_proj_ok(x, tab) else (_MDS_BWD, x.contiguous())
+    return _NO_GRAD, (x if _nhwc_proj_ok(x, tab) or tc16_nhwc else x.contiguous())
+
+
 class _MdsProjOhemCE(torch.autograd.Function):
     """MdsOhemCELoss(project -> upsample -> CE) of loss_cross_datasets.py:1006-1007,1074 in four kernels.  channels_last
     logits with sparse graphs are projected as they are and get a channels_last gradient (mdseg_proj_*_nhwc); so are
     channels_last 16-bit logits / features with dense graphs (folded prototypes, trainable graphs) when the backward takes
-    the tc16 route (mdseg_proj_*_tc16 with layout NHWC)."""
+    the tc16 route (mdseg_proj_*_tc16 with layout NHWC).  The backward route is chosen once, here (_mds_route)."""
 
     @staticmethod
     def forward(ctx, logits_uni, labels, dataset_ids, thresh, ignore, cache, per_dataset, *graphs):
@@ -758,29 +819,17 @@ class _MdsProjOhemCE(torch.autograd.Function):
         if tab.C_uni != Cu:
             raise ValueError(f"graphs have C_uni={tab.C_uni}, logits have {Cu}")
         Cs = [g.shape[0] for g in graphs]
-        cmax = max(Cs)
         ids = _ids32(dataset_ids, B, dev)
-        ef = err_flag(dev)
-        y = torch.empty(B, cmax, h, w, dtype=torch.float32, device=dev)
+        y = torch.empty(B, max(Cs), h, w, dtype=torch.float32, device=dev)
         ymax = torch.empty(B, h, w, dtype=torch.float32, device=dev)  # channel maximum of y: the softmax shift
         all_sparse = all(not tab.g[i].dense for i in range(len(Cs)))
-        n_seg = len(Cs) if per_dataset else 1
-        src = _src_table([y.data_ptr()] * len(Cs), [cmax * h * w] * len(Cs), Cs, N.F32, per_dataset, c_alloc=cmax,
-                         cmax=ymax, cmax_ready=all_sparse)
-        tc16 = _dense_tc16(tab)
-        if not (_nhwc_proj_ok(x, tab)
-                or (tc16 and _tc16_layout(x) == N.NHWC and _tc16_bwd_nhwc_ok(ctx, len(Cs), src, h, w, H, W))):
-            x = x.contiguous()
-        _proj_fwd(x, tab, graphs, ids, y, ymax, ef, tc16 and _tc16_layout(x) is not None)
-        P = B * H * W
-        loss_px = torch.empty(P, dtype=torch.float32, device=dev)
-        lse_px = torch.empty(P, dtype=torch.float32, device=dev)
-        st = _new_states(n_seg, thresh, dev)
-        N.call("mdseg_up_ce_fwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, int(ignore),
-               _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(ef), _stream())
-        out = _select(loss_px, B, H * W, ids if per_dataset else None, st, n_seg)
+        src = _planes_table(y, Cs, per_dataset, cmax=ymax, cmax_ready=all_sparse)
+        route, x = _mds_route(x, tab, Cs, (h, w, H, W), ctx.needs_input_grad[0],
+                              any(ctx.needs_input_grad[7:]))
+        _proj_fwd(x, tab, graphs, ids, y, ymax, err_flag(dev), _dense_tc16(tab) and _tc16_layout(x) is not None)
+        out, loss_px, lse_px, st = _up_ce_select(src, ids, labels, (B, h, w, H, W), ignore, thresh)
         ctx.save_for_backward(x, labels, ids, y, loss_px, lse_px, st, *graphs)
-        ctx.meta = (int(ignore), cache, Cs, cmax, (h, w, H, W), bool(per_dataset))
+        ctx.meta = (int(ignore), cache, Cs, (h, w, H, W), bool(per_dataset), route)
         ctx.states = st
         ctx.mark_non_differentiable(st)
         return (out if per_dataset else out[0]), st
@@ -788,87 +837,40 @@ class _MdsProjOhemCE(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_out, _grad_states=None):
         x, labels, ids, y, loss_px, lse_px, st, *graphs = ctx.saved_tensors
-        ignore, cache, Cs, cmax, (h, w, H, W), per_dataset = ctx.meta
+        ignore, cache, Cs, (h, w, H, W), per_dataset, route = ctx.meta
         B = x.shape[0]
-        dev = x.device
         n = len(Cs)
         g = _grad_scalar(grad_out, n if per_dataset else 1)
         tab, keep = cache.table(list(graphs))
-        scratch = torch.empty(1, dtype=torch.float32, device=dev)  # non-NULL cmax selects the TMA kernels
-        src = _src_table([y.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, per_dataset, c_alloc=cmax, cmax=scratch,
-                         cmax_ready=True)
+        scratch = torch.empty(1, dtype=torch.float32, device=x.device)  # non-NULL cmax selects the TMA kernels
+        src = _planes_table(y, Cs, per_dataset, cmax=scratch, cmax_ready=True)
         adj = (src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g)
-        want_dg = any(ctx.needs_input_grad[7 + i] for i in range(n))
-        dx = None
-        if not want_dg:
-            if ctx.needs_input_grad[0] and _channels_last(x):
-                # channels_last logits (sparse graphs, see forward): d loss / d y from the upsample + CE adjoint, then the
-                # broadcast through G^T written pixel-major
-                dx = torch.empty_like(x)  # channels_last
-                _proj_bwd(*_mds_dy(*adj, y, Cs, cmax), graphs, tab, ids, dx)
-            elif ctx.needs_input_grad[0]:
-                # one call: softmax recompute + adjoint of the upsample + broadcast through G^T (fused when it applies)
-                nbytes = N.lib.mdseg_mds_bwd_workspace_bytes(C.byref(src), C.byref(tab), B, h, w, H, W)
-                ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-                dx = torch.empty_like(x)
-                N.call("mdseg_mds_bwd", C.byref(src), C.byref(tab), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h,
-                       w, H, W, ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, _ptr(dx), _DT[x.dtype],
-                       _ptr(ws), nbytes, _stream())
+        dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None  # the layout of x
+        if route == _MDS_BWD:
+            # one call: softmax recompute + adjoint of the upsample + broadcast through G^T (fused when it applies)
+            nbytes = N.lib.mdseg_mds_bwd_workspace_bytes(C.byref(src), C.byref(tab), B, h, w, H, W)
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+            N.call("mdseg_mds_bwd", C.byref(src), C.byref(tab), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H,
+                   W, ignore, _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, _ptr(dx), _DT[x.dtype], _ptr(ws),
+                   nbytes, _stream())
             return (dx, None, None, None, None, None, None, *([None] * n))
-        if (N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W) and _tc16_layout(x) is not None
-                and _dense_tc16(tab)):
+        if route == _NHWC_BWD:
+            # d loss / d y from the upsample + CE adjoint, then the broadcast through G^T written pixel-major
+            _proj_bwd(*_mds_dy(*adj, y, Cs), graphs, tab, ids, dx)
+            return (dx, None, None, None, None, None, None, *([None] * n))
+        if route == _TC16_BWD:
             # 16-bit logits / features with dense graphs (AMP GNN stage, folded prototypes): d loss / d y leaves the fused
             # kernel in the dtype of x (what autocast's backward rounds it to) and both adjoints of the projection run
             # on the TMA-fed tcgen05 kernels — no register-staged conversion, one launch for all datasets each.
-            dy, dyB = torch.zeros(B, cmax, h, w, dtype=x.dtype, device=dev), None  # planes >= C_ds of an image stay 0
-            _up_ce_adjoint(*adj, _src_table([dy.data_ptr()] * n, [cmax * h * w] * n, Cs, _DT[x.dtype], False))
+            dy, dyB = torch.zeros(B, y.shape[1], h, w, dtype=x.dtype, device=x.device), None  # planes >= C_ds stay 0
+            _up_ce_adjoint(*adj, _planes_table(dy, Cs))
         else:
-            dy, dyB = _mds_dy(*adj, y, Cs, cmax)
-        if ctx.needs_input_grad[0]:
-            dx = torch.empty_like(x)
+            dy, dyB = _mds_dy(*adj, y, Cs)
+        if dx is not None:
             _proj_bwd(dy, dyB, graphs, tab, ids, dx)
         dG = _proj_bwd_graph(x, dy, dyB, graphs, tab, ids)
         dgs = [dG[i, :Cs[i]].to(graphs[i].dtype) if ctx.needs_input_grad[7 + i] else None for i in range(n)]
         return (dx, None, None, None, None, None, None, *dgs)
-
-
-def _tc16_bwd_nhwc_ok(ctx, n, src, h, w, H, W):
-    """_MdsProjOhemCE with channels_last x in the tc16 route of the forward: the backward reads x only on its tc16 branch — taken
-    when a graph wants a gradient and the upsample + CE adjoint is the fused kernel — or never runs (no input wants a
-    gradient).  A d x without d graphs goes through mdseg_mds_bwd, which writes dx planar, so x is copied then."""
-    want_dg = any(ctx.needs_input_grad[7 + i] for i in range(n))
-    if not want_dg:
-        return not ctx.needs_input_grad[0]
-    return bool(N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W))
-
-
-def _up_ce_adjoint(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, dst):
-    """mdseg_up_ce_bwd_direct: d loss / d (the low-resolution rows src describes) of the fused upsample + CE under the
-    selection in st, into the rows dst describes."""
-    B, h, w, H, W = shape
-    nbytes = N.lib.mdseg_up_ce_bwd_direct_workspace_bytes(C.byref(src), B, h, w, H, W)
-    ws = torch.empty(nbytes, dtype=torch.uint8, device=labels.device)
-    N.call("mdseg_up_ce_bwd_direct", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
-           _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
-
-
-def _mds_dy(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, y, Cs, cmax):
-    """d loss / d y of the fused loss as fp32 planes shaped like y: (dyA, None) from the fused single-pass kernel with
-    the identity in place of G^T when it applies, else the two planes (dyA, dyB) of mdseg_up_ce_bwd, whose sum it is."""
-    B, h, w, H, W = shape
-    n = len(Cs)
-    if N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W):
-        dyA, dyB = torch.empty_like(y), None  # only the first C_ds planes of an image are written — and read
-        _up_ce_adjoint(src, ids, labels, shape, ignore, loss_px, lse_px, st, g,
-                       _src_table([dyA.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False))
-    else:
-        dyA = torch.empty_like(y)
-        dyB = torch.empty_like(y)
-        dA = _src_table([dyA.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
-        dB = _src_table([dyB.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False)
-        N.call("mdseg_up_ce_bwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
-               _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dA), C.byref(dB), _stream())
-    return dyA, dyB
 
 
 def mds_proj_ohem_ce(logits_uni, labels, dataset_ids, graphs, thresh, ignore=255, cache=None, per_dataset=False):
@@ -905,7 +907,6 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
         n = len(graphs) // n_heads
         Cs = [graphs[d].shape[0] for d in range(n)]
         labels = _compact_labels(labels, max(Cs), ignore)
-        cmax2 = n_heads * max(Cs)
         stacked = [torch.cat([graphs[k * n + d].detach().to(torch.float32) for k in range(n_heads)], 0) for d in range(n)]
         cache = BipartiteGraphs(assume_dense=True)
         tab, keep = cache.table(stacked)
@@ -914,46 +915,35 @@ class _MdsProjOhemCEHeads(torch.autograd.Function):
             x = x.contiguous()
         tc16 = tc16 and _tc16_layout(x) is not None  # the route of both directions
         ids = _ids32(dataset_ids, B, dev)
-        ef = err_flag(dev)
-        y = torch.empty(B, cmax2, h, w, dtype=torch.float32, device=dev)
-        _proj_fwd(x, tab, stacked, ids, y, None, ef, tc16)
-        P = B * H * W
+        y = torch.empty(B, n_heads * max(Cs), h, w, dtype=torch.float32, device=dev)
+        _proj_fwd(x, tab, stacked, ids, y, None, err_flag(dev), tc16)
         outs, saved = [], []
         for k in range(n_heads):
             ymax = torch.empty(B, h, w, dtype=torch.float32, device=dev)
-            src = _src_table([y.data_ptr() + k * c * h * w * 4 for c in Cs], [cmax2 * h * w] * n, Cs, N.F32, False,
-                             c_alloc=[cmax2 - k * c for c in Cs], cmax=ymax, cmax_ready=False)
-            loss_px = torch.empty(P, dtype=torch.float32, device=dev)
-            lse_px = torch.empty(P, dtype=torch.float32, device=dev)
-            st = _new_states(1, thresh, dev)
-            N.call("mdseg_up_ce_fwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, int(ignore),
-                   _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(ef), _stream())
-            outs.append(_select(loss_px, B, H * W, None, st, 1)[0])
-            saved += [loss_px, lse_px, st]
+            out, *head = _up_ce_select(_planes_table(y, Cs, head=k, cmax=ymax), ids, labels, (B, h, w, H, W), ignore,
+                                       thresh)
+            outs.append(out[0])
+            saved += head
         ctx.save_for_backward(x, labels, ids, y, *saved, *stacked)
-        ctx.meta = (int(ignore), Cs, cmax2, (h, w, H, W), n_heads, [g.dtype for g in graphs], tc16)
+        ctx.meta = (int(ignore), Cs, (h, w, H, W), n_heads, [g.dtype for g in graphs], tc16)
         return torch.stack(outs)
 
     @staticmethod
     def backward(ctx, grad_out):
-        ignore, Cs, cmax2, (h, w, H, W), n_heads, gdt, tc16 = ctx.meta
+        ignore, Cs, (h, w, H, W), n_heads, gdt, tc16 = ctx.meta
         n = len(Cs)
         x, labels, ids, y = ctx.saved_tensors[:4]
         saved = ctx.saved_tensors[4:4 + 3 * n_heads]
         stacked = ctx.saved_tensors[4 + 3 * n_heads:]
         B = x.shape[0]
-        dev = x.device
         g = _grad_scalar(grad_out, n_heads)
-        ddt = x.dtype if tc16 else torch.float32
-        esz = 2 if tc16 else 4
-        dy = torch.zeros(B, cmax2, h, w, dtype=ddt, device=dev)  # planes past the heads of an image's dataset stay zero
-        scratch = torch.empty(1, dtype=torch.float32, device=dev)
+        # planes past the heads of an image's dataset stay zero
+        dy = torch.zeros(y.shape, dtype=x.dtype if tc16 else torch.float32, device=x.device)
+        scratch = torch.empty(1, dtype=torch.float32, device=x.device)
         for k in range(n_heads):
             loss_px, lse_px, st = saved[3 * k:3 * k + 3]
-            src = _src_table([y.data_ptr() + k * c * h * w * 4 for c in Cs], [cmax2 * h * w] * n, Cs, N.F32, False,
-                             c_alloc=[cmax2 - k * c for c in Cs], cmax=scratch, cmax_ready=True)
-            dst = _src_table([dy.data_ptr() + k * c * h * w * esz for c in Cs], [cmax2 * h * w] * n, Cs, _DT[ddt], False)
-            _up_ce_adjoint(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g[k:k + 1], dst)
+            _up_ce_adjoint(_planes_table(y, Cs, head=k, cmax=scratch, cmax_ready=True), ids, labels, (B, h, w, H, W),
+                           ignore, loss_px, lse_px, st, g[k:k + 1], _planes_table(dy, Cs, head=k))
         tab, keep = (None, None) if tc16 else BipartiteGraphs(assume_dense=True).table(list(stacked))
         dx = None
         if ctx.needs_input_grad[0]:
@@ -981,12 +971,8 @@ def mds_proj_ohem_ce_heads(x, labels, dataset_ids, graph_sets, thresh, ignore=25
     B, Cu, h, w = x.shape
     Hh, Ww = labels.shape[1:]
     Cs = [g.shape[0] for g in sets[0]]
-    ok = (len(sets) > 1 and all(len(gs) == n and [g.shape[0] for g in gs] == Cs for gs in sets)
-          and _tc16_envelope(Cu, Cs, len(sets)) and x.is_cuda)
-    if ok:
-        probe = _src_table([x.data_ptr() & ~15] * n, [4 * h * w] * n, Cs, N.F32, False, cmax=x)
-        ok = bool(N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(probe), h, w, Hh, Ww))
-    if not ok:
+    if not (len(sets) > 1 and all(len(gs) == n and [g.shape[0] for g in gs] == Cs for gs in sets)
+            and _tc16_envelope(Cu, Cs, len(sets)) and x.is_cuda and _fused_adjoint(Cs, h, w, Hh, Ww)):
         return torch.stack([mds_proj_ohem_ce(x, labels, dataset_ids, gs, thresh, ignore,
                                              BipartiteGraphs(assume_dense=all(g.requires_grad for g in gs)))
                             for gs in sets])
@@ -1085,7 +1071,7 @@ class _MdsNLLPlus(torch.autograd.Function):
         N.call("mdseg_softmax_nchw", _ptr(x), _DT[x.dtype], B, Cu, h * w, _ptr(pred), _stream())
         q = torch.empty(B, cmax, h, w, dtype=torch.float32, device=dev)
         _proj_fwd(pred, tab, graphs, ids, q, None, ef, False)
-        src = _src_table([q.data_ptr()] * len(Cs), [cmax * h * w] * len(Cs), Cs, N.F32, False, c_alloc=cmax)
+        src = _planes_table(q, Cs)
         loss_px = torch.empty(B * H * W, dtype=torch.float32, device=dev)
         st = _new_states(1, thresh, dev)
         N.call("mdseg_up_nll_fwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, int(ignore),
@@ -1105,9 +1091,9 @@ class _MdsNLLPlus(torch.autograd.Function):
         n = len(Cs)
         g = _grad_scalar(grad_out)
         tab, keep = cache.table(list(graphs))
-        src = _src_table([q.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False, c_alloc=cmax)
+        src = _planes_table(q, Cs)
         dq = torch.zeros_like(q)
-        dst = _src_table([dq.data_ptr()] * n, [cmax * h * w] * n, Cs, N.F32, False, c_alloc=cmax)
+        dst = _planes_table(dq, Cs)
         N.call("mdseg_up_nll_bwd", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
                _ptr(loss_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _stream())
         dx = None
@@ -1162,85 +1148,48 @@ class _UpOhemCE(torch.autograd.Function):
         ids = _ids32(dataset_ids, B, dev) if n > 1 else None
         smax = torch.empty(B, h, w, dtype=torch.float32, device=dev) if dt == torch.float32 and not ac0 else None
         if nhwc:
-            cm = max(Cs)
-            planar = torch.empty(B, cm, h, w, dtype=dt, device=dev)
-            src = _src_table([planar.data_ptr()] * n, [cm * h * w] * n, Cs, _DT[dt], seg_per_dataset, c_alloc=cm,
-                             cmax=smax)
-            nt = _src_table([s.data_ptr() for s in srcs], [s.stride(0) for s in srcs], Cs, _DT[dt], seg_per_dataset)
-            N.call("mdseg_nhwc_to_planar", C.byref(nt), _ptr(ids), B, h, w, C.byref(src), _stream())
+            planar = torch.empty(B, max(Cs), h, w, dtype=dt, device=dev)
+            src = _planes_table(planar, Cs, seg_per_dataset, cmax=smax)
+            N.call("mdseg_nhwc_to_planar", C.byref(_tensors_table(srcs, seg_per_dataset)), _ptr(ids), B, h, w,
+                   C.byref(src), _stream())
             srcs = [planar]
         else:
-            src = _src_table([s.data_ptr() for s in srcs], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset,
-                             cmax=smax)
-        n_seg = n if seg_per_dataset else 1
-        P = B * H * W
-        loss_px = torch.empty(P, dtype=torch.float32, device=dev)
-        lse_px = torch.empty(P, dtype=torch.float32, device=dev)
-        st = _new_states(n_seg, thresh, dev)
-        N.call("mdseg_up_ce_fwd_ac0" if ac0 else "mdseg_up_ce_fwd", C.byref(src), _ptr(ids), _ptr(labels),
-               _DT[labels.dtype], B, h, w, H, W, int(ignore), _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(err_flag(dev)),
-               _stream())
-        out = _select(loss_px, B, H * W, ids if seg_per_dataset else None, st, n_seg)
+            src = _tensors_table(srcs, seg_per_dataset, cmax=smax)
+        out, loss_px, lse_px, st = _up_ce_select(src, ids, labels, (B, h, w, H, W), ignore, thresh, ac0)
         ctx.save_for_backward(labels, ids, loss_px, lse_px, st, *srcs)
-        ctx.meta = (int(ignore), bool(seg_per_dataset), Cs, dt, (h, w, H, W), nhwc, ac0)
+        ctx.meta = (int(ignore), bool(seg_per_dataset), Cs, (h, w, H, W), nhwc, ac0)
         ctx.states = st
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         labels, ids, loss_px, lse_px, st, *srcs = ctx.saved_tensors
-        ignore, seg_per_dataset, Cs, dt, (h, w, H, W), nhwc, ac0 = ctx.meta
+        ignore, seg_per_dataset, Cs, (h, w, H, W), nhwc, ac0 = ctx.meta
         B = labels.shape[0]
-        n = len(Cs)
-        n_seg = n if seg_per_dataset else 1
-        g = _grad_scalar(grad_out, n_seg)
-        scratch = torch.empty(1, dtype=torch.float32, device=labels.device) if dt == torch.float32 else None
-        if nhwc:
-            return (None, None, None, None, None, None,
-                    *_up_ohem_ce_bwd_nhwc(srcs[0], labels, ids, loss_px, lse_px, st, g, scratch, ignore, seg_per_dataset,
-                                          Cs, dt, (h, w, H, W), ac0))
-        src = _src_table([s.data_ptr() for s in srcs], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset,
-                         cmax=scratch, cmax_ready=True)
-        # images of other datasets get a zero gradient (their rows are never selected, :1051): zero-initialised
-        # outputs, the kernel writes only the rows of a head's own images
-        grads = [torch.zeros_like(s) for s in srcs]
-        dst = _src_table([t.data_ptr() for t in grads], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset)
-        (_up_ce_adjoint_ac0 if ac0 else _up_ce_adjoint)(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st,
-                                                        g, dst)
+        dt, dev = srcs[0].dtype, labels.device
+        g = _grad_scalar(grad_out, len(Cs) if seg_per_dataset else 1)
+        scratch = torch.empty(1, dtype=torch.float32, device=dev) if dt == torch.float32 else None
+        if nhwc:  # d loss / d (the forward's planar rows), scattered into channels_last gradients at the end
+            src = _planes_table(srcs[0], Cs, seg_per_dataset, cmax=scratch, cmax_ready=True)
+        else:
+            src = _tensors_table(srcs, seg_per_dataset, cmax=scratch, cmax_ready=True)
+        if nhwc and not ac0 and _fused_adjoint(Cs, h, w, H, W, dt):
+            dp = torch.empty_like(srcs[0])  # the rows of image b's own head are written — and read
+            dst = _planes_table(dp, Cs, seg_per_dataset)
+        else:
+            # the routes that add two planes per head write dense [B, C_d, h, w] destinations whole; the fused kernel
+            # writes only the rows of a head's own images, so NCHW gradients start as zeros (images of other datasets
+            # get a zero gradient: their rows are never selected, :1051)
+            alloc = torch.empty if nhwc else torch.zeros
+            dp = [alloc(B, c, h, w, dtype=dt, device=dev) for c in Cs]
+            dst = _tensors_table(dp, seg_per_dataset)
+        _up_ce_adjoint(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g, dst, ac0)
+        if not nhwc:
+            return (None, None, None, None, None, None, *dp)
+        grads = [torch.empty((B, c, h, w), dtype=dt, device=dev, memory_format=torch.channels_last) for c in Cs]
+        N.call("mdseg_planar_to_nhwc", C.byref(dst), _ptr(ids), B, h, w, C.byref(_tensors_table(grads, seg_per_dataset)),
+               _stream())
         return (None, None, None, None, None, None, *grads)
-
-
-def _up_ohem_ce_bwd_nhwc(planar, labels, ids, loss_px, lse_px, st, g, scratch, ignore, seg_per_dataset, Cs, dt, shape,
-                         ac0=False):
-    """Gradients of _UpOhemCE's channels_last sources: d loss / d (planar rows) from mdseg_up_ce_bwd_direct (or
-    mdseg_up_ce_bwd_ac0), scattered into channels_last tensors (zeros for the images of other datasets)."""
-    h, w, H, W = shape
-    B, cm = planar.shape[:2]
-    n = len(Cs)
-    dev = planar.device
-    src = _src_table([planar.data_ptr()] * n, [cm * h * w] * n, Cs, _DT[dt], seg_per_dataset, c_alloc=cm, cmax=scratch,
-                     cmax_ready=True)
-    if not ac0 and N.lib.mdseg_up_ce_bwd_direct_is_fused(C.byref(src), h, w, H, W):
-        dp = torch.empty_like(planar)  # the rows of image b's own head are written — and read
-        dst = _src_table([dp.data_ptr()] * n, [cm * h * w] * n, Cs, _DT[dt], seg_per_dataset, c_alloc=cm)
-    else:  # the routes that add two planes per head: dense [B, C_d, h, w] destinations
-        dp = [torch.empty(B, c, h, w, dtype=dt, device=dev) for c in Cs]
-        dst = _src_table([t.data_ptr() for t in dp], [c * h * w for c in Cs], Cs, _DT[dt], seg_per_dataset)
-    (_up_ce_adjoint_ac0 if ac0 else _up_ce_adjoint)(src, ids, labels, (B, h, w, H, W), ignore, loss_px, lse_px, st, g,
-                                                    dst)
-    grads = [torch.empty((B, c, h, w), dtype=dt, device=dev, memory_format=torch.channels_last) for c in Cs]
-    gt = _src_table([t.data_ptr() for t in grads], [t.stride(0) for t in grads], Cs, _DT[dt], seg_per_dataset)
-    N.call("mdseg_planar_to_nhwc", C.byref(dst), _ptr(ids), B, h, w, C.byref(gt), _stream())
-    return grads
-
-
-def _up_ce_adjoint_ac0(src, ids, labels, shape, ignore, loss_px, lse_px, st, g, dst):
-    """mdseg_up_ce_bwd_ac0: the align_corners=False counterpart of _up_ce_adjoint (dense destinations)."""
-    B, h, w, H, W = shape
-    nbytes = N.lib.mdseg_up_ce_bwd_ac0_workspace_bytes(C.byref(src), B, h, w, H, W)
-    ws = torch.empty(nbytes, dtype=torch.uint8, device=labels.device)
-    N.call("mdseg_up_ce_bwd_ac0", C.byref(src), _ptr(ids), _ptr(labels), _DT[labels.dtype], B, h, w, H, W, ignore,
-           _ptr(loss_px), _ptr(lse_px), _ptr(st), _ptr(g), 1.0, C.byref(dst), _ptr(ws), nbytes, _stream())
 
 
 AC0_FACTORS = (2, 4, 8, 16)
