@@ -61,6 +61,97 @@ static inline int dtype_size(int d) {
   return 0;
 }
 
+// Type dispatch of a dtype code: f(type_tag<T>{}) for the C++ type T the code names, or error 2 naming the entry
+// point (who) and the parameter (what) for a code outside the set.
+template <typename T> struct type_tag { using type = T; };
+
+template <typename F>
+inline int with_float_type(int code, const char* who, const char* what, F&& f) {
+  switch (code) {
+    case MDSEG_F32: return f(type_tag<float>{});
+    case MDSEG_BF16: return f(type_tag<__nv_bfloat16>{});
+    case MDSEG_F16: return f(type_tag<__half>{});
+  }
+  set_error("%s: unsupported %s %d", who, what, code);
+  return 2;
+}
+
+template <typename F>
+inline int with_int_type(int code, const char* who, const char* what, F&& f) {
+  switch (code) {
+    case MDSEG_U8: return f(type_tag<uint8_t>{});
+    case MDSEG_I32: return f(type_tag<int32_t>{});
+    case MDSEG_I64: return f(type_tag<int64_t>{});
+  }
+  set_error("%s: unsupported %s %d", who, what, code);
+  return 2;
+}
+
+// Source tables: 1..MDSEG_MAX_DATASETS datasets ...
+inline bool src_count_ok(const mdseg_src_table* s) {
+  return s && s->n_datasets > 0 && s->n_datasets <= MDSEG_MAX_DATASETS;
+}
+// ... each with classes and a base pointer.
+inline int check_src(const mdseg_src_table* s, const char* who) {
+  MDSEG_REQUIRE(src_count_ok(s), "%s: bad source table", who);
+  for (int i = 0; i < s->n_datasets; ++i)
+    MDSEG_REQUIRE(s->C[i] > 0 && s->base[i] != nullptr, "%s: dataset %d has no source", who, i);
+  return 0;
+}
+// the widest class count of a source table
+inline int max_c(const mdseg_src_table* s) {
+  int m = 0;
+  for (int i = 0; i < s->n_datasets; ++i) m = s->C[i] > m ? s->C[i] : m;
+  return m;
+}
+
+// Graph tables: 1..MDSEG_MAX_DATASETS datasets onto C_uni > 0 unified classes.
+inline bool graph_header_ok(const mdseg_graph_table* t) {
+  return t && t->n_datasets > 0 && t->n_datasets <= MDSEG_MAX_DATASETS && t->C_uni > 0;
+}
+// the widest dataset class count C_ds of a graph table
+inline int max_c_ds(const mdseg_graph_table* t) {
+  int m = 0;
+  for (int i = 0; i < t->n_datasets; ++i) m = t->g[i].C_ds > m ? t->g[i].C_ds : m;
+  return m;
+}
+
+// The adjoint of a bilinear up-sampling writes the two vertical taps of every low-resolution cell into two fp32 planes
+// per dataset, A_d and B_d, each [n_images, C_d, h, w]; the gradient is their sum.  Bytes of that workspace:
+inline size_t two_plane_bytes(const mdseg_src_table* src, int n_images, int h, int w) {
+  size_t planes = 0;
+  for (int i = 0; i < src->n_datasets; ++i) planes += 2 * (size_t)n_images * src->C[i] * h * w * 4;
+  return planes + 256;
+}
+// Carves [A_d, B_d] out of the workspace, zeroes them when `zero`, runs adjoint(dA, dB) on the fp32 tables of the
+// planes and adds every pair into dst (dense [n_images, C_d, h, w] tensors of dst->dtype).
+template <typename Adjoint>
+int two_plane_adjoint(const char* who, const mdseg_src_table* src, const mdseg_src_table* dst, int n_images, int h,
+                      int w, void* workspace, bool zero, cudaStream_t s, Adjoint&& adjoint) {
+  const int64_t hw = (int64_t)h * w;
+  float* ws = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+  mdseg_src_table dA = *src, dB = *src;
+  dA.dtype = MDSEG_F32; dB.dtype = MDSEG_F32; dA.cmax = nullptr; dB.cmax = nullptr;
+  size_t off = 0;
+  for (int i = 0; i < src->n_datasets; ++i) {
+    const size_t n = (size_t)n_images * src->C[i] * hw;
+    dA.base[i] = ws + off; dB.base[i] = ws + off + n;
+    dA.image_stride[i] = (long long)src->C[i] * hw; dB.image_stride[i] = dA.image_stride[i];
+    dA.C_alloc[i] = src->C[i]; dB.C_alloc[i] = src->C[i];
+    off += 2 * n;
+  }
+  if (zero) MDSEG_CUDA_OK(cudaMemsetAsync(ws, 0, off * 4, s));
+  if (int rc = adjoint(dA, dB)) return rc;
+  for (int i = 0; i < src->n_datasets; ++i) {
+    MDSEG_REQUIRE(dst->image_stride[i] == (long long)src->C[i] * hw,
+                  "%s: the two-plane route needs dense [n_images, C, h, w] destinations", who);
+    if (int rc = mdseg_add_planes((const float*)dA.base[i], (const float*)dB.base[i], const_cast<void*>(dst->base[i]),
+                                  dst->dtype, (int64_t)n_images * src->C[i] * hw, s))
+      return rc;
+  }
+  return 0;
+}
+
 // ---- device side ---------------------------------------------------------
 constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;

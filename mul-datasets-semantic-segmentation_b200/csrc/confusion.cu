@@ -318,19 +318,6 @@ int launch_images(const void* label, const void* pred, const uint8_t* luts, cons
   return 0;
 }
 
-template <typename L>
-int dispatch_pred_images(const void* label, const void* pred, int pred_dtype, const uint8_t* luts, const int32_t* ids,
-                         int n_images, int64_t ppi, int64_t* hist, const mdseg_hist_table& tab, int ignore,
-                         int32_t* err_flag, cudaStream_t st) {
-  switch (pred_dtype) {
-    case MDSEG_U8: return launch_images<L, uint8_t>(label, pred, luts, ids, n_images, ppi, hist, tab, ignore, err_flag, st);
-    case MDSEG_I32: return launch_images<L, int32_t>(label, pred, luts, ids, n_images, ppi, hist, tab, ignore, err_flag, st);
-    case MDSEG_I64: return launch_images<L, int64_t>(label, pred, luts, ids, n_images, ppi, hist, tab, ignore, err_flag, st);
-  }
-  set_error("mdseg_confusion_images: unsupported pred_dtype %d", pred_dtype);
-  return 2;
-}
-
 template <typename L, typename P>
 int launch(const void* label, const void* pred, const uint8_t* lut, int64_t* hist, int Ca, int Cb, int ignore,
            int64_t n, int32_t* err_flag, cudaStream_t st) {
@@ -358,18 +345,6 @@ int launch(const void* label, const void* pred, const uint8_t* lut, int64_t* his
                                                   err_flag, replicas, aligned ? 1 : 0);
   MDSEG_LAUNCH_OK();
   return 0;
-}
-
-template <typename L>
-int dispatch_pred(const void* label, const void* pred, int pred_dtype, const uint8_t* lut, int64_t* hist, int Ca,
-                  int Cb, int ignore, int64_t n, int32_t* err_flag, cudaStream_t st) {
-  switch (pred_dtype) {
-    case MDSEG_U8: return launch<L, uint8_t>(label, pred, lut, hist, Ca, Cb, ignore, n, err_flag, st);
-    case MDSEG_I32: return launch<L, int32_t>(label, pred, lut, hist, Ca, Cb, ignore, n, err_flag, st);
-    case MDSEG_I64: return launch<L, int64_t>(label, pred, lut, hist, Ca, Cb, ignore, n, err_flag, st);
-  }
-  set_error("mdseg_confusion: unsupported pred_dtype %d", pred_dtype);
-  return 2;
 }
 
 // iou / mIoU on the device: one CTA; the final nanmean is a sequential double
@@ -407,13 +382,12 @@ extern "C" int mdseg_confusion(const void* label, int label_dtype, const void* p
   if (n == 0) return 0;
   MDSEG_REQUIRE(label && pred && hist && err_flag, "mdseg_confusion: null pointer (err_flag is required)");
   cudaStream_t st = (cudaStream_t)stream;
-  switch (label_dtype) {
-    case MDSEG_U8: return dispatch_pred<uint8_t>(label, pred, pred_dtype, lut256, hist, Ca, Cb, ignore, n, err_flag, st);
-    case MDSEG_I32: return dispatch_pred<int32_t>(label, pred, pred_dtype, lut256, hist, Ca, Cb, ignore, n, err_flag, st);
-    case MDSEG_I64: return dispatch_pred<int64_t>(label, pred, pred_dtype, lut256, hist, Ca, Cb, ignore, n, err_flag, st);
-  }
-  set_error("mdseg_confusion: unsupported label_dtype %d", label_dtype);
-  return 2;
+  return with_int_type(label_dtype, "mdseg_confusion", "label_dtype", [&](auto l) {
+    return with_int_type(pred_dtype, "mdseg_confusion", "pred_dtype", [&](auto p) {
+      return launch<typename decltype(l)::type, typename decltype(p)::type>(label, pred, lut256, hist, Ca, Cb, ignore,
+                                                                            n, err_flag, st);
+    });
+  });
 }
 
 extern "C" int mdseg_miou(const int64_t* hist, int C, float* iou, float* miou, void* stream) {
@@ -438,13 +412,12 @@ extern "C" int mdseg_confusion_images(const void* label, int label_dtype, const 
   MDSEG_REQUIRE(px_per_image % 16 == 0 && (((uintptr_t)label | (uintptr_t)pred) & 15) == 0,
                 "mdseg_confusion_images: images must be 16-element multiples and 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
-  switch (label_dtype) {
-    case MDSEG_U8: return dispatch_pred_images<uint8_t>(label, pred, pred_dtype, luts, dataset_ids, n_images, px_per_image, hist, *tab, ignore, err_flag, st);
-    case MDSEG_I32: return dispatch_pred_images<int32_t>(label, pred, pred_dtype, luts, dataset_ids, n_images, px_per_image, hist, *tab, ignore, err_flag, st);
-    case MDSEG_I64: return dispatch_pred_images<int64_t>(label, pred, pred_dtype, luts, dataset_ids, n_images, px_per_image, hist, *tab, ignore, err_flag, st);
-  }
-  set_error("mdseg_confusion_images: unsupported label_dtype %d", label_dtype);
-  return 2;
+  return with_int_type(label_dtype, "mdseg_confusion_images", "label_dtype", [&](auto l) {
+    return with_int_type(pred_dtype, "mdseg_confusion_images", "pred_dtype", [&](auto p) {
+      return launch_images<typename decltype(l)::type, typename decltype(p)::type>(
+          label, pred, luts, dataset_ids, n_images, px_per_image, hist, *tab, ignore, err_flag, st);
+    });
+  });
 }
 
 extern "C" int mdseg_miou_images(const int64_t* hist, const mdseg_hist_table* tab, float* iou, int iou_stride,

@@ -437,14 +437,12 @@ extern "C" int mdseg_eval_accum(const void* logits, int dtype, int C, int h, int
   AxisMap ym{axis_scale(h, H), h}, xm{axis_scale(w, W), w};
   cudaStream_t s = (cudaStream_t)stream;
   const int g = grid_for((int64_t)H * W);
-  switch (dtype) {
-    case MDSEG_F32: eval_accum_kernel<float><<<g, 256, 0, s>>>((const float*)logits, C, h, w, probs, H, W, ym, xm, flip, first); break;
-    case MDSEG_BF16: eval_accum_kernel<__nv_bfloat16><<<g, 256, 0, s>>>((const __nv_bfloat16*)logits, C, h, w, probs, H, W, ym, xm, flip, first); break;
-    case MDSEG_F16: eval_accum_kernel<__half><<<g, 256, 0, s>>>((const __half*)logits, C, h, w, probs, H, W, ym, xm, flip, first); break;
-    default: set_error("mdseg_eval_accum: unsupported dtype %d", dtype); return 2;
-  }
-  MDSEG_LAUNCH_OK();
-  return 0;
+  return with_float_type(dtype, "mdseg_eval_accum", "dtype", [&](auto t) {
+    using T = typename decltype(t)::type;
+    eval_accum_kernel<T><<<g, 256, 0, s>>>((const T*)logits, C, h, w, probs, H, W, ym, xm, flip, first);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 
 extern "C" int mdseg_argmax_hist(const float* probs, int C, int64_t n_px, int64_t* pred, const void* label,
@@ -457,13 +455,9 @@ extern "C" int mdseg_argmax_hist(const float* probs, int C, int64_t n_px, int64_
   if (n_px == 0) return 0;
   cudaStream_t s = (cudaStream_t)stream;
   if (!hist) return launch_argmax<uint8_t>(probs, C, n_px, pred, nullptr, nullptr, nullptr, ignore, err_flag, s);
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_argmax<uint8_t>(probs, C, n_px, pred, label, lut256, hist, ignore, err_flag, s);
-    case MDSEG_I32: return launch_argmax<int32_t>(probs, C, n_px, pred, label, lut256, hist, ignore, err_flag, s);
-    case MDSEG_I64: return launch_argmax<int64_t>(probs, C, n_px, pred, label, lut256, hist, ignore, err_flag, s);
-  }
-  set_error("mdseg_argmax_hist: unsupported label dtype %d", label_dtype);
-  return 2;
+  return with_int_type(label_dtype, "mdseg_argmax_hist", "label dtype", [&](auto l) {
+    return launch_argmax<typename decltype(l)::type>(probs, C, n_px, pred, label, lut256, hist, ignore, err_flag, s);
+  });
 }
 
 extern "C" int mdseg_label_nearest(const void* in, int dtype, int Hin, int Win, void* out, int Hout, int Wout,
@@ -475,14 +469,12 @@ extern "C" int mdseg_label_nearest(const void* in, int dtype, int Hin, int Win, 
   const float sy = (float)Hin / (float)Hout, sx = (float)Win / (float)Wout;
   const int g = grid_for((int64_t)n_images * Hout * Wout);
   cudaStream_t s = (cudaStream_t)stream;
-  switch (dtype) {
-    case MDSEG_U8: label_nearest_kernel<uint8_t><<<g, 256, 0, s>>>((const uint8_t*)in, Hin, Win, (uint8_t*)out, Hout, Wout, n_images, sy, sx); break;
-    case MDSEG_I32: label_nearest_kernel<int32_t><<<g, 256, 0, s>>>((const int32_t*)in, Hin, Win, (int32_t*)out, Hout, Wout, n_images, sy, sx); break;
-    case MDSEG_I64: label_nearest_kernel<int64_t><<<g, 256, 0, s>>>((const int64_t*)in, Hin, Win, (int64_t*)out, Hout, Wout, n_images, sy, sx); break;
-    default: set_error("mdseg_label_nearest: unsupported dtype %d", dtype); return 2;
-  }
-  MDSEG_LAUNCH_OK();
-  return 0;
+  return with_int_type(dtype, "mdseg_label_nearest", "dtype", [&](auto l) {
+    using L = typename decltype(l)::type;
+    label_nearest_kernel<L><<<g, 256, 0, s>>>((const L*)in, Hin, Win, (L*)out, Hout, Wout, n_images, sy, sx);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 
 namespace mdseg {
@@ -496,25 +488,17 @@ int launch_eval_fused(const EvalPassesDev& ps, int C, int H, int W, float2* stat
   if (staged) eval_stats_staged_kernel<T><<<dim3(grid.x, grid.y, (unsigned)ps.n), kEvThreads, 0, s>>>(ps, C, H, W, stats);
   else eval_stats_kernel<T><<<dim3(grid.x, grid.y, (unsigned)ps.n), kEvThreads, 0, s>>>(ps, C, H, W, stats);
   MDSEG_LAUNCH_OK();
-#define MDSEG_EVF(LT)                                                                                              \
-  do {                                                                                                             \
-    if (staged)                                                                                                    \
-      eval_fused_staged_kernel<T, LT><<<grid, kEvThreads, 0, s>>>(ps, C, H, W, stats, (long long*)pred,            \
-                                                                  (const LT*)label, lut, (unsigned long long*)hist, \
-                                                                  ignore, ef);                                     \
-    else                                                                                                           \
-      eval_fused_kernel<T, LT><<<grid, kEvThreads, 0, s>>>(ps, C, H, W, stats, (long long*)pred, (const LT*)label, \
-                                                           lut, (unsigned long long*)hist, ignore, ef);            \
-  } while (0)
-  switch (hist ? label_dtype : MDSEG_U8) {
-    case MDSEG_U8: MDSEG_EVF(uint8_t); break;
-    case MDSEG_I32: MDSEG_EVF(int32_t); break;
-    case MDSEG_I64: MDSEG_EVF(int64_t); break;
-    default: set_error("mdseg_eval_fused: unsupported label dtype %d", label_dtype); return 2;
-  }
-#undef MDSEG_EVF
-  MDSEG_LAUNCH_OK();
-  return 0;
+  return with_int_type(hist ? label_dtype : MDSEG_U8, "mdseg_eval_fused", "label dtype", [&](auto l) {
+    using L = typename decltype(l)::type;
+    if (staged)
+      eval_fused_staged_kernel<T, L><<<grid, kEvThreads, 0, s>>>(ps, C, H, W, stats, (long long*)pred, (const L*)label,
+                                                                 lut, (unsigned long long*)hist, ignore, ef);
+    else
+      eval_fused_kernel<T, L><<<grid, kEvThreads, 0, s>>>(ps, C, H, W, stats, (long long*)pred, (const L*)label, lut,
+                                                          (unsigned long long*)hist, ignore, ef);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 }  // namespace
 }  // namespace mdseg
@@ -549,10 +533,8 @@ extern "C" int mdseg_eval_fused(const mdseg_eval_passes* passes, int C, int H, i
   }
   float2* stats = reinterpret_cast<float2*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
   cudaStream_t s = (cudaStream_t)stream;
-  switch (passes->dtype) {
-    case MDSEG_F32: return launch_eval_fused<float>(ps, C, H, W, stats, pred, label, label_dtype, lut256, hist, ignore, err_flag, s);
-    case MDSEG_BF16: return launch_eval_fused<__nv_bfloat16>(ps, C, H, W, stats, pred, label, label_dtype, lut256, hist, ignore, err_flag, s);
-    case MDSEG_F16: return launch_eval_fused<__half>(ps, C, H, W, stats, pred, label, label_dtype, lut256, hist, ignore, err_flag, s);
-  }
-  return 2;
+  return with_float_type(passes->dtype, "mdseg_eval_fused", "dtype", [&](auto t) {
+    return launch_eval_fused<typename decltype(t)::type>(ps, C, H, W, stats, pred, label, label_dtype, lut256, hist,
+                                                         ignore, err_flag, s);
+  });
 }

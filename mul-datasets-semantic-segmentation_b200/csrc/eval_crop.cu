@@ -79,24 +79,13 @@ extern "C" int mdseg_eval_chip_accum(const void* logits, const void* logits_flip
   cudaStream_t s = (cudaStream_t)stream;
   int64_t bx = ceil_div64((int64_t)ch * cw, 256);
   if (bx > 8 * (int64_t)sm_count()) bx = 8 * (int64_t)sm_count();
-  switch (dtype) {
-    case MDSEG_F32:
-      chip_accum_kernel<float><<<(unsigned)bx, 256, 0, s>>>((const float*)logits, (const float*)logits_flip, C, ch, cw, probs,
-                                                            PH, PW, y0, x0, exp_after);
-      break;
-    case MDSEG_BF16:
-      chip_accum_kernel<__nv_bfloat16><<<(unsigned)bx, 256, 0, s>>>((const __nv_bfloat16*)logits,
-                                                                    (const __nv_bfloat16*)logits_flip, C, ch, cw, probs, PH,
-                                                                    PW, y0, x0, exp_after);
-      break;
-    case MDSEG_F16:
-      chip_accum_kernel<__half><<<(unsigned)bx, 256, 0, s>>>((const __half*)logits, (const __half*)logits_flip, C, ch, cw,
-                                                             probs, PH, PW, y0, x0, exp_after);
-      break;
-    default: MDSEG_REQUIRE(false, "mdseg_eval_chip_accum: unsupported dtype %d", dtype);
-  }
-  MDSEG_LAUNCH_OK();
-  return 0;
+  return with_float_type(dtype, "mdseg_eval_chip_accum", "dtype", [&](auto t) {
+    using T = typename decltype(t)::type;
+    chip_accum_kernel<T><<<(unsigned)bx, 256, 0, s>>>((const T*)logits, (const T*)logits_flip, C, ch, cw, probs, PH, PW,
+                                                      y0, x0, exp_after);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 
 extern "C" int mdseg_prob_resize_accum(const float* src, int C, int PH, int PW, int y0, int x0, int sh, int sw, float* dst,

@@ -259,18 +259,6 @@ int launch(const void* in, void* out, const uint8_t* lut, int oob, int64_t n, cu
   return 0;
 }
 
-template <typename In>
-int dispatch_out(const void* in, void* out, int out_dtype, const uint8_t* lut, int oob, int64_t n, cudaStream_t st,
-                 const int32_t* lut_ids = nullptr, int n_luts = 1, int n_images = 1, int* err_flag = nullptr) {
-  switch (out_dtype) {
-    case MDSEG_U8: return launch<In, uint8_t>(in, out, lut, oob, n, st, lut_ids, n_luts, n_images, err_flag);
-    case MDSEG_I32: return launch<In, int32_t>(in, out, lut, oob, n, st, lut_ids, n_luts, n_images, err_flag);
-    case MDSEG_I64: return launch<In, int64_t>(in, out, lut, oob, n, st, lut_ids, n_luts, n_images, err_flag);
-  }
-  set_error("mdseg_lut_remap: unsupported out_dtype %d", out_dtype);
-  return 2;
-}
-
 }  // namespace
 }  // namespace mdseg
 
@@ -280,13 +268,11 @@ extern "C" int mdseg_lut_remap(const void* in, int in_dtype, void* out, int out_
   MDSEG_REQUIRE(n >= 0, "mdseg_lut_remap: n < 0");
   MDSEG_REQUIRE(n == 0 || (in && out && lut256), "mdseg_lut_remap: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  switch (in_dtype) {
-    case MDSEG_U8: return dispatch_out<uint8_t>(in, out, out_dtype, lut256, oob, n, st);
-    case MDSEG_I32: return dispatch_out<int32_t>(in, out, out_dtype, lut256, oob, n, st);
-    case MDSEG_I64: return dispatch_out<int64_t>(in, out, out_dtype, lut256, oob, n, st);
-  }
-  set_error("mdseg_lut_remap: unsupported in_dtype %d", in_dtype);
-  return 2;
+  return with_int_type(in_dtype, "mdseg_lut_remap", "in_dtype", [&](auto i) {
+    return with_int_type(out_dtype, "mdseg_lut_remap", "out_dtype", [&](auto o) {
+      return launch<typename decltype(i)::type, typename decltype(o)::type>(in, out, lut256, oob, n, st);
+    });
+  });
 }
 
 extern "C" int mdseg_lut_remap_images(const void* in, int in_dtype, void* out, int out_dtype, const uint8_t* luts,
@@ -298,11 +284,10 @@ extern "C" int mdseg_lut_remap_images(const void* in, int in_dtype, void* out, i
   if (n_images == 0 || px_per_image == 0) return 0;
   MDSEG_REQUIRE(in && out && luts, "mdseg_lut_remap_images: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  switch (in_dtype) {
-    case MDSEG_U8: return dispatch_out<uint8_t>(in, out, out_dtype, luts, oob, px_per_image, st, lut_ids, n_luts, n_images, err_flag);
-    case MDSEG_I32: return dispatch_out<int32_t>(in, out, out_dtype, luts, oob, px_per_image, st, lut_ids, n_luts, n_images, err_flag);
-    case MDSEG_I64: return dispatch_out<int64_t>(in, out, out_dtype, luts, oob, px_per_image, st, lut_ids, n_luts, n_images, err_flag);
-  }
-  set_error("mdseg_lut_remap_images: unsupported in_dtype %d", in_dtype);
-  return 2;
+  return with_int_type(in_dtype, "mdseg_lut_remap_images", "in_dtype", [&](auto i) {
+    return with_int_type(out_dtype, "mdseg_lut_remap_images", "out_dtype", [&](auto o) {
+      return launch<typename decltype(i)::type, typename decltype(o)::type>(in, out, luts, oob, px_per_image, st,
+                                                                            lut_ids, n_luts, n_images, err_flag);
+    });
+  });
 }

@@ -856,15 +856,12 @@ bool row_route(const Args& a, bool ents_fit) {
 }
 
 template <typename TO>
-int launch(int label_dtype, const Maps& maps, const Args& a, int n_images, int max_c, bool ents_fit, cudaStream_t s) {
-  int rc = 2;
-  switch (label_dtype) {
-    case MDSEG_U8: rc = launch_prep<uint8_t>(a, n_images, s); break;
-    case MDSEG_I32: rc = launch_prep<int32_t>(a, n_images, s); break;
-    case MDSEG_I64: rc = launch_prep<int64_t>(a, n_images, s); break;
-    default: set_error("mdseg_mds_bwd: unsupported label dtype %d", label_dtype);
-  }
-  if (rc) return rc;
+int launch(const char* who, int label_dtype, const Maps& maps, const Args& a, int n_images, int max_c, bool ents_fit,
+           cudaStream_t s) {
+  if (int rc = with_int_type(label_dtype, who, "label dtype", [&](auto l) {
+        return launch_prep<typename decltype(l)::type>(a, n_images, s);
+      }))
+    return rc;
   if (row_route(a, ents_fit)) {
     const int n_w = a.gm.w / 32;
     if (a.col5 != nullptr && a.n_lite > 0) {
@@ -978,8 +975,8 @@ int setup_fused(const char* who, const mdseg_src_table* src, const int32_t* data
 extern "C" size_t mdseg_mds_bwd_workspace_bytes(const mdseg_src_table* src, const mdseg_graph_table* graphs,
                                                 int n_images, int h, int w, int H, int W) {
   using namespace mdseg;
-  if (!src || !graphs || src->n_datasets <= 0 || src->n_datasets > MDSEG_MAX_DATASETS ||
-      graphs->n_datasets != src->n_datasets || n_images <= 0 || h <= 0 || w <= 0 || H <= 0 || W <= 0)
+  if (!src_count_ok(src) || !graphs || graphs->n_datasets != src->n_datasets || n_images <= 0 || h <= 0 || w <= 0 ||
+      H <= 0 || W <= 0)
     return 256;
   const int c_max = max_c(src);
   const Geom gm = make_geom(h, w, H, W);
@@ -994,8 +991,7 @@ extern "C" int mdseg_mds_bwd(const mdseg_src_table* src, const mdseg_graph_table
                              const float* grad_out, float grad_scale, void* dx, int dx_dtype, void* workspace,
                              size_t workspace_bytes, void* stream) {
   using namespace mdseg;
-  MDSEG_REQUIRE(src && graphs && src->n_datasets > 0 && src->n_datasets <= MDSEG_MAX_DATASETS &&
-                    graphs->n_datasets == src->n_datasets && graphs->C_uni > 0,
+  MDSEG_REQUIRE(src_count_ok(src) && graph_header_ok(graphs) && graphs->n_datasets == src->n_datasets,
                 "mdseg_mds_bwd: bad source / graph table");
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && h > 0 && w > 0 && H > 0 && W > 0 && h <= 65535,
                 "mdseg_mds_bwd: bad shape");
@@ -1047,31 +1043,24 @@ extern "C" int mdseg_mds_bwd(const mdseg_src_table* src, const mdseg_graph_table
   a.zero_invalid = 1;
   bool ents_fit = true;  // a class group's (class, channel) pairs, each chunk padded to quads, within kEnt
   for (int i = 0; i < src->n_datasets; ++i) ents_fit = ents_fit && graphs->g[i].nnz + 8 <= kEnt;
-  switch (dx_dtype) {
-    case MDSEG_F32: return launch<float>(label_dtype, maps, a, n_images, c_max, ents_fit, s);
-    case MDSEG_BF16: return launch<__nv_bfloat16>(label_dtype, maps, a, n_images, c_max, ents_fit, s);
-    case MDSEG_F16: return launch<__half>(label_dtype, maps, a, n_images, c_max, ents_fit, s);
-  }
-  return 2;
+  return with_float_type(dx_dtype, "mdseg_mds_bwd", "gradient dtype", [&](auto t) {
+    return launch<typename decltype(t)::type>("mdseg_mds_bwd", label_dtype, maps, a, n_images, c_max, ents_fit, s);
+  });
 }
 
 // ---- the same kernel without a projection: aux heads (a10) and any direct upsample + CE --------------------
 extern "C" size_t mdseg_up_ce_bwd_direct_workspace_bytes(const mdseg_src_table* src, int n_images, int h, int w, int H,
                                                          int W) {
   using namespace mdseg;
-  if (!src || src->n_datasets <= 0 || src->n_datasets > MDSEG_MAX_DATASETS || n_images <= 0 || h <= 0 || w <= 0 ||
-      H <= 0 || W <= 0)
-    return 256;
+  if (!src_count_ok(src) || n_images <= 0 || h <= 0 || w <= 0 || H <= 0 || W <= 0) return 256;
   const Geom gm = make_geom(h, w, H, W);
   if (fused_geometry(src, gm)) return fused_workspace_bytes(n_images, gm, max_c(src));
-  size_t planes = 0;  // generic route: two fp32 planes per dataset, [n_images, C_d, h, w] each
-  for (int i = 0; i < src->n_datasets; ++i) planes += 2 * (size_t)n_images * src->C[i] * h * w * 4;
-  return planes + 256;
+  return two_plane_bytes(src, n_images, h, w);
 }
 
 extern "C" int mdseg_up_ce_bwd_direct_is_fused(const mdseg_src_table* src, int h, int w, int H, int W) {
   using namespace mdseg;
-  if (!src || src->n_datasets <= 0 || src->n_datasets > MDSEG_MAX_DATASETS || h <= 0 || w <= 0 || H <= 0 || W <= 0) return 0;
+  if (!src_count_ok(src) || h <= 0 || w <= 0 || H <= 0 || W <= 0) return 0;
   return fused_geometry(src, make_geom(h, w, H, W)) ? 1 : 0;
 }
 
@@ -1081,8 +1070,7 @@ extern "C" int mdseg_up_ce_bwd_direct(const mdseg_src_table* src, const int32_t*
                                       const float* grad_out, float grad_scale, const mdseg_src_table* dst,
                                       void* workspace, size_t workspace_bytes, void* stream) {
   using namespace mdseg;
-  MDSEG_REQUIRE(src && dst && src->n_datasets > 0 && src->n_datasets <= MDSEG_MAX_DATASETS &&
-                    dst->n_datasets == src->n_datasets && is_float_dtype(dst->dtype),
+  MDSEG_REQUIRE(src_count_ok(src) && dst && dst->n_datasets == src->n_datasets && is_float_dtype(dst->dtype),
                 "mdseg_up_ce_bwd_direct: bad source / destination table");
   for (int i = 0; i < src->n_datasets; ++i)
     MDSEG_REQUIRE(dst->base[i] && dst->C[i] == src->C[i], "mdseg_up_ce_bwd_direct: destination %d does not match", i);
@@ -1093,36 +1081,19 @@ extern "C" int mdseg_up_ce_bwd_direct(const mdseg_src_table* src, const int32_t*
   MDSEG_REQUIRE(workspace_bytes >= mdseg_up_ce_bwd_direct_workspace_bytes(src, n_images, h, w, H, W),
                 "mdseg_up_ce_bwd_direct: workspace too small");
   cudaStream_t s = (cudaStream_t)stream;
-  const int64_t hw = (int64_t)h * w;
   const Geom gm = make_geom(h, w, H, W);
-  float* ws = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
 
   if (!fused_geometry(src, gm)) {
     // generic route: two planes per dataset (zero for the images of other datasets), then their sum
-    mdseg_src_table dA = *src, dB = *src;
-    dA.dtype = MDSEG_F32; dB.dtype = MDSEG_F32; dA.cmax = nullptr; dB.cmax = nullptr;
-    size_t off = 0;
-    for (int i = 0; i < src->n_datasets; ++i) {
-      const size_t n = (size_t)n_images * src->C[i] * hw;
-      dA.base[i] = ws + off; dB.base[i] = ws + off + n;
-      dA.image_stride[i] = (long long)src->C[i] * hw; dB.image_stride[i] = dA.image_stride[i];
-      dA.C_alloc[i] = src->C[i]; dB.C_alloc[i] = src->C[i];
-      off += 2 * n;
-    }
-    MDSEG_CUDA_OK(cudaMemsetAsync(ws, 0, off * 4, s));
-    if (int rc = mdseg_up_ce_bwd(src, dataset_ids, labels, label_dtype, n_images, h, w, H, W, ignore, loss_px, lse_px,
-                                 states, grad_out, grad_scale, &dA, &dB, stream))
-      return rc;
-    for (int i = 0; i < src->n_datasets; ++i) {
-      MDSEG_REQUIRE(dst->image_stride[i] == (long long)src->C[i] * hw,
-                    "mdseg_up_ce_bwd_direct: the generic route needs dense [n_images, C, h, w] destinations");
-      if (int rc = mdseg_add_planes((const float*)dA.base[i], (const float*)dB.base[i], const_cast<void*>(dst->base[i]),
-                                    dst->dtype, (int64_t)n_images * src->C[i] * hw, stream))
-        return rc;
-    }
-    return 0;
+    return two_plane_adjoint("mdseg_up_ce_bwd_direct", src, dst, n_images, h, w, workspace, true, s,
+                             [&](const mdseg_src_table& dA, const mdseg_src_table& dB) {
+                               return mdseg_up_ce_bwd(src, dataset_ids, labels, label_dtype, n_images, h, w, H, W,
+                                                      ignore, loss_px, lse_px, states, grad_out, grad_scale, &dA, &dB,
+                                                      stream);
+                             });
   }
 
+  float* ws = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
   Args a;
   Maps maps;
   if (int rc = setup_fused("mdseg_up_ce_bwd_direct", src, dataset_ids, labels, gm, n_images, ignore, loss_px, lse_px,
@@ -1137,10 +1108,8 @@ extern "C" int mdseg_up_ce_bwd_direct(const mdseg_src_table* src, const int32_t*
   }
   a.zero_invalid = 0;  // rows of images that do not belong to a head stay as the caller initialised them
   const int c_max = max_c(src);
-  switch (dst->dtype) {  // identity channel lists: 16 entries per class group
-    case MDSEG_F32: return launch<float>(label_dtype, maps, a, n_images, c_max, true, s);
-    case MDSEG_BF16: return launch<__nv_bfloat16>(label_dtype, maps, a, n_images, c_max, true, s);
-    case MDSEG_F16: return launch<__half>(label_dtype, maps, a, n_images, c_max, true, s);
-  }
-  return 2;
+  // identity channel lists: 16 entries per class group
+  return with_float_type(dst->dtype, "mdseg_up_ce_bwd_direct", "destination dtype", [&](auto t) {
+    return launch<typename decltype(t)::type>("mdseg_up_ce_bwd_direct", label_dtype, maps, a, n_images, c_max, true, s);
+  });
 }

@@ -86,11 +86,7 @@ extern "C" int mdseg_multihot_remap(const void* labels, int label_dtype, const u
   MDSEG_REQUIRE(labels && table && out, "mdseg_multihot_remap: null pointer");
   MDSEG_REQUIRE(((uintptr_t)out & 15) == 0, "mdseg_multihot_remap: out must be 16-byte aligned");
   cudaStream_t s = (cudaStream_t)stream;
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_multihot<uint8_t>(labels, table, C_uni, n_px, out, s);
-    case MDSEG_I32: return launch_multihot<int32_t>(labels, table, C_uni, n_px, out, s);
-    case MDSEG_I64: return launch_multihot<int64_t>(labels, table, C_uni, n_px, out, s);
-  }
-  set_error("mdseg_multihot_remap: unsupported label dtype %d", label_dtype);
-  return 2;
+  return with_int_type(label_dtype, "mdseg_multihot_remap", "label dtype", [&](auto l) {
+    return launch_multihot<typename decltype(l)::type>(labels, table, C_uni, n_px, out, s);
+  });
 }

@@ -195,14 +195,12 @@ extern "C" int mdseg_softmax_nchw(const void* x, int dtype, int n_images, int C,
   int64_t bx = ceil_div64(hw, 256);
   if (bx > 65535) bx = 65535;
   dim3 grid((unsigned)bx, (unsigned)n_images);
-  switch (dtype) {
-    case MDSEG_F32: softmax_nchw_kernel<float><<<grid, 256, 0, s>>>((const float*)x, C, hw, pred); break;
-    case MDSEG_BF16: softmax_nchw_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>((const __nv_bfloat16*)x, C, hw, pred); break;
-    case MDSEG_F16: softmax_nchw_kernel<__half><<<grid, 256, 0, s>>>((const __half*)x, C, hw, pred); break;
-    default: MDSEG_REQUIRE(false, "mdseg_softmax_nchw: unsupported dtype %d", dtype);
-  }
-  MDSEG_LAUNCH_OK();
-  return 0;
+  return with_float_type(dtype, "mdseg_softmax_nchw", "dtype", [&](auto t) {
+    using T = typename decltype(t)::type;
+    softmax_nchw_kernel<T><<<grid, 256, 0, s>>>((const T*)x, C, hw, pred);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 
 extern "C" int mdseg_softmax_bwd_nchw(const float* pred, const float* dpred, int n_images, int C, int64_t hw, void* dx,
@@ -215,21 +213,19 @@ extern "C" int mdseg_softmax_bwd_nchw(const float* pred, const float* dpred, int
   int64_t bx = ceil_div64(hw, 256);
   if (bx > 65535) bx = 65535;
   dim3 grid((unsigned)bx, (unsigned)n_images);
-  switch (dx_dtype) {
-    case MDSEG_F32: softmax_bwd_nchw_kernel<float><<<grid, 256, 0, s>>>(pred, dpred, C, hw, (float*)dx); break;
-    case MDSEG_BF16: softmax_bwd_nchw_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(pred, dpred, C, hw, (__nv_bfloat16*)dx); break;
-    case MDSEG_F16: softmax_bwd_nchw_kernel<__half><<<grid, 256, 0, s>>>(pred, dpred, C, hw, (__half*)dx); break;
-    default: MDSEG_REQUIRE(false, "mdseg_softmax_bwd_nchw: unsupported dtype %d", dx_dtype);
-  }
-  MDSEG_LAUNCH_OK();
-  return 0;
+  return with_float_type(dx_dtype, "mdseg_softmax_bwd_nchw", "dx_dtype", [&](auto t) {
+    using T = typename decltype(t)::type;
+    softmax_bwd_nchw_kernel<T><<<grid, 256, 0, s>>>(pred, dpred, C, hw, (T*)dx);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 
 extern "C" int mdseg_up_nll_fwd(const mdseg_src_table* src, const int32_t* dataset_ids, const void* labels, int label_dtype,
                                 int n_images, int h, int w, int H, int W, int ignore, float* loss_px,
                                 mdseg_ohem_state* states, int32_t* err_flag, void* stream) {
   using namespace mdseg;
-  MDSEG_REQUIRE(src && src->n_datasets > 0 && src->n_datasets <= MDSEG_MAX_DATASETS && src->dtype == MDSEG_F32,
+  MDSEG_REQUIRE(src_count_ok(src) && src->dtype == MDSEG_F32,
                 "mdseg_up_nll_fwd: the projected probabilities must be an fp32 source table");
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && h > 0 && w > 0 && H > 0 && W > 0, "mdseg_up_nll_fwd: bad shape");
   if (n_images == 0) return 0;
@@ -239,12 +235,8 @@ extern "C" int mdseg_up_nll_fwd(const mdseg_src_table* src, const int32_t* datas
   a.ignore = ignore; a.loss_px = loss_px; a.states = states; a.grad_out = nullptr; a.grad_scale = 1.f;
   a.err_flag = err_flag;
   cudaStream_t s = (cudaStream_t)stream;
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_fwd<uint8_t>(a, n_images, s);
-    case MDSEG_I32: return launch_fwd<int32_t>(a, n_images, s);
-    case MDSEG_I64: return launch_fwd<int64_t>(a, n_images, s);
-  }
-  MDSEG_REQUIRE(false, "mdseg_up_nll_fwd: unsupported label dtype %d", label_dtype);
+  return with_int_type(label_dtype, "mdseg_up_nll_fwd", "label dtype",
+                       [&](auto l) { return launch_fwd<typename decltype(l)::type>(a, n_images, s); });
 }
 
 extern "C" int mdseg_up_nll_bwd(const mdseg_src_table* src, const int32_t* dataset_ids, const void* labels, int label_dtype,
@@ -252,8 +244,7 @@ extern "C" int mdseg_up_nll_bwd(const mdseg_src_table* src, const int32_t* datas
                                 const mdseg_ohem_state* states, const float* grad_out, float grad_scale,
                                 const mdseg_src_table* dst, void* stream) {
   using namespace mdseg;
-  MDSEG_REQUIRE(src && dst && src->n_datasets > 0 && src->n_datasets <= MDSEG_MAX_DATASETS &&
-                    dst->n_datasets == src->n_datasets && dst->dtype == MDSEG_F32,
+  MDSEG_REQUIRE(src_count_ok(src) && dst && dst->n_datasets == src->n_datasets && dst->dtype == MDSEG_F32,
                 "mdseg_up_nll_bwd: bad source / destination table");
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && h > 0 && h <= 65535 && w > 0 && H > 0 && W > 0,
                 "mdseg_up_nll_bwd: bad shape");
@@ -264,10 +255,6 @@ extern "C" int mdseg_up_nll_bwd(const mdseg_src_table* src, const int32_t* datas
   a.ignore = ignore; a.loss_px = const_cast<float*>(loss_px); a.states = const_cast<mdseg_ohem_state*>(states);
   a.grad_out = grad_out; a.grad_scale = grad_scale; a.err_flag = nullptr;
   cudaStream_t s = (cudaStream_t)stream;
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_bwd<uint8_t>(a, n_images, s);
-    case MDSEG_I32: return launch_bwd<int32_t>(a, n_images, s);
-    case MDSEG_I64: return launch_bwd<int64_t>(a, n_images, s);
-  }
-  MDSEG_REQUIRE(false, "mdseg_up_nll_bwd: unsupported label dtype %d", label_dtype);
+  return with_int_type(label_dtype, "mdseg_up_nll_bwd", "label dtype",
+                       [&](auto l) { return launch_bwd<typename decltype(l)::type>(a, n_images, s); });
 }

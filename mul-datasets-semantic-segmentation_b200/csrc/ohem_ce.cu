@@ -484,30 +484,6 @@ int launch_bwd(const void* logits, int layout, const void* labels, int N, int C,
   return 0;
 }
 
-template <typename T>
-int fwd_labels(int label_dtype, const void* logits, int layout, const void* labels, int N, int C, int H, int W,
-               int ignore, float* loss_px, float* lse_px, mdseg_ohem_state* st, int32_t* ef, cudaStream_t s) {
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_fwd<T, uint8_t>(logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, st, ef, s);
-    case MDSEG_I32: return launch_fwd<T, int32_t>(logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, st, ef, s);
-    case MDSEG_I64: return launch_fwd<T, int64_t>(logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, st, ef, s);
-  }
-  set_error("mdseg_ohem_ce_fwd: unsupported label dtype %d", label_dtype);
-  return 2;
-}
-template <typename T>
-int bwd_labels(int label_dtype, const void* logits, int layout, const void* labels, int N, int C, int H, int W,
-               int ignore, const float* loss_px, const float* lse_px, mdseg_ohem_state* st, const float* go, float gs,
-               void* dl, cudaStream_t s) {
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_bwd<T, uint8_t>(logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, st, go, gs, dl, s);
-    case MDSEG_I32: return launch_bwd<T, int32_t>(logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, st, go, gs, dl, s);
-    case MDSEG_I64: return launch_bwd<T, int64_t>(logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, st, go, gs, dl, s);
-  }
-  set_error("mdseg_ohem_ce_bwd: unsupported label dtype %d", label_dtype);
-  return 2;
-}
-
 }  // namespace
 }  // namespace mdseg
 
@@ -520,13 +496,12 @@ extern "C" int mdseg_ohem_ce_fwd(const void* logits, int dtype, int layout, cons
   if ((int64_t)N * H * W == 0) return 0;
   MDSEG_REQUIRE(logits && labels && loss_px && lse_px && state && err_flag, "mdseg_ohem_ce_fwd: null pointer");
   cudaStream_t s = (cudaStream_t)stream;
-  switch (dtype) {
-    case MDSEG_F32: return fwd_labels<float>(label_dtype, logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, state, err_flag, s);
-    case MDSEG_BF16: return fwd_labels<__nv_bfloat16>(label_dtype, logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, state, err_flag, s);
-    case MDSEG_F16: return fwd_labels<__half>(label_dtype, logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, state, err_flag, s);
-  }
-  set_error("mdseg_ohem_ce_fwd: unsupported dtype %d", dtype);
-  return 2;
+  return with_float_type(dtype, "mdseg_ohem_ce_fwd", "dtype", [&](auto t) {
+    return with_int_type(label_dtype, "mdseg_ohem_ce_fwd", "label dtype", [&](auto l) {
+      return launch_fwd<typename decltype(t)::type, typename decltype(l)::type>(
+          logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, state, err_flag, s);
+    });
+  });
 }
 
 extern "C" int mdseg_ohem_ce_bwd(const void* logits, int dtype, int layout, const void* labels, int label_dtype,
@@ -539,11 +514,10 @@ extern "C" int mdseg_ohem_ce_bwd(const void* logits, int dtype, int layout, cons
   if ((int64_t)N * H * W == 0) return 0;
   MDSEG_REQUIRE(logits && labels && loss_px && lse_px && state && dlogits, "mdseg_ohem_ce_bwd: null pointer");
   cudaStream_t s = (cudaStream_t)stream;
-  switch (dtype) {
-    case MDSEG_F32: return bwd_labels<float>(label_dtype, logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, state, grad_out, grad_scale, dlogits, s);
-    case MDSEG_BF16: return bwd_labels<__nv_bfloat16>(label_dtype, logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, state, grad_out, grad_scale, dlogits, s);
-    case MDSEG_F16: return bwd_labels<__half>(label_dtype, logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, state, grad_out, grad_scale, dlogits, s);
-  }
-  set_error("mdseg_ohem_ce_bwd: unsupported dtype %d", dtype);
-  return 2;
+  return with_float_type(dtype, "mdseg_ohem_ce_bwd", "dtype", [&](auto t) {
+    return with_int_type(label_dtype, "mdseg_ohem_ce_bwd", "label dtype", [&](auto l) {
+      return launch_bwd<typename decltype(t)::type, typename decltype(l)::type>(
+          logits, layout, labels, N, C, H, W, ignore, loss_px, lse_px, state, grad_out, grad_scale, dlogits, s);
+    });
+  });
 }

@@ -327,15 +327,8 @@ bool any_sparse(const mdseg_graph_table* t) {
     if (!t->g[i].dense) return true;
   return false;
 }
-int max_cds(const mdseg_graph_table* t) {
-  int m = 0;
-  for (int i = 0; i < t->n_datasets; ++i) m = t->g[i].C_ds > m ? t->g[i].C_ds : m;
-  return m;
-}
-
 int check_table(const mdseg_graph_table* t, const char* who) {
-  MDSEG_REQUIRE(t && t->n_datasets > 0 && t->n_datasets <= MDSEG_MAX_DATASETS && t->C_uni > 0,
-                "%s: bad graph table", who);
+  MDSEG_REQUIRE(graph_header_ok(t), "%s: bad graph table", who);
   for (int i = 0; i < t->n_datasets; ++i) {
     const mdseg_sparse_graph& g = t->g[i];
     MDSEG_REQUIRE(g.C_ds > 0, "%s: dataset %d has C_ds <= 0", who, i);
@@ -361,7 +354,7 @@ int launch_fwd(const void* x, const mdseg_graph_table* t, const int32_t* ids, in
     MDSEG_LAUNCH_OK();
   }
   if (any_dense(t, skip_mask)) {
-    dim3 grid((unsigned)ceil_div64(hw, kTP), (unsigned)((max_cds(t) + kTO - 1) / kTO), (unsigned)n_images);
+    dim3 grid((unsigned)ceil_div64(hw, kTP), (unsigned)((max_c_ds(t) + kTO - 1) / kTO), (unsigned)n_images);
     proj_dense_kernel<T, float, true><<<grid, 256, 0, s>>>((const T*)x, nullptr, *t, ids, hw, t->C_uni, y_cmax, y,
                                                            skip_mask);
     MDSEG_LAUNCH_OK();
@@ -399,7 +392,7 @@ int launch_dgraph(const void* x, const float* dyA, const float* dyB, int y_cmax,
   // pixel slabs: enough CTAs to fill the chip, at least 2048 px each
   int64_t slab = 2048;
   const int n_slabs = (int)ceil_div64(hw, slab);
-  dim3 grid((unsigned)((t->C_uni + 31) / 32), (unsigned)((max_cds(t) + 31) / 32), (unsigned)(n_images * n_slabs));
+  dim3 grid((unsigned)((t->C_uni + 31) / 32), (unsigned)((max_c_ds(t) + 31) / 32), (unsigned)(n_images * n_slabs));
   proj_dgraph_kernel<T><<<grid, 256, 0, s>>>((const T*)x, dyA, dyB, y_cmax, *t, ids, hw, slab, dG, dg_stride,
                                              skip_mask);
   MDSEG_LAUNCH_OK();
@@ -416,17 +409,14 @@ int proj_fwd_rest(const void* x, int dtype, const mdseg_graph_table* graphs, con
                   cudaStream_t s) {
   if (int rc = check_table(graphs, "mdseg_proj_fwd")) return rc;
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && h > 0 && w > 0, "mdseg_proj_fwd: bad shape");
-  MDSEG_REQUIRE(y_cmax >= max_cds(graphs), "mdseg_proj_fwd: y_cmax %d < max C_ds %d", y_cmax, max_cds(graphs));
+  MDSEG_REQUIRE(y_cmax >= max_c_ds(graphs), "mdseg_proj_fwd: y_cmax %d < max C_ds %d", y_cmax, max_c_ds(graphs));
   if (n_images == 0) return 0;
   MDSEG_REQUIRE(x && y, "mdseg_proj_fwd: null pointer");
   const int64_t hw = (int64_t)h * w;
-  switch (dtype) {
-    case MDSEG_F32: return launch_fwd<float>(x, graphs, dataset_ids, n_images, hw, y, y_cmax, cmax_out, err_flag, skip_mask, s);
-    case MDSEG_BF16: return launch_fwd<__nv_bfloat16>(x, graphs, dataset_ids, n_images, hw, y, y_cmax, cmax_out, err_flag, skip_mask, s);
-    case MDSEG_F16: return launch_fwd<__half>(x, graphs, dataset_ids, n_images, hw, y, y_cmax, cmax_out, err_flag, skip_mask, s);
-  }
-  set_error("mdseg_proj_fwd: unsupported dtype %d", dtype);
-  return 2;
+  return with_float_type(dtype, "mdseg_proj_fwd", "dtype", [&](auto t) {
+    return launch_fwd<typename decltype(t)::type>(x, graphs, dataset_ids, n_images, hw, y, y_cmax, cmax_out, err_flag,
+                                                  skip_mask, s);
+  });
 }
 }  // namespace mdseg
 
@@ -447,13 +437,10 @@ int proj_bwd_rest(const float* dyA, const float* dyB, int y_cmax, const mdseg_gr
   if (n_images == 0) return 0;
   MDSEG_REQUIRE(dyA && dx, "mdseg_proj_bwd: null pointer");
   const int64_t hw = (int64_t)h * w;
-  switch (dtype) {
-    case MDSEG_F32: return launch_bwd<float>(dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dx, skip_mask, s);
-    case MDSEG_BF16: return launch_bwd<__nv_bfloat16>(dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dx, skip_mask, s);
-    case MDSEG_F16: return launch_bwd<__half>(dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dx, skip_mask, s);
-  }
-  set_error("mdseg_proj_bwd: unsupported dtype %d", dtype);
-  return 2;
+  return with_float_type(dtype, "mdseg_proj_bwd", "dtype", [&](auto t) {
+    return launch_bwd<typename decltype(t)::type>(dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dx, skip_mask,
+                                                  s);
+  });
 }
 }  // namespace mdseg
 
@@ -477,13 +464,10 @@ int proj_dgraph_rest(const void* x, int dtype, const float* dyA, const float* dy
   bool any = false;
   for (int i = 0; i < graphs->n_datasets; ++i) any = any || !((skip_mask >> i) & 1u);
   if (!any) return 0;
-  switch (dtype) {
-    case MDSEG_F32: return launch_dgraph<float>(x, dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dG, dg_stride, skip_mask, s);
-    case MDSEG_BF16: return launch_dgraph<__nv_bfloat16>(x, dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dG, dg_stride, skip_mask, s);
-    case MDSEG_F16: return launch_dgraph<__half>(x, dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dG, dg_stride, skip_mask, s);
-  }
-  set_error("mdseg_proj_bwd_graph: unsupported dtype %d", dtype);
-  return 2;
+  return with_float_type(dtype, "mdseg_proj_bwd_graph", "dtype", [&](auto t) {
+    return launch_dgraph<typename decltype(t)::type>(x, dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dG,
+                                                     dg_stride, skip_mask, s);
+  });
 }
 }  // namespace mdseg
 

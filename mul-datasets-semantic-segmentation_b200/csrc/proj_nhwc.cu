@@ -229,8 +229,7 @@ nhwc_planar_kernel(const mdseg_src_table nhwc, const mdseg_src_table planar, con
 }
 
 int check_sparse_table(const mdseg_graph_table* t, const char* who) {
-  MDSEG_REQUIRE(t && t->n_datasets > 0 && t->n_datasets <= MDSEG_MAX_DATASETS && t->C_uni > 0 &&
-                    t->C_uni <= MDSEG_NHWC_MAX_CUNI,
+  MDSEG_REQUIRE(graph_header_ok(t) && t->C_uni <= MDSEG_NHWC_MAX_CUNI,
                 "%s: bad graph table (C_uni must be in [1, %d])", who, MDSEG_NHWC_MAX_CUNI);
   for (int i = 0; i < t->n_datasets; ++i) {
     const mdseg_sparse_graph& g = t->g[i];
@@ -240,12 +239,6 @@ int check_sparse_table(const mdseg_graph_table* t, const char* who) {
                   "%s: dataset %d needs a sparse graph (dense graphs take the NCHW kernels)", who, i);
   }
   return 0;
-}
-
-int max_c_ds(const mdseg_graph_table* t) {
-  int m = 0;
-  for (int i = 0; i < t->n_datasets; ++i) m = t->g[i].C_ds > m ? t->g[i].C_ds : m;
-  return m;
 }
 
 template <typename T>
@@ -276,8 +269,7 @@ int launch_bwd(const float* dyA, const float* dyB, int y_cmax, const mdseg_graph
 template <bool kToPlanar>
 int launch_move(const mdseg_src_table* nhwc, const mdseg_src_table* planar, const int32_t* ids, int n_images, int h,
                 int w, cudaStream_t s, const char* who) {
-  MDSEG_REQUIRE(nhwc && planar && nhwc->n_datasets > 0 && nhwc->n_datasets <= MDSEG_MAX_DATASETS &&
-                    planar->n_datasets == nhwc->n_datasets && planar->dtype == nhwc->dtype,
+  MDSEG_REQUIRE(src_count_ok(nhwc) && planar && planar->n_datasets == nhwc->n_datasets && planar->dtype == nhwc->dtype,
                 "%s: bad source / destination table", who);
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && h > 0 && w > 0, "%s: bad shape", who);
   if (n_images == 0) return 0;
@@ -291,14 +283,11 @@ int launch_move(const mdseg_src_table* nhwc, const mdseg_src_table* planar, cons
   }
   MDSEG_REQUIRE(ceil_div64(hw, 32) <= 0x7fffffff, "%s: image too large", who);
   dim3 grid((unsigned)ceil_div64(hw, 32), (unsigned)((cm + 31) / 32), (unsigned)n_images);
-  switch (nhwc->dtype) {
-    case MDSEG_F32: nhwc_planar_kernel<float, kToPlanar><<<grid, kThreads, 0, s>>>(*nhwc, *planar, ids, hw); break;
-    case MDSEG_BF16: nhwc_planar_kernel<__nv_bfloat16, kToPlanar><<<grid, kThreads, 0, s>>>(*nhwc, *planar, ids, hw); break;
-    case MDSEG_F16: nhwc_planar_kernel<__half, kToPlanar><<<grid, kThreads, 0, s>>>(*nhwc, *planar, ids, hw); break;
-    default: set_error("%s: unsupported dtype %d", who, nhwc->dtype); return 2;
-  }
-  MDSEG_LAUNCH_OK();
-  return 0;
+  return with_float_type(nhwc->dtype, who, "dtype", [&](auto t) {
+    nhwc_planar_kernel<typename decltype(t)::type, kToPlanar><<<grid, kThreads, 0, s>>>(*nhwc, *planar, ids, hw);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 
 }  // namespace
@@ -315,13 +304,10 @@ extern "C" int mdseg_proj_fwd_nhwc(const void* x, int dtype, const mdseg_graph_t
   MDSEG_REQUIRE(x && y, "mdseg_proj_fwd_nhwc: null pointer");
   const int64_t hw = (int64_t)h * w;
   cudaStream_t s = (cudaStream_t)stream;
-  switch (dtype) {
-    case MDSEG_F32: return launch_fwd<float>(x, graphs, dataset_ids, n_images, hw, y, y_cmax, cmax_out, err_flag, s);
-    case MDSEG_BF16: return launch_fwd<__nv_bfloat16>(x, graphs, dataset_ids, n_images, hw, y, y_cmax, cmax_out, err_flag, s);
-    case MDSEG_F16: return launch_fwd<__half>(x, graphs, dataset_ids, n_images, hw, y, y_cmax, cmax_out, err_flag, s);
-  }
-  set_error("mdseg_proj_fwd_nhwc: unsupported dtype %d", dtype);
-  return 2;
+  return with_float_type(dtype, "mdseg_proj_fwd_nhwc", "dtype", [&](auto t) {
+    return launch_fwd<typename decltype(t)::type>(x, graphs, dataset_ids, n_images, hw, y, y_cmax, cmax_out, err_flag,
+                                                  s);
+  });
 }
 
 extern "C" int mdseg_proj_bwd_nhwc(const float* dyA, const float* dyB, int y_cmax, const mdseg_graph_table* graphs,
@@ -335,13 +321,9 @@ extern "C" int mdseg_proj_bwd_nhwc(const float* dyA, const float* dyB, int y_cma
   MDSEG_REQUIRE(dyA && dx, "mdseg_proj_bwd_nhwc: null pointer");
   const int64_t hw = (int64_t)h * w;
   cudaStream_t s = (cudaStream_t)stream;
-  switch (dtype) {
-    case MDSEG_F32: return launch_bwd<float>(dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dx, s);
-    case MDSEG_BF16: return launch_bwd<__nv_bfloat16>(dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dx, s);
-    case MDSEG_F16: return launch_bwd<__half>(dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dx, s);
-  }
-  set_error("mdseg_proj_bwd_nhwc: unsupported dtype %d", dtype);
-  return 2;
+  return with_float_type(dtype, "mdseg_proj_bwd_nhwc", "dtype", [&](auto t) {
+    return launch_bwd<typename decltype(t)::type>(dyA, dyB, y_cmax, graphs, dataset_ids, n_images, hw, dx, s);
+  });
 }
 
 extern "C" int mdseg_nhwc_to_planar(const mdseg_src_table* nhwc, const int32_t* dataset_ids, int n_images, int h, int w,

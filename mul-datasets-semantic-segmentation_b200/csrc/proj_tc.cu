@@ -19,6 +19,8 @@
 // products of weight >= 2^-16 are accumulated (relative error ~2^-21, inside the 1e-5 parity bar without
 // giving up fp32's range); bf16 / fp16 inputs take ONE product in their own type, G rounded to it — what
 // autocast does to the reference einsum.
+#include <type_traits>
+
 #include "tma_util.cuh"
 
 namespace mdseg {
@@ -348,7 +350,7 @@ int terms_of(int dtype) { return dtype == MDSEG_F32 ? 3 : 1; }
 
 extern "C" size_t mdseg_proj_fwd_tc_workspace_bytes(const mdseg_graph_table* graphs, int dtype) {
   using namespace mdseg;
-  if (!graphs || graphs->n_datasets <= 0 || graphs->n_datasets > MDSEG_MAX_DATASETS || graphs->C_uni <= 0) return 256;
+  if (!graph_header_ok(graphs)) return 256;
   const int n_chunks = (graphs->C_uni + kKB - 1) / kKB;
   size_t total = 256;
   for (int i = 0; i < graphs->n_datasets; ++i)
@@ -364,8 +366,7 @@ extern "C" int mdseg_proj_fwd_tc(const void* x, int dtype, const mdseg_graph_tab
                                  int n_images, int h, int w, float* y, int y_cmax, float* cmax_out, void* workspace,
                                  size_t workspace_bytes, int32_t* err_flag, void* stream) {
   using namespace mdseg;
-  MDSEG_REQUIRE(graphs && graphs->n_datasets > 0 && graphs->n_datasets <= MDSEG_MAX_DATASETS && graphs->C_uni > 0,
-                "mdseg_proj_fwd_tc: bad graph table");
+  MDSEG_REQUIRE(graph_header_ok(graphs), "mdseg_proj_fwd_tc: bad graph table");
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && h > 0 && w > 0, "mdseg_proj_fwd_tc: bad shape");
   MDSEG_REQUIRE(is_float_dtype(dtype), "mdseg_proj_fwd_tc: unsupported dtype %d", dtype);
   if (n_images == 0) return 0;
@@ -411,23 +412,18 @@ extern "C" int mdseg_proj_fwd_tc(const void* x, int dtype, const mdseg_graph_tab
   const size_t smem = (size_t)kStagesTc * (a.a_stage_bytes + a.b_stage_bytes);
   const dim3 pgrid((unsigned)((groups_max + 255) / 256), (unsigned)graphs->n_datasets);
   const dim3 grid((unsigned)((a.hw + kTM - 1) / kTM), (unsigned)n_images, (unsigned)tiles_max);
-#define MDSEG_TC_LAUNCH(T, TERMS)                                                                                  \
-  do {                                                                                                             \
-    proj_tc_prep_kernel<TERMS><<<pgrid, 256, 0, s>>>(*graphs, a.tc_mask, a.n_chunks, a.fmt,                        \
-                                                     const_cast<unsigned char*>(a.gw), a);                         \
-    MDSEG_LAUNCH_OK();                                                                                             \
-    auto k = proj_tc_kernel<T, TERMS, false>;                                                                      \
-    MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                \
-    k<<<grid, kTcThreads, smem, s>>>(a);                                                                                  \
-    MDSEG_LAUNCH_OK();                                                                                             \
-  } while (0)
-  switch (dtype) {
-    case MDSEG_F32: MDSEG_TC_LAUNCH(float, 3); break;
-    case MDSEG_BF16: MDSEG_TC_LAUNCH(__nv_bfloat16, 1); break;
-    case MDSEG_F16: MDSEG_TC_LAUNCH(__half, 1); break;
-  }
-#undef MDSEG_TC_LAUNCH
-  return 0;
+  return with_float_type(dtype, "mdseg_proj_fwd_tc", "dtype", [&](auto t) {
+    using T = typename decltype(t)::type;
+    constexpr int kTerms = std::is_same_v<T, float> ? 3 : 1;
+    proj_tc_prep_kernel<kTerms><<<pgrid, 256, 0, s>>>(*graphs, a.tc_mask, a.n_chunks, a.fmt,
+                                                      const_cast<unsigned char*>(a.gw), a);
+    MDSEG_LAUNCH_OK();
+    auto k = proj_tc_kernel<T, kTerms, false>;
+    MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<grid, kTcThreads, smem, s>>>(a);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 
 // ---- adjoint on the tensor cores ---------------------------------------------------------------------------
@@ -446,7 +442,7 @@ void bwd_tiling(int C_uni, int* n_tiles, int* nt) {
 
 extern "C" size_t mdseg_proj_bwd_tc_workspace_bytes(const mdseg_graph_table* graphs, int dtype) {
   using namespace mdseg;
-  if (!graphs || graphs->n_datasets <= 0 || graphs->n_datasets > MDSEG_MAX_DATASETS || graphs->C_uni <= 0) return 256;
+  if (!graph_header_ok(graphs)) return 256;
   int n_tiles, nt;
   bwd_tiling(graphs->C_uni, &n_tiles, &nt);
   size_t total = 256;
@@ -460,8 +456,7 @@ extern "C" int mdseg_proj_bwd_tc(const float* dyA, const float* dyB, int y_cmax,
                                  const int32_t* dataset_ids, int n_images, int h, int w, void* dx, int dtype,
                                  void* workspace, size_t workspace_bytes, void* stream) {
   using namespace mdseg;
-  MDSEG_REQUIRE(graphs && graphs->n_datasets > 0 && graphs->n_datasets <= MDSEG_MAX_DATASETS && graphs->C_uni > 0,
-                "mdseg_proj_bwd_tc: bad graph table");
+  MDSEG_REQUIRE(graph_header_ok(graphs), "mdseg_proj_bwd_tc: bad graph table");
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && h > 0 && w > 0, "mdseg_proj_bwd_tc: bad shape");
   MDSEG_REQUIRE(is_float_dtype(dtype), "mdseg_proj_bwd_tc: unsupported dtype %d", dtype);
   if (n_images == 0) return 0;
@@ -505,22 +500,17 @@ extern "C" int mdseg_proj_bwd_tc(const float* dyA, const float* dyB, int y_cmax,
   const size_t smem = (size_t)(a.a_stage_bytes + a.b_stage_bytes);  // one stage (kNS == 1 in the adjoint)
   const dim3 pgrid((unsigned)((max_groups + 255) / 256), (unsigned)graphs->n_datasets);
   const dim3 grid((unsigned)((a.hw + kTM - 1) / kTM), (unsigned)n_images, (unsigned)n_tiles);
-#define MDSEG_TCB_LAUNCH(T, TERMS)                                                                                 \
-  do {                                                                                                             \
-    proj_tc_prep_bwd_kernel<TERMS><<<pgrid, 256, 0, s>>>(*graphs, n_tiles, a.fmt, const_cast<unsigned char*>(a.gw), a); \
-    MDSEG_LAUNCH_OK();                                                                                             \
-    auto k = proj_tc_kernel<T, TERMS, true>;                                                                       \
-    MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                \
-    k<<<grid, kTcThreads, smem, s>>>(a);                                                                           \
-    MDSEG_LAUNCH_OK();                                                                                             \
-  } while (0)
-  switch (dtype) {
-    case MDSEG_F32: MDSEG_TCB_LAUNCH(float, 3); break;
-    case MDSEG_BF16: MDSEG_TCB_LAUNCH(__nv_bfloat16, 1); break;
-    case MDSEG_F16: MDSEG_TCB_LAUNCH(__half, 1); break;
-  }
-#undef MDSEG_TCB_LAUNCH
-  return 0;
+  return with_float_type(dtype, "mdseg_proj_bwd_tc", "dtype", [&](auto t) {
+    using T = typename decltype(t)::type;
+    constexpr int kTerms = std::is_same_v<T, float> ? 3 : 1;
+    proj_tc_prep_bwd_kernel<kTerms><<<pgrid, 256, 0, s>>>(*graphs, n_tiles, a.fmt, const_cast<unsigned char*>(a.gw), a);
+    MDSEG_LAUNCH_OK();
+    auto k = proj_tc_kernel<T, kTerms, true>;
+    MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<grid, kTcThreads, smem, s>>>(a);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }
 
 // ---- d bi_graph on the tensor cores ------------------------------------------------------------------------
@@ -811,8 +801,7 @@ extern "C" int mdseg_proj_bwd_graph_tc(const void* x, int dtype, const float* dy
                                        int w, float* dG, long long dg_stride, void* workspace, size_t workspace_bytes,
                                        void* stream) {
   using namespace mdseg;
-  MDSEG_REQUIRE(graphs && graphs->n_datasets > 0 && graphs->n_datasets <= MDSEG_MAX_DATASETS && graphs->C_uni > 0,
-                "mdseg_proj_bwd_graph_tc: bad graph table");
+  MDSEG_REQUIRE(graph_header_ok(graphs), "mdseg_proj_bwd_graph_tc: bad graph table");
   MDSEG_REQUIRE(n_images >= 0 && n_images <= 65535 && h > 0 && w > 0, "mdseg_proj_bwd_graph_tc: bad shape");
   MDSEG_REQUIRE(is_float_dtype(dtype), "mdseg_proj_bwd_graph_tc: unsupported dtype %d", dtype);
   if (n_images == 0) return 0;
@@ -855,19 +844,15 @@ extern "C" int mdseg_proj_bwd_graph_tc(const void* x, int dtype, const float* dy
   MDSEG_REQUIRE(smem <= 220 * 1024, "mdseg_proj_bwd_graph_tc: C_uni too large for the staged operands");
   const dim3 grid((unsigned)a.n_slabs, (unsigned)(a.n_mt * a.n_nt), (unsigned)n_images);
   const dim3 rgrid((unsigned)(((long long)cmax * a.C_uni + 255) / 256), (unsigned)graphs->n_datasets);
-#define MDSEG_DG_LAUNCH(T, TERMS)                                                                       \
-  do {                                                                                                  \
-    auto k = proj_tc_dgraph_kernel<T, TERMS>;                                                           \
-    MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));     \
-    k<<<grid, kTcThreads, smem, s>>>(a);                                                                \
-    MDSEG_LAUNCH_OK();                                                                                  \
-  } while (0)
-  switch (dtype) {
-    case MDSEG_F32: MDSEG_DG_LAUNCH(float, 3); break;
-    case MDSEG_BF16: MDSEG_DG_LAUNCH(__nv_bfloat16, 1); break;
-    case MDSEG_F16: MDSEG_DG_LAUNCH(__half, 1); break;
-  }
-#undef MDSEG_DG_LAUNCH
+  if (int rc = with_float_type(dtype, "mdseg_proj_bwd_graph_tc", "dtype", [&](auto t) {
+        using T = typename decltype(t)::type;
+        auto k = proj_tc_dgraph_kernel<T, std::is_same_v<T, float> ? 3 : 1>;
+        MDSEG_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k<<<grid, kTcThreads, smem, s>>>(a);
+        MDSEG_LAUNCH_OK();
+        return 0;
+      }))
+    return rc;
   proj_tc_dgraph_reduce_kernel<<<rgrid, 256, 0, s>>>(a, n_images, dG, dg_stride);
   MDSEG_LAUNCH_OK();
   return 0;

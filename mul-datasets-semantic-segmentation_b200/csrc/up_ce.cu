@@ -29,6 +29,7 @@
 // The per-(pixel,class) cost is ~6 issue slots forward and ~9 backward; HBM
 // traffic per label pixel is C*4/16 (low-res logits) + L (label) + 8 (loss, lse).
 #include <float.h>
+#include <type_traits>
 
 #include "up_ce_internal.cuh"
 
@@ -548,12 +549,6 @@ up_ce_bwd_kernel(const BwdArgs a) {
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-int check_src(const mdseg_src_table* s, const char* who) {
-  MDSEG_REQUIRE(s && s->n_datasets > 0 && s->n_datasets <= MDSEG_MAX_DATASETS, "%s: bad source table", who);
-  for (int i = 0; i < s->n_datasets; ++i)
-    MDSEG_REQUIRE(s->C[i] > 0 && s->base[i] != nullptr, "%s: dataset %d has no source", who, i);
-  return 0;
-}
 constexpr size_t kSmemBudget = 56 * 1024;  // per CTA: keeps 3-4 CTAs resident per SM
 
 template <typename T, typename L>
@@ -594,27 +589,6 @@ int launch_bwd(const BwdArgs& a0, int n_images, cudaStream_t s) {
   return 0;
 }
 
-template <typename T>
-int fwd_labels(int label_dtype, const FwdArgs& a, int n_images, cudaStream_t s) {
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_fwd<T, uint8_t>(a, n_images, s);
-    case MDSEG_I32: return launch_fwd<T, int32_t>(a, n_images, s);
-    case MDSEG_I64: return launch_fwd<T, int64_t>(a, n_images, s);
-  }
-  set_error("mdseg_up_ce_fwd: unsupported label dtype %d", label_dtype);
-  return 2;
-}
-template <typename T>
-int bwd_labels(int label_dtype, const BwdArgs& a, int n_images, cudaStream_t s) {
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_bwd<T, uint8_t>(a, n_images, s);
-    case MDSEG_I32: return launch_bwd<T, int32_t>(a, n_images, s);
-    case MDSEG_I64: return launch_bwd<T, int64_t>(a, n_images, s);
-  }
-  set_error("mdseg_up_ce_bwd: unsupported label dtype %d", label_dtype);
-  return 2;
-}
-
 __global__ void add_planes_kernel_f32(const float* __restrict__ a, const float* __restrict__ b, float* __restrict__ o,
                                       int64_t n) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
@@ -652,13 +626,11 @@ extern "C" int mdseg_up_ce_fwd(const mdseg_src_table* src, const int32_t* datase
     const int rc = up_ce_fwd_tma(a, label_dtype, n_images, s);  // fp32, w % 4 == 0, factor <= 5, cmax workspace
     if (rc >= 0) return rc;
   }
-  switch (src->dtype) {
-    case MDSEG_F32: return fwd_labels<float>(label_dtype, a, n_images, s);
-    case MDSEG_BF16: return fwd_labels<__nv_bfloat16>(label_dtype, a, n_images, s);
-    case MDSEG_F16: return fwd_labels<__half>(label_dtype, a, n_images, s);
-  }
-  set_error("mdseg_up_ce_fwd: unsupported dtype %d", src->dtype);
-  return 2;
+  return with_float_type(src->dtype, "mdseg_up_ce_fwd", "dtype", [&](auto t) {
+    return with_int_type(label_dtype, "mdseg_up_ce_fwd", "label dtype", [&](auto l) {
+      return launch_fwd<typename decltype(t)::type, typename decltype(l)::type>(a, n_images, s);
+    });
+  });
 }
 
 extern "C" int mdseg_up_ce_bwd(const mdseg_src_table* src, const int32_t* dataset_ids, const void* labels,
@@ -684,13 +656,11 @@ extern "C" int mdseg_up_ce_bwd(const mdseg_src_table* src, const int32_t* datase
     const int rc = up_ce_bwd_tma(a, label_dtype, n_images, s);
     if (rc >= 0) return rc;
   }
-  switch (src->dtype) {
-    case MDSEG_F32: return bwd_labels<float>(label_dtype, a, n_images, s);
-    case MDSEG_BF16: return bwd_labels<__nv_bfloat16>(label_dtype, a, n_images, s);
-    case MDSEG_F16: return bwd_labels<__half>(label_dtype, a, n_images, s);
-  }
-  set_error("mdseg_up_ce_bwd: unsupported dtype %d", src->dtype);
-  return 2;
+  return with_float_type(src->dtype, "mdseg_up_ce_bwd", "dtype", [&](auto t) {
+    return with_int_type(label_dtype, "mdseg_up_ce_bwd", "label dtype", [&](auto l) {
+      return launch_bwd<typename decltype(t)::type, typename decltype(l)::type>(a, n_images, s);
+    });
+  });
 }
 
 extern "C" int mdseg_add_planes(const float* a, const float* b, void* out, int out_dtype, int64_t n, void* stream) {
@@ -702,12 +672,13 @@ extern "C" int mdseg_add_planes(const float* a, const float* b, void* out, int o
   int64_t cap = (int64_t)sm_count() * 8;
   if (blocks > cap) blocks = cap;
   cudaStream_t s = (cudaStream_t)stream;
-  switch (out_dtype) {
-    case MDSEG_F32: add_planes_kernel_f32<<<(unsigned)blocks, 256, 0, s>>>(a, b, (float*)out, n); break;
-    case MDSEG_BF16: add_planes_kernel<__nv_bfloat16><<<(unsigned)blocks, 256, 0, s>>>(a, b, (__nv_bfloat16*)out, n); break;
-    case MDSEG_F16: add_planes_kernel<__half><<<(unsigned)blocks, 256, 0, s>>>(a, b, (__half*)out, n); break;
-    default: set_error("mdseg_add_planes: unsupported dtype %d", out_dtype); return 2;
-  }
-  MDSEG_LAUNCH_OK();
-  return 0;
+  return with_float_type(out_dtype, "mdseg_add_planes", "out_dtype", [&](auto t) {
+    using T = typename decltype(t)::type;
+    if constexpr (std::is_same_v<T, float>)
+      add_planes_kernel_f32<<<(unsigned)blocks, 256, 0, s>>>(a, b, (float*)out, n);
+    else
+      add_planes_kernel<T><<<(unsigned)blocks, 256, 0, s>>>(a, b, (T*)out, n);
+    MDSEG_LAUNCH_OK();
+    return 0;
+  });
 }

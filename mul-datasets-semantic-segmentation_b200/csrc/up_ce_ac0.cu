@@ -376,17 +376,6 @@ up_ce_ac0_bwd_kernel(const Ac0Bwd a) {
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-int check_src(const mdseg_src_table* s, const char* who) {
-  MDSEG_REQUIRE(s && s->n_datasets > 0 && s->n_datasets <= MDSEG_MAX_DATASETS, "%s: bad source table", who);
-  for (int i = 0; i < s->n_datasets; ++i)
-    MDSEG_REQUIRE(s->C[i] > 0 && s->base[i] != nullptr, "%s: dataset %d has no source", who, i);
-  return 0;
-}
-int max_c(const mdseg_src_table* s) {
-  int m = 0;
-  for (int i = 0; i < s->n_datasets; ++i) m = s->C[i] > m ? s->C[i] : m;
-  return m;
-}
 bool pow2_factor(int f) { return f == 2 || f == 4 || f == 8 || f == 16; }
 
 // The geometry these kernels take: H = fy h and W = fx w with fy, fx in {2, 4, 8, 16}.
@@ -448,34 +437,20 @@ int launch_bwd(const Ac0Bwd& a0, int n_images, cudaStream_t s) {
 // source dtype x label dtype x horizontal factor
 template <bool kFwd, typename Args>
 int run(const Args& a, int dtype, int label_dtype, int fx, int n_images, cudaStream_t s, const char* who) {
-  auto go = [&](auto tz, auto lz) -> int {
-    using T = decltype(tz);
-    using L = decltype(lz);
-    switch (fx) {
+  return with_float_type(dtype, who, "dtype", [&](auto t) {
+    return with_int_type(label_dtype, who, "label dtype", [&](auto l) -> int {
+      using T = typename decltype(t)::type;
+      using L = typename decltype(l)::type;
+      switch (fx) {
 #define MDSEG_AC0_FX(F) \
   case F:               \
     if constexpr (kFwd) return launch_fwd<T, L, F>(a, n_images, s); else return launch_bwd<T, L, F>(a, n_images, s);
-      MDSEG_AC0_FX(2) MDSEG_AC0_FX(4) MDSEG_AC0_FX(8) MDSEG_AC0_FX(16)
+        MDSEG_AC0_FX(2) MDSEG_AC0_FX(4) MDSEG_AC0_FX(8) MDSEG_AC0_FX(16)
 #undef MDSEG_AC0_FX
-    }
-    return 2;
-  };
-  auto by_label = [&](auto tz) -> int {
-    switch (label_dtype) {
-      case MDSEG_U8: return go(tz, uint8_t());
-      case MDSEG_I32: return go(tz, int32_t());
-      case MDSEG_I64: return go(tz, int64_t());
-    }
-    set_error("%s: unsupported label dtype %d", who, label_dtype);
-    return 2;
-  };
-  switch (dtype) {
-    case MDSEG_F32: return by_label(float());
-    case MDSEG_BF16: return by_label(__nv_bfloat16());
-    case MDSEG_F16: return by_label(__half());
-  }
-  set_error("%s: unsupported dtype %d", who, dtype);
-  return 2;
+      }
+      return 2;
+    });
+  });
 }
 
 }  // namespace
@@ -501,12 +476,10 @@ extern "C" int mdseg_up_ce_fwd_ac0(const mdseg_src_table* src, const int32_t* da
 
 extern "C" size_t mdseg_up_ce_bwd_ac0_workspace_bytes(const mdseg_src_table* src, int n_images, int h, int w, int H,
                                                       int W) {
-  if (!src || src->n_datasets <= 0 || src->n_datasets > MDSEG_MAX_DATASETS || n_images <= 0 || h <= 0 || w <= 0)
-    return 256;
+  using namespace mdseg;
+  if (!src_count_ok(src) || n_images <= 0 || h <= 0 || w <= 0) return 256;
   (void)H; (void)W;
-  size_t planes = 0;  // two fp32 planes per dataset, [n_images, C_d, h, w] each
-  for (int i = 0; i < src->n_datasets; ++i) planes += 2 * (size_t)n_images * src->C[i] * h * w * 4;
-  return planes + 256;
+  return two_plane_bytes(src, n_images, h, w);
 }
 
 extern "C" int mdseg_up_ce_bwd_ac0(const mdseg_src_table* src, const int32_t* dataset_ids, const void* labels,
@@ -532,27 +505,15 @@ extern "C" int mdseg_up_ce_bwd_ac0(const mdseg_src_table* src, const int32_t* da
   MDSEG_REQUIRE(workspace_bytes >= mdseg_up_ce_bwd_ac0_workspace_bytes(src, n_images, h, w, H, W),
                 "%s: workspace too small", who);
   cudaStream_t s = (cudaStream_t)stream;
-  float* ws = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-  mdseg_src_table dA = *src, dB = *src;
-  dA.dtype = MDSEG_F32; dB.dtype = MDSEG_F32; dA.cmax = nullptr; dB.cmax = nullptr;
-  size_t off = 0;
-  for (int i = 0; i < src->n_datasets; ++i) {
-    const size_t n = (size_t)n_images * src->C[i] * hw;
-    dA.base[i] = ws + off; dB.base[i] = ws + off + n;
-    dA.image_stride[i] = (long long)src->C[i] * hw; dB.image_stride[i] = dA.image_stride[i];
-    dA.C_alloc[i] = src->C[i]; dB.C_alloc[i] = src->C[i];
-    off += 2 * n;
-  }
-  // the kernel writes both planes of every image of a valid dataset id; with several datasets (or ids) the planes
-  // of the other heads' images are zero, so the sum below writes exact zeros there
-  if (dataset_ids || src->n_datasets > 1) MDSEG_CUDA_OK(cudaMemsetAsync(ws, 0, off * 4, s));
-  a.src = *src; a.dstA = dA; a.dstB = dB; a.dataset_ids = dataset_ids; a.labels = labels; a.ignore = ignore;
+  a.src = *src; a.dataset_ids = dataset_ids; a.labels = labels; a.ignore = ignore;
   a.cc = 0; a.loss_px = loss_px; a.lse_px = lse_px; a.states = states; a.grad_out = grad_out;
   a.grad_scale = grad_scale;
-  if (int rc = run<false>(a, src->dtype, label_dtype, fx, n_images, s, who)) return rc;
-  for (int i = 0; i < src->n_datasets; ++i)
-    if (int rc = mdseg_add_planes((const float*)dA.base[i], (const float*)dB.base[i], const_cast<void*>(dst->base[i]),
-                                  dst->dtype, (int64_t)n_images * src->C[i] * hw, stream))
-      return rc;
-  return 0;
+  // the kernel writes both planes of every image of a valid dataset id; with several datasets (or ids) the planes
+  // of the other heads' images are zero, so the sum writes exact zeros there
+  const bool zero = dataset_ids || src->n_datasets > 1;
+  return two_plane_adjoint(who, src, dst, n_images, h, w, workspace, zero, s,
+                           [&](const mdseg_src_table& dA, const mdseg_src_table& dB) {
+                             a.dstA = dA; a.dstB = dB;
+                             return run<false>(a, src->dtype, label_dtype, fx, n_images, s, who);
+                           });
 }

@@ -19,13 +19,6 @@ inline Geom make_geom(int h, int w, int H, int W) {
   return g;
 }
 
-// the widest class count of a source table
-inline int max_c(const mdseg_src_table* s) {
-  int m = 0;
-  for (int i = 0; i < s->n_datasets; ++i) m = s->C[i] > m ? s->C[i] : m;
-  return m;
-}
-
 // smallest dst in [0, n_out] whose source floor is >= target (n_out if none)
 __device__ __forceinline__ int first_dst_ge(const AxisMap& m, int target, int n_out) {
   if (target <= 0) return 0;

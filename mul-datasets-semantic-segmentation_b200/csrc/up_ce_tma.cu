@@ -588,24 +588,16 @@ int up_ce_fwd_tma(const FwdArgs& a, int label_dtype, int n_images, cudaStream_t 
   if (int rc = tma::make_maps(a.src, a.gm, n_images, kBoxW, 2, kKC, &maps)) return rc;
   if (!a.src.cmax_ready)
     if (int rc = tma::channel_max(a.src, a.dataset_ids, n_images, (int64_t)a.gm.h * a.gm.w, s)) return rc;
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_fwd<uint8_t>(maps, a, n_images, s);
-    case MDSEG_I32: return launch_fwd<int32_t>(maps, a, n_images, s);
-    case MDSEG_I64: return launch_fwd<int64_t>(maps, a, n_images, s);
-  }
-  return -1;
+  return with_int_type(label_dtype, "mdseg_up_ce_fwd", "label dtype",
+                       [&](auto l) { return launch_fwd<typename decltype(l)::type>(maps, a, n_images, s); });
 }
 
 int up_ce_bwd_tma(const BwdArgs& a, int label_dtype, int n_images, cudaStream_t s) {
   if (!tma_applicable(a.src, a.gm)) return -1;
   Maps maps;
   if (int rc = tma::make_maps(a.src, a.gm, n_images, kBoxW, 2, kKC, &maps)) return rc;
-  switch (label_dtype) {
-    case MDSEG_U8: return launch_bwd<uint8_t>(maps, a, n_images, s);
-    case MDSEG_I32: return launch_bwd<int32_t>(maps, a, n_images, s);
-    case MDSEG_I64: return launch_bwd<int64_t>(maps, a, n_images, s);
-  }
-  return -1;
+  return with_int_type(label_dtype, "mdseg_up_ce_bwd", "label dtype",
+                       [&](auto l) { return launch_bwd<typename decltype(l)::type>(maps, a, n_images, s); });
 }
 
 }  // namespace mdseg
